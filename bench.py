@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # ours (torchrun launches N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port), rank 0 only
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's neighbour lists, sampled rows, as .npy
 
 One step = one all-pairs similarity-kNN build (K0 normalise -> [all-gather of x-hat at N>1] -> K1 tensor-core
 stage + FP32 rescore + exact fallback) of the pokec-shaped synthetic feature matrix (1,632,803 x 65, top_k=10),
@@ -49,7 +50,12 @@ def parse():
     ap.add_argument("--skip-configs", action="store_true", help="only the headline shape")
     ap.add_argument("--cpu-rows", type=int, default=2048, help="query-row slab of the CPU baseline sample")
     ap.add_argument("--parity-rows", type=int, default=4096, help="sampled query rows of the headline parity gate")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the neighbour lists of the last timed step of the headline build "
+                                                          "(a fixed sample of query rows) to DIR/{rows,idx,sim,cnt}.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def peaks():
@@ -190,22 +196,30 @@ def sample_rows(n, world, count, seed=7):
     return torch.tensor(sorted(set(fixed + rest)), dtype=torch.long)
 
 
+def rows_of_shards(cx, rows, lo, hi, *shards):
+    """Global query rows `rows` of tensors whose rows [lo, hi) this rank holds: every rank contributes the rows of its
+    shard and every rank receives all of them (integers padded with -2, floats with -inf, combined by MAX)."""
+    mine = (rows >= lo) & (rows < hi)
+    sel = (rows[mine] - lo).to(cx.dev)
+    out = []
+    for t in shards:
+        fill = float("-inf") if t.is_floating_point() else -2
+        got = torch.full((rows.numel(),) + tuple(t.shape[1:]), fill, dtype=t.dtype, device=cx.dev)
+        got[mine.to(cx.dev)] = t[sel]
+        if cx.world > 1:
+            cx.dist.all_reduce(got, op=cx.dist.ReduceOp.MAX)
+        out.append(got)
+    return out
+
+
 def knn_parity(cx, x, idx, cnt, lo, hi, k, thr, count, n_fallback, n_retry):
     """Index parity of a (sharded) build on sampled rows: every rank contributes the sampled rows of its shard, rank 0
     compares with the FP64 oracle (exact / in-band (FP64 gap < 1e-6) / out-of-band, which must be 0)."""
     n = x.size(0)
     rows = sample_rows(n, cx.world, count)
-    mine = (rows >= lo) & (rows < hi)
-    got_i = torch.full((rows.numel(), k), -2, dtype=torch.int32, device=cx.dev)
-    got_c = torch.full((rows.numel(),), -2, dtype=torch.int32, device=cx.dev)
-    if bool(mine.any()):
-        sel = (rows[mine] - lo).to(cx.dev)
-        got_i[mine.to(cx.dev)] = idx[sel]
-        got_c[mine.to(cx.dev)] = cnt[sel]
+    got_i, got_c = rows_of_shards(cx, rows, lo, hi, idx, cnt)
     fb = torch.tensor([n_fallback, n_retry], device=cx.dev, dtype=torch.int64)
     if cx.world > 1:
-        cx.dist.all_reduce(got_i, op=cx.dist.ReduceOp.MAX)
-        cx.dist.all_reduce(got_c, op=cx.dist.ReduceOp.MAX)
         cx.dist.all_reduce(fb, op=cx.dist.ReduceOp.SUM)
     if cx.rank != 0:
         return None
@@ -222,8 +236,26 @@ def knn_parity(cx, x, idx, cnt, lo, hi, k, thr, count, n_fallback, n_retry):
     return res
 
 
+DUMP_BYTES = 48 << 20
+
+
+def dump_outputs(cx, out_dir, n, lo, hi, idx, sim, cnt):
+    """The neighbour lists one build step returns (idx -1 padded, sim 0 padded, cnt), on a fixed sample of query rows that
+    depends only on n, so that runs on any number of GPUs and two builds of the library can be compared file for file:
+    rows / idx / cnt as float64 (exact integers), sim as float32, at most DUMP_BYTES in all."""
+    import numpy as np
+    k = idx.size(1)
+    rows = sample_rows(n, 1, min(n, 1 << 18, DUMP_BYTES // (12 * k + 16)), seed=13)
+    got_i, got_s, got_c = rows_of_shards(cx, rows, lo, hi, idx, sim, cnt)
+    if cx.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, dt in (("rows", rows, np.float64), ("idx", got_i, np.float64), ("sim", got_s, np.float32), ("cnt", got_c, np.float64)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(dt))
+
+
 def build_case(cx, pk, n, d, k, thr, features, steps, warmup, parity_rows, zscore=False, e2e=False, kernel_alone=False, cpu_rows=0,
-               phases=True):
+               phases=True, dump_dir=None):
     """One all-pairs similarity-kNN build configuration: timing (max over ranks), optional end-to-end timing from pinned host
     memory, the tensor-core main pass alone (roofline), index parity on sampled rows."""
     import ctypes
@@ -256,6 +288,8 @@ def build_case(cx, pk, n, d, k, thr, features, steps, warmup, parity_rows, zscor
 
     cx.barrier()
     ms = timed(step_resident, steps, warmup, cx.barrier)
+    if dump_dir:
+        dump_outputs(cx, dump_dir, n, lo, hi, *out["r"][:3])
     res = {"n": n, "d": d, "top_k": k, "thr": thr, "features": features, "steps": steps, "warmup": warmup}
     ms_e2e = None
     if e2e:
@@ -508,7 +542,7 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     head = build_case(cx, pk, N, Fd, k, thr, args.features, args.steps, args.warmup, args.parity_rows, zscore=(args.workload == "pokec"),
-                      e2e=True, kernel_alone=True, cpu_rows=0 if args.skip_cpu else args.cpu_rows)
+                      e2e=True, kernel_alone=True, cpu_rows=0 if args.skip_cpu else args.cpu_rows, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- the other BASELINE.json configurations (build) --------------------------------------------------------

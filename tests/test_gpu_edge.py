@@ -4,7 +4,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import load_golden, golden_inputs
+from conftest import load_golden, golden_inputs, golden_state_dict, golden_grad
 from parity import compare_lists
 
 pytestmark = pytest.mark.gpu
@@ -16,7 +16,7 @@ def _models():
     return M
 
 
-def _build(M, run, x, y):
+def _build(M, g, run, x, y):
     cfg, kind = run["cfg"], run["kind"]
     N, Fd = x.shape
     C = int(y.max()) + 1
@@ -28,7 +28,7 @@ def _build(M, run, x, y):
     else:
         m = M.SNGNN_Plus_Plus(Fd, cfg["hidden"], C, N, cfg["layers"], cfg["top_k"], cfg["thr"], cfg["beta"], cfg["rsl"], 0.0,
                               bn=cfg.get("bn", False))
-    m.load_state_dict(run["state_dict"])
+    m.load_state_dict(golden_state_dict(g, run))
     return m.to(DEV).train()
 
 
@@ -43,7 +43,7 @@ def test_models_match_reference_golden(fname):
     mask = (torch.arange(x.size(0)) % 2 == 0).to(DEV)
     worst = 0.0
     for run in g["runs"]:
-        m = _build(M, run, x, y)
+        m = _build(M, g, run, x, y)
         out = m(data)
         loss = F.nll_loss(out[mask], yd[mask])
         loss.backward()
@@ -51,9 +51,8 @@ def test_models_match_reference_golden(fname):
         torch.testing.assert_close(out.detach().cpu(), run["logp"], rtol=1e-5, atol=2e-6, msg=lambda s: f"{tag}: {s}")
         torch.testing.assert_close(loss.detach().cpu(), run["loss"], rtol=1e-5, atol=1e-6, msg=lambda s: f"{tag} loss: {s}")
         for k, p in m.named_parameters():
-            ref = run["grads"][k]
-            scale = ref.abs().max().item() + 1e-12
-            err = (p.grad.detach().cpu() - ref).abs().max().item() / scale
+            got, ref, scale = golden_grad(p.grad.detach().cpu(), run["grads"][k])
+            err = (got - ref).abs().max().item() / (scale.item() + 1e-12)
             worst = max(worst, err)
             assert err < 1e-5, f"{tag} grad {k}: rel-to-max err {err:.3e}"
     print(f"{fname}: worst grad error relative to max {worst:.2e}")

@@ -4,13 +4,13 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import load_golden, golden_inputs
+from conftest import load_golden, golden_inputs, golden_state_dict, golden_grad
 from oracle import sn_ref, toolbox_ref
 
 
-def _run_oracle(run, x, ei, y):
+def _run_oracle(g, run, x, ei, y):
     cfg = run["cfg"]
-    sd = {k: v.clone().requires_grad_(v.is_floating_point() and "running" not in k) for k, v in run["state_dict"].items()}
+    sd = {k: v.clone().requires_grad_(v.is_floating_point() and "running" not in k) for k, v in golden_state_dict(g, run).items()}
     params = sn_ref.params_from_state_dict(sd, cfg["layers"])
     bns = None
     if cfg.get("bn"):
@@ -31,12 +31,13 @@ def test_models_match_reference(fname):
     g = load_golden(fname)
     x, ei, y = golden_inputs(g)
     for run in g["runs"]:
-        out, loss, grads = _run_oracle(run, x, ei, y)
+        out, loss, grads = _run_oracle(g, run, x, ei, y)
         tag = f"{fname} {run['kind']} {run['cfg']}"
         torch.testing.assert_close(out, run["logp"], rtol=1e-5, atol=1e-6, msg=lambda m: f"{tag}: {m}")
         torch.testing.assert_close(loss, run["loss"], rtol=1e-5, atol=1e-6)
         for k, gref in run["grads"].items():
-            torch.testing.assert_close(grads[k], gref, rtol=1e-4, atol=1e-6, msg=lambda m: f"{tag} grad {k}: {m}")
+            got, ref, _ = golden_grad(grads[k], gref)
+            torch.testing.assert_close(got, ref, rtol=1e-4, atol=1e-6, msg=lambda m: f"{tag} grad {k}: {m}")
 
 
 def test_edge_select_matches_iterated_scatter_max():
