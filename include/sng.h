@@ -236,7 +236,6 @@ SNG_API int sng_sddmm_dot(const float* xhat, int64_t n, int64_t d, int64_t ld,
  *   exact common-neighbour counts and the scales apply 1 / (|a_i| |a_j|).
  * sng_sparse_col_cos: the same cosine between two COLUMNS of a CSC matrix (sorted, duplicate-free indices) at given column
  *   pairs, by merging the two index lists -- the edge metrics of R: SimGFAToolbox/sparse.py:44-119 without densifying.
- * sng_allpairs_dense_f32: out[n,n] = xhat xhat^T on the FP32 CUDA cores (kept as the cross-check of the tensor-core route).
  * sng_class_sums_f64: sums[c, :] += sum_{i: y[i]==c} xhat[i, :] and counts[c] += |class c| (both zero-initialised,
  *   FP64); y may be NULL when num_classes == 1.  Every "sum over all pairs" metric is <S_a, S_b>
  *   (R: SimGFAToolbox/dense.py:9-30, 104-130, 167-179 materialise N x N blocks for the same sums).
@@ -245,7 +244,6 @@ SNG_API int sng_gemm_nt_f16(const uint16_t* a, int64_t lda, const uint16_t* b, i
                     const float* row_scale, const float* col_scale, float* out, int64_t ldo, void* stream);
 SNG_API int sng_sparse_col_cos(const int32_t* indptr, const int32_t* indices, const float* data, const float* inv_norm,
                        const int32_t* a, const int32_t* b, int64_t num_pairs, float* s, void* stream);
-SNG_API int sng_allpairs_dense_f32(const float* xhat, int64_t n, int64_t d, int64_t ld, float* out, void* stream);
 SNG_API int sng_class_sums_f64(const float* xhat, const int32_t* y, int64_t n, int64_t d, int64_t ld, int num_classes,
                        double* sums, double* counts, void* stream);
 

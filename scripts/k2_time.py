@@ -3,7 +3,7 @@ deterministic backward, scatter backward.  python scripts/k2_time.py [shape] [C]
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
-from sngnn_b200 import synth, graph as G, functional as SF, _C
+from sngnn_b200 import synth, graph as G, functional as SF
 
 shape = sys.argv[1] if len(sys.argv) > 1 else "pokec"
 C = int(sys.argv[2]) if len(sys.argv) > 2 else 32
@@ -58,15 +58,6 @@ res["bwd_det_ms"] = timed(lambda: bwd(False))
 res["bwd_det_fused_ms"] = timed(lambda: bwd(True))
 b_bwd = nsel * (3 * 4 * C + 16) + 5 * N * 4 * C
 res["bwd_det_frac_hbm"] = b_bwd / res["bwd_det_ms"] / 1e6 / hbm
-dval, dnrm, dh = torch.zeros_like(h), torch.zeros_like(h), torch.empty_like(h)
-
-
-def bwd_scatter():
-    dval.zero_(); dnrm.zero_()
-    _C.call("sng_edge_agg_bwd", h, _C.ptr(h), _C.ptr(inv), _C.ptr(gg), N, N, 0, C, C, _C.ptr(g.rowptr_in), _C.ptr(g.col_in), k, _C.ptr(ss),
-            _C.ptr(sw), _C.ptr(sc), _C.ptr(g.inv_deg), _C.ptr(dval), _C.ptr(dnrm), _C.ptr(dh))
-
-
-res["bwd_scatter_ms"] = timed(bwd_scatter)
+res["bwd_scatter_ms"] = timed(lambda: SF.edge_agg_bwd_scatter(h, inv, gg, g.rowptr_in, g.col_in, N, 0, k, ss, sw, sc, g.inv_deg))
 res["spmm_ms"] = timed(lambda: SF.spmm(gg, g.rowptr_in, g.col_in_shift, N))
 print(json.dumps(res))

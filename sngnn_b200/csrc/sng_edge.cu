@@ -2088,44 +2088,7 @@ extern "C" int sng_sddmm_dot(const float* xhat, int64_t n, int64_t d, int64_t ld
 }
 
 // ------------------------------------------------------------------------------------------ toolbox helpers
-// Dense all-pairs cosine S = Xhat Xhat^T in FP32 for the toolbox's *_small variants, which RETURN the N x N values
-// (R: SimGFAToolbox/dense.py:138-149).  64x64 output tile per CTA, 16-wide K slices through shared memory, 4x4 micro-tile
-// per thread.  Only meant for matrices that are materialised anyway; the kNN builder never forms S.
 namespace sng {
-__global__ void __launch_bounds__(256) allpairs_dense_kernel(const float* __restrict__ xh, int n, int d, int64_t ld, float* __restrict__ out) {
-    __shared__ float As[16][64 + 4];
-    __shared__ float Bs[16][64 + 4];
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int i0 = blockIdx.y * 64, j0 = blockIdx.x * 64;
-    float acc[4][4] = {};
-    for (int k0 = 0; k0 < d; k0 += 16) {
-        for (int t = threadIdx.x; t < 64 * 16; t += 256) {
-            const int r = t >> 4, k = t & 15;
-            As[k][r] = (i0 + r < n && k0 + k < d) ? __ldg(xh + (int64_t)(i0 + r) * ld + k0 + k) : 0.f;
-            Bs[k][r] = (j0 + r < n && k0 + k < d) ? __ldg(xh + (int64_t)(j0 + r) * ld + k0 + k) : 0.f;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < 16; ++k) {
-            float a[4], b[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) { a[u] = As[k][ty * 4 + u]; b[u] = Bs[k][tx * 4 + u]; }
-#pragma unroll
-            for (int u = 0; u < 4; ++u)
-#pragma unroll
-                for (int v = 0; v < 4; ++v) acc[u][v] = fmaf(a[u], b[v], acc[u][v]);
-        }
-        __syncthreads();
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u)
-#pragma unroll
-        for (int v = 0; v < 4; ++v) {
-            const int i = i0 + ty * 4 + u, j = j0 + tx * 4 + v;
-            if (i < n && j < n) out[(int64_t)i * n + j] = acc[u][v];
-        }
-}
-
 // Per-class sums of unit rows, S[c] = sum_{i: y_i = c} xhat_i  (FP64 accumulation): the closed form behind every
 // "sum of all pairwise similarities" metric, sum_{i in a, j in b} <xhat_i, xhat_j> = <S_a, S_b>
 // (R: SimGFAToolbox/dense.py:9-30, 104-130, 167-179 compute the same sums by materialising N x N blocks).
@@ -2153,13 +2116,6 @@ __global__ void __launch_bounds__(256) class_sum_kernel(const float* __restrict_
     if (cur >= 0 && counter) atomicAdd(counts + cur, run);
 }
 }  // namespace sng
-
-extern "C" int sng_allpairs_dense_f32(const float* xhat, int64_t n, int64_t d, int64_t ld, float* out, void* stream) {
-    SNG_REQUIRE(xhat && out && n > 0 && d > 0 && ld >= d && n < 65536 * 64ll, "sng_allpairs_dense_f32: bad arguments");
-    dim3 grid((unsigned)((n + 63) / 64), (unsigned)((n + 63) / 64));
-    sng::allpairs_dense_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(xhat, (int)n, (int)d, ld, out);
-    return check_launch("sng_allpairs_dense_f32");
-}
 
 extern "C" int sng_class_sums_f64(const float* xhat, const int32_t* y, int64_t n, int64_t d, int64_t ld, int num_classes, double* sums,
                                   double* counts, void* stream) {

@@ -12,6 +12,8 @@ the compute callables default to the CUDA kernels and can be injected by the tes
 import torch
 import torch.distributed as dist
 
+from . import functional as SF
+
 
 def world():
     if dist.is_available() and dist.is_initialized():
@@ -86,7 +88,6 @@ def edge_agg_forward_sharded(h_local, graph, top_k=None, thr=None, agg=None):
     h_all = all_gather_rows(h_local, n)
     shard = graph.row_slice(lo, hi)
     if agg is None:
-        from . import functional as SF
         agg = SF.edge_topk_agg_rows
     return agg(h_all, shard, lo, top_k, thr)
 
@@ -138,7 +139,6 @@ def edge_agg_sharded(h_local, graph, top_k=None, thr=None, agg=None):
     h_all = AllGatherRows.apply(h_local, n)
     shard = graph.row_slice(lo, hi)
     if agg is None:
-        from . import functional as SF
         agg = SF.ShardedEdgeTopkAgg.apply
     return agg(h_all, shard, lo, top_k, thr), shard
 
@@ -147,16 +147,11 @@ def pp_fuse_sharded(out1_local, w_weight, w_bias, beta, bias, shard, n, lo, fuse
     """SNGNN++ fusion on a row shard: out rows [lo, hi) = beta * (A[lo:hi] @ W^T + b_w) + (1 - beta) * out_1 (+ bias), with
     the replicated parameter W^T [n, C] gathered over the shard's out-neighbours.  The parameter gradients this produces
     are PARTIAL (this rank's rows only), like every other parameter gradient of a sharded step: `allreduce_grads` sums them.
-    `fuse` defaults to functional.PPFuse on the shard's by-source CSR (its backward needs g0 of ALL rows for dL/dW^T rows
-    [lo, hi), so that variant all-gathers g0); the gloo tests inject a differentiable dense CPU version."""
+    `fuse` defaults to _ShardedPPFuse (K4 on the shard's by-source CSR; it completes dL/dw.weight on every rank itself); the
+    gloo tests inject a differentiable dense CPU version."""
     if fuse is not None:
         return fuse(out1_local, w_weight, w_bias, beta, bias, shard, n, lo)
     return _ShardedPPFuse.apply(out1_local, w_weight, w_bias, beta, bias, shard, n, lo)
-
-
-def _gather_row_blocks(local, n):
-    """[n, ld] from every rank's [hi - lo, ld] block (no autograd)."""
-    return all_gather_rows(local.contiguous(), n)
 
 
 class _ShardedPPFuse(torch.autograd.Function):
@@ -166,35 +161,21 @@ class _ShardedPPFuse(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, out1, w_weight, w_bias, beta, bias, shard, n, lo):
-        import torch.nn.functional as F
-        from . import _C, functional as SF
         out1 = SF._check_h(out1)
-        nl, cp = out1.shape
-        c = w_weight.size(0)
-        wt = SF._padded_wt(w_weight, cp)                                          # [n, Cp], replicated
-        bw = F.pad(w_bias.detach(), (0, cp - c)).contiguous()
-        bb = None if bias is None else F.pad(bias.detach(), (0, cp - c)).contiguous()
-        out0, out = torch.empty_like(out1), torch.empty_like(out1)
-        if nl:
-            _C.call("sng_pp_fuse_fwd", out1, _C.ptr(wt), nl, cp, cp, _C.ptr(shard.rowptr_out), _C.ptr(shard.col_out), _C.ptr(bw),
-                    _C.ptr(beta), _C.ptr(out1), _C.ptr(bb), _C.ptr(out0), _C.ptr(out))
-        ctx.shard, ctx.c, ctx.n, ctx.lo, ctx.has_bias = shard, c, n, lo, bias is not None
+        operands = SF._structural_operands(w_weight, w_bias, beta, bias, out1.size(1))      # W^T [n, Cp] replicated
+        out0, out = SF.pp_fuse_fwd(out1, *operands, shard.rowptr_out, shard.col_out)
+        ctx.shard, ctx.c, ctx.n, ctx.has_bias = shard, w_weight.size(0), n, bias is not None
         ctx.save_for_backward(out0, out1, beta)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        from . import _C, functional as SF
         out0, out1, beta = ctx.saved_tensors
-        shard, c, n = ctx.shard, ctx.c, ctx.n
-        nl, cp = out1.shape
+        c = ctx.c
         g = g.contiguous()
-        dbeta = torch.zeros(1, dtype=torch.float32, device=g.device)
-        if nl:
-            part = torch.empty(_C.PARTIALS, dtype=torch.float32, device=g.device)
-            _C.call("sng_pp_beta_grad", g, _C.ptr(out0), _C.ptr(out1), _C.ptr(g), g.numel(), _C.ptr(dbeta), _C.ptr(part))
+        dbeta = SF.pp_beta_grad(out0, out1, g)
         g0 = g * beta
-        dw = _complete_dw(g0, shard, n, nl, c, cp)
+        dw = _complete_dw(g0, ctx.shard, ctx.n, c)
         dbias = g.sum(0)[:c] if ctx.has_bias else None
         return g - g0, dw, g0.sum(0)[:c], dbeta, dbias, None, None, None
 
@@ -219,23 +200,21 @@ def _gather_row_blocks_async(local, n):
     return work, out[:n], (pad, out)
 
 
-def _complete_dw(g0, shard, n, nl, c, cp, pending=None):
+def _complete_dw(g0, shard, n, c, pending=None):
     """dL/dw.weight [C, N] (complete, identical on every rank) from this shard's g0 = beta * dL/dout rows: row t of dL/dW^T
     gathers g0 over the (shifted) sources of t's in-edges -- any row of g0, hence the all-gather.  `pending` = an all-gather of
     g0 the caller already started (`_gather_row_blocks_async`), so that it overlaps the caller's kernels."""
-    from . import functional as SF
     if pending is None:
-        g0_all = _gather_row_blocks(g0, n)
+        g0_all = all_gather_rows(g0, n)
     else:
         work, g0_all, _keep = pending
         if work is not None:
             work.wait()
-    if nl:
-        dwt_local = SF.spmm(g0_all.contiguous(), shard.rowptr_in, shard.col_in_shift, nl)
+    if shard.n:
+        dwt_local = SF.spmm(g0_all.contiguous(), shard.rowptr_in, shard.col_in_shift, shard.n)
     else:
-        dwt_local = g0.new_zeros(0, cp)
-    dwt = _gather_row_blocks(dwt_local, n)                                        # [n, Cp]
-    return (dwt if cp == c else dwt[:, :c]).t()
+        dwt_local = g0.new_zeros(0, g0.size(1))
+    return SF._weight_grad(all_gather_rows(dwt_local, n), c)                     # row blocks of dL/dW^T [n, Cp]
 
 
 class _ShardedFusedAgg(torch.autograd.Function):
@@ -245,36 +224,25 @@ class _ShardedFusedAgg(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, h_all, w_weight, w_bias, beta, bias, shard, n, lo, top_k, thr):
-        import torch.nn.functional as F
-        from . import functional as SF
         h_all = SF._check_h(h_all)
-        cp = h_all.size(1)
-        c = w_weight.size(0)
-        fuse = (SF._padded_wt(w_weight, cp), F.pad(w_bias.detach(), (0, cp - c)).contiguous(), beta.detach().contiguous(),
-                None if bias is None else F.pad(bias.detach(), (0, cp - c)).contiguous())
+        fuse = SF._structural_operands(w_weight, w_bias, beta, bias, h_all.size(1))
         train = any(ctx.needs_input_grad)
         out, sel_src, sel_w, _, sel_cnt, inv_norm, diff = SF._edge_fwd(h_all, shard, lo, int(top_k), thr, train, fuse)
-        ctx.shard, ctx.c, ctx.n, ctx.lo, ctx.k, ctx.has_bias = shard, c, n, lo, int(top_k), bias is not None
+        ctx.shard, ctx.c, ctx.n, ctx.lo, ctx.k, ctx.has_bias = shard, w_weight.size(0), n, lo, int(top_k), bias is not None
         ctx.save_for_backward(h_all, sel_src, sel_w, sel_cnt, inv_norm, diff, beta)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        from . import _C
         h_all, sel_src, sel_w, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
-        shard, c, n, k = ctx.shard, ctx.c, ctx.n, ctx.k
-        n_total, cp = h_all.shape
-        nl = shard.n
+        shard, c = ctx.shard, ctx.c
         g = g.contiguous()
         g0 = g * beta
-        pending = _gather_row_blocks_async(g0, n)                 # needed only for dL/dW^T below: overlaps the aggregation backward
-        g1 = (g - g0).contiguous()
-        dval, dnrm, dh = torch.zeros_like(h_all), torch.zeros_like(h_all), torch.empty_like(h_all)
-        _C.call("sng_edge_agg_bwd", h_all, _C.ptr(h_all), _C.ptr(inv_norm), _C.ptr(g1), n_total, nl, ctx.lo, cp, cp,
-                _C.ptr(shard.rowptr_in), _C.ptr(shard.col_in), k, _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_cnt),
-                _C.ptr(shard.inv_deg), _C.ptr(dval), _C.ptr(dnrm), _C.ptr(dh))
+        pending = _gather_row_blocks_async(g0, ctx.n)             # needed only for dL/dW^T below: overlaps the aggregation backward
+        dh = SF.edge_agg_bwd_scatter(h_all, inv_norm, g - g0, shard.rowptr_in, shard.col_in, shard.n, ctx.lo, ctx.k,
+                                     sel_src, sel_w, sel_cnt, shard.inv_deg)
         dbeta = (diff * g).sum().reshape(1)
-        dw = _complete_dw(g0, shard, n, nl, c, cp, pending)
+        dw = _complete_dw(g0, shard, ctx.n, c, pending)
         dbias = g.sum(0)[:c] if ctx.has_bias else None
         return dh, dw, g0.sum(0)[:c], dbeta, dbias, None, None, None, None, None
 

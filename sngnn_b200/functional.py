@@ -142,6 +142,18 @@ def _padded_wt(w_weight, cp):
     return wt.contiguous()
 
 
+def _structural_operands(w_weight, w_bias, beta, bias, cp):
+    """(wt [N, Cp], b_w [Cp], beta [1], bias [Cp] | None): the SNGNN++ structural parameters, detached, padded to Cp."""
+    c = w_weight.size(0)
+    return (_padded_wt(w_weight, cp), F.pad(w_bias.detach(), (0, cp - c)).contiguous(), beta.detach().contiguous(),
+            None if bias is None else F.pad(bias.detach(), (0, cp - c)).contiguous())
+
+
+def _weight_grad(dwt, c):
+    """dL/dw.weight [C, N] from dL/dW^T [N, Cp]: a view in the parameter's own (transposed) storage."""
+    return (dwt if dwt.size(1) == c else dwt[:, :c]).t()
+
+
 class EdgeAgg(torch.autograd.Function):
     """The similarity-navigated aggregation of one layer: out_1 of R: models/models.py:132 / :239 / :326 and -- when the
     structural parameters are given and the graph's in-lists equal its out-lists -- the whole of
@@ -166,8 +178,7 @@ class EdgeAgg(torch.autograd.Function):
                                    "(R builds w = Linear(num_nodes, out_channels), models.py:95)")
             if not graph.symmetric:
                 raise RuntimeError("the fused SNGNN++ pass needs a graph whose in-lists equal its out-lists")
-            fuse = (_padded_wt(w_weight, cp), F.pad(w_bias.detach(), (0, cp - c)).contiguous(), beta.detach().contiguous(),
-                    None if bias is None else F.pad(bias.detach(), (0, cp - c)).contiguous())
+            fuse = _structural_operands(w_weight, w_bias, beta, bias, cp)
             ctx.c = c
         out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = _edge_fwd(h, graph, 0, k, thr, train, fuse, want_q=True, inv_norm=inv_norm)
         ctx.graph, ctx.k, ctx.fused, ctx.has_bias = graph, k, fused, bias is not None
@@ -182,15 +193,13 @@ class EdgeAgg(torch.autograd.Function):
     def backward(ctx, g, *_):
         h, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
         graph, k, fused = ctx.graph, ctx.k, ctx.fused
-        cp = h.size(1)
         g = g.contiguous()
         dh, dwt, dbeta = edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta if fused else None, diff)
         if not fused:
             return dh, None, None, None, None, None, None, None, None
         c = ctx.c
         gsum = g.sum(0)[:c]
-        dw = (dwt if cp == c else dwt[:, :c]).t()           # [C, N] in the parameter's own (transposed) layout
-        return dh, None, None, None, dw, gsum * beta, dbeta, (gsum if ctx.has_bias else None), None
+        return dh, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None
 
 
 def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None):
@@ -224,6 +233,18 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
     return dh, dwt, dbeta
 
 
+def edge_agg_bwd_scatter(h_all, inv_norm, g, rowptr, col, n, row_offset, k, sel_src, sel_w, sel_cnt, inv_denom):
+    """sng_edge_agg_bwd (scatter form, FP32 atomics: row shards and explicit neighbour lists have no transpose index).
+    `g` = dL/dout of target rows [row_offset, row_offset + n) of `h_all`; returns their contribution to dL/dh_all (the
+    contributions of different row ranges add).  k > 0: selection lists + inv_denom; k == 0: every edge of rowptr / col."""
+    n_total, c = h_all.shape
+    g = g.contiguous()
+    dval, dnrm, dh = torch.zeros_like(h_all), torch.zeros_like(h_all), torch.empty_like(h_all)
+    _C.call("sng_edge_agg_bwd", h_all, _C.ptr(h_all), _C.ptr(inv_norm), _C.ptr(g), n_total, n, row_offset, c, c, _C.ptr(rowptr),
+            _C.ptr(col), k, _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_cnt), _C.ptr(inv_denom), _C.ptr(dval), _C.ptr(dnrm), _C.ptr(dh))
+    return dh
+
+
 def edge_topk_agg_rows(h_all, shard, row_offset, top_k=None, thr=None):
     """Forward-only K2 on a row shard: targets [row_offset, row_offset + shard.n) of `h_all` (all nodes, e.g. after an
     all-gather), `shard` = PreparedGraph.row_slice(lo, hi).  Returns (out [shard.n, C], sel_src, sel_w, sel_cnt)."""
@@ -236,7 +257,7 @@ class ShardedEdgeTopkAgg(torch.autograd.Function):
     """K2 / K2b on a ROW SHARD: forward computes out_1 for target rows [row_offset, row_offset + shard.n) from `h_all` (all
     nodes); backward returns this shard's contribution to dL/dh_all [N, C] -- contributions of different shards add
     (SURVEY.md §8(e): the caller reduce-scatters them, see dist.AllGatherRows).  A shard has no transpose index, so its
-    backward is the scatter form (sng_edge_agg_bwd)."""
+    backward is the scatter form (edge_agg_bwd_scatter)."""
 
     @staticmethod
     def forward(ctx, h_all, shard, row_offset, top_k, thr):
@@ -250,13 +271,9 @@ class ShardedEdgeTopkAgg(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         h_all, sel_src, sel_w, sel_cnt, inv_norm = ctx.saved_tensors
-        shard, k = ctx.shard, ctx.k
-        n_total, c = h_all.shape
-        g = g.contiguous()
-        dval, dnrm, dh = torch.zeros_like(h_all), torch.zeros_like(h_all), torch.empty_like(h_all)
-        _C.call("sng_edge_agg_bwd", h_all, _C.ptr(h_all), _C.ptr(inv_norm), _C.ptr(g), n_total, shard.n, ctx.row_offset, c, c,
-                _C.ptr(shard.rowptr_in), _C.ptr(shard.col_in), k, _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_cnt),
-                _C.ptr(shard.inv_deg), _C.ptr(dval), _C.ptr(dnrm), _C.ptr(dh))
+        shard = ctx.shard
+        dh = edge_agg_bwd_scatter(h_all, inv_norm, g, shard.rowptr_in, shard.col_in, shard.n, ctx.row_offset, ctx.k,
+                                  sel_src, sel_w, sel_cnt, shard.inv_deg)
         return dh, None, None, None, None
 
 
@@ -286,14 +303,11 @@ class ListAgg(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         h, idx, sim, cnt, inv_denom = ctx.saved_tensors
-        n, c = h.shape
+        n = h.size(0)
         if idx.size(0) != n:
             raise RuntimeError("backward through a row-sharded list aggregation is not supported")
-        g = g.contiguous()
-        dval, dnrm, dh = torch.zeros_like(h), torch.zeros_like(h), torch.empty_like(h)
         _, _, inv_norm = rownorm(h, want_f32=False, want_inv=True)
-        _C.call("sng_edge_agg_bwd", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n, n, 0, c, c, None, None, idx.size(1), _C.ptr(idx), _C.ptr(sim),
-                _C.ptr(cnt), _C.ptr(inv_denom), _C.ptr(dval), _C.ptr(dnrm), _C.ptr(dh))
+        dh = edge_agg_bwd_scatter(h, inv_norm, g, None, None, n, 0, idx.size(1), idx, sim, cnt, inv_denom)
         return dh, None, None, None, None
 
 
@@ -318,13 +332,7 @@ class PPFuse(torch.autograd.Function):
         if w_weight.size(1) != n:
             raise RuntimeError(f"w.weight is [{c},{w_weight.size(1)}] but the graph has {n} nodes "
                                "(R builds w = Linear(num_nodes, out_channels), models.py:95)")
-        wt = _padded_wt(w_weight, cp)                                             # [N, Cp]
-        bw = F.pad(w_bias.detach(), (0, cp - c)).contiguous()
-        bb = None if bias is None else F.pad(bias.detach(), (0, cp - c)).contiguous()
-        out0 = torch.empty_like(out1)
-        out = torch.empty_like(out1)
-        _C.call("sng_pp_fuse_fwd", out1, _C.ptr(wt), n, cp, cp, _C.ptr(graph.rowptr_out), _C.ptr(graph.col_out), _C.ptr(bw),
-                _C.ptr(beta), _C.ptr(out1), _C.ptr(bb), _C.ptr(out0), _C.ptr(out))
+        out0, out = pp_fuse_fwd(out1, *_structural_operands(w_weight, w_bias, beta, bias, cp), graph.rowptr_out, graph.col_out)
         ctx.graph, ctx.c, ctx.has_bias = graph, c, bias is not None
         ctx.save_for_backward(out0, out1, beta)
         return out
@@ -341,10 +349,29 @@ class PPFuse(torch.autograd.Function):
         # dL/dW^T = A^T g0: row t gathers g0 over the (shifted) sources of t's in-edges
         _C.call("sng_pp_fuse_bwd", g, _C.ptr(out0), _C.ptr(out1), _C.ptr(g), _C.ptr(beta), n, cp, cp, _C.ptr(graph.rowptr_in),
                 _C.ptr(graph.col_in_shift), _C.ptr(dbeta), _C.ptr(part), _C.ptr(g0), _C.ptr(dout1), _C.ptr(dwt))
-        dw = (dwt if cp == c else dwt[:, :c]).t()
         db_w = g0.sum(0)[:c]
         dbias = g.sum(0)[:c] if ctx.has_bias else None
-        return dout1, dw, db_w, dbeta, dbias, None
+        return dout1, _weight_grad(dwt, c), db_w, dbeta, dbias, None
+
+
+def pp_fuse_fwd(out1, wt, b_w, beta, bias, rowptr_out, col_out):
+    """sng_pp_fuse_fwd (K4) on the rows of out1 [n, Cp]: (out0 = A W^T + b_w with A's rows given by rowptr_out / col_out,
+    out = beta out0 + (1 - beta) out1 + bias).  The operands are those of _structural_operands; a shard may have no rows."""
+    n, cp = out1.shape
+    out0, out = torch.empty_like(out1), torch.empty_like(out1)
+    if n:
+        _C.call("sng_pp_fuse_fwd", out1, _C.ptr(wt), n, cp, cp, _C.ptr(rowptr_out), _C.ptr(col_out), _C.ptr(b_w), _C.ptr(beta),
+                _C.ptr(out1), _C.ptr(bias), _C.ptr(out0), _C.ptr(out))
+    return out0, out
+
+
+def pp_beta_grad(out0, out1, g):
+    """dL/dbeta [1] = sum((out0 - out1) g) of the K4 blend, summed in a fixed order (sng_pp_beta_grad); 0 for no rows."""
+    dbeta = torch.zeros(1, dtype=torch.float32, device=g.device)
+    if g.numel():
+        part = torch.empty(_C.PARTIALS, dtype=torch.float32, device=g.device)
+        _C.call("sng_pp_beta_grad", g, _C.ptr(out0), _C.ptr(out1), _C.ptr(g), g.numel(), _C.ptr(dbeta), _C.ptr(part))
+    return dbeta
 
 
 def rownorm(x, want_f32=True, want_f16=False, f16_ld=None, want_inv=False):
