@@ -23,13 +23,16 @@ int check_launch(const char* what) {
     return SNG_OK;
 }
 
+// Without a device every launch fails anyway; the host-side plans (sng_simknn_plan, the workspace sizes) then report what
+// they would be on a B200.
 int sm_count() {
+    constexpr int kNoDevice = 148;
     static int cached[64] = {0};
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return 0; }
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { cudaGetLastError(); return kNoDevice; }
     if (cached[dev] == 0) {
         int v = 0;
-        if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { cudaGetLastError(); return 0; }
+        if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) { cudaGetLastError(); return kNoDevice; }
         cached[dev] = v;
     }
     return cached[dev];

@@ -10,7 +10,7 @@ namespace sng {
 
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);   // cudaPeekAtLastError -> SNG_ERR_CUDA + message
-int sm_count();                       // cached; <=0 if no device
+int sm_count();                       // cached; 148 (a B200's) if there is no device, see sng_api.cu
 int debug_env_int(const char* name, int lo, int hi);   // tuning override; always 0 unless sng_set_debug_env(1) was called
 
 #define SNG_REQUIRE(cond, ...)                                  \
@@ -23,6 +23,7 @@ int debug_env_int(const char* name, int lo, int hi);   // tuning override; alway
 
 constexpr float kNormEps = 1e-12f;   // F.normalize eps, R: models/models.py:122
 
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ float dot4(const float4& a, const float4& b) {
     return fmaf(a.x, b.x, fmaf(a.y, b.y, fmaf(a.z, b.z, a.w * b.w)));
@@ -53,6 +54,22 @@ inline int group_lanes(int64_t c) {
     int g = 1;
     while (g * 4 < c) g <<= 1;
     return g;
+}
+
+// Grid of a grid-stride kernel: the blocks `items` need, at most ctas_per_sm CTAs per SM, at least one.
+inline int grid_capped(int64_t items, int64_t items_per_block, int64_t ctas_per_sm) {
+    const int64_t need = (items + items_per_block - 1) / items_per_block, cap = sm_count() * ctas_per_sm;
+    const int64_t g = need < cap ? need : cap;
+    return (int)(g < 1 ? 1 : g);
+}
+// Grid of a grid-stride row kernel = exactly the number of CTAs that are resident at once (SMs x occupancy of THIS kernel):
+// every CTA then gets the same share of rows and there is no partial second wave (a fixed 8 CTAs per SM left the gather
+// kernels, which fit 5-6, with a 1.3-1.6 wave launch whose tail ran on a half-empty GPU).
+template <typename Kernel>
+int grid_resident(Kernel kernel, int64_t items, int items_per_block, size_t smem = 0, int threads = 256) {
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem) != cudaSuccess || occ < 1) { cudaGetLastError(); occ = 1; }
+    return grid_capped(items, items_per_block, occ);
 }
 
 }  // namespace sng

@@ -18,8 +18,6 @@ constexpr int kWarpsPerBlock = 8;
 constexpr int kThreads = kWarpsPerBlock * 32;
 
 template <int G> struct Unroll { static constexpr int value = (G >= 4) ? 4 : G; };
-// forward scoring: all loads of a 32-edge chunk in flight at once while that fits in registers (G <= 8)
-template <int G> struct UnrollFwd { static constexpr int value = (G <= 8) ? G : 8; };
 
 // ------------------------------------------------------------------------------------------ K0
 __global__ void __launch_bounds__(kThreads) rownorm_kernel(const float* __restrict__ x, int64_t n, int d, int64_t ldx,
@@ -153,7 +151,6 @@ constexpr int kStWarps = 4;
 #ifndef SNG_BWDS_MINB
 #define SNG_BWDS_MINB 8
 #endif
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void cp_async16(uint32_t dst, const float* src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
@@ -169,8 +166,6 @@ __device__ __forceinline__ float lds32(uint32_t addr) {
 }
 // bytes of a staged row slot: the row padded by one 16-byte chunk (G > 1), so that slot strides are odd multiples of 16 B
 template <int G> constexpr int staged_row_bytes() { return G == 1 ? 16 : 16 * G + 16; }
-template <int G, bool FUSE>
-constexpr int staged_stage_bytes() { return (FUSE ? 65 : 33) * staged_row_bytes<G>(); }   // 32 source rows + the target row (+ 32 Wt rows)
 
 template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK>
 __global__ void __launch_bounds__(kStWarps * 32, SNG_FWD_MINB) edge_fwd_staged_kernel(const EdgeFwdArgs a) {
@@ -1749,26 +1744,6 @@ __global__ void __launch_bounds__(kThreads) sddmm_dot_kernel(const float* __rest
     }
 }
 
-static int grid_for_rows(int64_t rows, int rows_per_block) {
-    int64_t need = (rows + rows_per_block - 1) / rows_per_block;
-    int64_t cap = (int64_t)(sm_count() > 0 ? sm_count() : 1) * 8;   // 8 resident 256-thread CTAs per SM, grid-stride
-    int64_t g = need < cap ? need : cap;
-    return (int)(g < 1 ? 1 : g);
-}
-
-// Grid of a grid-stride row kernel = exactly the number of CTAs that are resident at once (SMs x occupancy of THIS kernel):
-// every CTA then gets the same share of rows and there is no partial second wave (a fixed 8 CTAs per SM left the gather
-// kernels, which fit 5-6, with a 1.3-1.6 wave launch whose tail ran on a half-empty GPU).
-template <typename Kernel>
-static int grid_resident(Kernel kernel, int64_t rows, int rows_per_block, size_t smem = 0, int threads = kThreads) {
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem) != cudaSuccess || occ < 1) { cudaGetLastError(); occ = 1; }
-    const int64_t need = (rows + rows_per_block - 1) / rows_per_block;
-    const int64_t cap = (int64_t)(sm_count() > 0 ? sm_count() : 1) * occ;
-    const int64_t g = need < cap ? need : cap;
-    return (int)(g < 1 ? 1 : g);
-}
-
 #define SNG_DISPATCH_G(cexpr, ...)                                              \
     switch (group_lanes(cexpr)) {                                               \
         case 1: { constexpr int G = 1; __VA_ARGS__; } break;                    \
@@ -1846,8 +1821,7 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
     edge_fwd_long_kernel<G, FUSE, SELECT_ALL><<<grid_resident(edge_fwd_long_kernel<G, FUSE, SELECT_ALL>, a.n, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
     if (a.skip_deg) {
         a.rows = rows_hub; a.n_rows = (int)n_hub; a.skip_deg = 0;
-        const int64_t cap = (int64_t)(sm_count() > 0 ? sm_count() : 148) * 4;
-        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL><<<(unsigned)(n_hub < cap ? n_hub : cap), kThreads, hs, st>>>(a);
+        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL><<<grid_capped(n_hub, 1, 4), kThreads, hs, st>>>(a);
     }
 }
 }  // namespace sng
@@ -2053,7 +2027,7 @@ extern "C" int sng_pp_fuse_fwd(const float* wt, int64_t n, int64_t c, int64_t ld
 extern "C" int sng_pp_beta_grad(const float* out0, const float* out1, const float* g, int64_t numel, float* dbeta, float* partials,
                                 void* stream) {
     SNG_REQUIRE(out0 && out1 && g && dbeta && partials && numel >= 0 && numel % 4 == 0, "sng_pp_beta_grad: bad arguments (numel must be a multiple of 4)");
-    int grid = grid_for_rows(numel / 4, 256);
+    int grid = grid_capped(numel / 4, 256, 8);
     if (grid > SNG_PARTIALS) grid = SNG_PARTIALS;
     if (numel == 0) { return cudaMemsetAsync(dbeta, 0, sizeof(float), (cudaStream_t)stream) == cudaSuccess ? SNG_OK : check_launch("sng_pp_beta_grad"); }
     pp_beta_grad_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(out0, out1, g, numel, partials);
@@ -2064,7 +2038,7 @@ extern "C" int sng_pp_beta_grad(const float* out0, const float* out1, const floa
 extern "C" int sng_nll_loss_fwd(const float* logp, int64_t n, int64_t c, int64_t ld, const int64_t* y, float* loss, float* count,
                                float* partials, void* stream) {
     SNG_REQUIRE(logp && y && loss && count && partials && n >= 0 && c > 0 && ld >= c && c < (1ll << 30), "sng_nll_loss_fwd: bad arguments");
-    int grid = grid_for_rows(n > 0 ? n : 1, 256);
+    int grid = grid_capped(n, 256, 8);
     if (grid > SNG_PARTIALS / 2) grid = SNG_PARTIALS / 2;
     nll_loss_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(logp, n, (int)c, ld, y, partials, partials + SNG_PARTIALS / 2);
     nll_loss_finish_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(partials, partials + SNG_PARTIALS / 2, grid, loss, count);
@@ -2075,7 +2049,7 @@ extern "C" int sng_nll_loss_bwd(int64_t n, int64_t c, int64_t ld, const int64_t*
                                void* stream) {
     SNG_REQUIRE(y && gscale && count && dlogp && n >= 0 && c > 0 && ld >= c, "sng_nll_loss_bwd: bad arguments");
     if (n == 0) return SNG_OK;
-    nll_loss_bwd_kernel<<<grid_for_rows(n * c, 256), 256, 0, (cudaStream_t)stream>>>(n, (int)c, ld, y, gscale, count, dlogp);
+    nll_loss_bwd_kernel<<<grid_capped(n * c, 256, 8), 256, 0, (cudaStream_t)stream>>>(n, (int)c, ld, y, gscale, count, dlogp);
     return check_launch("sng_nll_loss_bwd");
 }
 

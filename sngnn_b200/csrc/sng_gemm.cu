@@ -10,8 +10,7 @@
 // (tcgen05.mma.cta_group::1, M = 128, N = 128, accumulator = 128 TMEM columns), warps 2-5 = epilogue (tcgen05.ld, one
 // output row per thread).  Unlike the kNN builder this kernel materialises its output -- it exists for the functions
 // whose contract is the matrix itself.
-#include "sng_common.cuh"
-#include <cuda.h>
+#include "sng_sm100.cuh"
 #include <cuda_fp16.h>
 
 namespace sng {
@@ -21,29 +20,8 @@ constexpr int TM = 128, TN = 128, TK = 64;
 constexpr int kStages = 3;
 constexpr int kTile = 128 * TK * 2;          // 16 KiB: 128 rows x 64 FP16
 constexpr int kThreads = 192;
+static_assert(TK == 64 && TM == 128 && TN == 128, "make_tma_map_f16 loads 64 (K) x 128 (rows) boxes");
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done, polls = 0;
-    unsigned long long t0 = 0;
-    while (true) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) return;
-        if (++polls > 4096u) {                 // a protocol bug must trap (error returned to the caller), never hang the GPU
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ull) __trap();
-        }
-    }
-}
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1) : "memory");
@@ -55,22 +33,7 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr) : "memory");
-}
-// K-major, 128-byte-swizzled shared-memory matrix descriptor: rows 128 B apart, 8-row groups 1024 B apart
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(1024u >> 4) << 32) | (1ull << 46) | (2ull << 61);
-}
-// kind::f16: A, B = FP16, D = FP32, both K-major, N / 8 at [17, 23), M / 16 at [24, 29)
-constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(TN >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
+constexpr uint32_t kIdesc = f16_idesc(TM, TN);
 
 struct Params {
     int m, n, kblocks, accumulate;         // accumulate != 0: out += result (K segments of a long contraction, see the host entry)
@@ -97,9 +60,9 @@ __global__ void __launch_bounds__(kThreads) gemm_nt_f16_kernel(const __grid_cons
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 128;" ::"r"(smem_u32(tmem_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     const uint32_t tmem = *tmem_slot;
 
     if (warp == 0) {
@@ -118,7 +81,7 @@ __global__ void __launch_bounds__(kThreads) gemm_nt_f16_kernel(const __grid_cons
             int stage = 0; uint32_t phase = 0;
             for (int kb = 0; kb < p.kblocks; ++kb) {
                 mbar_wait(bar_full + 8 * stage, phase);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tc_fence_after();
                 const uint64_t adesc = make_smem_desc(base + a_off + (uint32_t)stage * kTile);
                 const uint64_t bdesc = make_smem_desc(base + b_off + (uint32_t)stage * kTile);
 #pragma unroll
@@ -135,14 +98,14 @@ __global__ void __launch_bounds__(kThreads) gemm_nt_f16_kernel(const __grid_cons
         const int r = quarter * 32 + lane;
         const int row = m0 + r;
         mbar_wait(bar_acc, 0);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         const float rs = (p.row_scale && row < p.m) ? __ldg(p.row_scale + row) : 1.0f;
         const bool vec = (p.ldo % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.out) & 15) == 0);
 #pragma unroll 1
         for (int c = 0; c < TN / 32; ++c) {
             uint32_t v[32];
             tmem_ld32(tmem + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(c * 32), v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_ld_wait();
             if (row < p.m) {
                 const int col0 = n0 + c * 32;
                 float* o = p.out + (int64_t)row * p.ldo + col0;
@@ -167,37 +130,12 @@ __global__ void __launch_bounds__(kThreads) gemm_nt_f16_kernel(const __grid_cons
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
     if (warp == 1) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" ::"r"(tmem) : "memory");
     }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int make_map(CUtensorMap* map, const uint16_t* ptr, int64_t rows, int64_t k, int64_t ld) {
-    static EncodeTiledFn enc = nullptr;
-    if (!enc) {
-        void* fp = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            enc = reinterpret_cast<EncodeTiledFn>(fp);
-        else
-            cudaGetLastError();
-    }
-    if (!enc) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return SNG_ERR_CUDA; }
-    cuuint64_t gdim[2] = {(cuuint64_t)k, (cuuint64_t)rows};          // columns beyond k and rows beyond `rows` read as zero
-    cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
-    cuuint32_t box[2] = {(cuuint32_t)TK, 128u};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<uint16_t*>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld k=%lld ld=%lld)", (int)r, (long long)rows, (long long)k, (long long)ld); return SNG_ERR_CUDA; }
-    return SNG_OK;
 }
 
 }  // namespace gemm
@@ -222,8 +160,8 @@ extern "C" int sng_gemm_nt_f16(const uint16_t* a, int64_t lda, const uint16_t* b
     for (int64_t k0 = 0; k0 < k; k0 += kseg) {
         const int64_t kk = k - k0 < kseg ? k - k0 : kseg;
         CUtensorMap ma, mb;
-        if (int rc = gemm::make_map(&ma, a + k0, m, kk, lda)) return rc;
-        if (int rc = gemm::make_map(&mb, b + k0, n, kk, ldb)) return rc;
+        if (int rc = make_tma_map_f16(&ma, a + k0, m, kk, lda, 1)) return rc;
+        if (int rc = make_tma_map_f16(&mb, b + k0, n, kk, ldb, 1)) return rc;
         gemm::Params p;
         p.m = (int)m; p.n = (int)n; p.kblocks = (int)((kk + gemm::TK - 1) / gemm::TK); p.accumulate = k0 > 0;
         p.row_scale = row_scale; p.col_scale = col_scale; p.out = out; p.ldo = ldo;
@@ -260,7 +198,6 @@ extern "C" int sng_sparse_col_cos(const int32_t* indptr, const int32_t* indices,
                                   const int32_t* b, int64_t num_pairs, float* s, void* stream) {
     SNG_REQUIRE(indptr && indices && data && inv_norm && a && b && s && num_pairs >= 0, "sng_sparse_col_cos: bad arguments");
     if (num_pairs == 0) return SNG_OK;
-    const int64_t cap = (int64_t)(sm_count() > 0 ? sm_count() : 148) * 8, need = (num_pairs + 255) / 256;
-    sng::sparse_col_cos_kernel<<<(unsigned)(need < cap ? need : cap), 256, 0, (cudaStream_t)stream>>>(indptr, indices, data, inv_norm, a, b, num_pairs, s);
+    sng::sparse_col_cos_kernel<<<grid_capped(num_pairs, 256, 8), 256, 0, (cudaStream_t)stream>>>(indptr, indices, data, inv_norm, a, b, num_pairs, s);
     return check_launch("sng_sparse_col_cos");
 }

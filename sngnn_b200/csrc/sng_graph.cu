@@ -137,8 +137,7 @@ extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, i
     int* min_src = reinterpret_cast<int*>(w); w += 256;
     void* temp = w;
     size_t temp_bytes = sort_temp_bytes(total, bits);
-    const int sms = sm_count() > 0 ? sm_count() : 148;
-    const int grid = (int)((total + 255) / 256 < (int64_t)sms * 16 ? (total + 255) / 256 : (int64_t)sms * 16);
+    const int grid = grid_capped(total, 256, 16);
     if (cudaMemsetAsync(min_src, 0x7f, sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");   // 0x7f7f7f7f
     if (cudaMemsetAsync(info, 0, 8 * sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");
     if (structural && cudaMemsetAsync(info + 2, 0xff, sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");
@@ -148,7 +147,7 @@ extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, i
     if (cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_dst, key_sorted, eid, perm_in, total, 0, bits, st) != cudaSuccess)
         return check_launch("sng_graph_prepare sort by target");
     graph_ends_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, total, perm_in, 0, col_in, nullptr);
-    const int rgrid = (int)((n + 256) / 256 < (int64_t)sms * 16 ? (n + 256) / 256 : (int64_t)sms * 16);
+    const int rgrid = grid_capped(n + 1, 256, 16);
     graph_rowptr_kernel<<<rgrid, 256, 0, st>>>(key_sorted, total, (int)n, nullptr, rowptr_in);
     if (structural) {
         if (cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_src, key_sorted, eid, perm_out, total, 0, bits, st) != cudaSuccess)

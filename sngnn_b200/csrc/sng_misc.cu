@@ -49,12 +49,6 @@ __global__ void __launch_bounds__(256) segment_finish_kernel(const double* __res
         out[i] = (float)(sums[i] / (double)max(counts[i], 1));
 }
 
-static int grid_1d(int64_t items) {
-    const int64_t cap = (int64_t)(sm_count() > 0 ? sm_count() : 148) * 8;
-    const int64_t need = (items + 255) / 256;
-    return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-}
-
 }  // namespace sng
 
 using namespace sng;
@@ -76,9 +70,9 @@ extern "C" int sng_knn_to_csr(const int32_t* idx, const float* sim, const int32_
     void* temp = reinterpret_cast<uint8_t*>(clamped) + (((size_t)(nq + 1) * 4 + 255) & ~(size_t)255);
     size_t temp_bytes = 0;
     cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, (const int*)nullptr, (int*)nullptr, (int)(nq + 1));
-    clamp_counts_kernel<<<grid_1d(nq + 1), 256, 0, st>>>(cnt, nq, top_k, clamped);
+    clamp_counts_kernel<<<grid_capped(nq + 1, 256, 8), 256, 0, st>>>(cnt, nq, top_k, clamped);
     if (cub::DeviceScan::ExclusiveSum(temp, temp_bytes, clamped, rowptr, (int)(nq + 1), st) != cudaSuccess) return check_launch("sng_knn_to_csr scan");
-    if (nq > 0) knn_compact_kernel<<<grid_1d(nq * top_k), 256, 0, st>>>(rowptr, idx, sim, nq, top_k, col, val);
+    if (nq > 0) knn_compact_kernel<<<grid_capped(nq * top_k, 256, 8), 256, 0, st>>>(rowptr, idx, sim, nq, top_k, col, val);
     return check_launch("sng_knn_to_csr");
 }
 
@@ -89,7 +83,7 @@ extern "C" int sng_pp_fuse_bwd(const float* out0, const float* out1, const float
     SNG_REQUIRE(n >= 0 && c > 0 && c % 4 == 0 && ld == c, "sng_pp_fuse_bwd: rows must be contiguous with a multiple of 4 channels");
     if (n == 0) return SNG_OK;
     if (int rc = sng_pp_beta_grad(out0, out1, g, n * c, dbeta, partials, stream)) return rc;
-    beta_split_kernel<<<grid_1d(n * c / 4), 256, 0, (cudaStream_t)stream>>>(g, beta, n * c / 4, g0, dout1);
+    beta_split_kernel<<<grid_capped(n * c / 4, 256, 8), 256, 0, (cudaStream_t)stream>>>(g, beta, n * c / 4, g0, dout1);
     if (int rc = check_launch("sng_pp_fuse_bwd split")) return rc;
     return sng_spmm_fwd(g0, n, c, c, rowptr_in, col_in_shift, nullptr, nullptr, nullptr, dwt, c, stream);   // dL/dW^T = A^T g0
 }
@@ -102,8 +96,8 @@ extern "C" int sng_segment_mean(const float* val, const int32_t* seg, int64_t nu
     double* sums = reinterpret_cast<double*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     int* counts = reinterpret_cast<int*>(sums + n_seg);
     if (cudaMemsetAsync(sums, 0, (size_t)n_seg * 12, st) != cudaSuccess) return check_launch("sng_segment_mean memset");
-    if (num > 0) segment_accum_kernel<<<grid_1d(num), 256, 0, st>>>(val, seg, num, (int)n_seg, sums, counts);
-    segment_finish_kernel<<<grid_1d(n_seg), 256, 0, st>>>(sums, counts, (int)n_seg, out);
+    if (num > 0) segment_accum_kernel<<<grid_capped(num, 256, 8), 256, 0, st>>>(val, seg, num, (int)n_seg, sums, counts);
+    segment_finish_kernel<<<grid_capped(n_seg, 256, 8), 256, 0, st>>>(sums, counts, (int)n_seg, out);
     return check_launch("sng_segment_mean");
 }
 
@@ -420,12 +414,7 @@ static LinBwdPlan lin_bwd_plan(int64_t n, int64_t f, int64_t c, bool flat) {
     p.smem = tiles > red ? tiles : red;
     int occ = 1;
     SNG_LB_DISPATCH(p, p, &occ, false, nullptr, 0, nullptr, 0, 0, 0, 0, 0, nullptr, nullptr, nullptr)
-    const int64_t sms = sm_count() > 0 ? sm_count() : 148;
-    int64_t want = sms * occ;                                                      // one resident wave of CTAs
-    const int64_t max_chunks = (n + 4 * kLbRows - 1) / (4 * kLbRows);              // at least 4 tiles per CTA
-    if (want > max_chunks) want = max_chunks;
-    if (want < 1) want = 1;
-    p.nchunk = (int)want;
+    p.nchunk = grid_capped(n, 4 * kLbRows, occ);                                    // one resident wave, at least 4 tiles per CTA
     return p;
 }
 }  // namespace sng
@@ -437,9 +426,8 @@ extern "C" int sng_lin_bwd_supported(int64_t f, int64_t c) { return f > 0 && c >
 extern "C" size_t sng_lin_bwd_workspace_bytes(int64_t n, int64_t f, int64_t c) {
     if (n <= 0 || !sng_lin_bwd_supported(f, c)) return 256;
     // chunk count bound that does not depend on the staging mode: one resident wave is at most 32 CTAs per SM
-    const int64_t sms = sng::sm_count() > 0 ? sng::sm_count() : 148;
     const size_t f4 = (size_t)(f + 3) / 4 * 4, c4 = (size_t)(c + 3) / 4 * 4;
-    return (size_t)(sms * 32) * c4 * (f4 + 1) * sizeof(float) + 256;
+    return (size_t)sng::sm_count() * 32 * c4 * (f4 + 1) * sizeof(float) + 256;
 }
 
 extern "C" int sng_lin_bwd(const float* g, int64_t ldg, const float* x, int64_t ldx, int64_t n, int64_t f, int64_t c, float* dw, int64_t lddw,
@@ -486,10 +474,7 @@ extern "C" int sng_lin_norm_fwd(const float* x, int64_t n, int64_t f, int64_t ld
         constexpr int R = (256 / CGV) * 4;                                                                                       \
         const size_t smem = (size_t)2 * (CGV <= 2 ? 16 : kLinKC) * (R + CGV * 4) * sizeof(float);                                                  \
         cudaFuncSetAttribute(lin_norm_kernel<CGV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                      \
-        int occ = 1;                                                                                                             \
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lin_norm_kernel<CGV>, 256, smem) != cudaSuccess || occ < 1) { cudaGetLastError(); occ = 1; } \
-        const int64_t need = (n + R - 1) / R, cap = (int64_t)(sm_count() > 0 ? sm_count() : 148) * occ;                         \
-        lin_norm_kernel<CGV><<<(unsigned)(need < cap ? need : cap), 256, smem, st>>>(x, n, (int)f, ldx, w, (int)c, ldw, bias, h, inv_norm); \
+        lin_norm_kernel<CGV><<<grid_resident(lin_norm_kernel<CGV>, n, R, smem), 256, smem, st>>>(x, n, (int)f, ldx, w, (int)c, ldw, bias, h, inv_norm); \
     }
     switch (cgn) {
         case 1: SNG_LIN_LAUNCH(1) break;

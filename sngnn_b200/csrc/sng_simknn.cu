@@ -20,8 +20,7 @@
 // Operands are FP16 (not BF16): unit-norm rows live in [-1,1] where FP16 has 3 more mantissa bits, so the
 // worst-case score error is 2^-10 instead of 2^-8 and the candidate margin needed for exact indices is 4x
 // smaller; kind::f16 runs FP16 and BF16 at the same rate.
-#include "sng_common.cuh"
-#include <cuda.h>        // CUtensorMap + enums only; cuTensorMapEncodeTiled is resolved at run time
+#include "sng_sm100.cuh"
 #include <cuda_fp16.h>
 #include <math_constants.h>
 #include <stdlib.h>
@@ -33,6 +32,7 @@ constexpr int BM = 128;                 // query rows per CTA = TMEM lanes (a CT
 constexpr int BN = 256;                 // database columns per pair tile = UMMA N
 constexpr int BK = 64;                  // K elements per smem tile row = 128 bytes = one swizzle span
 constexpr int kTileBytes = 128 * BK * 2;// 16 KiB: one K block of 128 rows (A block, or this CTA's half of a B tile)
+static_assert(BK == 64 && BM == 128, "make_tma_map_f16 loads 64 (K) x 128 (rows) boxes");
 constexpr int kUmmaK = 16;
 constexpr int kNonEpiThreads = 128;
 constexpr int kMaxStages = 10;
@@ -66,7 +66,6 @@ __device__ __forceinline__ unsigned short q_of(float v) {
 __device__ __forceinline__ float q_upper(unsigned q) { return ((float)q + 1.5f) * kQBin - kQOff; }
 
 // ------------------------------------------------------------------------------------------ PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -77,22 +76,10 @@ __device__ __forceinline__ bool elect_one() {
     asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(p));
     return p != 0;
 }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
 // arrive on the barrier at the same shared-memory offset in CTA `cta` of the cluster
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t cta) {
     asm volatile("{\n\t.reg .b32 ra;\n\tmapa.shared::cluster.u32 ra, %0, %1;\n\tmbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}"
                  ::"r"(bar), "r"(cta) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    return done != 0;
 }
 __device__ __forceinline__ uint32_t mapa_cluster(uint32_t addr, uint32_t cta) {
     uint32_t ra;
@@ -102,33 +89,11 @@ __device__ __forceinline__ uint32_t mapa_cluster(uint32_t addr, uint32_t cta) {
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-// Bounded wait: a protocol bug must trap (error returned to the caller) instead of hanging the GPU.
-__device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
-    uint32_t done, polls = 0;
-    unsigned long long t0 = 0;
-    while (true) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (done) return;
-        if (++polls > 4096u) {
-            unsigned long long now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ull) __trap();     // 4 s
-        }
-    }
-}
-// hot-loop form: one inline try (it suspends in hardware for a while), the bounded polling loop stays out of line
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    if (!mbar_try(bar, parity)) mbar_wait_slow(bar, parity);
-}
 // TMA load issued by either CTA of the pair into its OWN shared memory; the bytes are credited to the LEADER's barrier
 __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map, uint32_t bar_leader, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_leader), "r"(c0), "r"(c1) : "memory");
 }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 // D[tmem] (+)= A[smem] * B[smem]^T over the CTA pair: M = 256 (128 rows per CTA), N = 256 (128 B rows per CTA), K = 16
 __device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
     asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
@@ -139,43 +104,12 @@ __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                  ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ float max3(float a, float b, float c) {
     float r;
     asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
     return r;
 }
-// v[i] for a warp-uniform runtime i, without local memory: 31 selects
-__device__ __forceinline__ float select32(const uint32_t (&v)[32], int i) {
-    uint32_t a[16], b[8], c[4], d[2];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) a[j] = (i & 1) ? v[2 * j + 1] : v[2 * j];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) b[j] = (i & 2) ? a[2 * j + 1] : a[2 * j];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) c[j] = (i & 4) ? b[2 * j + 1] : b[2 * j];
-#pragma unroll
-    for (int j = 0; j < 2; ++j) d[j] = (i & 8) ? c[2 * j + 1] : c[2 * j];
-    return __uint_as_float((i & 16) ? d[1] : d[0]);
-}
-
-// K-major, 128-byte-swizzled shared-memory matrix descriptor (sm_100 "version 1"):
-// rows are 128 B apart, 8-row groups 1024 B apart (SBO); LBO unused for swizzled K-major.
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
-    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(1024u >> 4) << 32) | (1ull << 46) | (2ull << 61);
-}
-// kind::f16 instruction descriptor: A,B = FP16 (0), D = FP32 (1 at bit 4), both K-major, N/8 at [17,23), M/16 at [24,29); M = 256 spans the pair
-constexpr uint32_t kIdesc = (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+constexpr uint32_t kIdesc = f16_idesc(256, BN);            // M = 256 spans the pair
 
 struct Stage1Params {
     int nq, n, q_offset;          // query rows in this call, database rows, global id of query row 0
@@ -208,7 +142,7 @@ struct Stage1Params {
 template <int W, int NI>
 __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base, uint32_t a_off, uint32_t b_off, uint32_t bar_full, uint32_t bar_empty,
                                             uint32_t bar_tfull, uint32_t bar_tempty, int t_beg, int t_end, bool issuer, int lane) {
-    constexpr uint32_t kIdescHalf = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+    constexpr uint32_t kIdescHalf = f16_idesc(256, 128);
     long long* const trc = kInstr ? p.trace : nullptr;
     const uint64_t adesc0 = make_smem_desc(base + a_off);
     const uint64_t bdesc0 = make_smem_desc(base + b_off);
@@ -1045,39 +979,6 @@ __global__ void __launch_bounds__(256) simknn_fb_stream_kernel(
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-        else
-            cudaGetLastError();
-    }
-    return fn;
-}
-
-// [rows, ld] FP16 row-major, box = 64 (K) x 128 (rows), 128-byte swizzle, zero fill out of bounds.  `row_stride` > 1
-// maps every row_stride-th row of the matrix (the seed pass's column sample); `ld` stays the K extent.
-static int make_map(CUtensorMap* map, const uint16_t* ptr, int64_t rows, int64_t ld, int64_t row_stride = 1) {
-    EncodeTiledFn enc = get_encode_fn();
-    if (!enc) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return SNG_ERR_CUDA; }
-    cuuint64_t gdim[2] = {(cuuint64_t)ld, (cuuint64_t)rows};
-    cuuint64_t gstr[1] = {(cuuint64_t)ld * 2 * (cuuint64_t)row_stride};
-    cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)BM};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<uint16_t*>(ptr), gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld ld=%lld)", (int)r, (long long)rows, (long long)ld); return SNG_ERR_CUDA; }
-    return SNG_OK;
-}
-
 struct Plan {
     int ew, stages, cand, qcap, nsplit, kblocks, ksteps_last, tiles, stream_a;
     int seed_stride, seed_q;      // 0 = no seed pass
@@ -1184,9 +1085,8 @@ static int make_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int top_k, int 
     if (!pl->ew) { set_error("simknn: d=%lld top_k=%d does not fit in shared memory", (long long)d, top_k); return SNG_ERR_UNSUPPORTED; }
     // the pair kernel allocates all 512 TMEM columns: a CTA must own its SM, so never request less than half the shared memory
     if (pl->smem <= kMaxSmem / 2) pl->smem = kMaxSmem / 2 + 1024;
-    const int sms = sm_count() > 0 ? sm_count() : 148;
     const int64_t ctas = 2 * ((nq + 2 * BM - 1) / (2 * BM));
-    int ns = (int)((3ll * sms + ctas - 1) / ctas);
+    int ns = (int)((3ll * sm_count() + ctas - 1) / ctas);
     if (ns > 8) ns = 8;
     if (ns > pl->tiles) ns = pl->tiles;
     while (ns > 1 && ns * pl->cand > kMaxCandTotal) --ns;
@@ -1233,8 +1133,8 @@ static int launch_stage1(const Plan& pl, const uint16_t* xq, const uint16_t* xal
     const bool seed_pass = seed_out != nullptr;
     const int64_t n_db = seed_pass ? (n + pl.seed_stride - 1) / pl.seed_stride : n;
     CUtensorMap mq, mdb;
-    if (int rc = make_map(&mq, xq, nq, ldb)) return rc;
-    if (int rc = make_map(&mdb, xall, n_db, ldb, seed_pass ? pl.seed_stride : 1)) return rc;
+    if (int rc = make_tma_map_f16(&mq, xq, nq, ldb, ldb, 1)) return rc;
+    if (int rc = make_tma_map_f16(&mdb, xall, n_db, ldb, ldb, seed_pass ? pl.seed_stride : 1)) return rc;   // seed pass: the column sample
     Stage1Params p;
     p.nq = (int)nq; p.n = (int)n_db; p.q_offset = (int)q_offset;
     p.kblocks = pl.kblocks; p.ksteps_last = pl.ksteps_last; p.stages = pl.stages; p.stream_a = pl.stream_a; p.cand = seed_pass ? 0 : pl.cand; p.qcap = pl.qcap;
@@ -1430,8 +1330,7 @@ extern "C" int sng_simknn_build(const uint16_t* xq, const uint16_t* xall, int64_
     int* flag_rows = retry ? fb_rows : fb2_rows;
     int* flag_cnt = retry ? n_fb1 : n_fallback;
     {
-        const int blocks = (int)((nq + 7) / 8 < (int64_t)sm_count() * 8 ? (nq + 7) / 8 : (int64_t)sm_count() * 8);
-        simknn_rescore_kernel<<<blocks > 0 ? blocks : 1, 256, (size_t)8 * 2 * 3 * m_total * 4, st>>>(
+        simknn_rescore_kernel<<<grid_capped(nq, 8, 8), 256, (size_t)8 * 2 * 3 * m_total * 4, st>>>(
             xq32, xall32, ld32, d4, (int)nq, (int)n, (int)q_offset, remove_self, m_total, pl.lists(), top_k, thr, eps, cand_val, cand_idx, cand_min,
             idx, sim, cnt, flag_rows, flag_cnt, nullptr, nullptr);
         if (int rc = check_launch("simknn stage 2")) return rc;
@@ -1469,7 +1368,7 @@ extern "C" int sng_simknn_build(const uint16_t* xq, const uint16_t* xall, int64_
             // rows of this round: exact on the host unless capturing (then the grid covers `cap` rows and the device count trims it)
             const int n_r = capturing ? cap : (flagged - r * cap < cap ? flagged - r * cap : cap);
             const int n_launch = (n_r + 2 * BM - 1) / (2 * BM) * (2 * BM);
-            simknn_retry_gather_kernel<<<(sm_count() > 0 ? sm_count() : 148) * 2, 256, 0, st>>>(xq, ldb, rows_r, round_cnt + r, xq_retry);
+            simknn_retry_gather_kernel<<<sm_count() * 2, 256, 0, st>>>(xq, ldb, rows_r, round_cnt + r, xq_retry);
             if (int rc = launch_stage1(pr, xq_retry, xall, ldb, n_launch, q_offset, n, thr_lo, remove_self, rcand_val, rcand_idx, rcand_min,
                                        pl.seed_stride > 0 ? seeds : nullptr, nullptr, nullptr, st, round_cnt + r, rows_r)) return rc;
             const int rblocks = (n_launch + 7) / 8 < 4096 ? (n_launch + 7) / 8 : 4096;
@@ -1483,7 +1382,7 @@ extern "C" int sng_simknn_build(const uint16_t* xq, const uint16_t* xall, int64_
         if (cudaMemcpyAsync(n_retry, retry ? n_fb1 : n_fallback, sizeof(int), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
             return check_launch("sng_simknn_build n_retry");
     }
-    const int fb_grid = (sm_count() > 0 ? sm_count() : 148) * 4;
+    const int fb_grid = sm_count() * 4;                          // one resident wave: the flagged-row count is on the device
     for (int wave = 0; wave < kFbWaves; ++wave) {
         simknn_fb_scan_kernel<<<fb_grid, 256, 0, st>>>(xq32, xall32, ld32, d4, (int)n, (int)q_offset, top_k, thr, remove_self, fb2_rows, n_fallback,
                                                       wave, n_chunks, part_s, part_i);
