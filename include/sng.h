@@ -40,6 +40,8 @@ extern "C" {
 #define SNG_ERR_WORKSPACE (-4)   /* workspace too small */
 
 #define SNG_MAX_TOPK 64          /* edge path: top_k <= 64; top_k <= 0 means "select every edge" */
+#define SNG_MAX_CHANNELS 512     /* padded row width c of sng_edge_fwd / _bwd, sng_edge_agg_bwd, sng_list_agg_fwd, sng_spmm_fwd,
+                                    sng_pp_fuse_fwd / _bwd; wider rows return SNG_ERR_UNSUPPORTED */
 #define SNG_KNN_MAX_TOPK 64      /* all-pairs builder */
 
 SNG_API int sng_version(void);
@@ -81,9 +83,10 @@ SNG_API int sng_rownorm_f32(const float* x, int64_t n, int64_t d, int64_t ldx,
  * sel_w [n,top_k] (s_e), sel_cnt [n], sel_q [n,top_k] = tpos of the selected edges (needs tpos; input of sng_edge_bwd).
  * Degree dispatch (tables built once per graph by the caller, sngnn_b200/graph.py): rows with more than 32 in-edges are cut
  * into chunks of <= 32 consecutive edges.  chunk_tab [n_chunks, 4] int32 = (first edge position, edges, local row id, 0);
- * lrows [n_lrows] = those rows in ascending order, lrow_ptr [n_lrows + 1] = their chunk ranges; rows_hub [n_hub] = the rows
- * with more than 1024 in-edges (used for c > 32 only).  workspace >= sng_edge_fwd_workspace_bytes(n_chunks, c, top_k) holds
- * the per-chunk candidates.  n_chunks < 0 = tables unknown: one general kernel then runs every row.
+ * lrows [n_lrows] = those rows in ascending order, lrow_ptr [n_lrows + 1] = their chunk ranges (both used for c <= 32 only);
+ * rows_hub [n_hub] = the rows with more than 1024 in-edges (used for 32 < c <= SNG_MAX_CHANNELS, where one general kernel
+ * runs every other row).  workspace >= sng_edge_fwd_workspace_bytes(n_chunks, c, top_k) holds the per-chunk candidates.
+ * n_chunks < 0 = tables unknown: the general kernel then runs every row.
  * Row sharding: the call covers target rows [row_offset, row_offset + n) of `h`, which holds ALL n_total nodes
  * (sources are arbitrary); rowptr / out / sel_* / the chunk tables are local to the shard, `col` holds global source ids.
  * inv_norm [n_total] is filled with 1/max(||h_i||, 1e-12) (a pre-pass of this call, skipped when inv_norm_ready != 0: the

@@ -91,6 +91,7 @@ def ptr(t):
 
 
 PARTIALS = 4096          # SNG_PARTIALS of include/sng.h
+MAX_CHANNELS = 512       # SNG_MAX_CHANNELS of include/sng.h
 
 
 def stream(t=None):

@@ -2,8 +2,9 @@
 //
 // All of these are HBM/L2-gather bound (SURVEY.md §8(d)): one warp owns one target row; a group of
 // G = C/4 lanes owns one in-edge at a time and fetches its source row with ONE 128-bit load per lane, so
-// a warp step touches 32/G full rows (coalesced 16..512-byte segments).  Scores, selection and the
-// weighted reduction never leave registers / shared memory; nothing of size E is written.
+// a warp step touches 32/G full rows (coalesced 16..512-byte segments).  Wider rows (C > 128, up to SNG_MAX_CHANNELS) take the
+// whole warp, G/32 loads per lane (RowShape).  Scores, selection and the weighted reduction never leave registers / shared
+// memory; nothing of size E is written.
 //
 // Reference call sites replaced: R: models/models.py:121-137,139-158 (++), :233-263 (+), :322-334 (base).
 #include "sng_common.cuh"
@@ -17,7 +18,26 @@ namespace sng {
 constexpr int kWarpsPerBlock = 8;
 constexpr int kThreads = kWarpsPerBlock * 32;
 
-template <int G> struct Unroll { static constexpr int value = (G >= 4) ? 4 : G; };
+// Row layout of the lane-group kernels for G float4 slots per row (4 G channels).  G <= 32: a group of L = G lanes owns a row,
+// one slot per lane, EPW = 32 / G rows per warp step.  G > 32 (wide rows, up to SNG_MAX_CHANNELS): the warp owns the row and
+// lane l holds the V = G / 32 slots l, l + 32, ... (channels 4 (32 v + l) .. + 3), so each load instruction of the warp is one
+// contiguous 512-byte segment of the row.
+template <int G> struct RowShape {
+    static constexpr int L = G < 32 ? G : 32;
+    static constexpr int V = G / L;
+    static constexpr int EPW = 32 / L;
+};
+// first channel of slot v of the lane with group index q
+__device__ __forceinline__ int slot_c4(int q, int v) { return 4 * (q + 32 * v); }
+template <int V> __device__ __forceinline__ float dotv(const float4 (&a)[V], const float4 (&b)[V]) {
+    float d = dot4(a[0], b[0]);
+#pragma unroll
+    for (int v = 1; v < V; ++v) d += dot4(a[v], b[v]);
+    return d;
+}
+
+// rows in flight per lane group: four (one 16-byte load each) for G <= 32; wide rows keep the same four loads per lane
+template <int G> struct Unroll { static constexpr int value = G > 32 ? 128 / G : (G >= 4) ? 4 : G; };
 
 // ------------------------------------------------------------------------------------------ K0
 __global__ void __launch_bounds__(kThreads) rownorm_kernel(const float* __restrict__ x, int64_t n, int d, int64_t ldx,
@@ -43,11 +63,12 @@ __global__ void __launch_bounds__(kThreads) rownorm_kernel(const float* __restri
 }
 
 // inv_r[i] = 1 / max(||h_i||, 1e-12).  The edge kernels gather this scalar per edge (the array is L2 resident) instead of
-// recomputing every source row's norm from its gathered features.  G = C/4 lanes per row, four rows in flight per group.
+// recomputing every source row's norm from its gathered features.  Row layout RowShape<G>, four rows in flight per group.
 template <int G>
 __global__ void __launch_bounds__(kThreads) row_inv_norm_kernel(const float* __restrict__ h, int64_t n, int c, int64_t ld, float* __restrict__ inv) {
-    constexpr int RPW = 32 / G;                                        // rows per warp step
-    const int lane = threadIdx.x & 31, q = lane % G, grp = lane / G;
+    using S = RowShape<G>;
+    constexpr int RPW = S::EPW;                                        // rows per warp step
+    const int lane = threadIdx.x & 31, q = lane % S::L, grp = lane / S::L;
     const bool ch_ok = q * 4 < c;
     const int64_t nw = (int64_t)gridDim.x * kWarpsPerBlock;
     for (int64_t r0 = ((int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5)) * RPW * 4; r0 < n; r0 += nw * RPW * 4) {
@@ -56,11 +77,18 @@ __global__ void __launch_bounds__(kThreads) row_inv_norm_kernel(const float* __r
         for (int u = 0; u < 4; ++u) {
             const int64_t row = r0 + u * RPW + grp;
             ss[u] = 0.f;
-            if (row < n && ch_ok) { const float4 v = ldg4(h + row * ld + q * 4); ss[u] = dot4(v, v); }
+            if (row < n && ch_ok) {
+                const float4 v = ldg4(h + row * ld + q * 4);
+                ss[u] = dot4(v, v);
+#pragma unroll
+                for (int s = 1; s < S::V; ++s) {
+                    if (slot_c4(q, s) < c) { const float4 w = ldg4(h + row * ld + slot_c4(q, s)); ss[u] += dot4(w, w); }
+                }
+            }
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            const float t = group_sum<G>(ss[u]);
+            const float t = group_sum<S::L>(ss[u]);
             const int64_t row = r0 + u * RPW + grp;
             if (q == 0 && row < n) inv[row] = inv_norm_of(t);
         }
@@ -520,14 +548,18 @@ struct TopList {
 };
 
 // One warp scans the 32-edge chunks first, first + step, ... of a row: lane e owns edge e of the chunk (source id, 1/norm,
-// score); a group of G lanes fetches one source row per step.  SELECT_ALL accumulates the weighted rows on the fly, the
-// selection variant only maintains the warp's top-k list (winners are re-gathered afterwards: they were loaded moments ago).
+// score); a group of RowShape<G>::L lanes fetches one source row per step.  SELECT_ALL accumulates the weighted rows on the
+// fly, the selection variant only maintains the warp's top-k list (winners are re-gathered afterwards: they were loaded
+// moments ago).  hb / wb / ni / ch_ok / acc / a0 hold one entry per float4 slot of the lane (RowShape<G>::V).
 template <int G, bool FUSE, bool SELECT_ALL>
-__device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* hb, const float* wb, int grow, int end, int first, int step,
-                                         const float4& ni, bool ch_ok, int lane, TopList& L, float4& acc, float4& a0) {
-    constexpr int EPW = 32 / G;
-    constexpr int U = (G <= 8) ? G : 8;         // steps whose loads are issued together
-    const int grp = lane / G;
+__device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* const (&hb)[RowShape<G>::V], const float* const (&wb)[RowShape<G>::V],
+                                         int grow, int end, int first, int step, const float4 (&ni)[RowShape<G>::V],
+                                         const bool (&ch_ok)[RowShape<G>::V], int lane, TopList& L, float4 (&acc)[RowShape<G>::V],
+                                         float4 (&a0)[RowShape<G>::V]) {
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
+    constexpr int U = (G <= 8) ? G : 8 / V;     // steps whose loads are issued together (eight 16-byte loads per lane from G = 8 on)
+    const int grp = lane / S::L;
     for (int base = first; base < end; base += step) {
         const int nchunk = min(32, end - base);
         const bool has = lane < nchunk;
@@ -535,23 +567,29 @@ __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* hb, 
         const float irl = __ldg(a.inv_r + jl);
         float my_d = 0.f;                                                               // <n_i, h_j> of edge base + lane
         for (int st = 0; st < nchunk; st += EPW * U) {
-            float4 v[U];
+            float4 v[U][V];
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int e = st + u * EPW + grp;
                 const int j = __shfl_sync(kFull, jl, e & 31);
-                v[u] = ldg4(hb + (int64_t)j * a.ldh);
-                if (FUSE && e < nchunk) add4(a0, ldg4(wb + (int64_t)j * a.ldw));
+#pragma unroll
+                for (int s = 0; s < V; ++s) v[u][s] = ldg4(hb[s] + (int64_t)j * a.ldh);
+                if (FUSE && e < nchunk) {
+#pragma unroll
+                    for (int s = 0; s < V; ++s) add4(a0[s], ldg4(wb[s] + (int64_t)j * a.ldw));
+                }
             }
 #pragma unroll
             for (int u = 0; u < U; ++u) {
-                const float d = group_sum<G>(dot4(ni, v[u]));
+                const float d = group_sum<S::L>(dotv<V>(ni, v[u]));
                 if (SELECT_ALL) {
                     const int e = st + u * EPW + grp;
                     const float w = __shfl_sync(kFull, irl, e & 31);
-                    if (e < nchunk && ch_ok) fma4(acc, d * w + 0.0f, v[u]);
+#pragma unroll
+                    for (int s = 0; s < V; ++s)
+                        if (e < nchunk && ch_ok[s]) fma4(acc[s], d * w + 0.0f, v[u][s]);
                 } else {
-                    const float t = __shfl_sync(kFull, d, (lane % EPW) * G);             // hand (step, group) to the edge's lane
+                    const float t = __shfl_sync(kFull, d, (lane % EPW) * S::L);          // hand (step, group) to the edge's lane
                     if (lane / EPW == st / EPW + u) my_d = t;
                 }
             }
@@ -587,14 +625,17 @@ __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* hb, 
 
 // weighted sum of the <= top_k winners of a finished list (source ids re-read through their positions) + the saved lists
 template <int G>
-__device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* hb, int row, const float* ls, const int* lp, int cnt, int lane,
-                                            float4& acc) {
-    constexpr int EPW = 32 / G;
-    const int grp = lane / G;
+__device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* const (&hb)[RowShape<G>::V], int row, const float* ls,
+                                            const int* lp, int cnt, int lane, float4 (&acc)[RowShape<G>::V]) {
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW;
+    const int grp = lane / S::L;
     for (int st = 0; st < cnt; st += EPW) {
         const int t = min(st + grp, cnt - 1);                                            // clamp: the duplicate gets weight 0
         const float w = st + grp < cnt ? ls[t] : 0.f;
-        fma4(acc, w, ldg4(hb + (int64_t)__ldg(a.col + lp[t]) * a.ldh));
+        const int64_t o = (int64_t)__ldg(a.col + lp[t]) * a.ldh;
+#pragma unroll
+        for (int s = 0; s < S::V; ++s) fma4(acc[s], w, ldg4(hb[s] + o));
     }
     if (a.sel_cnt) {
         const int64_t lo = (int64_t)row * a.top_k;
@@ -611,17 +652,27 @@ __device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* h
 
 template <int G, bool FUSE, bool SELECT_ALL>
 __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdArgs a) {
+    using S = RowShape<G>;
+    constexpr int V = S::V;
     extern __shared__ float smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G;
-    const bool ch_ok = q * 4 < a.c;
-    const int c4 = ch_ok ? q * 4 : 0;
-    const float* hb = a.h + c4;
-    const float* wb = FUSE ? a.wt + c4 : nullptr;
+    const int q = lane % S::L, grp = lane / S::L;
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    bool ch_ok[V];
+    const float* hb[V];
+    const float* wb[V];
     float beta = 0.f;
-    float4 bw = z4, bb = z4;
-    if (FUSE) { beta = __ldg(a.beta); if (ch_ok) { bw = ldg4(a.b_w + c4); if (a.bias) bb = ldg4(a.bias + c4); } }
+    float4 bw[V], bb[V];
+    if (FUSE) beta = __ldg(a.beta);
+#pragma unroll
+    for (int s = 0; s < V; ++s) {
+        ch_ok[s] = slot_c4(q, s) < a.c;
+        const int c4 = ch_ok[s] ? slot_c4(q, s) : 0;
+        hb[s] = a.h + c4;
+        wb[s] = FUSE ? a.wt + c4 : nullptr;
+        bw[s] = z4; bb[s] = z4;
+        if (FUSE && ch_ok[s]) { bw[s] = ldg4(a.b_w + c4); if (a.bias) bb[s] = ldg4(a.bias + c4); }
+    }
     TopList L;
     L.s = smem + (size_t)warp * 2 * max(a.top_k, 1);
     L.p = reinterpret_cast<int*>(L.s + max(a.top_k, 1));
@@ -631,15 +682,22 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdAr
         const int grow = a.row_offset + row;
         const int beg = __ldg(a.rowptr + row), end = __ldg(a.rowptr + row + 1);
         if (a.skip_deg && end - beg > a.skip_deg) continue;
-        float4 ni = scale4(ldg4(hb + (int64_t)grow * a.ldh), __ldg(a.inv_r + grow));
-        if (!ch_ok) ni = z4;
-        float4 acc = z4, a0 = z4;
+        float4 ni[V], acc[V], a0[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            ni[s] = scale4(ldg4(hb[s] + (int64_t)grow * a.ldh), __ldg(a.inv_r + grow));
+            if (!ch_ok[s]) ni[s] = z4;
+            acc[s] = z4; a0[s] = z4;
+        }
         L.cnt = 0; L.kth = -CUDART_INF_F;
         scan_row<G, FUSE, SELECT_ALL>(a, hb, wb, grow, end, beg, 32, ni, ch_ok, lane, L, acc, a0);
         if (!SELECT_ALL) { finish_list<G>(a, hb, row, L.s, L.p, L.cnt, lane, acc); __syncwarp(); }
-        cross_group_sum4<G>(acc);
-        if (FUSE) cross_group_sum4<G>(a0);
-        if (grp == 0 && ch_ok) write_row<FUSE>(a, row, q * 4, acc, a0, end - beg, beta, bw, bb);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            cross_group_sum4<G>(acc[s]);
+            if (FUSE) cross_group_sum4<G>(a0[s]);
+            if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), acc[s], a0[s], end - beg, beta, bw[s], bb[s]);
+        }
     }
 }
 
@@ -772,22 +830,33 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
 // strict order and the ranks are the final ranks); warp 0 then finishes the row exactly like the long-row kernel.
 template <int G, bool FUSE, bool SELECT_ALL>
 __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArgs a) {
+    using S = RowShape<G>;
+    constexpr int V = S::V;
+    constexpr int PW = 128 * V;                 // channels of a partial-sum row: a warp's 32 lanes x V slots x 4
     extern __shared__ float smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G;
-    const bool ch_ok = q * 4 < a.c;
-    const int c4 = ch_ok ? q * 4 : 0;
-    const float* hb = a.h + c4;
-    const float* wb = FUSE ? a.wt + c4 : nullptr;
+    const int q = lane % S::L, grp = lane / S::L;
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     const int k1 = max(a.top_k, 1);
+    bool ch_ok[V];
+    const float* hb[V];
+    const float* wb[V];
     float beta = 0.f;
-    float4 bw = z4, bb = z4;
-    if (FUSE) { beta = __ldg(a.beta); if (ch_ok) { bw = ldg4(a.b_w + c4); if (a.bias) bb = ldg4(a.bias + c4); } }
-    // shared memory: the warps' partial sums (acc, a0: 128 channels each; first, so they stay 16-byte aligned), 8 warp lists,
+    float4 bw[V], bb[V];
+    if (FUSE) beta = __ldg(a.beta);
+#pragma unroll
+    for (int s = 0; s < V; ++s) {
+        ch_ok[s] = slot_c4(q, s) < a.c;
+        const int c4 = ch_ok[s] ? slot_c4(q, s) : 0;
+        hb[s] = a.h + c4;
+        wb[s] = FUSE ? a.wt + c4 : nullptr;
+        bw[s] = z4; bb[s] = z4;
+        if (FUSE && ch_ok[s]) { bw[s] = ldg4(a.b_w + c4); if (a.bias) bb[s] = ldg4(a.bias + c4); }
+    }
+    // shared memory: the warps' partial sums (acc, a0: PW channels each; first, so they stay 16-byte aligned), 8 warp lists,
     // the final list, the list lengths
     float* part = smem;
-    float* lists = smem + (size_t)kWarpsPerBlock * 2 * 128;
+    float* lists = smem + (size_t)kWarpsPerBlock * 2 * PW;
     float* fin_s = lists + (size_t)kWarpsPerBlock * 2 * k1;
     int* fin_p = reinterpret_cast<int*>(fin_s + k1);
     int* wcnt = fin_p + k1;
@@ -798,16 +867,26 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
         const int row = __ldg(a.rows + ri);
         const int grow = a.row_offset + row;
         const int beg = __ldg(a.rowptr + row), end = __ldg(a.rowptr + row + 1);
-        float4 ni = scale4(ldg4(hb + (int64_t)grow * a.ldh), __ldg(a.inv_r + grow));
-        if (!ch_ok) ni = z4;
-        float4 acc = z4, a0 = z4;
+        float4 ni[V], acc[V], a0[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            ni[s] = scale4(ldg4(hb[s] + (int64_t)grow * a.ldh), __ldg(a.inv_r + grow));
+            if (!ch_ok[s]) ni[s] = z4;
+            acc[s] = z4; a0[s] = z4;
+        }
         L.cnt = 0; L.kth = -CUDART_INF_F;
         scan_row<G, FUSE, SELECT_ALL>(a, hb, wb, grow, end, beg + 32 * warp, 32 * kWarpsPerBlock, ni, ch_ok, lane, L, acc, a0);
-        cross_group_sum4<G>(acc);
-        cross_group_sum4<G>(a0);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            cross_group_sum4<G>(acc[s]);
+            cross_group_sum4<G>(a0[s]);
+        }
         if (grp == 0) {
-            *reinterpret_cast<float4*>(part + (size_t)(warp * 2) * 128 + q * 4) = acc;
-            *reinterpret_cast<float4*>(part + (size_t)(warp * 2 + 1) * 128 + q * 4) = a0;
+#pragma unroll
+            for (int s = 0; s < V; ++s) {
+                *reinterpret_cast<float4*>(part + (size_t)(warp * 2) * PW + slot_c4(q, s)) = acc[s];
+                *reinterpret_cast<float4*>(part + (size_t)(warp * 2 + 1) * PW + slot_c4(q, s)) = a0[s];
+            }
         }
         if (lane == 0) wcnt[warp] = L.cnt;
         __syncthreads();
@@ -832,15 +911,25 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
             __syncthreads();
         }
         if (warp == 0) {
-            float4 sacc = z4, sa0 = z4;
-            if (grp == 0) {
-                for (int w = 0; w < kWarpsPerBlock; ++w) {
-                    if (SELECT_ALL) add4(sacc, *reinterpret_cast<const float4*>(part + (size_t)(w * 2) * 128 + q * 4));
-                    if (FUSE) add4(sa0, *reinterpret_cast<const float4*>(part + (size_t)(w * 2 + 1) * 128 + q * 4));
+            float4 sacc[V], sa0[V];
+#pragma unroll
+            for (int s = 0; s < V; ++s) {
+                sacc[s] = z4; sa0[s] = z4;
+                if (grp == 0) {
+                    for (int w = 0; w < kWarpsPerBlock; ++w) {
+                        if (SELECT_ALL) add4(sacc[s], *reinterpret_cast<const float4*>(part + (size_t)(w * 2) * PW + slot_c4(q, s)));
+                        if (FUSE) add4(sa0[s], *reinterpret_cast<const float4*>(part + (size_t)(w * 2 + 1) * PW + slot_c4(q, s)));
+                    }
                 }
             }
-            if (!SELECT_ALL) { finish_list<G>(a, hb, row, fin_s, fin_p, cnt, lane, sacc); cross_group_sum4<G>(sacc); }
-            if (grp == 0 && ch_ok) write_row<FUSE>(a, row, q * 4, sacc, sa0, end - beg, beta, bw, bb);
+            if (!SELECT_ALL) {
+                finish_list<G>(a, hb, row, fin_s, fin_p, cnt, lane, sacc);
+#pragma unroll
+                for (int s = 0; s < V; ++s) cross_group_sum4<G>(sacc[s]);
+            }
+#pragma unroll
+            for (int s = 0; s < V; ++s)
+                if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), sacc[s], sa0[s], end - beg, beta, bw[s], bb[s]);
         }
         __syncthreads();
     }
@@ -852,24 +941,33 @@ __global__ void __launch_bounds__(kThreads) list_agg_fwd_kernel(
     const float* __restrict__ h, int n_rows, int c, int64_t ldh, int list_k, const int* __restrict__ sel_src,
     const float* __restrict__ sel_w, const int* __restrict__ sel_cnt, const float* __restrict__ inv_denom,
     float* __restrict__ out, int64_t ldo) {
-    constexpr int EPW = 32 / G;
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
+    const int q = lane % S::L, grp = lane / S::L, c4 = q * 4;
     const bool ch_ok = c4 < c;
     for (int row = blockIdx.x * kWarpsPerBlock + warp; row < n_rows; row += gridDim.x * kWarpsPerBlock) {
         const int cnt = min(__ldg(sel_cnt + row), list_k);
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+        float4 acc[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) acc[s] = make_float4(0.f, 0.f, 0.f, 0.f);
         for (int st = 0; st < cnt; st += EPW) {
             const int t = st + grp;
-            if (t < cnt && ch_ok) {
+            if (t < cnt && ch_ok) {                                  // ch_ok = slot 0 holds data; a lane's later slots may not
                 const int j = __ldg(sel_src + (int64_t)row * list_k + t);
-                fma4(acc, __ldg(sel_w + (int64_t)row * list_k + t), ldg4(h + (int64_t)j * ldh + c4));
+                const float w = __ldg(sel_w + (int64_t)row * list_k + t);
+#pragma unroll
+                for (int s = 0; s < V; ++s)
+                    if (s == 0 || slot_c4(q, s) < c) fma4(acc[s], w, ldg4(h + (int64_t)j * ldh + slot_c4(q, s)));
             }
         }
-        acc.x = cross_group_sum<G>(acc.x); acc.y = cross_group_sum<G>(acc.y);
-        acc.z = cross_group_sum<G>(acc.z); acc.w = cross_group_sum<G>(acc.w);
-        if (grp == 0 && ch_ok)
-            *reinterpret_cast<float4*>(out + (int64_t)row * ldo + c4) = scale4(acc, inv_denom ? __ldg(inv_denom + row) : 1.f);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            acc[s].x = cross_group_sum<G>(acc[s].x); acc[s].y = cross_group_sum<G>(acc[s].y);
+            acc[s].z = cross_group_sum<G>(acc[s].z); acc[s].w = cross_group_sum<G>(acc[s].w);
+            if (grp == 0 && slot_c4(q, s) < c)
+                *reinterpret_cast<float4*>(out + (int64_t)row * ldo + slot_c4(q, s)) = scale4(acc[s], inv_denom ? __ldg(inv_denom + row) : 1.f);
+        }
     }
 }
 
@@ -879,11 +977,15 @@ __global__ void __launch_bounds__(kThreads) edge_agg_bwd_scatter_kernel(
     const float* __restrict__ h, const float* __restrict__ inv_r, const float* __restrict__ g, int n, int row_offset, int c, int64_t ld, const int* __restrict__ rowptr,
     const int* __restrict__ col, int top_k, const int* __restrict__ sel_src, const float* __restrict__ sel_w,
     const int* __restrict__ sel_cnt, const float* __restrict__ inv_denom, float* __restrict__ dval, float* __restrict__ dnrm) {
-    constexpr int EPW = 32 / G;
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
     constexpr int U = Unroll<G>::value;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < c;
+    const int q = lane % S::L, grp = lane / S::L;
+    bool ok[V];                                                  // slot holds data; ok[s] implies ok[0]
+    int c4[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < c; }
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int row = blockIdx.x * kWarpsPerBlock + warp; row < n; row += gridDim.x * kWarpsPerBlock) {
         int beg, cnt;
@@ -899,12 +1001,16 @@ __global__ void __launch_bounds__(kThreads) edge_agg_bwd_scatter_kernel(
         }
         if (cnt == 0) continue;
         const int grow = row_offset + row;                       // h / inv_r / dval / dnrm hold all nodes, g and the lists are shard-local
-        const float4 hi = ch_ok ? ldg4(h + (int64_t)grow * ld + c4) : z4;
-        const float4 ni = scale4(hi, __ldg(inv_r + grow));
-        const float4 gs = ch_ok ? scale4(ldg4(g + (int64_t)row * ld + c4), invd) : z4;     // g_i / deg_i
-        float4 dni = z4;
+        float4 ni[V], gs[V], dni[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            const float4 hi = ok[s] ? ldg4(h + (int64_t)grow * ld + c4[s]) : z4;
+            ni[s] = scale4(hi, __ldg(inv_r + grow));
+            gs[s] = ok[s] ? scale4(ldg4(g + (int64_t)row * ld + c4[s]), invd) : z4;    // g_i / deg_i
+            dni[s] = z4;
+        }
         for (int st = 0; st < cnt; st += EPW * U) {
-            float4 v[U]; int j[U]; float w[U];
+            float4 v[U][V]; int j[U]; float w[U];
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int t = st + u * EPW + grp;
@@ -913,24 +1019,32 @@ __global__ void __launch_bounds__(kThreads) edge_agg_bwd_scatter_kernel(
                     if (SELECT_ALL) j[u] = __ldg(col + beg + t);
                     else { j[u] = __ldg(sel_src + (int64_t)row * top_k + t); w[u] = __ldg(sel_w + (int64_t)row * top_k + t); }
                 }
-                v[u] = (j[u] >= 0 && ch_ok) ? ldg4(h + (int64_t)j[u] * ld + c4) : z4;
+#pragma unroll
+                for (int s = 0; s < V; ++s) v[u][s] = (j[u] >= 0 && ok[s]) ? ldg4(h + (int64_t)j[u] * ld + c4[s]) : z4;
             }
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 if (st + u * EPW >= cnt) break;
                 const float inv_rj = j[u] >= 0 ? __ldg(inv_r + j[u]) : 0.f;
-                const float s = SELECT_ALL ? group_sum<G>(dot4(ni, v[u])) * inv_rj + 0.0f : w[u];
-                const float ds = group_sum<G>(dot4(v[u], gs));                 // dL/ds_e = (h_j . g_i)/deg_i
-                if (j[u] >= 0 && ch_ok) {
-                    atomicAdd(reinterpret_cast<float4*>(dval + (int64_t)j[u] * ld + c4), scale4(gs, s));
-                    atomicAdd(reinterpret_cast<float4*>(dnrm + (int64_t)j[u] * ld + c4), scale4(ni, ds));
-                    fma4(dni, ds * inv_rj, v[u]);                              // ds * n_j
+                const float sc = SELECT_ALL ? group_sum<S::L>(dotv<V>(ni, v[u])) * inv_rj + 0.0f : w[u];
+                const float ds = group_sum<S::L>(dotv<V>(v[u], gs));           // dL/ds_e = (h_j . g_i)/deg_i
+                if (j[u] >= 0 && ok[0]) {
+#pragma unroll
+                    for (int s = 0; s < V; ++s) {
+                        if (s > 0 && !ok[s]) continue;
+                        atomicAdd(reinterpret_cast<float4*>(dval + (int64_t)j[u] * ld + c4[s]), scale4(gs[s], sc));
+                        atomicAdd(reinterpret_cast<float4*>(dnrm + (int64_t)j[u] * ld + c4[s]), scale4(ni[s], ds));
+                        fma4(dni[s], ds * inv_rj, v[u][s]);                    // ds * n_j
+                    }
                 }
             }
         }
-        dni.x = cross_group_sum<G>(dni.x); dni.y = cross_group_sum<G>(dni.y);
-        dni.z = cross_group_sum<G>(dni.z); dni.w = cross_group_sum<G>(dni.w);
-        if (grp == 0 && ch_ok) atomicAdd(reinterpret_cast<float4*>(dnrm + (int64_t)grow * ld + c4), dni);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            dni[s].x = cross_group_sum<G>(dni[s].x); dni[s].y = cross_group_sum<G>(dni[s].y);
+            dni[s].z = cross_group_sum<G>(dni[s].z); dni[s].w = cross_group_sum<G>(dni[s].w);
+            if (grp == 0 && ok[s]) atomicAdd(reinterpret_cast<float4*>(dnrm + (int64_t)grow * ld + c4[s]), dni[s]);
+        }
     }
 }
 
@@ -939,25 +1053,38 @@ template <int G>
 __global__ void __launch_bounds__(kThreads) norm_bwd_finish_kernel(const float* __restrict__ h, const float* __restrict__ inv_rv, int n, int c, int64_t ld,
                                                                   const float* __restrict__ dval, const float* __restrict__ dnrm,
                                                                   float* __restrict__ dh) {
-    constexpr int RPW = 32 / G;
+    using S = RowShape<G>;
+    constexpr int RPW = S::EPW, V = S::V;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < c;
+    const int q = lane % S::L, grp = lane / S::L;
+    int c4[V];
+    bool ch_ok[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ch_ok[s] = c4[s] < c; }
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int r0 = (blockIdx.x * kWarpsPerBlock + warp) * RPW; r0 < n; r0 += gridDim.x * kWarpsPerBlock * RPW) {
         const int row = r0 + grp;
-        const bool ok = row < n && ch_ok;
-        const float4 hi = ok ? ldg4(h + (int64_t)row * ld + c4) : z4;
+        bool ok[V];
+        float4 hi[V], ni[V], dn[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) ok[s] = row < n && ch_ok[s];
+#pragma unroll
+        for (int s = 0; s < V; ++s) hi[s] = ok[s] ? ldg4(h + (int64_t)row * ld + c4[s]) : z4;
         const float inv_r = row < n ? __ldg(inv_rv + row) : 0.f;
-        const float4 ni = scale4(hi, inv_r);
-        const float4 dn = ok ? ldg4(dnrm + (int64_t)row * ld + c4) : z4;
-        const float proj = group_sum<G>(dot4(ni, dn));
-        if (ok) {
-            const float4 dv = ldg4(dval + (int64_t)row * ld + c4);
-            float4 o;
-            o.x = dv.x + (dn.x - ni.x * proj) * inv_r; o.y = dv.y + (dn.y - ni.y * proj) * inv_r;
-            o.z = dv.z + (dn.z - ni.z * proj) * inv_r; o.w = dv.w + (dn.w - ni.w * proj) * inv_r;
-            *reinterpret_cast<float4*>(dh + (int64_t)row * ld + c4) = o;
+#pragma unroll
+        for (int s = 0; s < V; ++s) ni[s] = scale4(hi[s], inv_r);
+#pragma unroll
+        for (int s = 0; s < V; ++s) dn[s] = ok[s] ? ldg4(dnrm + (int64_t)row * ld + c4[s]) : z4;
+        const float proj = group_sum<S::L>(dotv<V>(ni, dn));
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            if (ok[s]) {
+                const float4 dv = ldg4(dval + (int64_t)row * ld + c4[s]);
+                float4 o;
+                o.x = dv.x + (dn[s].x - ni[s].x * proj) * inv_r; o.y = dv.y + (dn[s].y - ni[s].y * proj) * inv_r;
+                o.z = dv.z + (dn[s].z - ni[s].z * proj) * inv_r; o.w = dv.w + (dn[s].w - ni[s].w * proj) * inv_r;
+                *reinterpret_cast<float4*>(dh + (int64_t)row * ld + c4[s]) = o;
+            }
         }
     }
 }
@@ -991,11 +1118,15 @@ struct EdgeBwdArgs {
 
 template <int G, bool SELECT_ALL>
 __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwdArgs a) {
-    constexpr int EPW = 32 / G;
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
     constexpr int U = Unroll<G>::value;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < a.c;
+    const int q = lane % S::L, grp = lane / S::L;
+    bool ok[V];                                                              // slot holds data; ok[s] implies ok[0]
+    int c4[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < a.c; }
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     const float gscale = a.beta ? 1.0f - __ldg(a.beta) : 1.0f;
     float bpart = 0.f;
@@ -1005,13 +1136,24 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
         const int cnt = SELECT_ALL ? deg : __ldg(a.sel_cnt + row);
         const float invd = 1.0f / (float)max(deg, 1);
         const float iri = __ldg(a.inv_r + grow);
-        const float4 graw = ch_ok ? ldg4(a.g + (int64_t)row * a.ldg + c4) : z4;
-        const float4 gs = scale4(graw, invd * gscale);                     // g1_i / deg_i
-        const float4 ni = ch_ok ? scale4(ldg4(a.h + (int64_t)grow * a.ld + c4), iri) : z4;
-        if (a.diff && grp == 0 && ch_ok) bpart += dot4(ldg4(a.diff + (int64_t)row * a.lddiff + c4), graw);   // dL/dbeta
-        float4 dni = z4;
+        float4 graw[V], gs[V], ni[V], dni[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            graw[s] = ok[s] ? ldg4(a.g + (int64_t)row * a.ldg + c4[s]) : z4;
+            gs[s] = scale4(graw[s], invd * gscale);                           // g1_i / deg_i
+            ni[s] = ok[s] ? scale4(ldg4(a.h + (int64_t)grow * a.ld + c4[s]), iri) : z4;
+        }
+        if (a.diff && grp == 0 && ok[0]) {                                   // dL/dbeta
+            float b = dot4(ldg4(a.diff + (int64_t)row * a.lddiff + c4[0]), graw[0]);
+#pragma unroll
+            for (int s = 1; s < V; ++s)
+                if (ok[s]) b += dot4(ldg4(a.diff + (int64_t)row * a.lddiff + c4[s]), graw[s]);
+            bpart += b;
+        }
+#pragma unroll
+        for (int s = 0; s < V; ++s) dni[s] = z4;
         for (int st = 0; st < cnt; st += EPW * U) {
-            float4 v[U]; int j[U], qp[U]; float w[U];
+            float4 v[U][V]; int j[U], qp[U]; float w[U];
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int t = st + u * EPW + grp;
@@ -1023,22 +1165,27 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
                         j[u] = __ldg(a.sel_src + o); w[u] = __ldg(a.sel_w + o); qp[u] = __ldg(a.sel_q + o);
                     }
                 }
-                v[u] = (j[u] >= 0 && ch_ok) ? ldg4(a.h + (int64_t)j[u] * a.ld + c4) : z4;
+#pragma unroll
+                for (int s = 0; s < V; ++s) v[u][s] = (j[u] >= 0 && ok[s]) ? ldg4(a.h + (int64_t)j[u] * a.ld + c4[s]) : z4;
             }
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 if (st + u * EPW >= cnt) break;                              // warp-uniform
                 const float irj = j[u] >= 0 ? __ldg(a.inv_r + j[u]) : 0.f;
-                const float ds = group_sum<G>(dot4(v[u], gs));               // dL/ds_e
-                const float s = SELECT_ALL ? group_sum<G>(dot4(ni, v[u])) * irj + 0.0f : w[u];
+                const float ds = group_sum<S::L>(dotv<V>(v[u], gs));         // dL/ds_e
+                const float sc = SELECT_ALL ? group_sum<S::L>(dotv<V>(ni, v[u])) * irj + 0.0f : w[u];
                 if (j[u] >= 0) {
-                    fma4(dni, ds * irj, v[u]);                               // ds_e n_j
-                    if (q == 0) a.coef[qp[u]] = make_float2(s * invd * gscale, ds * iri);
+#pragma unroll
+                    for (int s = 0; s < V; ++s) fma4(dni[s], ds * irj, v[u][s]);   // ds_e n_j
+                    if (q == 0) a.coef[qp[u]] = make_float2(sc * invd * gscale, ds * iri);
                 }
             }
         }
-        cross_group_sum4<G>(dni);
-        if (grp == 0 && ch_ok) *reinterpret_cast<float4*>(a.dnT + (int64_t)grow * a.ld + c4) = dni;
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            cross_group_sum4<G>(dni[s]);
+            if (grp == 0 && ok[s]) *reinterpret_cast<float4*>(a.dnT + (int64_t)grow * a.ld + c4[s]) = dni[s];
+        }
     }
     if (a.dbeta_part) {                                                      // fixed-order block sum -> one partial per block
         bpart = group_sum<32>(bpart);
@@ -1055,58 +1202,78 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
 
 template <int G, bool FUSE>
 __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwdArgs a) {
-    constexpr int EPW = 32 / G;
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
     constexpr int U = Unroll<G>::value;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < a.c;
+    const int q = lane % S::L, grp = lane / S::L;
+    bool ok[V];                                                              // slot holds data; ok[s] implies ok[0]
+    int c4[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < a.c; }
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     const float beta = FUSE ? __ldg(a.beta) : 0.f;
     for (int j = blockIdx.x * kWarpsPerBlock + warp; j < a.n_total; j += gridDim.x * kWarpsPerBlock) {
         const int jr = j - a.shift;                                          // rows of the by-source CSR are shifted source ids
         int beg = 0, end = 0;
         if (jr >= 0) { beg = __ldg(a.rowptr_out + jr); end = __ldg(a.rowptr_out + jr + 1); }
-        float4 dval = z4, dnj = z4, dw = z4;
+        float4 dval[V], dnj[V], dw[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) { dval[s] = z4; dnj[s] = z4; dw[s] = z4; }
         for (int base = beg; base < end; base += 32) {
             const int nchunk = min(32, end - base);
             const int il = lane < nchunk ? __ldg(a.col_out + base + lane) : 0;
             const float2 cf = lane < nchunk ? __ldg(a.coef + base + lane) : make_float2(0.f, 0.f);
             for (int st = 0; st < nchunk; st += EPW * U) {
-                float4 gv[U], hv[U]; float ca[U], cb[U];
+                float4 gv[U][V], hv[U][V]; float ca[U], cb[U];
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
                     const int e = st + u * EPW + grp;
                     const int i = __shfl_sync(kFull, il, e & 31);
                     ca[u] = __shfl_sync(kFull, cf.x, e & 31);
                     cb[u] = __shfl_sync(kFull, cf.y, e & 31);
-                    const bool on = e < nchunk && ch_ok;
+                    const bool on = e < nchunk && ok[0];
                     const bool sel = on && (ca[u] != 0.f || cb[u] != 0.f);   // an unselected edge has both coefficients 0
                     if (!on) { ca[u] = 0.f; cb[u] = 0.f; }
-                    gv[u] = (FUSE ? on : sel) ? ldg4(a.g + (int64_t)i * a.ldg + c4) : z4;
-                    hv[u] = sel ? ldg4(a.h + (int64_t)i * a.ld + c4) : z4;
+#pragma unroll
+                    for (int s = 0; s < V; ++s) {
+                        const bool sok = s == 0 || ok[s];
+                        gv[u][s] = ((FUSE ? on : sel) && sok) ? ldg4(a.g + (int64_t)i * a.ldg + c4[s]) : z4;
+                        hv[u][s] = (sel && sok) ? ldg4(a.h + (int64_t)i * a.ld + c4[s]) : z4;
+                    }
                 }
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
-                    fma4(dval, ca[u], gv[u]);
-                    fma4(dnj, cb[u], hv[u]);
-                    if (FUSE) add4(dw, gv[u]);
+#pragma unroll
+                    for (int s = 0; s < V; ++s) {
+                        fma4(dval[s], ca[u], gv[u][s]);
+                        fma4(dnj[s], cb[u], hv[u][s]);
+                        if (FUSE) add4(dw[s], gv[u][s]);
+                    }
                 }
             }
         }
-        cross_group_sum4<G>(dval);
-        cross_group_sum4<G>(dnj);
-        if (FUSE) cross_group_sum4<G>(dw);
         const float irj = __ldg(a.inv_r + j);
-        const float4 nj = ch_ok ? scale4(ldg4(a.h + (int64_t)j * a.ld + c4), irj) : z4;
-        float4 dn = ch_ok ? ldg4(a.dnT + (int64_t)j * a.ld + c4) : z4;
-        add4(dn, dnj);
-        const float proj = group_sum<G>(dot4(nj, dn));
-        if (grp == 0 && ch_ok) {
-            float4 o;
-            o.x = dval.x + (dn.x - nj.x * proj) * irj; o.y = dval.y + (dn.y - nj.y * proj) * irj;
-            o.z = dval.z + (dn.z - nj.z * proj) * irj; o.w = dval.w + (dn.w - nj.w * proj) * irj;
-            *reinterpret_cast<float4*>(a.dh + (int64_t)j * a.ld + c4) = o;
-            if (FUSE) *reinterpret_cast<float4*>(a.dwt + (int64_t)j * a.lddw + c4) = scale4(dw, beta);
+        float4 nj[V], dn[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            cross_group_sum4<G>(dval[s]);
+            cross_group_sum4<G>(dnj[s]);
+            if (FUSE) cross_group_sum4<G>(dw[s]);
+            nj[s] = ok[s] ? scale4(ldg4(a.h + (int64_t)j * a.ld + c4[s]), irj) : z4;
+            dn[s] = ok[s] ? ldg4(a.dnT + (int64_t)j * a.ld + c4[s]) : z4;
+            add4(dn[s], dnj[s]);
+        }
+        const float proj = group_sum<S::L>(dotv<V>(nj, dn));
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            if (grp == 0 && ok[s]) {
+                float4 o;
+                o.x = dval[s].x + (dn[s].x - nj[s].x * proj) * irj; o.y = dval[s].y + (dn[s].y - nj[s].y * proj) * irj;
+                o.z = dval[s].z + (dn[s].z - nj[s].z * proj) * irj; o.w = dval[s].w + (dn[s].w - nj[s].w * proj) * irj;
+                *reinterpret_cast<float4*>(a.dh + (int64_t)j * a.ld + c4[s]) = o;
+                if (FUSE) *reinterpret_cast<float4*>(a.dwt + (int64_t)j * a.lddw + c4[s]) = scale4(dw[s], beta);
+            }
         }
     }
 }
@@ -1581,34 +1748,44 @@ __global__ void __launch_bounds__(256) sum_partials_kernel(const float* __restri
 }
 
 // ------------------------------------------------------------------------------------------ K3 / K4
+// acc[s] = sum over the row's edges of val[e] x[col[e]], slot s of the lane (c4[s] = its first channel, ok[s] = it holds data)
 template <int G>
-__device__ __forceinline__ float4 gather_sum(const float* __restrict__ x, int64_t ldx, const int* __restrict__ col,
-                                             const float* __restrict__ val, int beg, int end, int c4, bool ch_ok, int grp, int lane) {
-    constexpr int EPW = 32 / G;
+__device__ __forceinline__ void gather_sum(const float* __restrict__ x, int64_t ldx, const int* __restrict__ col,
+                                           const float* __restrict__ val, int beg, int end, const int (&c4)[RowShape<G>::V],
+                                           const bool (&ok)[RowShape<G>::V], int grp, int lane, float4 (&acc)[RowShape<G>::V]) {
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
     constexpr int U = Unroll<G>::value;
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 acc = z4;
+#pragma unroll
+    for (int s = 0; s < V; ++s) acc[s] = z4;
     for (int base = beg; base < end; base += 32) {
         const int nchunk = min(32, end - base);
         const int jl = lane < nchunk ? __ldg(col + base + lane) : -1;
         const float wl = (val && lane < nchunk) ? __ldg(val + base + lane) : 1.f;
         for (int st = 0; st < nchunk; st += EPW * U) {
-            float4 v[U]; float w[U];
+            float4 v[U][V]; float w[U];
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int e = st + u * EPW + grp;
                 int j = __shfl_sync(0xffffffffu, jl, e & 31);
                 w[u] = __shfl_sync(0xffffffffu, wl, e & 31);
                 if (e >= nchunk) j = -1;
-                v[u] = (j >= 0 && ch_ok) ? ldg4(x + (int64_t)j * ldx + c4) : z4;
+#pragma unroll
+                for (int s = 0; s < V; ++s) v[u][s] = (j >= 0 && ok[s]) ? ldg4(x + (int64_t)j * ldx + c4[s]) : z4;
             }
 #pragma unroll
-            for (int u = 0; u < U; ++u) fma4(acc, w[u], v[u]);
+            for (int u = 0; u < U; ++u) {
+#pragma unroll
+                for (int s = 0; s < V; ++s) fma4(acc[s], w[u], v[u][s]);
+            }
         }
     }
-    acc.x = cross_group_sum<G>(acc.x); acc.y = cross_group_sum<G>(acc.y);
-    acc.z = cross_group_sum<G>(acc.z); acc.w = cross_group_sum<G>(acc.w);
-    return acc;
+#pragma unroll
+    for (int s = 0; s < V; ++s) {
+        acc[s].x = cross_group_sum<G>(acc[s].x); acc[s].y = cross_group_sum<G>(acc[s].y);
+        acc[s].z = cross_group_sum<G>(acc[s].z); acc[s].w = cross_group_sum<G>(acc[s].w);
+    }
 }
 
 template <int G>
@@ -1616,16 +1793,25 @@ __global__ void __launch_bounds__(kThreads) spmm_fwd_kernel(const float* __restr
                                                            const int* __restrict__ rowptr, const int* __restrict__ col,
                                                            const float* __restrict__ val, const float* __restrict__ rowscale,
                                                            const float* __restrict__ bias, float* __restrict__ out, int64_t ldo) {
+    using S = RowShape<G>;
+    constexpr int V = S::V;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < c;
+    const int q = lane % S::L, grp = lane / S::L;
+    int c4[V];
+    bool ok[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < c; }
     for (int row = blockIdx.x * kWarpsPerBlock + warp; row < n_rows; row += gridDim.x * kWarpsPerBlock) {
         const int beg = __ldg(rowptr + row), end = __ldg(rowptr + row + 1);
-        float4 acc = gather_sum<G>(x, ldx, col, val, beg, end, c4, ch_ok, grp, lane);
-        if (grp == 0 && ch_ok) {
-            if (rowscale) acc = scale4(acc, __ldg(rowscale + row));
-            if (bias) { const float4 b = ldg4(bias + c4); acc.x += b.x; acc.y += b.y; acc.z += b.z; acc.w += b.w; }
-            *reinterpret_cast<float4*>(out + (int64_t)row * ldo + c4) = acc;
+        float4 acc[V];
+        gather_sum<G>(x, ldx, col, val, beg, end, c4, ok, grp, lane, acc);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            if (grp == 0 && ok[s]) {
+                if (rowscale) acc[s] = scale4(acc[s], __ldg(rowscale + row));
+                if (bias) { const float4 b = ldg4(bias + c4[s]); acc[s].x += b.x; acc[s].y += b.y; acc[s].z += b.z; acc[s].w += b.w; }
+                *reinterpret_cast<float4*>(out + (int64_t)row * ldo + c4[s]) = acc[s];
+            }
         }
     }
 }
@@ -1636,24 +1822,34 @@ __global__ void __launch_bounds__(kThreads) pp_fuse_fwd_kernel(const float* __re
                                                               const float* __restrict__ b_w, const float* __restrict__ beta_p,
                                                               const float* __restrict__ out1, const float* __restrict__ bias,
                                                               float* __restrict__ out0, float* __restrict__ out) {
+    using S = RowShape<G>;
+    constexpr int V = S::V;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int q = lane % G, grp = lane / G, c4 = q * 4;
-    const bool ch_ok = c4 < c;
+    const int q = lane % S::L, grp = lane / S::L;
+    int c4[V];
+    bool ok[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < c; }
     const float beta = __ldg(beta_p);
     for (int row = blockIdx.x * kWarpsPerBlock + warp; row < n; row += gridDim.x * kWarpsPerBlock) {
         const int beg = __ldg(rowptr + row), end = __ldg(rowptr + row + 1);
-        float4 a = gather_sum<G>(wt, ld, col, nullptr, beg, end, c4, ch_ok, grp, lane);
-        if (grp == 0 && ch_ok) {
-            const float4 b = ldg4(b_w + c4);
-            a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
-            const int64_t o = (int64_t)row * ld + c4;
-            *reinterpret_cast<float4*>(out0 + o) = a;
-            const float4 o1 = ldg4(out1 + o);
-            float4 r;
-            r.x = beta * a.x + (1.f - beta) * o1.x; r.y = beta * a.y + (1.f - beta) * o1.y;
-            r.z = beta * a.z + (1.f - beta) * o1.z; r.w = beta * a.w + (1.f - beta) * o1.w;
-            if (bias) { const float4 bb = ldg4(bias + c4); r.x += bb.x; r.y += bb.y; r.z += bb.z; r.w += bb.w; }
-            *reinterpret_cast<float4*>(out + o) = r;
+        float4 acc[V];
+        gather_sum<G>(wt, ld, col, nullptr, beg, end, c4, ok, grp, lane, acc);
+#pragma unroll
+        for (int s = 0; s < V; ++s) {
+            if (grp == 0 && ok[s]) {
+                float4 a = acc[s];
+                const float4 b = ldg4(b_w + c4[s]);
+                a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
+                const int64_t o = (int64_t)row * ld + c4[s];
+                *reinterpret_cast<float4*>(out0 + o) = a;
+                const float4 o1 = ldg4(out1 + o);
+                float4 r;
+                r.x = beta * a.x + (1.f - beta) * o1.x; r.y = beta * a.y + (1.f - beta) * o1.y;
+                r.z = beta * a.z + (1.f - beta) * o1.z; r.w = beta * a.w + (1.f - beta) * o1.w;
+                if (bias) { const float4 bb = ldg4(bias + c4[s]); r.x += bb.x; r.y += bb.y; r.z += bb.z; r.w += bb.w; }
+                *reinterpret_cast<float4*>(out + o) = r;
+            }
         }
     }
 }
@@ -1751,13 +1947,20 @@ __global__ void __launch_bounds__(kThreads) sddmm_dot_kernel(const float* __rest
         case 4: { constexpr int G = 4; __VA_ARGS__; } break;                    \
         case 8: { constexpr int G = 8; __VA_ARGS__; } break;                    \
         case 16: { constexpr int G = 16; __VA_ARGS__; } break;                  \
-        default: { constexpr int G = 32; __VA_ARGS__; } break;                  \
+        case 32: { constexpr int G = 32; __VA_ARGS__; } break;                  \
+        case 64: { constexpr int G = 64; __VA_ARGS__; } break;                  \
+        case 128: { constexpr int G = 128; __VA_ARGS__; } break;                \
+        default: set_error("c=%lld: no edge kernel for this width", (long long)(cexpr)); return SNG_ERR_UNSUPPORTED; \
     }
+static_assert(SNG_MAX_CHANNELS == 4 * 128, "SNG_DISPATCH_G instantiates the edge kernels up to G = 128 float4 slots per row");
 
 static int check_rows(const char* fn, int64_t n, int64_t c, int64_t ld) {
     if (n < 0 || n >= (1ll << 31)) { set_error("%s: n=%lld out of range", fn, (long long)n); return SNG_ERR_ARG; }
     if (c <= 0 || c % 4 != 0 || ld % 4 != 0 || ld < c) { set_error("%s: c=%lld ld=%lld must be multiples of 4, ld>=c", fn, (long long)c, (long long)ld); return SNG_ERR_ARG; }
-    if (c > 128) { set_error("%s: c=%lld > 128 channels not supported by the edge kernels", fn, (long long)c); return SNG_ERR_UNSUPPORTED; }
+    if (c > SNG_MAX_CHANNELS) {
+        set_error("%s: c=%lld > %d channels (SNG_MAX_CHANNELS) not supported by the edge kernels", fn, (long long)c, SNG_MAX_CHANNELS);
+        return SNG_ERR_UNSUPPORTED;
+    }
     return SNG_OK;
 }
 
@@ -1779,9 +1982,11 @@ extern "C" int sng_rownorm_f32(const float* x, int64_t n, int64_t d, int64_t ldx
 namespace sng {
 // dynamic shared memory of the long-row / hub kernels (see their carve-up)
 static size_t long_smem(int top_k) { return (size_t)kWarpsPerBlock * 2 * (top_k > 0 ? top_k : 1) * sizeof(float); }
+// (the partial sums take 128 V channels per warp: 8 KB for C <= 128, 32 KB at C = 512, inside the 48 KB default)
+template <int G>
 static size_t hub_smem(int top_k) {
     const size_t k1 = top_k > 0 ? top_k : 1;
-    return ((size_t)kWarpsPerBlock * 2 * k1 + 2 * k1 + kWarpsPerBlock + (size_t)kWarpsPerBlock * 2 * 128) * sizeof(float);
+    return ((size_t)kWarpsPerBlock * 2 * k1 + 2 * k1 + kWarpsPerBlock + (size_t)kWarpsPerBlock * 2 * 128 * RowShape<G>::V) * sizeof(float);
 }
 
 // row slots per warp of the staged forward kernel (see there); any single item (33 / fused 65 slots) must fit
@@ -1793,7 +1998,7 @@ static int forward_slots(bool fuse, int g) {
 }
 template <int G, bool FUSE, bool SELECT_ALL>
 static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hub, cudaStream_t st) {
-    const size_t ls = long_smem(a.top_k), hs = hub_smem(a.top_k);
+    const size_t ls = long_smem(a.top_k), hs = hub_smem<G>(a.top_k);
     if constexpr (G <= 8) {
         if (a.n_chunks >= 0) {
             // degree lists known, rows of <= 128 bytes: staged kernel over the short rows, then over the <= 32-edge chunks of the
@@ -1860,7 +2065,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
     }
     cudaStream_t st = (cudaStream_t)stream;
     if (!inv_norm_ready)                                     // (sng_lin_norm_fwd already produced it with h)
-        SNG_DISPATCH_G(c, row_inv_norm_kernel<G><<<grid_resident(row_inv_norm_kernel<G>, n_total, kWarpsPerBlock * (32 / G) * 4), kThreads, 0, st>>>(h, n_total, (int)c, ldh, inv_norm));
+        SNG_DISPATCH_G(c, row_inv_norm_kernel<G><<<grid_resident(row_inv_norm_kernel<G>, n_total, kWarpsPerBlock * RowShape<G>::EPW * 4), kThreads, 0, st>>>(h, n_total, (int)c, ldh, inv_norm));
     EdgeFwdArgs a;
     a.h = h; a.inv_r = inv_norm; a.n = (int)n; a.row_offset = (int)row_offset; a.c = (int)c; a.ldh = (int)ldh;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.rows = nullptr; a.n_rows = 0; a.skip_deg = 0;
@@ -2001,7 +2206,7 @@ extern "C" int sng_edge_agg_bwd(const float* h, const float* inv_norm, const flo
     SNG_DISPATCH_G(c,
         if (n > 0 && top_k > 0) edge_agg_bwd_scatter_kernel<G, false><<<grid_resident(edge_agg_bwd_scatter_kernel<G, false>, n, kWarpsPerBlock), kThreads, 0, st>>>(h, inv_norm, g, (int)n, (int)row_offset, (int)c, ld, rowptr, col, top_k, sel_src, sel_w, sel_cnt, inv_denom, dval, dnrm);
         else if (n > 0) edge_agg_bwd_scatter_kernel<G, true><<<grid_resident(edge_agg_bwd_scatter_kernel<G, true>, n, kWarpsPerBlock), kThreads, 0, st>>>(h, inv_norm, g, (int)n, (int)row_offset, (int)c, ld, rowptr, col, 0, nullptr, nullptr, nullptr, nullptr, dval, dnrm);
-        norm_bwd_finish_kernel<G><<<grid_resident(norm_bwd_finish_kernel<G>, n_total, kWarpsPerBlock * (32 / G)), kThreads, 0, st>>>(h, inv_norm, (int)n_total, (int)c, ld, dval, dnrm, dh));
+        norm_bwd_finish_kernel<G><<<grid_resident(norm_bwd_finish_kernel<G>, n_total, kWarpsPerBlock * RowShape<G>::EPW), kThreads, 0, st>>>(h, inv_norm, (int)n_total, (int)c, ld, dval, dnrm, dh));
     return check_launch("sng_edge_agg_bwd");
 }
 

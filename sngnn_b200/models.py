@@ -16,6 +16,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 from torch.nn.parameter import Parameter
 
+from . import _C
 from . import functional as SF
 from . import graph as G
 
@@ -28,10 +29,10 @@ def _as_bool(flag):
 class _SNConvBase(nn.Module):
     @staticmethod
     def _check_width(out_channels):
-        # the edge kernels hold a row in at most 32 lanes x 4 channels; fail at construction, not at the first forward
-        if SF.padded_channels(out_channels) > 128:
-            raise ValueError(f"out_channels={out_channels}: the B200 edge kernels support at most 128 channels per layer "
-                             "(the reference accepts any width)")
+        # the edge kernels are instantiated up to SNG_MAX_CHANNELS; fail at construction, not at the first forward
+        if SF.padded_channels(out_channels) > _C.MAX_CHANNELS:
+            raise ValueError(f"out_channels={out_channels}: the B200 edge kernels support at most {_C.MAX_CHANNELS} channels per "
+                             "layer (the reference accepts any width)")
 
     def _init_bias(self, bias, out_channels):
         if bias:
