@@ -48,9 +48,9 @@ SNG_API int sng_version(void);
 SNG_API const char* sng_last_error(void);
 /* SM count / compute capability of the current device; fails (SNG_ERR_CUDA) when there is no GPU. */
 SNG_API int sng_device_info(int* sm_count, int* cc_major, int* cc_minor);
-/* Tests / experiments only: while enabled, the similarity-kNN planner honours its SNG_KNN_* environment overrides (seed
- * stride / quantile, candidate slots, ring depth ...).  Off by default: the library then never reads the environment.
- * Returns the previous setting. */
+/* Tests / experiments only: while enabled, the similarity-kNN build honours four environment overrides: SNG_KNN_CAND
+ * (candidate slots per row), SNG_KNN_SEED_S / SNG_KNN_SEED_Q (seed stride / quantile) and SNG_KNN_NORETRY (no retry pass).
+ * Off by default: the library then never reads the environment.  Returns the previous setting. */
 SNG_API int sng_set_debug_env(int enabled);
 
 /* ------------------------------------------------------------------------------------------------
@@ -257,18 +257,18 @@ SNG_API int sng_class_sums_f64(const float* xhat, const int32_t* y, int64_t n, i
  *   N self loops are appended at the END; with remove_self_loops every src == dst edge is then dropped.
  *   rowptr_in [n+1], col_in [num_edges + n capacity]: CSR by target, sources in original edge-position order (the
  *   tie-break order of the selection); inv_deg [n] = 1/max(in-degree, 1).
- *   structural != 0: rowptr_out [n+1], col_out [capacity] = CSR by (src - min src) holding the targets
- *   (A of R: models.py:124-127), col_in_shift [capacity] = col_in - min src (its transpose).
- *   tpos [capacity] (may be NULL; needs structural) = position of by-target edge p in the by-source arrays (the transpose
+ *   rowptr_out [n+1], col_out [capacity] = CSR by (src - min src) holding the targets (A of R: models.py:124-127),
+ *   col_in_shift [capacity] = col_in - min src (its transpose).
+ *   tpos [capacity] (may be NULL) = position of by-target edge p in the by-source arrays (the transpose
  *   index of sng_edge_bwd).  long_rows [n] (may be NULL): local ids of the rows with 32 < in-degree <= 1024 from the
  *   front, of the rows with in-degree > 1024 from the back, in no particular order (the caller sorts them and derives the
  *   chunk tables of sng_edge_fwd).
- *   info (device int32[8]) = {number of kept edges E', min src, 1 if every in-list equals the out-list and min src == 0
- *   (structural only), rows in (32, 1024], rows > 1024, max in-degree, 0, 0}.  Only the first E' entries of col_* / tpos
+ *   info (device int32[8]) = {number of kept edges E', min src, 1 if every in-list equals the out-list and min src == 0,
+ *   rows in (32, 1024], rows > 1024, max in-degree, 0, 0}.  Only the first E' entries of col_* / tpos
  *   are meaningful.  The two stable sorts are cub::DeviceRadixSort (a library sort); everything else is kernels of this library.
  */
 SNG_API size_t sng_graph_prepare_workspace_bytes(int64_t num_edges, int64_t n);
-SNG_API int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, int64_t n, int remove_self_loops, int structural,
+SNG_API int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, int64_t n, int remove_self_loops,
                       int32_t* rowptr_in, int32_t* col_in, float* inv_deg,
                       int32_t* rowptr_out, int32_t* col_out, int32_t* col_in_shift,
                       int32_t* tpos, int32_t* long_rows,

@@ -1,4 +1,5 @@
-"""A/B timing of the edge kernels at the pokec shape: python scripts/edge_ab.py [lib path] (env SNG_K2_SLOTS / SNG_K2B_SLOTS honoured)."""
+"""A/B timing of the edge kernels at the pokec shape: python scripts/edge_ab.py [lib path] [C].  Run it once per library,
+alternating, and compare the JSON lines."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -26,19 +27,12 @@ def timed(fn, steps=10, warm=3):
     return round(a.elapsed_time(b) / steps, 4)
 
 
-_C.lib().sng_set_debug_env(1)
 res = {"lib": os.path.basename(_C._LIB_PATH), "C": C}
-for s in [int(x) for x in os.environ.get("FWD_SLOTS", "33,40").split(",")]:
-    os.environ["SNG_K2_SLOTS"] = str(s)
-    res[f"fwd_infer_s{s}"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, False))
-    res[f"fwd_train_s{s}"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, True, want_q=True))
-for s in [int(x) for x in os.environ.get("FUSE_SLOTS", "65,66").split(",")]:
-    os.environ["SNG_K2_SLOTS"] = str(s)
-    res[f"fwd_fused_infer_s{s}"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, False, fuse))
-    res[f"fwd_fused_train_s{s}"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, True, fuse, want_q=True))
+res["fwd_infer"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, False))
+res["fwd_train"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, True, want_q=True))
+res["fwd_fused_infer"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, False, fuse))
+res["fwd_fused_train"] = timed(lambda: SF._edge_fwd(h, g, 0, 10, 0.0, True, fuse, want_q=True))
 out, ss, sw, sq, sc, inv, diff = SF._edge_fwd(h, g, 0, 10, 0.0, True, fuse, want_q=True)
-for s in [int(x) for x in os.environ.get("BWD_SLOTS", "64").split(",")]:
-    os.environ["SNG_K2B_SLOTS"] = str(s)
-    res[f"bwd_plain_s{s}"] = timed(lambda: SF.edge_bwd(h, inv, gg, g, 10, ss, sw, sq, sc, None, None))
-    res[f"bwd_fused_s{s}"] = timed(lambda: SF.edge_bwd(h, inv, gg, g, 10, ss, sw, sq, sc, fuse[2], diff))
+res["bwd_plain"] = timed(lambda: SF.edge_bwd(h, inv, gg, g, 10, ss, sw, sq, sc, None, None))
+res["bwd_fused"] = timed(lambda: SF.edge_bwd(h, inv, gg, g, 10, ss, sw, sq, sc, fuse[2], diff))
 print(json.dumps(res))

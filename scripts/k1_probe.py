@@ -23,9 +23,9 @@ def run(n, d, kind, thr_lo, mb, ns, cand=16, reps=3, nq=None, seed_stride=0, see
         for _ in range(reps): g()
         b.record(); torch.cuda.synchronize()
         print(json.dumps(dict(seed_pass_ms=round(a.elapsed_time(b) / reps, 3), stride=seed_stride)), flush=True)
-    phase = torch.zeros(8, dtype=torch.int32, device=dev) if not os.environ.get('SNG_KNN_NOPHASE') else None
+    phase = torch.zeros(8, dtype=torch.int32, device=dev)
     def f():
-        if phase is not None: phase.zero_()
+        phase.zero_()
         _C.check(_C.lib().sng_simknn_stage1(_C.ptr(xh), _C.ptr(xh), xh.size(1), nq, 0, n, d, cand, thr_lo, 1, _C.ptr(ci), _C.ptr(cv), _C.ptr(cm), mb, ns, ctypes.byref(nsv), _C.ptr(seeds), seed_q, seed_stride, _C.ptr(phase), _C.stream()), "s1")
     f(); torch.cuda.synchronize()
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

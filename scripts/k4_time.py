@@ -7,7 +7,7 @@ C = int(sys.argv[1]) if len(sys.argv) > 1 else 32
 N, Fd, E, _ = synth.SHAPES["pokec"]
 dev = "cuda"
 ei = synth.make_graph(N, E, seed=1, device=dev, symmetric=True)
-g = G.prepare(ei, N, True, structural=True)
+g = G.prepare(ei, N, True)
 torch.manual_seed(0)
 x = torch.randn(N, C, device=dev)
 def timed(f, reps=10):

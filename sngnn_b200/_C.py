@@ -45,7 +45,7 @@ SIGNATURES = {
     "sng_sparse_col_cos": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _P, _P]),
     "sng_class_sums_f64": (_I32, [_P, _P, _I64, _I64, _I64, _I32, _P, _P, _P]),
     "sng_graph_prepare_workspace_bytes": (_SZ, [_I64, _I64]),
-    "sng_graph_prepare": (_I32, [_P, _I64, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "sng_graph_prepare": (_I32, [_P, _I64, _I64, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "sng_simknn_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I32]),
     "sng_simknn_build": (_I32, [_P, _P, _I64, _P, _P, _I64, _I64, _I64, _I64, _I64, _I32, _F32, _I32,
                                 _P, _P, _P, _P, _P, _P, _SZ, _P]),

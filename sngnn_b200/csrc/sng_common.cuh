@@ -11,7 +11,6 @@ namespace sng {
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);   // cudaPeekAtLastError -> SNG_ERR_CUDA + message
 int sm_count();                       // cached; 148 (a B200's) if there is no device, see sng_api.cu
-int debug_env_int(const char* name, int lo, int hi);   // tuning override; always 0 unless sng_set_debug_env(1) was called
 
 #define SNG_REQUIRE(cond, ...)                                  \
     do {                                                        \

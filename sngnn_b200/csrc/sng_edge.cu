@@ -170,15 +170,7 @@ __device__ __forceinline__ void write_row(const EdgeFwdArgs& a, int row, int c4,
 // keep the per-row instruction count down.
 constexpr int kStWarps = 4;
 // resident CTAs per SM the staged kernels are compiled for (register caps): they are latency / issue bound with few warps
-#ifndef SNG_FWD_MINB
-#define SNG_FWD_MINB 8
-#endif
-#ifndef SNG_BWDT_MINB
-#define SNG_BWDT_MINB 8
-#endif
-#ifndef SNG_BWDS_MINB
-#define SNG_BWDS_MINB 8
-#endif
+constexpr int kStMinBlocks = 8;
 __device__ __forceinline__ void cp_async16(uint32_t dst, const float* src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
@@ -196,7 +188,7 @@ __device__ __forceinline__ float lds32(uint32_t addr) {
 template <int G> constexpr int staged_row_bytes() { return G == 1 ? 16 : 16 * G + 16; }
 
 template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK>
-__global__ void __launch_bounds__(kStWarps * 32, SNG_FWD_MINB) edge_fwd_staged_kernel(const EdgeFwdArgs a) {
+__global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_kernel(const EdgeFwdArgs a) {
     constexpr int C = 4 * G;                    // channels of a padded row
     constexpr int RB = staged_row_bytes<G>();
     constexpr int EPW = 32 / G;                 // rows copied per cp.async instruction
@@ -1283,7 +1275,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwd
 // Pass T, item = target row: stage = its <= top_k selected source rows (lane = edge for ds_e = <h_j, g_i>, lane = channel for
 // dn_i = sum ds_e n_j), plus h_i and g_i.
 template <int G>
-__global__ void __launch_bounds__(kStWarps * 32, SNG_BWDT_MINB) edge_bwd_target_staged_kernel(const EdgeBwdArgs a) {
+__global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_staged_kernel(const EdgeBwdArgs a) {
     constexpr int C = 4 * G;
     constexpr int RB = staged_row_bytes<G>();
     constexpr int EPW = 32 / G;
@@ -1409,7 +1401,7 @@ __global__ void __launch_bounds__(kStWarps * 32, SNG_BWDT_MINB) edge_bwd_target_
 // is done (that item loses its prefetch, nothing else).  The pool is `slots` rows (launcher: 64 -> 8 KB per warp at C = 32,
 // 24+ warps per SM where the fixed two-stage layout allowed 12).
 template <int G, bool FUSE, bool CHUNK>
-__global__ void __launch_bounds__(kStWarps * 32, SNG_BWDS_MINB) edge_bwd_source_staged_kernel(const EdgeBwdArgs a) {
+__global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_source_staged_kernel(const EdgeBwdArgs a) {
     constexpr int C = 4 * G;
     constexpr int RB = 16 * G;                  // no lane-per-row reads here: no padding needed
     constexpr int EPW = 32 / G;
@@ -1990,10 +1982,7 @@ static size_t hub_smem(int top_k) {
 }
 
 // row slots per warp of the staged forward kernel (see there); any single item (33 / fused 65 slots) must fit
-static int forward_slots(bool fuse, int g) {
-    const int o = debug_env_int("SNG_K2_SLOTS", 33, 160);
-    if (o) return o < (fuse ? 65 : 33) ? (fuse ? 65 : 33) : o;
-    (void)g;
+static int forward_slots(bool fuse) {
     return fuse ? 66 : 40;                  // measured (pokec shape, C = 32): smaller pools win -- occupancy beats prefetch depth
 }
 template <int G, bool FUSE, bool SELECT_ALL>
@@ -2003,7 +1992,7 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
         if (a.n_chunks >= 0) {
             // degree lists known, rows of <= 128 bytes: staged kernel over the short rows, then over the <= 32-edge chunks of the
             // long rows, then the per-row merge of the chunk candidates
-            a.slots = forward_slots(FUSE, G);
+            a.slots = forward_slots(FUSE);
             const size_t ss = (size_t)kStWarps * a.slots * staged_row_bytes<G>();
             if constexpr (G == 1) {
                 // 16-byte rows: everything in registers (edge_fwd_narrow_kernel); the chunk pass of the long rows stays staged
@@ -2094,11 +2083,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
 
 namespace sng {
 // row slots per warp of the staged source pass (see edge_bwd_source_staged_kernel); >= 64 so that any single item fits
-static int source_slots(bool fuse) {
-    const int o = debug_env_int("SNG_K2B_SLOTS", 64, 128);
-    (void)fuse;
-    return o ? o : 64;                      // measured (pokec shape, C = 32): 64 / 72 equal, 80+ slower in both modes (occupancy)
-}
+constexpr int kSourceSlots = 64;            // measured (pokec shape, C = 32): 64 / 72 equal, 80+ slower in both modes (occupancy)
 template <int G>
 static int launch_bwd_target_staged(const EdgeBwdArgs& a, cudaStream_t st) {
     const size_t ss = (size_t)kStWarps * 2 * (size_t)((a.top_k < 32 ? a.top_k : 32) + 2) * staged_row_bytes<G>();
@@ -2109,7 +2094,7 @@ static int launch_bwd_target_staged(const EdgeBwdArgs& a, cudaStream_t st) {
 }
 template <int G, bool FUSE>
 static void launch_bwd_source_staged(EdgeBwdArgs a, cudaStream_t st) {
-    a.slots = source_slots(FUSE);
+    a.slots = kSourceSlots;
     const size_t ss = (size_t)kStWarps * a.slots * 16 * G;
     if constexpr (G == 1) {
         edge_bwd_source_narrow_kernel<FUSE><<<grid_resident(edge_bwd_source_narrow_kernel<FUSE>, a.n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);

@@ -114,14 +114,13 @@ extern "C" size_t sng_graph_prepare_workspace_bytes(int64_t num_edges, int64_t n
     return 7 * al256((size_t)total * 4) + al256(sort_temp_bytes(total, key_bits(n))) + 512;
 }
 
-extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, int64_t n, int remove_self_loops, int structural,
+extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, int64_t n, int remove_self_loops,
                                  int32_t* rowptr_in, int32_t* col_in, float* inv_deg, int32_t* rowptr_out, int32_t* col_out,
                                  int32_t* col_in_shift, int32_t* tpos, int32_t* long_rows, int32_t* info, void* workspace,
                                  size_t workspace_bytes, void* stream) {
     SNG_REQUIRE(n > 0 && num_edges >= 0 && num_edges + n < (1ll << 31), "sng_graph_prepare: graph too large for int32 CSR");
     SNG_REQUIRE((edge_index || num_edges == 0) && rowptr_in && col_in && inv_deg && info && workspace, "sng_graph_prepare: null pointer");
-    SNG_REQUIRE(!structural || (rowptr_out && col_out && col_in_shift), "sng_graph_prepare: structural outputs missing");
-    SNG_REQUIRE(!tpos || structural, "sng_graph_prepare: tpos needs the by-source CSR (structural != 0)");
+    SNG_REQUIRE(rowptr_out && col_out && col_in_shift, "sng_graph_prepare: by-source outputs missing");
     if (workspace_bytes < sng_graph_prepare_workspace_bytes(num_edges, n)) { set_error("sng_graph_prepare: workspace too small"); return SNG_ERR_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t total = num_edges + n;
@@ -140,23 +139,19 @@ extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, i
     const int grid = grid_capped(total, 256, 16);
     if (cudaMemsetAsync(min_src, 0x7f, sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");   // 0x7f7f7f7f
     if (cudaMemsetAsync(info, 0, 8 * sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");
-    if (structural && cudaMemsetAsync(info + 2, 0xff, sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");
-    graph_keys_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, (int)n, remove_self_loops, key_dst, structural ? key_src : nullptr, eid,
-                                           structural ? min_src : nullptr);
+    if (cudaMemsetAsync(info + 2, 0xff, sizeof(int), st) != cudaSuccess) return check_launch("sng_graph_prepare memset");
+    graph_keys_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, (int)n, remove_self_loops, key_dst, key_src, eid, min_src);
     if (int rc = check_launch("sng_graph_prepare keys")) return rc;
     if (cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_dst, key_sorted, eid, perm_in, total, 0, bits, st) != cudaSuccess)
         return check_launch("sng_graph_prepare sort by target");
     graph_ends_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, total, perm_in, 0, col_in, nullptr);
     const int rgrid = grid_capped(n + 1, 256, 16);
     graph_rowptr_kernel<<<rgrid, 256, 0, st>>>(key_sorted, total, (int)n, nullptr, rowptr_in);
-    if (structural) {
-        if (cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_src, key_sorted, eid, perm_out, total, 0, bits, st) != cudaSuccess)
-            return check_launch("sng_graph_prepare sort by source");
-        graph_ends_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, total, perm_out, 1, col_out, inv_out);
-        graph_rowptr_kernel<<<rgrid, 256, 0, st>>>(key_sorted, total, (int)n, min_src, rowptr_out);
-    }
-    graph_finish_kernel<<<grid, 256, 0, st>>>(rowptr_in, (int)n, inv_deg, col_in, structural ? col_in_shift : nullptr,
-                                             structural ? min_src : nullptr, structural ? rowptr_out : nullptr,
-                                             structural ? col_out : nullptr, perm_in, inv_out, tpos, long_rows, info);
+    if (cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_src, key_sorted, eid, perm_out, total, 0, bits, st) != cudaSuccess)
+        return check_launch("sng_graph_prepare sort by source");
+    graph_ends_kernel<<<grid, 256, 0, st>>>(edge_index, num_edges, total, perm_out, 1, col_out, inv_out);
+    graph_rowptr_kernel<<<rgrid, 256, 0, st>>>(key_sorted, total, (int)n, min_src, rowptr_out);
+    graph_finish_kernel<<<grid, 256, 0, st>>>(rowptr_in, (int)n, inv_deg, col_in, col_in_shift, min_src, rowptr_out, col_out, perm_in,
+                                             inv_out, tpos, long_rows, info);
     return check_launch("sng_graph_prepare");
 }

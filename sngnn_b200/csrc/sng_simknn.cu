@@ -39,19 +39,6 @@ constexpr int kMaxStages = 10;
 constexpr int kMaxD = 4096;             // feature width limit (d > ~640 streams the query block, see Stage1Params::stream_a)
 constexpr int kMaxCandTotal = 192;      // lists per row * cand <= this; stage 2 expands every candidate into 3 columns
 constexpr uint32_t kPeerMask = 0xFEFFFFFFu;   // clears the CTA-rank bit of a shared::cluster address -> leader CTA
-// Instrumented builds (make EXTRA=-DSNG_KNN_INSTRUMENT): the SNG_KNN_DEBUG work-skipping modes and the SNG_KNN_TRACE
-// per-tile clock stamps used for the pipeline analysis in DESIGN.md.  Compiled out of the product library: the checks
-// sit in the per-tile loops of every role.
-#ifdef SNG_KNN_INSTRUMENT
-constexpr bool kInstr = true;
-#else
-constexpr bool kInstr = false;
-#endif
-#ifdef SNG_KNN_EVTRACE
-constexpr bool kEvTrace = true;          // per-event statistics in SNG_KNN_TRACE runs (costs local memory in the epilogue)
-#else
-constexpr bool kEvTrace = false;
-#endif
 constexpr int kQueue = 256;             // hit queue entries per CTA (power of two; the plan may shrink it); one entry = 64 bytes
 constexpr int kSeedGroups = 16;         // disjoint column groups of the seed sample: (tile parity) x (32-column chunk of the tile)
 // Candidate scores are kept in shared memory as 16-bit bins (6 bytes per slot with the 32-bit column id instead of 8): at
@@ -121,8 +108,6 @@ struct Stage1Params {
     int nsplit, tiles_total;      // 256-column tiles are split across gridDim.y cluster columns
     float thr_lo;                 // approximate scores <= thr_lo can never be selected
     int remove_self;
-    int issuers;                  // MMA-issuing warps (1 or 2)
-    int debug;                    // profiling aid (SNG_KNN_DEBUG): 1 = skip the max tree / inserts, 2 = skip the TMEM loads, 4 = skip the B loads
     float* cand_val;              // [nq, nsplit, cand]
     int* cand_idx;                // [nq, nsplit, cand]   (-1 = empty)
     float* cand_min;              // [nq, nsplit]  largest threshold the row's list pruned with, -inf if it never left thr_lo
@@ -130,20 +115,20 @@ struct Stage1Params {
     const float* seeds;           // [nq, kSeedGroups] group maxima over a 1/seed_stride column sample, or nullptr
     float* seed_out;              // SEED kernel only
     int seed_q, seed_stride;      // row threshold = seed_q-th largest group maximum; sample = every seed_stride-th column
+    int issuers;                  // MMA-issuing warps (1 or 2).  Placed here, the padding keeps the block at 136 bytes: at 128,
+                                  // ptxas (CUDA 12.9) schedules and register-allocates every instance differently
     const int* nq_dev;            // retry pass: number of query rows actually present (device), or nullptr
     const int* row_ids;           // retry pass: global row id (minus q_offset) of query row r, or nullptr (= r)
     int* phase;                   // [nsplit] sweep phase shared by all CTAs of a column split (see "Phase alignment"), or nullptr
-    long long* trace;             // SNG_KNN_TRACE: [64 tiles][8] clock64 stamps of cluster 0's leader CTA, else nullptr
 };
 
 // MMA issue loop of the SPLIT (four 128-column accumulator stages) mode for issuer W of NI, kblocks <= 2.  W / NI are compile
 // time so that every address, descriptor and ring index below is provably warp-uniform and stays in uniform registers: on a
-// busy SM the issuer's dependent instruction chain, not the tensor pipe, sets the tile period (SNG_KNN_TRACE).
+// busy SM the issuer's dependent instruction chain, not the tensor pipe, sets the tile period (per-tile clock stamps).
 template <int W, int NI>
 __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base, uint32_t a_off, uint32_t b_off, uint32_t bar_full, uint32_t bar_empty,
-                                            uint32_t bar_tfull, uint32_t bar_tempty, int t_beg, int t_end, bool issuer, int lane) {
+                                            uint32_t bar_tfull, uint32_t bar_tempty, int t_beg, int t_end, bool issuer) {
     constexpr uint32_t kIdescHalf = f16_idesc(256, 128);
-    long long* const trc = kInstr ? p.trace : nullptr;
     const uint64_t adesc0 = make_smem_desc(base + a_off);
     const uint64_t bdesc0 = make_smem_desc(base + b_off);
     const int kb2 = p.kblocks == 2;                          // second K block present
@@ -162,7 +147,6 @@ __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base
         tc_fence_after();
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
-            if (h == 0 && trc && blockIdx.x == 0 && blockIdx.y == 0 && tt < 64 && lane == 0) trc[tt * 8 + 0] = clock64();
             const uint32_t tmem_d = (uint32_t)((acc0 + h) * 128);
             const uint64_t hb = (uint64_t)(h * (kTileBytes >> 5));                       // + 64 rows x 128 B
             if (issuer) {
@@ -177,7 +161,6 @@ __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base
             }
             __syncwarp();
         }
-        if (trc && blockIdx.x == 0 && blockIdx.y == 0 && tt < 64 && lane == 0) trc[tt * 8 + 1] = clock64();
         st0 += step;
         while (st0 >= nst) { st0 -= nst; ph0 ^= 1u; }
     }
@@ -202,8 +185,6 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     // sits on the critical path of every tile and any late epilogue warp stalls the tensor pipe; with four, each issuer owns
     // two stages and a stage is not needed again for a whole tile period after it was drained.
     constexpr bool SPLIT = (EW == 4);
-    const int dbg = kInstr ? p.debug : 0;
-    long long* const trc = kInstr ? p.trace : nullptr;
     // retry pass: the grid is sized for the maximum, the number of rows lives on the device; idle pairs leave together
     const int nq_eff = p.nq_dev ? min(__ldg(p.nq_dev), p.nq) : p.nq;
     if ((int)(blockIdx.x >> 1) * 2 * BM >= nq_eff) return;
@@ -315,9 +296,6 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                  : "=r"(t_start) : "r"(smem_u32(t0_slot)) : "memory");
     t_start += t_beg;
 
-    long long life_clk = 0; unsigned long long life_ns = 0;
-    const bool life = trc && threadIdx.x == 0 && blockIdx.y == 0 && (blockIdx.x == 0 || blockIdx.x == gridDim.x - 2);
-    if (life) { life_clk = clock64(); asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(life_ns)); }
     if (warp == 0) {
         // ------------------------------------------------------------------ TMA producer (both CTAs, whole warp, one lane issues)
         const bool issuer = elect_one();
@@ -337,14 +315,10 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 // pay one wait and one commit per tile instead of one per K block
                 mbar_wait(bar_empty + 8 * stage, phase ^ 1);
                 if (issuer) {
-                    if (!(dbg & 4)) {
-                        for (int kb = 0; kb < p.kblocks; ++kb)
-                            tma_load_2d_pair(base + b_off + (uint32_t)(stage + kb) * kTileBytes, &map_db, (bar_full + 8 * stage) & kPeerMask, kb * BK, brow);
-                        if (rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2u * (uint32_t)p.kblocks * kTileBytes);
-                        else mbar_arrive_cluster(bar_full + 8 * stage, 0);
-                    } else {
-                        mbar_arrive_cluster(bar_full + 8 * stage, 0);
-                    }
+                    for (int kb = 0; kb < p.kblocks; ++kb)
+                        tma_load_2d_pair(base + b_off + (uint32_t)(stage + kb) * kTileBytes, &map_db, (bar_full + 8 * stage) & kPeerMask, kb * BK, brow);
+                    if (rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2u * (uint32_t)p.kblocks * kTileBytes);
+                    else mbar_arrive_cluster(bar_full + 8 * stage, 0);
                 }
                 stage += p.kblocks;
                 if (stage >= p.stages) { stage = 0; phase ^= 1; }
@@ -352,15 +326,11 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             for (int kb = 0; kb < p.kblocks; ++kb) {
                 mbar_wait(bar_empty + 8 * stage, phase ^ 1);
                 if (issuer) {
-                    if (!(dbg & 4)) {
-                        const uint32_t sdst = base + b_off + (uint32_t)stage * stage_bytes;
-                        if (p.stream_a) tma_load_2d_pair(sdst, &map_q, (bar_full + 8 * stage) & kPeerMask, kb * BK, row0);
-                        tma_load_2d_pair(sdst + (p.stream_a ? (uint32_t)kTileBytes : 0u), &map_db, (bar_full + 8 * stage) & kPeerMask, kb * BK, brow);
-                        if (rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2u * stage_bytes);
-                        else mbar_arrive_cluster(bar_full + 8 * stage, 0);
-                    } else {                                        // profiling: no B traffic at all, the MMAs read stale shared memory
-                        mbar_arrive_cluster(bar_full + 8 * stage, 0);
-                    }
+                    const uint32_t sdst = base + b_off + (uint32_t)stage * stage_bytes;
+                    if (p.stream_a) tma_load_2d_pair(sdst, &map_q, (bar_full + 8 * stage) & kPeerMask, kb * BK, row0);
+                    tma_load_2d_pair(sdst + (p.stream_a ? (uint32_t)kTileBytes : 0u), &map_db, (bar_full + 8 * stage) & kPeerMask, kb * BK, brow);
+                    if (rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2u * stage_bytes);
+                    else mbar_arrive_cluster(bar_full + 8 * stage, 0);
                 }
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
@@ -369,7 +339,7 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
     } else if (warp == 1 || warp == 2) {
         // ------------------------------------------------------------------ MMA issuers (leader CTA; whole warp runs the loop, one lane issues)
         // The chain "accumulator free -> B landed -> issue -> commit" costs one thread ~1300 cycles per tile (mbarrier
-        // try_wait ~90 each even when complete, plus issue / commit latencies; measured with SNG_KNN_TRACE), twice the
+        // try_wait ~90 each even when complete, plus issue / commit latencies; measured with per-tile clock stamps), twice the
         // 640 cycles the tensor pipe needs for a K = 80 tile.  So TWO warps issue, each owning every other tile and one
         // of the two accumulator stages; their chains overlap and the pipe stays fed.  (tcgen05.commit tracks the MMAs
         // of the executing thread only, and each accumulator is only ever written by one of the two threads.)
@@ -384,16 +354,15 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             auto advance = [&](int steps) { for (int i = 0; i < steps; ++i) if (++stage == p.stages) { stage = 0; phase ^= 1; } };
             advance(w * p.kblocks);
             if constexpr (SPLIT) {
-                if (p.issuers == 1) issue_split<0, 1>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer, lane);
-                else if (warp == 1) issue_split<0, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer, lane);
-                else issue_split<1, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer, lane);
+                if (p.issuers == 1) issue_split<0, 1>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
+                else if (warp == 1) issue_split<0, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
+                else issue_split<1, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
             } else {
             for (int tt = w; tt < T; tt += p.issuers) {
                 const int acc = tt & 1;
                 const uint32_t acc_phase = (uint32_t)(tt >> 1) & 1u;
                 mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
                 tc_fence_after();
-                if (trc && blockIdx.x == 0 && blockIdx.y == 0 && tt < 64 && lane == 0) trc[tt * 8 + 0] = clock64();
                 const uint32_t tmem_d = (uint32_t)(acc * BN);
                 for (int kb = 0; kb < p.kblocks; ++kb) {
                     mbar_wait(bar_full + 8 * stage, phase);
@@ -411,7 +380,6 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                     __syncwarp();
                     advance(1);
                 }
-                if (trc && blockIdx.x == 0 && blockIdx.y == 0 && tt < 64 && lane == 0) trc[tt * 8 + 1] = clock64();
                 advance((p.issuers - 1) * p.kblocks);                   // the other issuer's tile
             }
             }
@@ -518,7 +486,6 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         const int self_col = p.remove_self ? p.q_offset + ((p.row_ids && grow < nq_eff) ? __ldg(p.row_ids + grow) : grow) : -1;
         const int n = p.n;
         float thr_cur = p.thr_lo;                                  // the row's pruning threshold as last read from shared memory
-        long long ev_chunks = 0, ev_n = 0, ev_cyc = 0, ev_max = 0, ev_push = 0;   // SNG_KNN_TRACE statistics of warp 4 of CTA 0
         float gmax[2 * CT];                                        // SEED: running maxima of this thread's column groups
 #pragma unroll
         for (int i = 0; i < 2 * CT; ++i) gmax[i] = -CUDART_INF_F;
@@ -527,7 +494,6 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         // was pruned with (cand_min) and stage 2 only accepts a row whose k-th exact score clears it.
         // `ci` = chunk index within the thread's tile slice (compile time after unrolling), `odd` = tile parity.
         auto process = [&](uint32_t (&v)[32], int col0, int ci, bool odd) {
-            if (dbg & 1) { if (__uint_as_float(v[0] ^ v[31]) == 12345.678f) thr_cur = 0.f; return; }
             float m[11];
             auto tree = [&]() {
 #pragma unroll
@@ -547,11 +513,7 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 gmax[CT + ci] = fmaxf(gmax[CT + ci], odd ? mx : -CUDART_INF_F);
                 return;
             }
-            const bool cnt_on = kEvTrace && trc && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == kNonEpiThreads;
-            if (cnt_on) ++ev_chunks;
             if (__any_sync(0xffffffffu, mx > thr_cur)) {           // rare slow path
-                const long long ev0 = cnt_on ? clock64() : 0;
-                if (dbg & 8) return;
                 if ((unsigned)(self_col - col0) < 32u || col0 + 32 > n) {
                     // the chunk holds the row's own column, or columns beyond n (zero filled): once per row / last tile only
 #pragma unroll
@@ -568,14 +530,9 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                     q_ent[4 * s + 3] = make_float4(__int_as_float(r), 0.f, 0.f, 0.f);
                     __threadfence_block();
                     q_flag[s] = 1;                                                   // publishes the entry
-                    if (cnt_on) ++ev_push;
                 }
                 __syncwarp();
                 thr_cur = fmaxf(thr_cur, row_thr[r]);                // the list warp may already have raised it
-                if (cnt_on) {
-                    const long long dt = clock64() - ev0;
-                    ++ev_n; ev_cyc += dt; ev_max = dt > ev_max ? dt : ev_max;
-                }
             }
         };
 
@@ -595,23 +552,18 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             const uint32_t acc_phase = (uint32_t)(tt >> 1) & 1u;
             mbar_wait(bar_tf_e + par * (SPLIT ? 16u : 8u), acc_phase);
             tc_fence_after();
-            const bool tr = trc && blockIdx.x == 0 && blockIdx.y == 0 && tt < 64 && threadIdx.x == kNonEpiThreads;
-            if (tr) trc[tt * 8 + 2] = clock64();
             if (!SEED) thr_cur = fmaxf(thr_cur, row_thr[r]);
             const uint32_t taddr = taddr_e + par * (uint32_t)(SPLIT ? 256 : BN);
             const int col0 = t * BN + tile_col;
             const bool odd = (t & 1) != 0;
             if (CPT == 64) {
                 // both loads in flight at once; the accumulator stage goes back to the MMA warp before any processing
-                if (!(dbg & 2)) {
-                    tmem_ld32(taddr, va);
-                    tmem_ld32(taddr + 32, vb);
-                    tmem_ld_wait();
-                }
+                tmem_ld32(taddr, va);
+                tmem_ld32(taddr + 32, vb);
+                tmem_ld_wait();
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive_remote(bar_te_e + 8u * par);
-                if (tr) trc[tt * 8 + 3] = clock64();
                 process(va, col0, 0, odd);
                 process(vb, col0 + 32, CT > 1 ? 1 : 0, odd);
             } else {
@@ -644,18 +596,10 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             __syncwarp();
             __threadfence_block();
             if (lane == 0) atomicAdd(q_done, 1u);                    // this warp will push nothing more
-            if (kEvTrace && trc && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == kNonEpiThreads) {
-                trc[525] = ev_chunks; trc[520] = ev_n; trc[521] = ev_push; trc[526] = ev_cyc; trc[527] = ev_max;
-            }
         }
     }
     tc_fence_before();
     __syncthreads();
-    if (life) {
-        unsigned long long ns1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns1));
-        long long* o = trc + 512 + (blockIdx.x == 0 ? 0 : 4);
-        o[0] = clock64() - life_clk; o[1] = (long long)(ns1 - life_ns); o[2] = T; o[3] = blockIdx.x;
-    }
     cluster_sync_all();                        // neither CTA may exit (or free TMEM) while the other can still signal / write it
     if (warp == 2) {
         tc_fence_after();
@@ -1006,9 +950,9 @@ static size_t smem_bytes(int ew, int kblocks, int stages, int cand, int qcap, bo
            16 + (size_t)qcap * 68 + 16 + 8 * (2 * kMaxStages + 9) + 16;
 }
 
-// Tuning / debugging overrides through environment variables are OFF unless a test or experiment switches them on with
-// sng_set_debug_env(1): the product call path reads no environment (one static flag is tested instead) and keeps no other
-// global state besides the cached SM count and driver entry point.
+// The overrides the tests use to reach the seeded and no-retry builds (SNG_KNN_CAND, SNG_KNN_SEED_S, SNG_KNN_SEED_Q,
+// SNG_KNN_NORETRY) are OFF unless switched on with sng_set_debug_env(1): the product call path reads no environment (one
+// static flag is tested instead) and keeps no other global state besides the cached SM count and driver entry point.
 static int g_debug_env = 0;
 static int env_int(const char* name, int lo, int hi) {
     if (!g_debug_env) return 0;
@@ -1018,10 +962,6 @@ static int env_int(const char* name, int lo, int hi) {
     return (v >= lo && v <= hi) ? v : 0;
 }
 static bool env_flag(const char* name) { return g_debug_env && getenv(name) != nullptr; }
-}  // namespace knn
-// the same switch for the other translation units (0 = not set / overrides off)
-int debug_env_int(const char* name, int lo, int hi) { return knn::env_int(name, lo, hi); }
-namespace knn {
 
 // Candidate slots per row list.  The list keeps the row's best `cand` FP16 scores; stage 2 proves a row only if its k-th
 // exact score clears the list's drop bound by the FP16 error, so cand - top_k is the number of near-cut columns a row may
@@ -1035,7 +975,6 @@ static int cand_for(int top_k, int margin) {
 // top_k > 0: derive cand from top_k;  top_k == 0: use the explicit `cand` (stage-1 test entry point)
 static int make_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int top_k, int cand, int force_ew) {
     const size_t kMaxSmem = 227 * 1024;
-    if (!force_ew) force_ew = env_int("SNG_KNN_EW", 1, 4) == 3 ? 0 : env_int("SNG_KNN_EW", 1, 4);
     const int d16 = (int)((d + 15) / 16 * 16);
     pl->kblocks = (d16 + BK - 1) / BK;
     pl->ksteps_last = (d16 - (pl->kblocks - 1) * BK) / kUmmaK;
@@ -1056,8 +995,7 @@ static int make_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int top_k, int 
                 const int c = top_k > 0 ? cand_for(top_k, kMargins[mi]) : cand;
                 if (c > kMaxCandTotal) continue;
                 for (int qc = kQueue; qc >= 64 && !pl->ew; qc /= 4) {
-                    int want = pl->kblocks * 4 < kMaxStages ? (pl->kblocks * 4 > 4 ? pl->kblocks * 4 : 4) : kMaxStages;
-                    if (env_int("SNG_KNN_STAGES", 2, kMaxStages)) want = env_int("SNG_KNN_STAGES", 2, kMaxStages);
+                    const int want = pl->kblocks * 4 < kMaxStages ? (pl->kblocks * 4 > 4 ? pl->kblocks * 4 : 4) : kMaxStages;
                     for (int st = want; st >= (pass ? 2 : 3); --st) {
                         if (ew == 4 && st % pl->kblocks != 0) continue;      // split mode: a tile's K blocks share one ring lap
                         const size_t sz = smem_bytes(ew, pl->kblocks, st, c, qc);
@@ -1098,7 +1036,7 @@ static int make_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int top_k, int 
     // a rank's share of a sharded build of a small database gets 3 splits, and measured there (arxiv shape, 1/8 of the rows)
     // the unseeded lists cost 9.4 ms against 2.3 ms seeded: without a threshold every list starts with its warm-up inserts.)
     const bool forced = env_int("SNG_KNN_SEED_S", 2, 256) != 0;
-    if (top_k > 0 && !env_flag("SNG_KNN_NOSEED")) {
+    if (top_k > 0) {
         if (forced) {
             const int stride = env_int("SNG_KNN_SEED_S", 2, 256);
             int q = env_int("SNG_KNN_SEED_Q", 1, kSeedGroups - 2);
@@ -1139,19 +1077,12 @@ static int launch_stage1(const Plan& pl, const uint16_t* xq, const uint16_t* xal
     p.nq = (int)nq; p.n = (int)n_db; p.q_offset = (int)q_offset;
     p.kblocks = pl.kblocks; p.ksteps_last = pl.ksteps_last; p.stages = pl.stages; p.stream_a = pl.stream_a; p.cand = seed_pass ? 0 : pl.cand; p.qcap = pl.qcap;
     p.nsplit = seed_pass ? 1 : pl.nsplit; p.tiles_total = (int)((n_db + BN - 1) / BN); p.thr_lo = thr_lo; p.remove_self = remove_self;
-    p.debug = env_int("SNG_KNN_DEBUG", 1, 63);
-    p.issuers = env_int("SNG_KNN_ISSUERS", 1, 2) ? env_int("SNG_KNN_ISSUERS", 1, 2) : (pl.kblocks <= 3 ? 2 : 1);
-    if (pl.stream_a) p.issuers = 1;
+    p.issuers = pl.stream_a ? 1 : (pl.kblocks <= 3 ? 2 : 1);
     p.cand_val = cand_val; p.cand_idx = cand_idx; p.cand_min = cand_min;
     p.phase = seed_pass ? nullptr : phase;
     p.nq_dev = nq_dev; p.row_ids = row_ids;
     p.seeds = seed_pass ? nullptr : seeds; p.seed_out = seed_out; p.seed_q = pl.seed_q; p.seed_stride = pl.seed_stride > 0 ? pl.seed_stride : 1;
     dim3 grid((unsigned)(2 * ((nq + 2 * BM - 1) / (2 * BM))), (unsigned)p.nsplit);        // x: CTA pairs (cluster of 2), y: column splits
-    p.trace = nullptr;
-    if (env_flag("SNG_KNN_TRACE") && !seed_pass) {              // debugging aid only: allocates, synchronises and prints
-        cudaMalloc(&p.trace, (64 * 8 + 16) * sizeof(long long));
-        cudaMemset(p.trace, 0, (64 * 8 + 16) * sizeof(long long));
-    }
     cudaError_t e;
     if (seed_pass) e = pl.ew == 4 ? launch_ew<4, true>(grid, pl.smem, st, mq, mdb, p)
                      : pl.ew == 2 ? launch_ew<2, true>(grid, pl.smem, st, mq, mdb, p)
@@ -1160,23 +1091,6 @@ static int launch_stage1(const Plan& pl, const uint16_t* xq, const uint16_t* xal
            : pl.ew == 2 ? launch_ew<2, false>(grid, pl.smem, st, mq, mdb, p)
                         : launch_ew<1, false>(grid, pl.smem, st, mq, mdb, p);
     if (e != cudaSuccess) { cudaGetLastError(); set_error("simknn stage 1: cudaFuncSetAttribute(%zu B smem): %s", pl.smem, cudaGetErrorString(e)); return SNG_ERR_CUDA; }
-    if (p.trace) {
-        long long h[64 * 8 + 16];
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h, p.trace, sizeof(h), cudaMemcpyDeviceToHost);
-        cudaFree(p.trace);
-        fprintf(stderr, "tile  mma:tempty_ok  [4]  [5]  [6]  mma:issued  epi:tfull_ok  epi:released   (cycles since tile 0's tempty_ok; split mode: [4] = half 0 issued, [5] = half 1 stage free)\n");
-        for (int t = 0; t < 64; ++t)
-            fprintf(stderr, "%4d %10lld %10lld %10lld %10lld %10lld %10lld %10lld\n", t, h[8 * t] - h[0], h[8 * t + 4] - h[0], h[8 * t + 5] - h[0],
-                    h[8 * t + 6] - h[0], h[8 * t + 1] - h[0], h[8 * t + 2] - h[0], h[8 * t + 3] - h[0]);
-        fprintf(stderr, "CTA 0 warp 4: %lld warp-chunks, %lld slow-path events, %lld pushes (%lld %lld %lld); "
-                "event cycles: mean %.0f max %lld\n", h[525], h[520], h[521], h[522], h[523], h[524], (double)h[526] / (double)(h[520] > 0 ? h[520] : 1), h[527]);
-        for (int c = 0; c < 2; ++c) {
-            const long long* o = h + 512 + 4 * c;
-            if (o[1] > 0) fprintf(stderr, "CTA %lld lifetime: %lld cycles, %lld ns -> %.0f MHz, %lld tiles, %.0f cycles/tile\n", o[3], o[0], o[1],
-                                  1e3 * (double)o[0] / (double)o[1], o[2], (double)o[0] / (double)(o[2] > 0 ? o[2] : 1));
-        }
-    }
     return check_launch(seed_pass ? "simknn seed pass" : "simknn stage 1");
 }
 
@@ -1324,7 +1238,7 @@ extern "C" int sng_simknn_build(const uint16_t* xq, const uint16_t* xall, int64_
     if (pl.seed_stride > 0)
         if (int rc = launch_stage1(pl, xq, xall, ldb, nq, q_offset, n, thr_lo, remove_self, nullptr, nullptr, nullptr, nullptr, seeds, nullptr, st)) return rc;
     if (int rc = launch_stage1(pl, xq, xall, ldb, nq, q_offset, n, thr_lo, remove_self, cand_val, cand_idx, cand_min,
-                               pl.seed_stride > 0 ? seeds : nullptr, nullptr, env_flag("SNG_KNN_NOPHASE") ? nullptr : phase, st)) return rc;
+                               pl.seed_stride > 0 ? seeds : nullptr, nullptr, phase, st)) return rc;
     const int d4 = (int)((d + 3) / 4);
     // stage 2 flags the rows it cannot prove: into the retry list when there is a retry pass, else straight into the scan list
     int* flag_rows = retry ? fb_rows : fb2_rows;

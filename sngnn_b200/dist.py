@@ -280,7 +280,7 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
             raise NotImplementedError("sharded_forward supports candidates='edges', denominator='candidates' only")
         if not base and conv.top_k <= 0:
             raise NotImplementedError("sharded_forward: top_k <= 0")
-        g = G.prepare(edge_index, n, remove_self_loops=False if base else bool(conv.is_remove_self_loops), structural=plus_plus)
+        g = G.prepare(edge_index, n, remove_self_loops=False if base else bool(conv.is_remove_self_loops))
         h = conv._hidden_norm(x)[0]                          # lin + bias in the library's kernel (its backward is the one-pass dW / db)
         injected = agg is not None or fuse is not None
         if plus_plus:

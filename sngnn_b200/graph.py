@@ -14,8 +14,7 @@ int32 CSR arrays the kernels consume:
     aggregation run as two gather passes without float atomics (sng_edge_bwd).
   * `rows_long` / `rows_hub`: target rows with 32 < in-degree <= 1024 / > 1024 (the forward's degree dispatch), and
     `symmetric`: every in-list equals the out-list with min(src) == 0, which lets SNGNN++ gather W^T rows in the same pass.
-The by-source arrays are always built (the deterministic backward of every model needs them), `structural` is kept for
-API compatibility.
+The by-source arrays are always built: the deterministic backward of every model needs them.
 
 CUDA `edge_index`: one call of `sng_graph_prepare` (stable radix sort by target / source, include/sng.h).  CPU tensors
 (the host-logic and gloo tests): the same construction in torch, with a stable argsort.
@@ -30,7 +29,7 @@ _CACHE_MAX = 8
 
 class PreparedGraph:
     __slots__ = ("n", "num_edges", "rowptr_in", "col_in", "inv_deg", "src_shift", "rowptr_out", "col_out",
-                 "col_in_shift", "dst_sorted", "_shards", "tpos", "rows_long", "rows_hub", "symmetric", "max_deg", "is_shard",
+                 "col_in_shift", "_shards", "tpos", "rows_long", "rows_hub", "symmetric", "max_deg", "is_shard",
                  "chunk_tab", "lrows", "lrow_ptr", "chunk_tab_out", "lrows_out", "lrow_ptr_out")
 
     @staticmethod
@@ -81,7 +80,7 @@ class PreparedGraph:
         g.inv_deg = self.inv_deg[lo:hi].contiguous()
         g.src_shift = self.src_shift
         g.col_in_shift = None if self.col_in_shift is None else self.col_in_shift[b:e].contiguous()
-        g.rowptr_out = g.col_out = g.dst_sorted = g.tpos = None      # no transpose index for a shard: its backward scatters
+        g.rowptr_out = g.col_out = g.tpos = None      # no transpose index for a shard: its backward scatters
         g.symmetric, g.max_deg, g.is_shard = False, self.max_deg, True
         g.rows_long = g.rows_hub = None
         if self.rows_long is not None:                       # shard-local degree lists
@@ -114,11 +113,10 @@ def process_edges(edge_index, num_nodes, remove_self_loops):
     return ei
 
 
-def prepare(edge_index, num_nodes, remove_self_loops, structural=False, processed=False):
+def prepare(edge_index, num_nodes, remove_self_loops, processed=False):
     """Build (or fetch from cache) the PreparedGraph of `edge_index` [2,E] int64.
 
     remove_self_loops: False for base SNConv (R: :323), the `is_remove_self_loops` flag otherwise.
-    structural: ignored (the by-source CSR is always built; kept for API compatibility).
     The cache is keyed on the tensor object, its storage address and `_version`; writes that bypass the version counter
     (`edge_index.data[...] = ...`) are not seen -- call `clear_cache()` after such an edit.
     processed: `edge_index` already went through `process_edges` (used by tests)."""
@@ -146,7 +144,7 @@ def prepare(edge_index, num_nodes, remove_self_loops, structural=False, processe
     g.col_in = col_in.to(torch.int32).contiguous()
     deg = (g.rowptr_in[1:] - g.rowptr_in[:-1])
     g.inv_deg = (1.0 / deg.to(torch.float32).clamp(min=1)).contiguous()
-    g.dst_sorted, g.is_shard = None, False
+    g.is_shard = False
     g.src_shift = int(src.min()) if src.numel() else 0                # R: models/models.py:125
     g.rowptr_out, col_out, perm_out = _csr_from_keys(src - g.src_shift, dst, g.n)
     g.col_out = col_out.to(torch.int32).contiguous()
@@ -187,7 +185,7 @@ def _prepare_cuda(edge_index, n, remove_self_loops):
     if wbytes == 0:
         raise ValueError("graph too large for int32 CSR")
     ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
-    _C.call("sng_graph_prepare", ei, _C.ptr(ei), e, n, int(remove_self_loops), 1, _C.ptr(rowptr_in), _C.ptr(col_in),
+    _C.call("sng_graph_prepare", ei, _C.ptr(ei), e, n, int(remove_self_loops), _C.ptr(rowptr_in), _C.ptr(col_in),
             _C.ptr(g.inv_deg), _C.ptr(rowptr_out), _C.ptr(col_out), _C.ptr(col_in_shift), _C.ptr(tpos), _C.ptr(long_rows), _C.ptr(info),
             _C.ptr(ws), wbytes)
     kept, shift, sym, n_long, n_hub, max_deg = (int(v) for v in info.tolist()[:6])   # one sync: the arrays are narrowed to the kept edges
@@ -198,7 +196,6 @@ def _prepare_cuda(edge_index, n, remove_self_loops):
     g.rows_long = long_rows[:n_long].clone()
     g.rows_hub = long_rows[n - n_hub:].clone() if n_hub else long_rows[:0].clone()
     g.symmetric, g.max_deg, g.is_shard = sym != 0, max_deg, False
-    g.dst_sorted = None
     g.build_chunks()
     return g
 

@@ -54,7 +54,7 @@ def test_graph_prepare_matches_reference_edge_processing():
     ei = synth.make_graph(n, 300, seed=9, hub_offset=2.0)
     ei = torch.cat([ei, torch.tensor([[3, 3], [3, 7]])], dim=1)        # an original self loop and a duplicate-able edge
     for rsl in (True, False):
-        g = G.prepare(ei, n, rsl, structural=True)
+        g = G.prepare(ei, n, rsl)
         pe = sn_ref.process_edges(ei, n, rsl)
         assert torch.equal(G.process_edges(ei, n, rsl), pe)
         # CSR by target keeps original positions
@@ -70,7 +70,7 @@ def test_graph_prepare_matches_reference_edge_processing():
             want = sorted(pe[1][pe[0] - m == i].tolist())
             got = sorted(g.col_out[g.rowptr_out[i]:g.rowptr_out[i + 1]].tolist())
             assert got == want
-        assert G.prepare(ei, n, rsl, structural=True) is g                # cache hit
+        assert G.prepare(ei, n, rsl) is g                                 # cache hit
     sl = g.row_slice(10, 30)
     assert sl.n == 20 and int(sl.rowptr_in[0]) == 0 and sl.col_in.numel() == int(g.rowptr_in[30] - g.rowptr_in[10])
 
