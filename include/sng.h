@@ -106,16 +106,23 @@ SNG_API int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t row
  * two gather passes (by target, then by source through the transpose index tpos), every sum in a fixed order, so the
  * result is bit-reproducible (closed form of SURVEY.md §3.4).  g = dL/dout [n, ldg] (dL/dout_1 when beta == NULL).
  *   top_k > 0: uses the saved lists (sel_src, sel_w, sel_q, sel_cnt);  top_k <= 0: every edge of the CSR (col, tpos).
- *   rowptr_out / col_out = CSR by (source - src_shift) of the same edges, num_edges of them.
+ *   rowptr_out [n_total + 1] / col_out = CSR by (source - src_shift) of the same edges, num_edges of them.
  *   beta != NULL: g is scaled by (1 - beta) for the aggregation; dbeta (may be NULL) = sum(diff * g) (needs diff, partials);
  *                 dwt (may be NULL) [n, lddw] = beta * sum over out-edges (j -> i) of g_i = dL/dwt.
  * Workspaces (caller-allocated, contents irrelevant): coef [2 * num_edges] floats, dn_target [n, ld], partials [SNG_PARTIALS].
  * chunk_tab_out / lrows_out / lrow_ptr_out: the degree tables of sng_edge_fwd built over the BY-SOURCE CSR (rows with more
  * than 32 out-edges cut into <= 32-edge chunks; lrows_out holds true source ids), chunk_partials [n_chunks_out, 3, 4*ceil_pow2(c/4)]
  * floats; n_chunks_out < 0 = tables unknown (the unstaged source pass then runs every row).
- * Output dh [n, ld] = dL/dh. */
+ * Output dh [n_total, ld]: every row is written.
+ * Row sharding (the convention of sng_edge_fwd): the call covers target rows [row_offset, row_offset + n) of `h`, which holds
+ * ALL n_total nodes, as does inv_norm; g, diff, the selection lists, rowptr / col / tpos and the by-source CSR are local to the
+ * shard -- the by-source CSR holds only the shard's in-edges, over all source rows, with targets as LOCAL ids.  dh is then
+ * this shard's CONTRIBUTION to dL/dh of every node (the map to dh is linear: the contributions of the shards add, e.g. in a
+ * reduce-scatter across ranks), dbeta its part of dL/dbeta.  n = 0 gives a zero contribution.  dwt needs a call over all rows
+ * (row_offset = 0, n = n_total); a row shard assembles dL/dwt from g elsewhere.  row_offset = 0, n = n_total: the whole graph. */
 #define SNG_PARTIALS 4096
-SNG_API int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n, int64_t c, int64_t ld, int64_t ldg,
+SNG_API int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                 int64_t c, int64_t ld, int64_t ldg,
                  const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
                  const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
                  int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
@@ -124,8 +131,8 @@ SNG_API int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, 
                  const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
                  int64_t n_lrows_out, float* chunk_partials, void* stream);
 
-/* Scatter form of the backward (float atomics; used for row shards and for explicit neighbour lists, where no
- * transpose index exists).
+/* Scatter form of the backward (float atomics; used for explicit neighbour lists -- the all-pairs mode -- which have no
+ * transpose index; edge-restricted layers, row shards included, use sng_edge_bwd).
  * Pass 1 scatters into the two zero-initialised accumulators dval, dnrm [n_total, c];
  * pass 2 writes dh [n_total, c] = dval + (dnrm - n (n . dnrm)) / r.   `g` = dL/dout_1 [n, c].
  * top_k > 0: uses the saved selection lists (inv_denom[i] = 1/max(deg_i,1));

@@ -27,7 +27,7 @@ SIGNATURES = {
     "sng_lin_bwd_supported": (_I32, [_I64, _I64]),
     "sng_lin_bwd_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
     "sng_lin_bwd": (_I32, [_P, _I64, _P, _I64, _I64, _I64, _I64, _P, _I64, _P, _P, _SZ, _P]),
-    "sng_edge_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P, _P, _P, _P,
+    "sng_edge_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P, _P, _P, _P,
                             _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _P]),
     "sng_edge_agg_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
     "sng_list_agg_fwd": (_I32, [_P, _I64, _I64, _I64, _I32, _P, _P, _P, _P, _P, _I64, _P]),

@@ -1092,6 +1092,9 @@ __global__ void __launch_bounds__(kThreads) norm_bwd_finish_kernel(const float* 
 // Pass S (by source, over the out-edges): dval_j = sum A_e g_i, dn_j = dnT_j + sum B_e h_i, then the normalisation
 //   backward, all in registers; under the fused epilogue the same walk also sums beta g_i over ALL out-edges = dL/dWt_j.
 // Every sum runs in a fixed order: the result is bit-reproducible.
+// Row shards: the call owns target rows [row_offset, row_offset + n) of h (all n_total rows); g, the lists, the CSR by
+// target, dnT and the by-source CSR (the shard's in-edges only, targets as local ids) are shard-local.  Pass S still runs
+// every source row j of n_total and writes dh_j = this shard's contribution; dnT_j exists only for the rows it owns.
 struct EdgeBwdArgs {
     const float* h; const float* inv_r; const float* g;
     int n_total, n, row_offset, c, ld, ldg;
@@ -1107,6 +1110,9 @@ struct EdgeBwdArgs {
     float* tmp_part;                         // [n_chunks, 3, 4G]
     int slots;                               // staged source pass: row slots per warp (>= 64: any single item fits)
 };
+
+// source row j is one of the call's target rows: pass T wrote its target-side dn at dnT[j - row_offset]
+__device__ __forceinline__ bool owns_row(const EdgeBwdArgs& a, int j) { return (unsigned)(j - a.row_offset) < (unsigned)a.n; }
 
 template <int G, bool SELECT_ALL>
 __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwdArgs a) {
@@ -1176,7 +1182,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
 #pragma unroll
         for (int s = 0; s < V; ++s) {
             cross_group_sum4<G>(dni[s]);
-            if (grp == 0 && ok[s]) *reinterpret_cast<float4*>(a.dnT + (int64_t)grow * a.ld + c4[s]) = dni[s];
+            if (grp == 0 && ok[s]) *reinterpret_cast<float4*>(a.dnT + (int64_t)row * a.ld + c4[s]) = dni[s];
         }
     }
     if (a.dbeta_part) {                                                      // fixed-order block sum -> one partial per block
@@ -1205,6 +1211,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwd
     for (int s = 0; s < V; ++s) { c4[s] = slot_c4(q, s); ok[s] = c4[s] < a.c; }
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     const float beta = FUSE ? __ldg(a.beta) : 0.f;
+    const float* ht = a.h + (int64_t)a.row_offset * a.ld;                  // h rows of the call's targets (col_out: local ids)
     for (int j = blockIdx.x * kWarpsPerBlock + warp; j < a.n_total; j += gridDim.x * kWarpsPerBlock) {
         const int jr = j - a.shift;                                          // rows of the by-source CSR are shifted source ids
         int beg = 0, end = 0;
@@ -1231,7 +1238,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwd
                     for (int s = 0; s < V; ++s) {
                         const bool sok = s == 0 || ok[s];
                         gv[u][s] = ((FUSE ? on : sel) && sok) ? ldg4(a.g + (int64_t)i * a.ldg + c4[s]) : z4;
-                        hv[u][s] = (sel && sok) ? ldg4(a.h + (int64_t)i * a.ld + c4[s]) : z4;
+                        hv[u][s] = (sel && sok) ? ldg4(ht + (int64_t)i * a.ld + c4[s]) : z4;
                     }
                 }
 #pragma unroll
@@ -1246,6 +1253,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwd
             }
         }
         const float irj = __ldg(a.inv_r + j);
+        const bool own = owns_row(a, j);
         float4 nj[V], dn[V];
 #pragma unroll
         for (int s = 0; s < V; ++s) {
@@ -1253,7 +1261,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_kernel(const EdgeBwd
             cross_group_sum4<G>(dnj[s]);
             if (FUSE) cross_group_sum4<G>(dw[s]);
             nj[s] = ok[s] ? scale4(ldg4(a.h + (int64_t)j * a.ld + c4[s]), irj) : z4;
-            dn[s] = ok[s] ? ldg4(a.dnT + (int64_t)j * a.ld + c4[s]) : z4;
+            dn[s] = (own && ok[s]) ? ldg4(a.dnT + (int64_t)(j - a.row_offset) * a.ld + c4[s]) : z4;
             add4(dn[s], dnj[s]);
         }
         const float proj = group_sum<S::L>(dotv<V>(nj, dn));
@@ -1369,7 +1377,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
 #pragma unroll 2
             for (int t = 0; t < cnt; ++t) dni = fmaf(__shfl_sync(kFull, wdn, t), lds32(rd + (uint32_t)(t * RB)), dni);
             if (lane < C && ch_ok) {
-                a.dnT[(int64_t)(a.row_offset + row) * a.ld + ch] = dni;
+                a.dnT[(int64_t)row * a.ld + ch] = dni;
                 if (a.diff) bpart = fmaf(dfA, lds32(rd + GI), bpart);                    // dL/dbeta: diff . g (raw g)
             }
         }
@@ -1413,7 +1421,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_source_s
     const bool cq_ok = q * 4 < a.c;
     const int ch = lane % C;
     const bool ch_ok = ch < a.c;
-    const char* hq = reinterpret_cast<const char*>(a.h + q * 4);
+    const char* hq = reinterpret_cast<const char*>(a.h + (int64_t)a.row_offset * a.ld + q * 4);   // targets' h rows (local ids)
     const char* gq = reinterpret_cast<const char*>(a.g + q * 4);
     const int64_t ldhb = (int64_t)a.ld * 4, ldgb = (int64_t)a.ldg * 4;
     const int egrp = cq_ok ? grp : 64;
@@ -1477,7 +1485,10 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_source_s
     float hjA = 0.f, dnA = 0.f, irA = 0.f;
     if (!CHUNK && degA >= 0 && degA <= 32) {
         irA = __ldg(a.inv_r + row0);
-        if (ch_ok) { hjA = __ldg(a.h + (int64_t)row0 * a.ld + ch); dnA = __ldg(a.dnT + (int64_t)row0 * a.ld + ch); }
+        if (ch_ok) {
+            hjA = __ldg(a.h + (int64_t)row0 * a.ld + ch);
+            if (owns_row(a, row0)) dnA = __ldg(a.dnT + (int64_t)(row0 - a.row_offset) * a.ld + ch);
+        }
     }
     for (int row = row0; row < n_items; row += stride) {
         load_rp(row + 3 * stride, begD, degD);
@@ -1491,7 +1502,10 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_source_s
         float hjB = 0.f, dnB = 0.f, irB = 0.f;
         if (!CHUNK && degB >= 0 && degB <= 32) {
             irB = __ldg(a.inv_r + row + stride);
-            if (ch_ok) { hjB = __ldg(a.h + (int64_t)(row + stride) * a.ld + ch); dnB = __ldg(a.dnT + (int64_t)(row + stride) * a.ld + ch); }
+            if (ch_ok) {
+                hjB = __ldg(a.h + (int64_t)(row + stride) * a.ld + ch);
+                if (owns_row(a, row + stride)) dnB = __ldg(a.dnT + (int64_t)(row + stride - a.row_offset) * a.ld + ch);
+            }
         }
         if (ahead) asm volatile("cp.async.wait_group 1;" ::: "memory");
         else asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -1599,7 +1613,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_narrow_kernel(const 
             float v[4] = {wdn * gA.hj.x, wdn * gA.hj.y, wdn * gA.hj.z, wdn * gA.hj.w};
             const float tot = lane_reduce_scatter<4>(v, lane);
             if (writer) {
-                a.dnT[(int64_t)(a.row_offset + row) * a.ld + wc] = tot;
+                a.dnT[(int64_t)row * a.ld + wc] = tot;
                 bpart = fmaf(gA.df, gA.gc, bpart);                                       // dL/dbeta: diff . g (raw g); df = 0 without diff
             }
         }
@@ -1620,8 +1634,9 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_narrow_kernel(const 
     }
 }
 
+// (5 blocks per SM: the row-shard operands would otherwise push it to 55-62 registers and 4 blocks; at 48 it does not spill)
 template <bool FUSE>
-__global__ void __launch_bounds__(kThreads) edge_bwd_source_narrow_kernel(const EdgeBwdArgs a) {
+__global__ void __launch_bounds__(kThreads, 5) edge_bwd_source_narrow_kernel(const EdgeBwdArgs a) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int stride = gridDim.x * kWarpsPerBlock;
     const int row0 = blockIdx.x * kWarpsPerBlock + warp;
@@ -1634,6 +1649,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_narrow_kernel(const 
     const int wc = (lane >> 3) & 3;
     const bool wwriter = (lane & 7) == 0 && wc < a.c;
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    const float* ht = a.h + (int64_t)a.row_offset * a.ld;                  // h rows of the call's targets (col_out: local ids)
     struct Gs { float4 gv, hv; float hj, dn, ir; };
     auto load_rp = [&](int item, int& beg, int& deg) {
         beg = 0; deg = -1;
@@ -1652,9 +1668,12 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_narrow_kernel(const 
         if ((unsigned)deg <= 32u) {
             const bool sel = cf.x != 0.f || cf.y != 0.f;                     // an unselected edge has both coefficients 0
             if (il >= 0 && (FUSE || sel)) g.gv = ldg4(a.g + (int64_t)il * a.ldg);
-            if (sel) g.hv = ldg4(a.h + (int64_t)il * a.ld);
+            if (sel) g.hv = ldg4(ht + (int64_t)il * a.ld);
             g.ir = __ldg(a.inv_r + item);
-            if (fin_ok) { g.hj = __ldg(a.h + (int64_t)item * a.ld + fc); g.dn = __ldg(a.dnT + (int64_t)item * a.ld + fc); }
+            if (fin_ok) {
+                g.hj = __ldg(a.h + (int64_t)item * a.ld + fc);
+                if (owns_row(a, item)) g.dn = __ldg(a.dnT + (int64_t)(item - a.row_offset) * a.ld + fc);
+            }
         }
     };
     int begA, degA, begB, degB, begC, degC, begD, degD;
@@ -1715,7 +1734,7 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_source_merge_kernel(const E
         }
         const float ir = __ldg(a.inv_r + row);
         const float nj = ch_ok ? __ldg(a.h + (int64_t)row * a.ld + ch) * ir : 0.f;
-        const float dn = (ch_ok ? __ldg(a.dnT + (int64_t)row * a.ld + ch) : 0.f) + dnj;
+        const float dn = (ch_ok && owns_row(a, row) ? __ldg(a.dnT + (int64_t)(row - a.row_offset) * a.ld + ch) : 0.f) + dnj;
         float proj = (lane < C && ch_ok) ? nj * dn : 0.f;
         proj = group_sum<32>(proj);
         if (lane < C && ch_ok) {
@@ -2035,7 +2054,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
                             const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
                             void* stream) {
     if (int rc = check_rows("sng_edge_fwd", n, c, ldh)) return rc;
-    SNG_REQUIRE(h && rowptr && col && out && ldo % 4 == 0 && ldo >= c, "sng_edge_fwd: null pointer or bad ldo");
+    SNG_REQUIRE(h && rowptr && ((col && out) || n == 0) && ldo % 4 == 0 && ldo >= c, "sng_edge_fwd: null pointer or bad ldo");   // (an empty shard has no edges, no rows)
     SNG_REQUIRE(row_offset >= 0 && row_offset + n <= n_total && n_total < (1ll << 31) && ldh < (1ll << 31) && ldo < (1ll << 31),
                 "sng_edge_fwd: bad row_offset / n_total");
     SNG_REQUIRE(inv_norm, "sng_edge_fwd: inv_norm [n_total] is required");
@@ -2047,7 +2066,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
     SNG_REQUIRE(n_hub >= 0 && (n_hub == 0 || rows_hub), "sng_edge_fwd: hub list missing");
     SNG_REQUIRE(!wt || (b_w && beta && ldw % 4 == 0 && ldw >= c && ldw < (1ll << 31)), "sng_edge_fwd: fused epilogue needs b_w, beta and a 16-byte aligned wt");
     SNG_REQUIRE(wt || !diff, "sng_edge_fwd: diff is an output of the fused epilogue");
-    if (n == 0) return SNG_OK;
+    if (n == 0 && (inv_norm_ready || n_total == 0)) return SNG_OK;     // (an empty row shard still fills inv_norm: the backward reads it)
     const bool staged = c <= 32 && n_chunks >= 0;
     if (staged && n_chunks > 0) {
         if (!workspace || workspace_bytes < sng_edge_fwd_workspace_bytes(n_chunks, c, top_k)) { set_error("sng_edge_fwd: workspace too small"); return SNG_ERR_WORKSPACE; }
@@ -2055,6 +2074,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
     cudaStream_t st = (cudaStream_t)stream;
     if (!inv_norm_ready)                                     // (sng_lin_norm_fwd already produced it with h)
         SNG_DISPATCH_G(c, row_inv_norm_kernel<G><<<grid_resident(row_inv_norm_kernel<G>, n_total, kWarpsPerBlock * RowShape<G>::EPW * 4), kThreads, 0, st>>>(h, n_total, (int)c, ldh, inv_norm));
+    if (n == 0) return check_launch("sng_edge_fwd");
     EdgeFwdArgs a;
     a.h = h; a.inv_r = inv_norm; a.n = (int)n; a.row_offset = (int)row_offset; a.c = (int)c; a.ldh = (int)ldh;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.rows = nullptr; a.n_rows = 0; a.skip_deg = 0;
@@ -2110,7 +2130,8 @@ static void launch_bwd_source_staged(EdgeBwdArgs a, cudaStream_t st) {
 }
 }  // namespace sng
 
-extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n, int64_t c, int64_t ld, int64_t ldg,
+extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                            int64_t c, int64_t ld, int64_t ldg,
                             const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
                             const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
                             int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
@@ -2118,21 +2139,26 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
                             float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
                             const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
                             int64_t n_lrows_out, float* chunk_partials, void* stream) {
-    if (int rc = check_rows("sng_edge_bwd", n, c, ld)) return rc;
-    SNG_REQUIRE(h && inv_norm && g && rowptr && rowptr_out && col_out && coef && dn_target && dh && ldg % 4 == 0 && ldg >= c,
-                "sng_edge_bwd: null pointer or bad ldg");
-    SNG_REQUIRE(top_k > 0 ? (sel_src && sel_w && sel_q && sel_cnt) : (col && tpos), "sng_edge_bwd: missing selection lists / CSR + tpos");
+    if (int rc = check_rows("sng_edge_bwd", n_total, c, ld)) return rc;
+    SNG_REQUIRE(n >= 0 && row_offset >= 0 && row_offset + n <= n_total, "sng_edge_bwd: bad n / row_offset / n_total");
+    // (an empty shard, n == 0, has no rows of g / dn_target / the lists, and possibly no edges: those may be NULL)
+    SNG_REQUIRE(h && inv_norm && rowptr && rowptr_out && (col_out || num_edges == 0) && coef && dh && ldg % 4 == 0 && ldg >= c &&
+                (n == 0 || (g && dn_target)), "sng_edge_bwd: null pointer or bad ldg");
+    SNG_REQUIRE(n == 0 || (top_k > 0 ? (sel_src && sel_w && sel_q && sel_cnt) : (col && tpos)), "sng_edge_bwd: missing selection lists / CSR + tpos");
     SNG_REQUIRE(!dwt || (beta && lddw % 4 == 0 && lddw >= c), "sng_edge_bwd: dwt needs beta and a 16-byte aligned leading dimension");
-    SNG_REQUIRE(!dbeta || (beta && diff && partials && lddiff % 4 == 0 && lddiff >= c), "sng_edge_bwd: dbeta needs beta, diff and the partials workspace");
+    SNG_REQUIRE(!dwt || (row_offset == 0 && n == n_total),
+                "sng_edge_bwd: dwt needs a call over all rows (row_offset = 0, n = n_total); a row shard's pass S sees only its own out-edges");
+    SNG_REQUIRE(!dbeta || (beta && (diff || n == 0) && partials && lddiff % 4 == 0 && lddiff >= c), "sng_edge_bwd: dbeta needs beta, diff and the partials workspace");
     SNG_REQUIRE(src_shift >= 0 && num_edges >= 0, "sng_edge_bwd: bad src_shift / num_edges");
     SNG_REQUIRE(n_chunks_out <= 0 || (chunk_tab_out && lrows_out && lrow_ptr_out && n_lrows_out > 0 && chunk_partials),
                 "sng_edge_bwd: by-source chunk tables / partials workspace missing");
-    if (n == 0) return SNG_OK;
+    if (n_total == 0) return SNG_OK;
     cudaStream_t st = (cudaStream_t)stream;
     if (top_k > 0 && num_edges > 0 &&
         cudaMemsetAsync(coef, 0, (size_t)num_edges * sizeof(float2), st) != cudaSuccess) return check_launch("sng_edge_bwd memset");
     EdgeBwdArgs a;
-    a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n; a.n = (int)n; a.row_offset = 0; a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
+    a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n_total; a.n = (int)n; a.row_offset = (int)row_offset;
+    a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.top_k = top_k > 0 ? top_k : 0;
     a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt;
     a.beta = beta; a.diff = dbeta ? diff : nullptr; a.lddiff = (int)lddiff; a.dbeta_part = dbeta ? partials : nullptr;
@@ -2141,6 +2167,8 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
     a.dh = dh; a.dwt = dwt; a.lddw = (int)lddw;
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab_out); a.n_chunks = (int)n_chunks_out; a.lrows = lrows_out; a.lrow_ptr = lrow_ptr_out;
     a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials;
+    // n == 0 (an empty shard) still runs both passes: pass T writes no row but its one block writes a zero dbeta partial,
+    // pass S writes the zero contribution of every row
     const bool staged_t = c <= 32 && top_k > 0 && top_k <= 32;      // pass T from the saved lists, rows staged in shared memory
     const bool staged_s = c <= 32 && n_chunks_out >= 0;              // pass S with the by-source chunk tables
     int grid_t = 1;
@@ -2162,8 +2190,8 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
             if (staged_s) { if (dwt) launch_bwd_source_staged<G, true>(a, st); else launch_bwd_source_staged<G, false>(a, st); done_s = true; }
         }
         if (!done_s) {
-            if (dwt) edge_bwd_source_kernel<G, true><<<grid_resident(edge_bwd_source_kernel<G, true>, n, kWarpsPerBlock), kThreads, 0, st>>>(a);
-            else edge_bwd_source_kernel<G, false><<<grid_resident(edge_bwd_source_kernel<G, false>, n, kWarpsPerBlock), kThreads, 0, st>>>(a);
+            if (dwt) edge_bwd_source_kernel<G, true><<<grid_resident(edge_bwd_source_kernel<G, true>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
+            else edge_bwd_source_kernel<G, false><<<grid_resident(edge_bwd_source_kernel<G, false>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
         });
     if (dbeta) sum_partials_kernel<<<1, 256, 0, st>>>(partials, grid_t, dbeta);
     return check_launch("sng_edge_bwd");

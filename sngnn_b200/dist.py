@@ -219,29 +219,28 @@ def _complete_dw(g0, shard, n, c, pending=None):
 
 class _ShardedFusedAgg(torch.autograd.Function):
     """SNGNN++ layer on a row shard of a SYMMETRIC graph: aggregation, structural term and beta blend in ONE pass over the
-    shard's in-edges (sng_edge_fwd with the fused epilogue; R: models/models.py:124-136).  Backward: scatter form of the
-    aggregation backward (contribution to dL/dh of every node, reduce-scattered by AllGatherRows), dL/dW^T as above."""
+    shard's in-edges (sng_edge_fwd with the fused epilogue; R: models/models.py:124-136).  Backward: sng_edge_bwd in its
+    row-shard form (the shard's contribution to dL/dh of every node, reduce-scattered by AllGatherRows, and its part of
+    dL/dbeta, both from fixed-order sums), dL/dW^T as above."""
 
     @staticmethod
     def forward(ctx, h_all, w_weight, w_bias, beta, bias, shard, n, lo, top_k, thr):
         h_all = SF._check_h(h_all)
         fuse = SF._structural_operands(w_weight, w_bias, beta, bias, h_all.size(1))
         train = any(ctx.needs_input_grad)
-        out, sel_src, sel_w, _, sel_cnt, inv_norm, diff = SF._edge_fwd(h_all, shard, lo, int(top_k), thr, train, fuse)
+        out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = SF._edge_fwd(h_all, shard, lo, int(top_k), thr, train, fuse, want_q=True)
         ctx.shard, ctx.c, ctx.n, ctx.lo, ctx.k, ctx.has_bias = shard, w_weight.size(0), n, lo, int(top_k), bias is not None
-        ctx.save_for_backward(h_all, sel_src, sel_w, sel_cnt, inv_norm, diff, beta)
+        ctx.save_for_backward(h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        h_all, sel_src, sel_w, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
+        h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
         shard, c = ctx.shard, ctx.c
         g = g.contiguous()
         g0 = g * beta
         pending = _gather_row_blocks_async(g0, ctx.n)             # needed only for dL/dW^T below: overlaps the aggregation backward
-        dh = SF.edge_agg_bwd_scatter(h_all, inv_norm, g - g0, shard.rowptr_in, shard.col_in, shard.n, ctx.lo, ctx.k,
-                                     sel_src, sel_w, sel_cnt, shard.inv_deg)
-        dbeta = (diff * g).sum().reshape(1)
+        dh, _, dbeta = SF.edge_bwd(h_all, inv_norm, g, shard, ctx.k, sel_src, sel_w, sel_q, sel_cnt, beta, diff, row_offset=ctx.lo)
         dw = _complete_dw(g0, shard, ctx.n, c, pending)
         dbias = g.sum(0)[:c] if ctx.has_bias else None
         return dh, dw, g0.sum(0)[:c], dbeta, dbias, None, None, None, None, None

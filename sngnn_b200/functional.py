@@ -202,20 +202,25 @@ class EdgeAgg(torch.autograd.Function):
         return dh, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None
 
 
-def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None):
+def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None, *, row_offset=0):
     """sng_edge_bwd: dL/dh [N, Cp] of the aggregation -- two gather passes, no float atomics -- and, with `beta` (the fused
-    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout."""
-    n, cp = h.shape
+    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout.
+    Row shard (`graph` = PreparedGraph.row_slice(lo, hi), row_offset = lo, `h` / `inv_norm` of all N nodes, `g` / `diff` / the
+    lists of the shard's rows): dh is the shard's contribution to dL/dh of every node and dbeta its part of dL/dbeta, both
+    bit-reproducible; dL/dW^T is not computed (None): the caller assembles it from the g0 of every shard."""
+    n_total, cp = h.shape
+    n = graph.n
     dev = h.device
     fused = beta is not None
     coef = torch.empty(max(graph.num_edges, 1) * 2, dtype=torch.float32, device=dev)
-    dnt = torch.empty_like(h)
+    dnt = torch.empty(n, cp, dtype=torch.float32, device=dev)
     dh = torch.empty_like(h)
     dbeta = dwt = part = None
     if fused:
         dbeta = torch.empty(1, dtype=torch.float32, device=dev)
         part = torch.empty(_C.PARTIALS, dtype=torch.float32, device=dev)
-        dwt = torch.empty(n, cp, dtype=torch.float32, device=dev)
+        if not graph.is_shard:
+            dwt = torch.empty(n, cp, dtype=torch.float32, device=dev)
     tab = graph.chunk_tab_out if cp <= 32 else None
     n_chunks = -1 if tab is None else int(tab.size(0))
     cpart = None
@@ -224,8 +229,9 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
         while cg < cp:
             cg *= 2
         cpart = torch.empty(n_chunks * 3 * cg, dtype=torch.float32, device=dev)
-    _C.call("sng_edge_bwd", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n, cp, cp, cp, _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
-            _C.ptr(graph.tpos), _C.ptr(graph.rowptr_out), _C.ptr(graph.col_out), graph.src_shift, graph.num_edges, k,
+    _C.call("sng_edge_bwd", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
+            _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
+            _C.ptr(graph.tpos), _C.ptr(graph.rowptr_tr), _C.ptr(graph.col_tr), graph.src_shift, graph.num_edges, k,
             _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_q), _C.ptr(sel_cnt), _C.ptr(beta), _C.ptr(diff if fused else None), cp,
             _C.ptr(dbeta), _C.ptr(coef), _C.ptr(dnt), _C.ptr(part), _C.ptr(dh), _C.ptr(dwt), cp,
             _C.ptr(tab), n_chunks, _C.ptr(graph.lrows_out if tab is not None else None),
@@ -234,7 +240,7 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
 
 
 def edge_agg_bwd_scatter(h_all, inv_norm, g, rowptr, col, n, row_offset, k, sel_src, sel_w, sel_cnt, inv_denom):
-    """sng_edge_agg_bwd (scatter form, FP32 atomics: row shards and explicit neighbour lists have no transpose index).
+    """sng_edge_agg_bwd (scatter form, FP32 atomics: explicit neighbour lists have no transpose index; it serves ListAgg).
     `g` = dL/dout of target rows [row_offset, row_offset + n) of `h_all`; returns their contribution to dL/dh_all (the
     contributions of different row ranges add).  k > 0: selection lists + inv_denom; k == 0: every edge of rowptr / col."""
     n_total, c = h_all.shape
@@ -256,24 +262,23 @@ def edge_topk_agg_rows(h_all, shard, row_offset, top_k=None, thr=None):
 class ShardedEdgeTopkAgg(torch.autograd.Function):
     """K2 / K2b on a ROW SHARD: forward computes out_1 for target rows [row_offset, row_offset + shard.n) from `h_all` (all
     nodes); backward returns this shard's contribution to dL/dh_all [N, C] -- contributions of different shards add
-    (SURVEY.md §8(e): the caller reduce-scatters them, see dist.AllGatherRows).  A shard has no transpose index, so its
-    backward is the scatter form (edge_agg_bwd_scatter)."""
+    (SURVEY.md §8(e): the caller reduce-scatters them, see dist.AllGatherRows).  The backward is sng_edge_bwd in its
+    row-shard form, through the shard's own transpose index: no float atomics, bit-reproducible."""
 
     @staticmethod
     def forward(ctx, h_all, shard, row_offset, top_k, thr):
         h_all = _check_h(h_all)
         k = int(top_k) if top_k is not None else 0
-        out, sel_src, sel_w, _, sel_cnt, inv_norm, _ = _edge_fwd(h_all, shard, int(row_offset), k, thr, ctx.needs_input_grad[0])
+        out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, _ = _edge_fwd(h_all, shard, int(row_offset), k, thr, ctx.needs_input_grad[0],
+                                                                     want_q=True)
         ctx.shard, ctx.k, ctx.row_offset = shard, k, int(row_offset)
-        ctx.save_for_backward(h_all, sel_src, sel_w, sel_cnt, inv_norm)
+        ctx.save_for_backward(h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        h_all, sel_src, sel_w, sel_cnt, inv_norm = ctx.saved_tensors
-        shard = ctx.shard
-        dh = edge_agg_bwd_scatter(h_all, inv_norm, g, shard.rowptr_in, shard.col_in, shard.n, ctx.row_offset, ctx.k,
-                                  sel_src, sel_w, sel_cnt, shard.inv_deg)
+        h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm = ctx.saved_tensors
+        dh, _, _ = edge_bwd(h_all, inv_norm, g.contiguous(), ctx.shard, ctx.k, sel_src, sel_w, sel_q, sel_cnt, row_offset=ctx.row_offset)
         return dh, None, None, None, None
 
 

@@ -11,7 +11,9 @@ int32 CSR arrays the kernels consume:
   * CSR by SHIFTED SOURCE (`rowptr_out`, `col_out`): out-neighbours t of node (src - min src), for
     out_0 = A @ W^T (R: :124-130);  `col_in_shift = col_in - min(src)` serves its transpose in backward.
   * `tpos[p]` = position of by-target edge p in the by-source arrays: the transpose index that lets the backward of the
-    aggregation run as two gather passes without float atomics (sng_edge_bwd).
+    aggregation run as two gather passes without float atomics (sng_edge_bwd).  `rowptr_tr` / `col_tr` name the by-source
+    CSR that `tpos` points into: the same tensors as `rowptr_out` / `col_out` for a whole graph, the shard's own
+    transpose for a row shard (`row_slice`).
   * `rows_long` / `rows_hub`: target rows with 32 < in-degree <= 1024 / > 1024 (the forward's degree dispatch), and
     `symmetric`: every in-list equals the out-list with min(src) == 0, which lets SNGNN++ gather W^T rows in the same pass.
 The by-source arrays are always built: the deterministic backward of every model needs them.
@@ -30,7 +32,7 @@ _CACHE_MAX = 8
 class PreparedGraph:
     __slots__ = ("n", "num_edges", "rowptr_in", "col_in", "inv_deg", "src_shift", "rowptr_out", "col_out",
                  "col_in_shift", "_shards", "tpos", "rows_long", "rows_hub", "symmetric", "max_deg", "is_shard",
-                 "chunk_tab", "lrows", "lrow_ptr", "chunk_tab_out", "lrows_out", "lrow_ptr_out")
+                 "chunk_tab", "lrows", "lrow_ptr", "chunk_tab_out", "lrows_out", "lrow_ptr_out", "rowptr_tr", "col_tr")
 
     @staticmethod
     def _chunk_tables(rowptr, lrows):
@@ -58,14 +60,20 @@ class PreparedGraph:
         lrows = torch.cat([self.rows_long, self.rows_hub]).long().sort().values
         self.chunk_tab, self.lrow_ptr = self._chunk_tables(self.rowptr_in, lrows)
         self.lrows = lrows.to(torch.int32).contiguous()
-        if self.rowptr_out is not None and not self.is_shard:
-            rp = self.rowptr_out.long()
+        if self.rowptr_tr is not None:
+            rp = self.rowptr_tr.long()
             lr = ((rp[1:] - rp[:-1]) > 32).nonzero().flatten()                             # rows of the by-source CSR = source id - shift
-            self.chunk_tab_out, self.lrow_ptr_out = self._chunk_tables(self.rowptr_out, lr)
+            self.chunk_tab_out, self.lrow_ptr_out = self._chunk_tables(self.rowptr_tr, lr)
             self.lrows_out = (lr + self.src_shift).to(torch.int32).contiguous()               # true source ids
 
     def row_slice(self, lo, hi):
-        """Row-sharded view (targets [lo, hi)) for multi-GPU aggregation: rowptr rebased to 0.  Cached per (lo, hi)."""
+        """Row-sharded view (targets [lo, hi)) for multi-GPU aggregation: rowptr rebased to 0.  Cached per (lo, hi).
+
+        The shard gets its own transpose index, so that its backward runs the same two gather passes as a whole graph's:
+        `rowptr_tr` [n + 1] / `col_tr` = CSR by (source - src_shift) over ALL n source rows holding only the shard's
+        in-edges, targets as shard-local ids; `tpos[p]` = position of shard by-target edge p in those arrays.  They are a
+        stable compaction of the whole graph's by-source arrays (no sort), so every source row lists its shard edges in the
+        whole graph's order, and the shard [0, n) has exactly the whole graph's transpose."""
         cache = getattr(self, "_shards", None)
         if cache is None:
             cache = self._shards = {}
@@ -80,7 +88,14 @@ class PreparedGraph:
         g.inv_deg = self.inv_deg[lo:hi].contiguous()
         g.src_shift = self.src_shift
         g.col_in_shift = None if self.col_in_shift is None else self.col_in_shift[b:e].contiguous()
-        g.rowptr_out = g.col_out = g.tpos = None      # no transpose index for a shard: its backward scatters
+        g.rowptr_out = g.col_out = g.tpos = g.rowptr_tr = g.col_tr = None
+        if self.tpos is not None:
+            keep = (self.col_out >= lo) & (self.col_out < hi)                # by-source edges whose target is in the shard
+            newpos = torch.zeros(keep.numel() + 1, dtype=torch.int64, device=keep.device)
+            torch.cumsum(keep, 0, out=newpos[1:])                             # newpos[q] = kept edges before by-source position q
+            g.rowptr_tr = newpos[self.rowptr_out.long()].to(torch.int32).contiguous()
+            g.col_tr = (self.col_out[keep] - lo).to(torch.int32).contiguous()
+            g.tpos = newpos[self.tpos[b:e].long()].to(torch.int32).contiguous()
         g.symmetric, g.max_deg, g.is_shard = False, self.max_deg, True
         g.rows_long = g.rows_hub = None
         if self.rows_long is not None:                       # shard-local degree lists
@@ -152,6 +167,7 @@ def prepare(edge_index, num_nodes, remove_self_loops, processed=False):
     inv_out = torch.empty_like(perm_out)
     inv_out[perm_out] = torch.arange(perm_out.numel(), device=perm_out.device)
     g.tpos = inv_out[perm_in].to(torch.int32).contiguous()
+    g.rowptr_tr, g.col_tr = g.rowptr_out, g.col_out
     g.rows_long = ((deg > 32) & (deg <= 1024)).nonzero().flatten().to(torch.int32)
     g.rows_hub = (deg > 1024).nonzero().flatten().to(torch.int32)
     g.max_deg = int(deg.max()) if g.n else 0
@@ -193,6 +209,7 @@ def _prepare_cuda(edge_index, n, remove_self_loops):
     g.rowptr_in, g.col_in = rowptr_in, col_in[:kept]
     g.src_shift = shift
     g.rowptr_out, g.col_out, g.col_in_shift, g.tpos = rowptr_out, col_out[:kept], col_in_shift[:kept], tpos[:kept]
+    g.rowptr_tr, g.col_tr = g.rowptr_out, g.col_out
     g.rows_long = long_rows[:n_long].clone()
     g.rows_hub = long_rows[n - n_hub:].clone() if n_hub else long_rows[:0].clone()
     g.symmetric, g.max_deg, g.is_shard = sym != 0, max_deg, False
