@@ -131,8 +131,36 @@ SNG_API int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, 
                  const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
                  int64_t n_lrows_out, float* chunk_partials, void* stream);
 
-/* Scatter form of the backward (float atomics; used for explicit neighbour lists -- the all-pairs mode -- which have no
- * transpose index; edge-restricted layers, row shards included, use sng_edge_bwd).
+/* Gather form of the backward of sng_list_agg_fwd (explicit neighbour lists: the all-pairs mode) -- the same two passes and
+ * kernels as sng_edge_bwd, no float atomics, bit-reproducible.  The lists are those of sng_simknn_build: idx / sim [n, top_k]
+ * (global column ids in rank order, sim = cosine of h_i and h_j), cnt [n]; entries t < cnt[i] <= top_k are node ids, the
+ * rest is padding.  inv_denom [n] = the forward's per-row factor (1 / denominator).  g = dL/dout [n, ldg].
+ * sel_q / rowptr_tr / col_tr: the transpose of the lists (sng_list_transpose), the by-source CSR over all n_total nodes.
+ * chunk_tab / lrows / lrow_ptr: the degree tables of sng_edge_bwd over rowptr_tr (source rows with more than 32 list entries
+ * cut into <= 32-entry chunks), chunk_partials as there; n_chunks < 0 = tables unknown (used for c <= 32 only).
+ * Workspaces (contents irrelevant): coef [2 * rowptr_tr[n_total]] floats, dn_target [n, ld].  Output dh [n_total, ld]: every
+ * row is written.  Row sharding as sng_edge_bwd: the lists are rows [row_offset, row_offset + n) of `h` (all n_total nodes,
+ * as is inv_norm), dh is their CONTRIBUTION to dL/dh of every node; n = 0 gives a zero contribution. */
+SNG_API int sng_list_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                 int64_t c, int64_t ld, int64_t ldg,
+                 int top_k, const int32_t* idx, const float* sim, const int32_t* cnt, const float* inv_denom,
+                 const int32_t* sel_q, const int32_t* rowptr_tr, const int32_t* col_tr,
+                 float* coef, float* dn_target, float* dh,
+                 const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                 float* chunk_partials, void* stream);
+
+/* Transpose of fixed-width neighbour lists idx [nq, k] / cnt [nq] (entries t < cnt[i] are column ids in [0, n_total), the
+ * rest padding) into the by-source index of sng_list_bwd: rowptr_tr [n_total + 1], col_tr [nq * k capacity; rowptr_tr[n_total]
+ * used] = the LOCAL row i of every entry whose column is the source, ordered by (i, rank) within a source -- a stable radix
+ * sort (cub::DeviceRadixSort), so the result is a pure function of the lists; sel_q [nq, k] = position of entry (i, t) in
+ * col_tr (-1 for padding).  workspace >= sng_list_transpose_workspace_bytes(nq, k, n_total) (0 = shape rejected). */
+SNG_API size_t sng_list_transpose_workspace_bytes(int64_t nq, int64_t k, int64_t n_total);
+SNG_API int sng_list_transpose(const int32_t* idx, const int32_t* cnt, int64_t nq, int64_t k, int64_t n_total,
+                       int32_t* rowptr_tr, int32_t* col_tr, int32_t* sel_q, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Scatter form of the backward (float atomics, so not bit-reproducible).  No layer of the package calls it since sng_list_bwd
+ * covers explicit neighbour lists; it is kept as the comparison baseline of the timing scripts (scripts/k2_time.py,
+ * scripts/shard_bwd_time.py, scripts/allpairs_bwd_time.py).
  * Pass 1 scatters into the two zero-initialised accumulators dval, dnrm [n_total, c];
  * pass 2 writes dh [n_total, c] = dval + (dnrm - n (n . dnrm)) / r.   `g` = dL/dout_1 [n, c].
  * top_k > 0: uses the saved selection lists (inv_denom[i] = 1/max(deg_i,1));

@@ -30,6 +30,10 @@ SIGNATURES = {
     "sng_edge_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P, _P, _P, _P,
                             _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _P]),
     "sng_edge_agg_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "sng_list_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                            _P, _I64, _P, _P, _I64, _P, _P]),
+    "sng_list_transpose_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
+    "sng_list_transpose": (_I32, [_P, _P, _I64, _I64, _I64, _P, _P, _P, _P, _SZ, _P]),
     "sng_list_agg_fwd": (_I32, [_P, _I64, _I64, _I64, _I32, _P, _P, _P, _P, _P, _I64, _P]),
     "sng_spmm_fwd": (_I32, [_P, _I64, _I64, _I64, _P, _P, _P, _P, _P, _P, _I64, _P]),
     "sng_pp_fuse_fwd": (_I32, [_P, _I64, _I64, _I64, _P, _P, _P, _P, _P, _P, _P, _P, _P]),

@@ -1095,11 +1095,14 @@ __global__ void __launch_bounds__(kThreads) norm_bwd_finish_kernel(const float* 
 // Row shards: the call owns target rows [row_offset, row_offset + n) of h (all n_total rows); g, the lists, the CSR by
 // target, dnT and the by-source CSR (the shard's in-edges only, targets as local ids) are shard-local.  Pass S still runs
 // every source row j of n_total and writes dh_j = this shard's contribution; dnT_j exists only for the rows it owns.
+// Neighbour lists (sng_list_bwd): the saved lists are fixed-width kNN lists, inv_denom[i] replaces 1 / deg_i (the pass-T
+// kernels then never read rowptr), and the by-source CSR is their transpose (sng_list_transpose, src_shift 0).
 struct EdgeBwdArgs {
     const float* h; const float* inv_r; const float* g;
     int n_total, n, row_offset, c, ld, ldg;
     const int* rowptr; const int* col; const int* tpos;
     int top_k; const int* sel_src; const float* sel_w; const int* sel_q; const int* sel_cnt;
+    const float* inv_denom;                  // NULL: 1 / max(deg_i, 1) from rowptr (edges); else per target row (lists)
     const float* beta; const float* diff; int lddiff; float* dbeta_part;
     float2* coef; float* dnT;
     const int* rowptr_out; const int* col_out; int shift;
@@ -1114,7 +1117,9 @@ struct EdgeBwdArgs {
 // source row j is one of the call's target rows: pass T wrote its target-side dn at dnT[j - row_offset]
 __device__ __forceinline__ bool owns_row(const EdgeBwdArgs& a, int j) { return (unsigned)(j - a.row_offset) < (unsigned)a.n; }
 
-template <int G, bool SELECT_ALL>
+// LIST: the saved lists are neighbour lists with a.inv_denom (a template flag: a runtime branch costs the edge instances at
+// C = 32 / 64 an 8-byte spill)
+template <int G, bool SELECT_ALL, bool LIST = false>
 __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwdArgs a) {
     using S = RowShape<G>;
     constexpr int EPW = S::EPW, V = S::V;
@@ -1130,9 +1135,13 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
     float bpart = 0.f;
     for (int row = blockIdx.x * kWarpsPerBlock + warp; row < a.n; row += gridDim.x * kWarpsPerBlock) {
         const int grow = a.row_offset + row;
-        const int beg = __ldg(a.rowptr + row), deg = __ldg(a.rowptr + row + 1) - beg;
-        const int cnt = SELECT_ALL ? deg : __ldg(a.sel_cnt + row);
-        const float invd = 1.0f / (float)max(deg, 1);
+        int beg = 0, cnt;
+        float invd;
+        if (SELECT_ALL) { beg = __ldg(a.rowptr + row); cnt = __ldg(a.rowptr + row + 1) - beg; invd = 1.0f / (float)max(cnt, 1); }
+        else {
+            cnt = __ldg(a.sel_cnt + row);
+            invd = LIST ? __ldg(a.inv_denom + row) : 1.0f / (float)max(__ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row), 1);
+        }
         const float iri = __ldg(a.inv_r + grow);
         float4 graw[V], gs[V], ni[V], dni[V];
 #pragma unroll
@@ -1309,9 +1318,12 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
     const int row0 = blockIdx.x * kStWarps + warp;
     float bpart = 0.f;
 
-    auto load_meta = [&](int row, int& cnt, int& deg) {
-        cnt = -1; deg = 1;
-        if (row < a.n) { cnt = __ldg(a.sel_cnt + row); deg = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row); }
+    auto load_meta = [&](int row, int& cnt, float& invd) {                            // invd = 1 / deg_i
+        cnt = -1; invd = 1.f;
+        if (row < a.n) {
+            cnt = __ldg(a.sel_cnt + row);
+            invd = a.inv_denom ? __ldg(a.inv_denom + row) : __fdividef(1.0f, (float)max(__ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row), 1));
+        }
     };
     auto load_list = [&](int row, int cnt, int& j, float& w, int& qp) {
         j = 0; w = 0.f; qp = 0;
@@ -1335,10 +1347,10 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
 
-    int cntA, degA, cntB, degB, cntC, degC, cntD, degD;
-    load_meta(row0, cntA, degA);
-    load_meta(row0 + stride, cntB, degB);
-    load_meta(row0 + 2 * stride, cntC, degC);
+    int cntA, cntB, cntC, cntD; float idA, idB, idC, idD;
+    load_meta(row0, cntA, idA);
+    load_meta(row0 + stride, cntB, idB);
+    load_meta(row0 + 2 * stride, cntC, idC);
     int jA, qA, jB, qB; float wA, wB;
     load_list(row0, cntA, jA, wA, qA);
     load_list(row0 + stride, cntB, jB, wB, qB);
@@ -1348,7 +1360,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
     float dfA = (a.diff && cntA >= 0 && ch_ok) ? __ldg(a.diff + (int64_t)row0 * a.lddiff + ch) : 0.f;
     uint32_t stA = sbase, stB = sbase + SB;
     for (int row = row0; row < a.n; row += stride) {
-        load_meta(row + 3 * stride, cntD, degD);
+        load_meta(row + 3 * stride, cntD, idD);
         int jC, qC; float wC;
         load_list(row + 2 * stride, cntC, jC, wC, qC);
         issue(stB, row + stride, cntB, jB);
@@ -1359,7 +1371,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
         __syncwarp();
         {
             const int cnt = cntA;
-            const float invd = __fdividef(1.0f, (float)max(degA, 1)) * gscale;           // g1_i / deg_i = g_i * invd
+            const float invd = idA * gscale;                                             // g1_i / deg_i = g_i * invd
             const uint32_t own = stA + own_off, gt = stA + GI;
             float d = 0.f;
 #pragma unroll
@@ -1382,9 +1394,9 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_bwd_target_s
             }
         }
         __syncwarp();
-        cntA = cntB; degA = degB; jA = jB; wA = wB; qA = qB; irjA = irjB; iriA = iriB; dfA = dfB;
-        cntB = cntC; degB = degC; jB = jC; wB = wC; qB = qC;
-        cntC = cntD; degC = degD;
+        cntA = cntB; idA = idB; jA = jB; wA = wB; qA = qB; irjA = irjB; iriA = iriB; dfA = dfB;
+        cntB = cntC; idB = idC; jB = jC; wB = wC; qB = qC;
+        cntC = cntD; idC = idD;
         const uint32_t t = stA; stA = stB; stB = t;
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -1573,9 +1585,12 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_narrow_kernel(const 
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
     float bpart = 0.f;
     struct Gt { float4 hj, hi, gi; float irj, iri, df, gc; };
-    auto load_meta = [&](int row, int& cnt, int& deg) {
-        cnt = -1; deg = 1;
-        if (row < a.n) { cnt = __ldg(a.sel_cnt + row); deg = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row); }
+    auto load_meta = [&](int row, int& cnt, float& invd) {                            // invd = 1 / deg_i
+        cnt = -1; invd = 1.f;
+        if (row < a.n) {
+            cnt = __ldg(a.sel_cnt + row);
+            invd = a.inv_denom ? __ldg(a.inv_denom + row) : __fdividef(1.0f, (float)max(__ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row), 1));
+        }
     };
     auto load_list = [&](int row, int cnt, int& j, float& w, int& qp) {
         j = -1; w = 0.f; qp = 0;
@@ -1590,22 +1605,22 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_narrow_kernel(const 
             if (a.diff && writer) { g.df = __ldg(a.diff + (int64_t)row * a.lddiff + wc); g.gc = __ldg(a.g + (int64_t)row * a.ldg + wc); }
         }
     };
-    int cntA, degA, cntB, degB, cntC, degC, cntD, degD;
-    load_meta(row0, cntA, degA);
-    load_meta(row0 + stride, cntB, degB);
-    load_meta(row0 + 2 * stride, cntC, degC);
+    int cntA, cntB, cntC, cntD; float idA, idB, idC, idD;
+    load_meta(row0, cntA, idA);
+    load_meta(row0 + stride, cntB, idB);
+    load_meta(row0 + 2 * stride, cntC, idC);
     int jA, qA, jB, qB; float wA, wB;
     load_list(row0, cntA, jA, wA, qA);
     load_list(row0 + stride, cntB, jB, wB, qB);
     Gt gA, gB;
     gather(row0, cntA, jA, gA);
     for (int row = row0; row < a.n; row += stride) {
-        load_meta(row + 3 * stride, cntD, degD);
+        load_meta(row + 3 * stride, cntD, idD);
         int jC, qC; float wC;
         load_list(row + 2 * stride, cntC, jC, wC, qC);
         gather(row + stride, cntB, jB, gB);
         {
-            const float invd = __fdividef(1.0f, (float)max(degA, 1)) * gscale;           // g1_i / deg_i = g_i * invd
+            const float invd = idA * gscale;                                             // g1_i / deg_i = g_i * invd
             const float d = fmaf(gA.hj.x, gA.gi.x, fmaf(gA.hj.y, gA.gi.y, fmaf(gA.hj.z, gA.gi.z, fmaf(gA.hj.w, gA.gi.w, 0.f))));
             const float ds = d * invd;                                                   // dL/ds_e (lane = selected edge)
             if (lane < cntA) a.coef[qA] = make_float2(wA * invd, ds * gA.iri);
@@ -1617,9 +1632,9 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_narrow_kernel(const 
                 bpart = fmaf(gA.df, gA.gc, bpart);                                       // dL/dbeta: diff . g (raw g); df = 0 without diff
             }
         }
-        cntA = cntB; degA = degB; jA = jB; wA = wB; qA = qB; gA = gB;
-        cntB = cntC; degB = degC; jB = jC; wB = wC; qB = qC;
-        cntC = cntD; degC = degD;
+        cntA = cntB; idA = idB; jA = jB; wA = wB; qA = qB; gA = gB;
+        cntB = cntC; idB = idC; jB = jC; wB = wC; qB = qC;
+        cntC = cntD; idC = idD;
     }
     if (a.dbeta_part) {                                                                  // fixed-order block sum -> one partial per block
         bpart = group_sum<32>(bpart);
@@ -2128,6 +2143,41 @@ static void launch_bwd_source_staged(EdgeBwdArgs a, cudaStream_t st) {
         edge_bwd_source_merge_kernel<G, FUSE><<<grid_resident(edge_bwd_source_merge_kernel<G, FUSE>, a.n_lrows, kWarpsPerBlock), kThreads, 0, st>>>(a);
     }
 }
+
+// launch body of sng_edge_bwd and sng_list_bwd: pass T (by target), pass S (by source), then the fixed-order dbeta sum
+static int launch_edge_bwd(const EdgeBwdArgs& a, float* dbeta, cudaStream_t st, const char* fn) {
+    const int c = a.c, top_k = a.top_k, n = a.n, n_total = a.n_total;
+    const bool fuse = a.dwt != nullptr;
+    // n == 0 (an empty shard) still runs both passes: pass T writes no row but its one block writes a zero dbeta partial,
+    // pass S writes the zero contribution of every row
+    const bool staged_t = c <= 32 && top_k > 0 && top_k <= 32;      // pass T from the saved lists, rows staged in shared memory
+    const bool staged_s = c <= 32 && a.n_chunks >= 0;               // pass S with the by-source chunk tables
+    int grid_t = 1;
+    SNG_DISPATCH_G(c,
+        if constexpr (G == 1) {
+            if (staged_t) {
+                grid_t = grid_resident(edge_bwd_target_narrow_kernel, n, kWarpsPerBlock);
+                edge_bwd_target_narrow_kernel<<<grid_t, kThreads, 0, st>>>(a);
+            }
+        } else if constexpr (G <= 8) {
+            if (staged_t) grid_t = launch_bwd_target_staged<G>(a, st);
+        }
+        if (!staged_t || G > 8) {
+            if (a.inv_denom) { grid_t = grid_resident(edge_bwd_target_kernel<G, false, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false, true><<<grid_t, kThreads, 0, st>>>(a); }
+            else if (top_k > 0) { grid_t = grid_resident(edge_bwd_target_kernel<G, false>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false><<<grid_t, kThreads, 0, st>>>(a); }
+            else { grid_t = grid_resident(edge_bwd_target_kernel<G, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, true><<<grid_t, kThreads, 0, st>>>(a); }
+        }
+        bool done_s = false;
+        if constexpr (G <= 8) {
+            if (staged_s) { if (fuse) launch_bwd_source_staged<G, true>(a, st); else launch_bwd_source_staged<G, false>(a, st); done_s = true; }
+        }
+        if (!done_s) {
+            if (fuse) edge_bwd_source_kernel<G, true><<<grid_resident(edge_bwd_source_kernel<G, true>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
+            else edge_bwd_source_kernel<G, false><<<grid_resident(edge_bwd_source_kernel<G, false>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
+        });
+    if (dbeta) sum_partials_kernel<<<1, 256, 0, st>>>(a.dbeta_part, grid_t, dbeta);
+    return check_launch(fn);
+}
 }  // namespace sng
 
 extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
@@ -2154,47 +2204,50 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
                 "sng_edge_bwd: by-source chunk tables / partials workspace missing");
     if (n_total == 0) return SNG_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    if (top_k > 0 && num_edges > 0 &&
+    if (top_k > 0 && num_edges > 0 &&                                // unselected edges keep both coefficients 0
         cudaMemsetAsync(coef, 0, (size_t)num_edges * sizeof(float2), st) != cudaSuccess) return check_launch("sng_edge_bwd memset");
     EdgeBwdArgs a;
     a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n_total; a.n = (int)n; a.row_offset = (int)row_offset;
     a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.top_k = top_k > 0 ? top_k : 0;
-    a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt;
+    a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt; a.inv_denom = nullptr;
     a.beta = beta; a.diff = dbeta ? diff : nullptr; a.lddiff = (int)lddiff; a.dbeta_part = dbeta ? partials : nullptr;
     a.coef = reinterpret_cast<float2*>(coef); a.dnT = dn_target;
     a.rowptr_out = rowptr_out; a.col_out = col_out; a.shift = (int)src_shift;
     a.dh = dh; a.dwt = dwt; a.lddw = (int)lddw;
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab_out); a.n_chunks = (int)n_chunks_out; a.lrows = lrows_out; a.lrow_ptr = lrow_ptr_out;
     a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials;
-    // n == 0 (an empty shard) still runs both passes: pass T writes no row but its one block writes a zero dbeta partial,
-    // pass S writes the zero contribution of every row
-    const bool staged_t = c <= 32 && top_k > 0 && top_k <= 32;      // pass T from the saved lists, rows staged in shared memory
-    const bool staged_s = c <= 32 && n_chunks_out >= 0;              // pass S with the by-source chunk tables
-    int grid_t = 1;
-    SNG_DISPATCH_G(c,
-        if constexpr (G == 1) {
-            if (staged_t) {
-                grid_t = grid_resident(edge_bwd_target_narrow_kernel, n, kWarpsPerBlock);
-                edge_bwd_target_narrow_kernel<<<grid_t, kThreads, 0, st>>>(a);
-            }
-        } else if constexpr (G <= 8) {
-            if (staged_t) grid_t = launch_bwd_target_staged<G>(a, st);
-        }
-        if (!staged_t || G > 8) {
-            if (top_k > 0) { grid_t = grid_resident(edge_bwd_target_kernel<G, false>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false><<<grid_t, kThreads, 0, st>>>(a); }
-            else { grid_t = grid_resident(edge_bwd_target_kernel<G, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, true><<<grid_t, kThreads, 0, st>>>(a); }
-        }
-        bool done_s = false;
-        if constexpr (G <= 8) {
-            if (staged_s) { if (dwt) launch_bwd_source_staged<G, true>(a, st); else launch_bwd_source_staged<G, false>(a, st); done_s = true; }
-        }
-        if (!done_s) {
-            if (dwt) edge_bwd_source_kernel<G, true><<<grid_resident(edge_bwd_source_kernel<G, true>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
-            else edge_bwd_source_kernel<G, false><<<grid_resident(edge_bwd_source_kernel<G, false>, n_total, kWarpsPerBlock), kThreads, 0, st>>>(a);
-        });
-    if (dbeta) sum_partials_kernel<<<1, 256, 0, st>>>(partials, grid_t, dbeta);
-    return check_launch("sng_edge_bwd");
+    return launch_edge_bwd(a, dbeta, st, "sng_edge_bwd");
+}
+
+extern "C" int sng_list_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                            int64_t c, int64_t ld, int64_t ldg,
+                            int top_k, const int32_t* idx, const float* sim, const int32_t* cnt, const float* inv_denom,
+                            const int32_t* sel_q, const int32_t* rowptr_tr, const int32_t* col_tr,
+                            float* coef, float* dn_target, float* dh,
+                            const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                            float* chunk_partials, void* stream) {
+    if (int rc = check_rows("sng_list_bwd", n_total, c, ld)) return rc;
+    SNG_REQUIRE(n >= 0 && row_offset >= 0 && row_offset + n <= n_total, "sng_list_bwd: bad n / row_offset / n_total");
+    SNG_REQUIRE(top_k > 0 && top_k <= SNG_MAX_TOPK, "sng_list_bwd: list width top_k=%d must be in [1, %d]", top_k, SNG_MAX_TOPK);
+    // (an empty shard, n == 0, has no rows of g / dn_target / the lists, and no transposed entries: those may be NULL)
+    SNG_REQUIRE(h && inv_norm && rowptr_tr && dh && ldg % 4 == 0 && ldg >= c, "sng_list_bwd: null pointer or bad ldg");
+    SNG_REQUIRE(n == 0 || (g && idx && sim && cnt && inv_denom && sel_q && col_tr && coef && dn_target), "sng_list_bwd: missing lists / transpose / workspace");
+    SNG_REQUIRE(n_chunks <= 0 || (chunk_tab && lrows && lrow_ptr && n_lrows > 0 && chunk_partials),
+                "sng_list_bwd: by-source chunk tables / partials workspace missing");
+    if (n_total == 0) return SNG_OK;
+    EdgeBwdArgs a;
+    a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n_total; a.n = (int)n; a.row_offset = (int)row_offset;
+    a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
+    a.rowptr = nullptr; a.col = nullptr; a.tpos = nullptr; a.top_k = top_k;
+    a.sel_src = idx; a.sel_w = sim; a.sel_q = sel_q; a.sel_cnt = cnt; a.inv_denom = inv_denom;
+    a.beta = nullptr; a.diff = nullptr; a.lddiff = 0; a.dbeta_part = nullptr;
+    a.coef = reinterpret_cast<float2*>(coef); a.dnT = dn_target;            // every list entry writes its coefficient: no memset
+    a.rowptr_out = rowptr_tr; a.col_out = col_tr; a.shift = 0;
+    a.dh = dh; a.dwt = nullptr; a.lddw = 0;
+    a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab); a.n_chunks = (int)n_chunks; a.lrows = lrows; a.lrow_ptr = lrow_ptr;
+    a.n_lrows = (int)n_lrows; a.tmp_part = chunk_partials;
+    return launch_edge_bwd(a, nullptr, (cudaStream_t)stream, "sng_list_bwd");
 }
 
 extern "C" int sng_list_agg_fwd(const float* h, int64_t n_rows, int64_t c, int64_t ldh, int list_k, const int32_t* sel_src,

@@ -94,6 +94,29 @@ __global__ void __launch_bounds__(256) graph_finish_kernel(const int* __restrict
     if (blockIdx.x == 0 && threadIdx.x == 0) { info[0] = kept; info[1] = shift; }
 }
 
+// ---- transpose of fixed-width neighbour lists (the by-source index of sng_list_bwd).  Entry p = i * k + s of the lists is
+// keyed by its column idx[p] (padding, s >= cnt[i]: the sentinel n_total); the stable sort of (key, p) orders every source
+// row's entries by p, i.e. by (target row, rank).
+__global__ void __launch_bounds__(256) list_keys_kernel(const int* __restrict__ idx, const int* __restrict__ cnt, int64_t total, int k,
+                                                       int n_total, int* __restrict__ key, int* __restrict__ pos) {
+    for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < total; p += (int64_t)gridDim.x * blockDim.x) {
+        const int i = (int)(p / k), s = (int)(p - (int64_t)i * k);
+        key[p] = s < __ldg(cnt + i) ? __ldg(idx + p) : n_total;
+        pos[p] = (int)p;
+    }
+}
+
+// col_tr[q] = local target row of sorted entry q, sel_q[p] = its position q (-1 for padding)
+__global__ void __launch_bounds__(256) list_place_kernel(const int* __restrict__ key_sorted, const int* __restrict__ pos_sorted, int64_t total,
+                                                        int k, int n_total, int* __restrict__ col_tr, int* __restrict__ sel_q) {
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < total; q += (int64_t)gridDim.x * blockDim.x) {
+        const int p = __ldg(pos_sorted + q);
+        const bool valid = __ldg(key_sorted + q) < n_total;
+        if (valid) col_tr[q] = p / k;
+        sel_q[p] = valid ? (int)q : -1;
+    }
+}
+
 static int key_bits(int64_t n) { int b = 1; while ((1ll << b) <= n) ++b; return b; }      // keys are in [0, n]
 
 static size_t sort_temp_bytes(int64_t total, int bits) {
@@ -154,4 +177,38 @@ extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, i
     graph_finish_kernel<<<grid, 256, 0, st>>>(rowptr_in, (int)n, inv_deg, col_in, col_in_shift, min_src, rowptr_out, col_out, perm_in,
                                              inv_out, tpos, long_rows, info);
     return check_launch("sng_graph_prepare");
+}
+
+extern "C" size_t sng_list_transpose_workspace_bytes(int64_t nq, int64_t k, int64_t n_total) {
+    if (nq < 0 || k <= 0 || k > SNG_MAX_TOPK || n_total < 0 || n_total >= (1ll << 31) || nq * k >= (1ll << 31)) return 0;
+    const int64_t total = nq * k;
+    return 4 * al256((size_t)total * 4) + al256(sort_temp_bytes(total, key_bits(n_total))) + 256;
+}
+
+extern "C" int sng_list_transpose(const int32_t* idx, const int32_t* cnt, int64_t nq, int64_t k, int64_t n_total,
+                                  int32_t* rowptr_tr, int32_t* col_tr, int32_t* sel_q, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+    const size_t need = sng_list_transpose_workspace_bytes(nq, k, n_total);
+    SNG_REQUIRE(need > 0, "sng_list_transpose: bad nq=%lld / k=%lld / n_total=%lld", (long long)nq, (long long)k, (long long)n_total);
+    SNG_REQUIRE(rowptr_tr && (nq == 0 || (idx && cnt && col_tr && sel_q)), "sng_list_transpose: null pointer");
+    if (!workspace || workspace_bytes < need) { set_error("sng_list_transpose: workspace too small"); return SNG_ERR_WORKSPACE; }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t total = nq * k;
+    const int bits = key_bits(n_total);
+    uint8_t* w = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    int* key = reinterpret_cast<int*>(w); w += al256((size_t)total * 4);
+    int* pos = reinterpret_cast<int*>(w); w += al256((size_t)total * 4);
+    int* key_sorted = reinterpret_cast<int*>(w); w += al256((size_t)total * 4);
+    int* pos_sorted = reinterpret_cast<int*>(w); w += al256((size_t)total * 4);
+    size_t temp_bytes = sort_temp_bytes(total, bits);
+    if (total > 0) {
+        const int grid = grid_capped(total, 256, 16);
+        list_keys_kernel<<<grid, 256, 0, st>>>(idx, cnt, total, (int)k, (int)n_total, key, pos);
+        if (int rc = check_launch("sng_list_transpose keys")) return rc;
+        if (cub::DeviceRadixSort::SortPairs(w, temp_bytes, key, key_sorted, pos, pos_sorted, total, 0, bits, st) != cudaSuccess)
+            return check_launch("sng_list_transpose sort");
+        list_place_kernel<<<grid, 256, 0, st>>>(key_sorted, pos_sorted, total, (int)k, (int)n_total, col_tr, sel_q);
+    }
+    graph_rowptr_kernel<<<grid_capped(n_total + 1, 256, 16), 256, 0, st>>>(key_sorted, total, (int)n_total, nullptr, rowptr_tr);
+    return check_launch("sng_list_transpose");
 }

@@ -263,9 +263,12 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
     feature rows [lo, hi) and returns the log-probabilities of those rows.  Mirrors _SNStack.forward / the conv forwards of
     models.py (R: models/models.py:76-86,116-137,233-242,322-329) with the aggregation and the ++ fusion replaced by their
     sharded forms.  BatchNorm needs statistics over all nodes and is not supported here (the reference default is bn=False);
-    neither are the non-reference options candidates='all_pairs' / denominator='selected'."""
+    neither is denominator='selected' with candidates='edges'.
+    candidates='all_pairs' (either denominator): h is all-gathered, the rank builds the kNN lists of its own rows over every
+    node (simknn.allpairs_topk_agg with rows = [lo, hi)) and aggregates them; the SNGNN++ structural term goes through
+    pp_fuse_sharded."""
     import torch.nn.functional as F
-    from . import graph as G, models as M
+    from . import graph as G, models as M, simknn
     if getattr(model, "bn", False):
         raise NotImplementedError("sharded_forward: bn=True needs cross-rank batch statistics")
     ws, rank = world()
@@ -275,8 +278,9 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
     for i, conv in enumerate(convs):
         base = type(conv) is M.SNConv
         plus_plus = isinstance(conv, M.SNConv_plus_plus)
-        if not base and (conv.candidates != "edges" or conv.denominator != "candidates"):
-            raise NotImplementedError("sharded_forward supports candidates='edges', denominator='candidates' only")
+        all_pairs = not base and conv.candidates == "all_pairs"
+        if not base and not all_pairs and conv.denominator != "candidates":
+            raise NotImplementedError("sharded_forward: candidates='edges' with denominator='selected'")
         if not base and conv.top_k <= 0:
             raise NotImplementedError("sharded_forward: top_k <= 0")
         g = G.prepare(edge_index, n, remove_self_loops=False if base else bool(conv.is_remove_self_loops))
@@ -284,13 +288,19 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
         injected = agg is not None or fuse is not None
         if plus_plus:
             conv.w.weight._sng_grad_complete = not injected      # the CUDA backward assembles the complete gradient itself
-        if plus_plus and not injected and g.symmetric:
+        if plus_plus and not all_pairs and not injected and g.symmetric:
             h_all = AllGatherRows.apply(h, n)
             out = _ShardedFusedAgg.apply(h_all, conv.w.weight, conv.w.bias, conv.beta, conv.bias, g.row_slice(lo, hi), n, lo,
                                          conv.top_k, conv.thr)
             out = out[:, :conv.lin.out_features]
         else:
-            out, shard = edge_agg_sharded(h, g, None if base else conv.top_k, None if base else conv.thr, agg=agg)
+            if all_pairs:
+                h_all = AllGatherRows.apply(h, n)
+                out = simknn.allpairs_topk_agg(h_all, conv.top_k, conv.thr, bool(conv.is_remove_self_loops), conv.denominator,
+                                               rows=(lo, hi))
+                shard = g.row_slice(lo, hi) if plus_plus else None
+            else:
+                out, shard = edge_agg_sharded(h, g, None if base else conv.top_k, None if base else conv.thr, agg=agg)
             if plus_plus:
                 out = pp_fuse_sharded(out, conv.w.weight, conv.w.bias, conv.beta, conv.bias, shard, n, lo, fuse=fuse)
                 out = out[:, :conv.lin.out_features]

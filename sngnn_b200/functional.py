@@ -240,7 +240,7 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
 
 
 def edge_agg_bwd_scatter(h_all, inv_norm, g, rowptr, col, n, row_offset, k, sel_src, sel_w, sel_cnt, inv_denom):
-    """sng_edge_agg_bwd (scatter form, FP32 atomics: explicit neighbour lists have no transpose index; it serves ListAgg).
+    """sng_edge_agg_bwd (scatter form, FP32 atomics): no layer uses it; the timing scripts compare the gather forms with it.
     `g` = dL/dout of target rows [row_offset, row_offset + n) of `h_all`; returns their contribution to dL/dh_all (the
     contributions of different row ranges add).  k > 0: selection lists + inv_denom; k == 0: every edge of rowptr / col."""
     n_total, c = h_all.shape
@@ -292,28 +292,112 @@ def edge_topk_agg(h, graph, top_k=None, thr=None, return_selection=False, struct
     return out
 
 
+class ListTranspose:
+    """By-source index of fixed-width neighbour lists (sng_list_transpose): rowptr_tr [n_total + 1] / col_tr = for every source
+    node, the LOCAL rows of the lists that hold it, ordered by (row, rank); sel_q [nq, k] = position of entry (i, t) in col_tr
+    (-1 for padding); chunk_tab / lrows / lrow_ptr = the degree tables of sng_list_bwd's staged source pass (None when not
+    asked for)."""
+    __slots__ = ("rowptr_tr", "col_tr", "sel_q", "chunk_tab", "lrows", "lrow_ptr")
+
+
+def list_transpose(idx, cnt, n_total, chunk_tables=False):
+    """Transpose of the lists idx [nq, k] / cnt [nq] (entries t < cnt[i] are node ids < n_total, the rest padding).
+    CUDA tensors: sng_list_transpose (a stable radix sort), and with `chunk_tables` the chunk tables over rowptr_tr, which
+    read two counts back (one host synchronisation).  CPU tensors (the host-logic tests): the same construction in torch."""
+    from .graph import PreparedGraph
+    nq, k = idx.shape
+    t = ListTranspose()
+    t.chunk_tab = t.lrows = t.lrow_ptr = None
+    dev = idx.device
+    if not idx.is_cuda:
+        valid = (torch.arange(k)[None, :] < cnt[:, None]).reshape(-1)
+        key = torch.where(valid, idx.reshape(-1).long(), torch.full_like(valid, n_total, dtype=torch.long))
+        perm = torch.argsort(key, stable=True)
+        nnz = int(valid.sum())
+        rowptr = torch.zeros(n_total + 1, dtype=torch.int64)
+        torch.cumsum(torch.bincount(key[valid], minlength=n_total), 0, out=rowptr[1:])
+        t.rowptr_tr = rowptr.to(torch.int32)
+        t.col_tr = (perm[:nnz] // k).to(torch.int32)
+        sel_q = torch.full((nq * k,), -1, dtype=torch.int32)
+        sel_q[perm[:nnz]] = torch.arange(nnz, dtype=torch.int32)
+        t.sel_q = sel_q.reshape(nq, k)
+    else:
+        _C.require_cuda(idx, cnt)
+        idx, cnt = idx.contiguous(), cnt.contiguous()
+        t.rowptr_tr = torch.empty(n_total + 1, dtype=torch.int32, device=dev)
+        t.col_tr = torch.empty(max(nq * k, 1), dtype=torch.int32, device=dev)
+        t.sel_q = torch.empty(nq, k, dtype=torch.int32, device=dev)
+        wbytes = _C.lib().sng_list_transpose_workspace_bytes(nq, k, n_total)
+        if wbytes == 0:
+            raise RuntimeError(f"sng_list_transpose_workspace_bytes rejected nq={nq} k={k} n_total={n_total}")
+        ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
+        _C.call("sng_list_transpose", idx, _C.ptr(idx), _C.ptr(cnt), nq, k, n_total, _C.ptr(t.rowptr_tr), _C.ptr(t.col_tr),
+                _C.ptr(t.sel_q), _C.ptr(ws), wbytes)
+    if chunk_tables:
+        rp = t.rowptr_tr.long()
+        deg = rp[1:] - rp[:-1]
+        long_rows = deg > 32
+        n_long, n_chunks = (int(v) for v in torch.stack([long_rows.sum(), torch.where(long_rows, (deg + 31) // 32, 0).sum()]).tolist())
+        slot = torch.where(long_rows, torch.cumsum(long_rows, 0) - 1, n_long)          # rank among the long rows; n_long = discard
+        lr = torch.zeros(n_long + 1, dtype=torch.int64, device=dev).scatter_(0, slot, torch.arange(n_total, device=dev))[:n_long]
+        t.chunk_tab, t.lrow_ptr = PreparedGraph._chunk_tables(t.rowptr_tr, lr, n_chunks)
+        t.lrows = lr.to(torch.int32).contiguous()
+    return t
+
+
+def list_bwd(h_all, inv_norm, g, idx, sim, cnt, inv_denom, row_offset=0):
+    """sng_list_bwd: dL/dh [N, Cp] of the list aggregation out[i] = inv_denom[i] sum_t sim[i, t] h[idx[i, t]] with sim the
+    cosines of h -- sng_edge_bwd's two gather passes through the lists' transpose (built here), no float atomics.  The
+    lists are rows [row_offset, row_offset + n) of `h_all` (all N nodes); dh is their contribution to dL/dh of every node."""
+    n_total, cp = h_all.shape
+    n, k = idx.shape
+    dev = h_all.device
+    tr = list_transpose(idx, cnt, n_total, chunk_tables=cp <= 32)
+    n_chunks = -1 if tr.chunk_tab is None else int(tr.chunk_tab.size(0))
+    cpart = None
+    if n_chunks > 0:
+        cg = 4
+        while cg < cp:
+            cg *= 2
+        cpart = torch.empty(n_chunks * 3 * cg, dtype=torch.float32, device=dev)
+    coef = torch.empty(max(n * k, 1) * 2, dtype=torch.float32, device=dev)
+    dnt = torch.empty(n, cp, dtype=torch.float32, device=dev)
+    dh = torch.empty_like(h_all)
+    _C.call("sng_list_bwd", h_all, _C.ptr(h_all), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
+            k, _C.ptr(idx), _C.ptr(sim), _C.ptr(cnt), _C.ptr(inv_denom), _C.ptr(tr.sel_q), _C.ptr(tr.rowptr_tr), _C.ptr(tr.col_tr),
+            _C.ptr(coef), _C.ptr(dnt), _C.ptr(dh), _C.ptr(tr.chunk_tab), n_chunks, _C.ptr(tr.lrows), _C.ptr(tr.lrow_ptr),
+            0 if tr.lrows is None else int(tr.lrows.numel()), _C.ptr(cpart))
+    return dh
+
+
 class ListAgg(torch.autograd.Function):
-    """Mean aggregation over an explicit neighbour list (all-pairs mode): forward sng_list_agg_fwd, backward K2b."""
+    """Mean aggregation over an explicit neighbour list (all-pairs mode): forward sng_list_agg_fwd, backward sng_list_bwd
+    (two gather passes through the lists' transpose, no float atomics, bit-reproducible).  With `row_offset` the lists are
+    rows [row_offset, row_offset + len(idx)) of `h`, which holds every node (a row shard): the backward then returns this
+    shard's contribution to dL/dh of every node -- contributions of different shards add (dist.AllGatherRows)."""
 
     @staticmethod
-    def forward(ctx, h, idx, sim, cnt, inv_denom):
+    def forward(ctx, h, idx, sim, cnt, inv_denom, row_offset=0):
         h = _check_h(h)
         n, c = h.shape
-        out = torch.empty(idx.size(0), c, dtype=h.dtype, device=h.device)
-        _C.call("sng_list_agg_fwd", h, _C.ptr(h), idx.size(0), c, c, idx.size(1), _C.ptr(idx), _C.ptr(sim), _C.ptr(cnt),
-                _C.ptr(inv_denom), _C.ptr(out), c)
+        nq = idx.size(0)
+        if row_offset < 0 or row_offset + nq > n:
+            raise RuntimeError(f"lists of rows [{row_offset}, {row_offset + nq}) but h has {n} rows")
+        out = torch.empty(nq, c, dtype=h.dtype, device=h.device)
+        if nq:
+            _C.call("sng_list_agg_fwd", h, _C.ptr(h), nq, c, c, idx.size(1), _C.ptr(idx), _C.ptr(sim), _C.ptr(cnt),
+                    _C.ptr(inv_denom), _C.ptr(out), c)
+        ctx.row_offset = int(row_offset)
         ctx.save_for_backward(h, idx, sim, cnt, inv_denom)
         return out
 
     @staticmethod
     def backward(ctx, g):
         h, idx, sim, cnt, inv_denom = ctx.saved_tensors
-        n = h.size(0)
-        if idx.size(0) != n:
-            raise RuntimeError("backward through a row-sharded list aggregation is not supported")
         _, _, inv_norm = rownorm(h, want_f32=False, want_inv=True)
-        dh = edge_agg_bwd_scatter(h, inv_norm, g, None, None, n, 0, idx.size(1), idx, sim, cnt, inv_denom)
-        return dh, None, None, None, None
+        idx, sim, cnt, inv_denom = idx.contiguous(), sim.contiguous(), cnt.contiguous(), inv_denom.contiguous()
+        dh = list_bwd(h, inv_norm, g.contiguous(), idx, sim, cnt, inv_denom, ctx.row_offset)
+        return dh, None, None, None, None, None
 
 
 def spmm(x, rowptr, col, n_rows, val=None, rowscale=None, bias=None):

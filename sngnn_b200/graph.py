@@ -35,15 +35,16 @@ class PreparedGraph:
                  "chunk_tab", "lrows", "lrow_ptr", "chunk_tab_out", "lrows_out", "lrow_ptr_out", "rowptr_tr", "col_tr")
 
     @staticmethod
-    def _chunk_tables(rowptr, lrows):
-        """(chunk_tab [n_chunks, 4] = first edge position, edges, row, 0; lrow_ptr) of the rows `lrows` (ascending) of a CSR."""
+    def _chunk_tables(rowptr, lrows, n_chunks=None):
+        """(chunk_tab [n_chunks, 4] = first edge position, edges, row, 0; lrow_ptr) of the rows `lrows` (ascending) of a CSR.
+        `n_chunks` (the total, when the caller knows it) spares the host synchronisation of sizing the table."""
         dev = rowptr.device
         rp = rowptr.long()
         beg, deg = rp[lrows], rp[lrows + 1] - rp[lrows]
         nch = (deg + 31) // 32
         ptr = torch.zeros(lrows.numel() + 1, dtype=torch.int64, device=dev)
         torch.cumsum(nch, 0, out=ptr[1:])
-        owner = torch.repeat_interleave(torch.arange(lrows.numel(), device=dev), nch)      # chunk -> index of its long row
+        owner = torch.repeat_interleave(torch.arange(lrows.numel(), device=dev), nch, output_size=n_chunks)   # chunk -> its long row
         within = torch.arange(owner.numel(), device=dev) - ptr[owner]
         cbeg = beg[owner] + 32 * within
         clen = torch.minimum(deg[owner] - 32 * within, torch.full_like(within, 32))

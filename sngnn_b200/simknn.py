@@ -124,14 +124,24 @@ def stage1_candidates(x, cand, thr_lo=-2.0, remove_self=True, force_ew=0, force_
     return ci[: n * s * cand].reshape(n, s, cand), cv[: n * s * cand].reshape(n, s, cand), cm[: n * s].reshape(n, s), xf, xh
 
 
-def allpairs_topk_agg(h, top_k, thr, remove_self, denominator="candidates"):
+def allpairs_topk_agg(h, top_k, thr, remove_self, denominator="candidates", rows=None):
     """All-pairs candidate mode of SNConv_plus(_plus): kNN on the layer's own h (similarity is on lin(x),
-    SURVEY.md D4), then the cosine-weighted mean.  `h` is the padded [N, Cp] hidden matrix."""
+    SURVEY.md D4), then the cosine-weighted mean.  `h` is the padded [N, Cp] hidden matrix.
+    rows = (lo, hi): only query rows [lo, hi) (a row shard; `h` still holds every node, e.g. after an all-gather).  The build
+    then runs on the same operands over those rows, so their lists and similarities equal the unsharded build's bit for bit;
+    the output has hi - lo rows and its backward is their contribution to dL/dh of every node (zero for an empty range)."""
     n = h.size(0)
-    idx, sim, cnt = build_knn(h.detach(), top_k, thr, remove_self)
+    lo, hi = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
+    if hi <= lo:                                          # empty shard: no build (it rejects empty ranges), zero contribution
+        idx = torch.empty(0, top_k, dtype=torch.int32, device=h.device)
+        sim = torch.empty(0, top_k, dtype=torch.float32, device=h.device)
+        cnt = torch.empty(0, dtype=torch.int32, device=h.device)
+    else:
+        xf, xh = normalize_operands(h.detach())
+        idx, sim, cnt = build_knn_normalized(xf, xh, h.size(1), top_k, thr, remove_self, lo, hi)
     if denominator == "candidates":
         cand = float(n - 1 if remove_self else n)
-        inv = torch.full((n,), 1.0 / max(cand, 1.0), dtype=torch.float32, device=h.device)
+        inv = torch.full((hi - lo,), 1.0 / max(cand, 1.0), dtype=torch.float32, device=h.device)
     else:
         inv = cnt.clamp(min=1).float().reciprocal()
-    return SF.ListAgg.apply(h, idx, sim, cnt, inv)
+    return SF.ListAgg.apply(h, idx, sim, cnt, inv, lo)
