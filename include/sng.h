@@ -74,7 +74,9 @@ SNG_API int sng_rownorm_f32(const float* x, int64_t n, int64_t d, int64_t ldx,
  * kept in original edge-position order):
  *   s_e    = <h_i/r_i , h_j/r_j>,  r = max(||h||, 1e-12)
  *   S_i    = first min(top_k, deg) edges under (s desc, position asc), cut at the first s < thr
- *   out_1[i] = (1/max(deg_i,1)) * sum_{e in S_i} s_e * h[src_e]
+ *   out_1[i] = (1/max(deg_i,1)) * sum_{e in S_i} s_e * h[src_e]                 denominator 0 ('candidates', PyG aggr='mean')
+ *   out_1[i] = (1/max(|S_i|,1)) * sum_{e in S_i} s_e * h[src_e]                 denominator 1 ('selected', sng_edge_fwd_denom)
+ *              (a row that selects nothing outputs 0)
  *   wt == NULL:  out = out_1
  *   wt != NULL:  out_0[i] = sum_{e in-list of i} wt[src_e] + b_w ;  out = beta*out_0 + (1-beta)*out_1 (+ bias) ;
  *                diff (may be NULL) = out_0 - out_1 = d out / d beta.  Only valid when the in-list of every node equals its
@@ -101,6 +103,19 @@ SNG_API int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t row
                  int32_t* sel_src, float* sel_w, int32_t* sel_q, int32_t* sel_cnt, float* inv_norm, int inv_norm_ready,
                  const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
                  void* stream);
+/* sng_edge_fwd with the mean's denominator as an argument (sng_edge_fwd = this with denominator 0, inv_denom NULL).
+ * denominator: 0 = candidates (1/max(deg_i,1)), 1 = selected (1/max(|S_i|,1); needs top_k > 0), in inference and training,
+ * with and without the fused epilogue (diff then holds out_0 - out_1 of this out_1).  inv_denom [n] (may be NULL; only with
+ * denominator 1) receives the factor 1/max(|S_i|,1) each row was scaled by: pass it to sng_edge_bwd_denom, which then uses the
+ * same floats.  Row sharding: inv_denom is indexed by LOCAL row, like out and sel_cnt. */
+SNG_API int sng_edge_fwd_denom(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
+                 const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                 const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                 const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
+                 int top_k, float thr, float* out, int64_t ldo,
+                 int32_t* sel_src, float* sel_w, int32_t* sel_q, int32_t* sel_cnt, float* inv_norm, int inv_norm_ready,
+                 const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
+                 int denominator, float* inv_denom, void* stream);
 
 /* K2b (+K4b) backward of the above w.r.t. h -- and, under the fused epilogue, w.r.t. wt and beta -- WITHOUT float atomics:
  * two gather passes (by target, then by source through the transpose index tpos), every sum in a fixed order, so the
@@ -130,6 +145,18 @@ SNG_API int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, 
                  float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
                  const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
                  int64_t n_lrows_out, float* chunk_partials, void* stream);
+/* sng_edge_bwd with the forward's per-row factor (sng_edge_bwd = this with inv_denom NULL).  inv_denom NULL: 1/max(deg_i,1)
+ * from rowptr (denominator 0); else inv_denom [n] as sng_edge_fwd_denom wrote it (denominator 1, needs top_k > 0), per LOCAL
+ * row under row sharding.  Everything else, the fused epilogue included, as sng_edge_bwd. */
+SNG_API int sng_edge_bwd_denom(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                 int64_t c, int64_t ld, int64_t ldg,
+                 const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                 const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
+                 int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
+                 const float* beta, const float* diff, int64_t lddiff, float* dbeta,
+                 float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
+                 const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
+                 int64_t n_lrows_out, float* chunk_partials, const float* inv_denom, void* stream);
 
 /* Gather form of the backward of sng_list_agg_fwd (explicit neighbour lists: the all-pairs mode) -- the same two passes and
  * kernels as sng_edge_bwd, no float atomics, bit-reproducible.  The lists are those of sng_simknn_build: idx / sim [n, top_k]

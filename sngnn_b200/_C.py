@@ -22,6 +22,8 @@ SIGNATURES = {
     "sng_edge_fwd_workspace_bytes": (_SZ, [_I64, _I64, _I32]),
     "sng_edge_fwd": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P, _P, _I64, _P, _I64, _P, _SZ, _I32, _F32, _P, _I64,
                             _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _P]),
+    "sng_edge_fwd_denom": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P, _P, _I64, _P, _I64, _P, _SZ, _I32, _F32, _P,
+                                  _I64, _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _I32, _P, _P]),
     "sng_lin_norm_supported": (_I32, [_I64, _I64]),
     "sng_lin_norm_fwd": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _P, _P, _P, _P]),
     "sng_lin_bwd_supported": (_I32, [_I64, _I64]),
@@ -29,6 +31,8 @@ SIGNATURES = {
     "sng_lin_bwd": (_I32, [_P, _I64, _P, _I64, _I64, _I64, _I64, _P, _I64, _P, _P, _SZ, _P]),
     "sng_edge_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P, _P, _P, _P,
                             _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _P]),
+    "sng_edge_bwd_denom": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _I32, _P, _P, _P, _P,
+                                  _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _P, _P]),
     "sng_edge_agg_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
     "sng_list_bwd": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
                             _P, _I64, _P, _P, _I64, _P, _P]),

@@ -99,6 +99,9 @@ __global__ void __launch_bounds__(kThreads) row_inv_norm_kernel(const float* __r
 // One launch family computes, for every target row i with in-edge list P_i (CSR by target, position order):
 //   s_e = <n_i, n_j>, S_i = first min(top_k, |P_i|) edges under (s desc, position asc) with s >= thr,
 //   out_1[i] = sum_{e in S_i} s_e h_j / max(|P_i|, 1)                                  (R: models/models.py:139-158, 244-263, 331-334)
+// or, with DSEL (denominator='selected', top_k > 0), out_1[i] = sum_{e in S_i} s_e h_j / max(|S_i|, 1): every variant
+// applies sel_factor(|S_i|) where it knows the final count, and writes that factor to inv_denom[i] (training) for the backward.
+// DSEL is a template flag: read at run time, it changed the registers or spills of 31 candidates-mode instances.
 // and, when `wt` is given (SNGNN++ on a graph whose in-lists equal its out-lists), in the SAME pass over the edges
 //   out_0[i] = sum_{e in P_i} Wt[j] + b_w,  out[i] = beta out_0 + (1 - beta) out_1 (+ bias)   (R: models/models.py:124-136)
 // Rows are dispatched by in-degree (tables built once per graph, sngnn_b200/graph.py):
@@ -119,6 +122,7 @@ struct EdgeFwdArgs {
     float* tmp_s; int* tmp_p; int* tmp_cnt; float* tmp_acc; float* tmp_a0;   // per-chunk candidates [n_chunks, min(top_k,32)], partial sums [n_chunks, 4G]
     int skip_deg;                            // long kernel over all rows: rows with more in-edges are left to the hub kernel (0 = none)
     int top_k; float thr;
+    float* inv_denom;                        // DSEL instances: the factor applied per row [n], or nullptr
     float* out; int ldo;
     int* sel_src; float* sel_w; int* sel_q; int* sel_cnt;      // saved for backward; all nullptr in inference
     const float* wt; int ldw; const float* b_w; const float* beta; const float* bias; float* diff;   // fused SNGNN++ epilogue
@@ -136,10 +140,14 @@ __device__ __forceinline__ void cross_group_sum4(float4& a) {
     a.x = cross_group_sum<G>(a.x); a.y = cross_group_sum<G>(a.y); a.z = cross_group_sum<G>(a.z); a.w = cross_group_sum<G>(a.w);
 }
 
+// denominator='selected': the per-row factor 1 / max(|S_i|, 1); the forward writes the same float to inv_denom for the backward
+__device__ __forceinline__ float sel_factor(int cnt) { return 1.0f / (float)max(cnt, 1); }
+
+// den = the row's in-degree (PyG aggr='mean': every candidate, selected or not) or, with DSEL, its selected count
 template <bool FUSE>
-__device__ __forceinline__ void write_row(const EdgeFwdArgs& a, int row, int c4, const float4& acc, const float4& a0, int deg, float beta,
+__device__ __forceinline__ void write_row(const EdgeFwdArgs& a, int row, int c4, const float4& acc, const float4& a0, int den, float beta,
                                           const float4& bw, const float4& bb) {
-    const float invd = 1.0f / (float)max(deg, 1);                    // PyG aggr='mean': the full in-degree, selected or not
+    const float invd = 1.0f / (float)max(den, 1);
     const float4 o1 = scale4(acc, invd);
     const int64_t o = (int64_t)row * a.ldo + c4;
     if (FUSE) {
@@ -187,7 +195,7 @@ __device__ __forceinline__ float lds32(uint32_t addr) {
 // bytes of a staged row slot: the row padded by one 16-byte chunk (G > 1), so that slot strides are odd multiples of 16 B
 template <int G> constexpr int staged_row_bytes() { return G == 1 ? 16 : 16 * G + 16; }
 
-template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK>
+template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK, bool DSEL = false>
 __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_kernel(const EdgeFwdArgs a) {
     constexpr int C = 4 * G;                    // channels of a padded row
     constexpr int RB = staged_row_bytes<G>();
@@ -338,7 +346,8 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_k
                 }
             } else {
                 if (lane < C && ch_ok) {
-                    const float o1 = __fdividef(acc, (float)max(deg, 1));                // PyG aggr='mean': the full in-degree
+                    // PyG aggr='mean': the full in-degree; denominator='selected': the selected count
+                    const float o1 = DSEL ? acc * sel_factor(cnt) : __fdividef(acc, (float)max(deg, 1));
                     const int64_t o = (int64_t)row * a.ldo + ch;
                     if (FUSE) {
                         const float o0 = a0 + bw;
@@ -360,6 +369,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_k
                     }
                     if (lane == 0) a.sel_cnt[row] = cnt;
                 }
+                if (DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(cnt);
             }
         }
         __syncwarp();                                                                    // A's slots are free from here
@@ -401,7 +411,7 @@ __device__ __forceinline__ float lane_reduce_scatter(float (&v)[K], int lane) {
 
 struct NarrowGather { float4 hj, wj, hi; float irl, iri; int tq; };
 
-template <bool FUSE, bool SELECT_ALL>
+template <bool FUSE, bool SELECT_ALL, bool DSEL = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_narrow_kernel(const EdgeFwdArgs a) {
     constexpr int K = FUSE ? 8 : 4;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -480,7 +490,8 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_narrow_kernel(const EdgeFwd
             const float tot = lane_reduce_scatter<K>(v, lane);
             const float a0 = FUSE ? __shfl_xor_sync(kFull, tot, 16) : 0.f;
             if (writer) {
-                const float o1 = __fdividef(tot, (float)max(deg, 1));                // PyG aggr='mean': the full in-degree
+                // PyG aggr='mean': the full in-degree; denominator='selected': the selected count
+                const float o1 = DSEL ? tot * sel_factor(cnt) : __fdividef(tot, (float)max(deg, 1));
                 const int64_t o = (int64_t)row * a.ldo + wc;
                 if (FUSE) {
                     const float o0 = a0 + bw;
@@ -502,6 +513,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_narrow_kernel(const EdgeFwd
                 }
                 if (lane == 0) a.sel_cnt[row] = cnt;
             }
+            if (DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(cnt);
         }
         begA = begB; degA = degB; jA = jB; gA = gB;
         begB = begC; degB = degC; jB = jC;
@@ -616,7 +628,7 @@ __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* cons
 }
 
 // weighted sum of the <= top_k winners of a finished list (source ids re-read through their positions) + the saved lists
-template <int G>
+template <int G, bool DSEL>
 __device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* const (&hb)[RowShape<G>::V], int row, const float* ls,
                                             const int* lp, int cnt, int lane, float4 (&acc)[RowShape<G>::V]) {
     using S = RowShape<G>;
@@ -640,9 +652,10 @@ __device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* c
         }
         if (lane == 0) a.sel_cnt[row] = cnt;
     }
+    if (DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(cnt);
 }
 
-template <int G, bool FUSE, bool SELECT_ALL>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdArgs a) {
     using S = RowShape<G>;
     constexpr int V = S::V;
@@ -683,12 +696,13 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdAr
         }
         L.cnt = 0; L.kth = -CUDART_INF_F;
         scan_row<G, FUSE, SELECT_ALL>(a, hb, wb, grow, end, beg, 32, ni, ch_ok, lane, L, acc, a0);
-        if (!SELECT_ALL) { finish_list<G>(a, hb, row, L.s, L.p, L.cnt, lane, acc); __syncwarp(); }
+        if (!SELECT_ALL) { finish_list<G, DSEL>(a, hb, row, L.s, L.p, L.cnt, lane, acc); __syncwarp(); }
+        const int den = DSEL ? L.cnt : end - beg;
 #pragma unroll
         for (int s = 0; s < V; ++s) {
             cross_group_sum4<G>(acc[s]);
             if (FUSE) cross_group_sum4<G>(a0[s]);
-            if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), acc[s], a0[s], end - beg, beta, bw[s], bb[s]);
+            if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), acc[s], a0[s], den, beta, bw[s], bb[s]);
         }
     }
 }
@@ -700,7 +714,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdAr
 // candidates of as many further chunks as fit, and top_k rounds of a warp max pick the new winners; lane order equals edge
 // position order, so the lowest lane among equal scores is the reference's tie-break.  Larger top_k: sorted insertion into
 // a shared-memory list (a newcomer loses every tie).
-template <int G, bool FUSE, bool SELECT_ALL>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdArgs a) {
     constexpr int C = 4 * G;
     extern __shared__ float smem[];
@@ -719,6 +733,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
         const int c0 = __ldg(a.lrow_ptr + li), c1 = __ldg(a.lrow_ptr + li + 1);
         const int deg = __ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row);
         float acc = 0.f, a0 = 0.f;
+        int nsel = 0;                                                        // the row's final selected count
         if (SELECT_ALL || FUSE) {
 #pragma unroll 4
             for (int ci = c0; ci < c1; ++ci) {
@@ -802,9 +817,11 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
                 }
                 if (lane == 0) a.sel_cnt[row] = nw;
             }
+            nsel = nw;
         }
+        if (DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(nsel);
         if (lane < C && ch_ok) {
-            const float o1 = __fdividef(acc, (float)max(deg, 1));
+            const float o1 = DSEL ? acc * sel_factor(nsel) : __fdividef(acc, (float)max(deg, 1));
             const int64_t o = (int64_t)row * a.ldo + ch;
             if (FUSE) {
                 const float o0 = a0 + bw;
@@ -820,7 +837,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
 // Hub rows (in-degree > 1024): one block per row.  Warp w scans chunks w, w + 8, ... with its own top-k list; the 8 lists
 // are merged by ranking their <= 8 top_k entries against each other (positions are unique, so (score, position) is a
 // strict order and the ranks are the final ranks); warp 0 then finishes the row exactly like the long-row kernel.
-template <int G, bool FUSE, bool SELECT_ALL>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArgs a) {
     using S = RowShape<G>;
     constexpr int V = S::V;
@@ -915,13 +932,13 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
                 }
             }
             if (!SELECT_ALL) {
-                finish_list<G>(a, hb, row, fin_s, fin_p, cnt, lane, sacc);
+                finish_list<G, DSEL>(a, hb, row, fin_s, fin_p, cnt, lane, sacc);
 #pragma unroll
                 for (int s = 0; s < V; ++s) cross_group_sum4<G>(sacc[s]);
             }
 #pragma unroll
             for (int s = 0; s < V; ++s)
-                if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), sacc[s], sa0[s], end - beg, beta, bw[s], bb[s]);
+                if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), sacc[s], sa0[s], DSEL ? cnt : end - beg, beta, bw[s], bb[s]);
         }
         __syncthreads();
     }
@@ -1097,12 +1114,14 @@ __global__ void __launch_bounds__(kThreads) norm_bwd_finish_kernel(const float* 
 // every source row j of n_total and writes dh_j = this shard's contribution; dnT_j exists only for the rows it owns.
 // Neighbour lists (sng_list_bwd): the saved lists are fixed-width kNN lists, inv_denom[i] replaces 1 / deg_i (the pass-T
 // kernels then never read rowptr), and the by-source CSR is their transpose (sng_list_transpose, src_shift 0).
+// Edges under denominator='selected' (sng_edge_bwd_denom): the same inv_denom, the factor the forward applied per row.  Selection
+// carries no gradient, so it is a per-row constant and the closed form holds with 1 / deg_i replaced by it.
 struct EdgeBwdArgs {
     const float* h; const float* inv_r; const float* g;
     int n_total, n, row_offset, c, ld, ldg;
     const int* rowptr; const int* col; const int* tpos;
     int top_k; const int* sel_src; const float* sel_w; const int* sel_q; const int* sel_cnt;
-    const float* inv_denom;                  // NULL: 1 / max(deg_i, 1) from rowptr (edges); else per target row (lists)
+    const float* inv_denom;                  // NULL: 1 / max(deg_i, 1) from rowptr (edges); else per target row (lists, 'selected')
     const float* beta; const float* diff; int lddiff; float* dbeta_part;
     float2* coef; float* dnT;
     const int* rowptr_out; const int* col_out; int shift;
@@ -1117,8 +1136,8 @@ struct EdgeBwdArgs {
 // source row j is one of the call's target rows: pass T wrote its target-side dn at dnT[j - row_offset]
 __device__ __forceinline__ bool owns_row(const EdgeBwdArgs& a, int j) { return (unsigned)(j - a.row_offset) < (unsigned)a.n; }
 
-// LIST: the saved lists are neighbour lists with a.inv_denom (a template flag: a runtime branch costs the edge instances at
-// C = 32 / 64 an 8-byte spill)
+// LIST: the saved lists come with a.inv_denom -- neighbour lists, or edges under denominator='selected' (a template flag: a
+// runtime branch costs the edge instances at C = 32 / 64 an 8-byte spill)
 template <int G, bool SELECT_ALL, bool LIST = false>
 __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwdArgs a) {
     using S = RowShape<G>;
@@ -2019,7 +2038,7 @@ static size_t hub_smem(int top_k) {
 static int forward_slots(bool fuse) {
     return fuse ? 66 : 40;                  // measured (pokec shape, C = 32): smaller pools win -- occupancy beats prefetch depth
 }
-template <int G, bool FUSE, bool SELECT_ALL>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL>
 static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hub, cudaStream_t st) {
     const size_t ls = long_smem(a.top_k), hs = hub_smem<G>(a.top_k);
     if constexpr (G <= 8) {
@@ -2030,15 +2049,15 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
             const size_t ss = (size_t)kStWarps * a.slots * staged_row_bytes<G>();
             if constexpr (G == 1) {
                 // 16-byte rows: everything in registers (edge_fwd_narrow_kernel); the chunk pass of the long rows stays staged
-                edge_fwd_narrow_kernel<FUSE, SELECT_ALL><<<grid_resident(edge_fwd_narrow_kernel<FUSE, SELECT_ALL>, a.n, kWarpsPerBlock), kThreads, 0, st>>>(a);
+                edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL>, a.n, kWarpsPerBlock), kThreads, 0, st>>>(a);
             } else {
-                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
-                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false>, a.n, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
+                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
+                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL>, a.n, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
             }
             if (a.n_chunks > 0) {
                 cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
                 edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true>, a.n_chunks, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
-                edge_fwd_merge_kernel<G, FUSE, SELECT_ALL><<<grid_resident(edge_fwd_merge_kernel<G, FUSE, SELECT_ALL>, a.n_lrows, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
+                edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL>, a.n_lrows, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
             }
             return;
         }
@@ -2046,10 +2065,10 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
     // wide rows (C > 32) or no degree lists: the chunked kernel runs every row; listed hubs still get their block kernel
     a.rows = nullptr; a.n_rows = 0;
     a.skip_deg = n_hub > 0 ? 1024 : 0;
-    edge_fwd_long_kernel<G, FUSE, SELECT_ALL><<<grid_resident(edge_fwd_long_kernel<G, FUSE, SELECT_ALL>, a.n, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
+    edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL>, a.n, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
     if (a.skip_deg) {
         a.rows = rows_hub; a.n_rows = (int)n_hub; a.skip_deg = 0;
-        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL><<<grid_capped(n_hub, 1, 4), kThreads, hs, st>>>(a);
+        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_capped(n_hub, 1, 4), kThreads, hs, st>>>(a);
     }
 }
 }  // namespace sng
@@ -2060,15 +2079,17 @@ extern "C" size_t sng_edge_fwd_workspace_bytes(int64_t n_chunks, int64_t c, int 
     return (size_t)n_chunks * (size_t)(2 * kk + 1 + 2 * cg) * 4 + 1024;
 }
 
-extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
-                            const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
-                            const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
-                            const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
-                            int top_k, float thr, float* out, int64_t ldo,
-                            int32_t* sel_src, float* sel_w, int32_t* sel_q, int32_t* sel_cnt, float* inv_norm, int inv_norm_ready,
-                            const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
-                            void* stream) {
+extern "C" int sng_edge_fwd_denom(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
+                                  const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                                  const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                                  const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
+                                  int top_k, float thr, float* out, int64_t ldo,
+                                  int32_t* sel_src, float* sel_w, int32_t* sel_q, int32_t* sel_cnt, float* inv_norm, int inv_norm_ready,
+                                  const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
+                                  int denominator, float* inv_denom, void* stream) {
     if (int rc = check_rows("sng_edge_fwd", n, c, ldh)) return rc;
+    SNG_REQUIRE(denominator == 0 || (denominator == 1 && top_k > 0), "sng_edge_fwd: denominator=%d must be 0 (candidates) or 1 (selected, needs top_k > 0)", denominator);
+    SNG_REQUIRE(!inv_denom || denominator == 1, "sng_edge_fwd: inv_denom is an output of denominator=1 (selected)");
     SNG_REQUIRE(h && rowptr && ((col && out) || n == 0) && ldo % 4 == 0 && ldo >= c, "sng_edge_fwd: null pointer or bad ldo");   // (an empty shard has no edges, no rows)
     SNG_REQUIRE(row_offset >= 0 && row_offset + n <= n_total && n_total < (1ll << 31) && ldh < (1ll << 31) && ldo < (1ll << 31),
                 "sng_edge_fwd: bad row_offset / n_total");
@@ -2094,6 +2115,7 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
     a.h = h; a.inv_r = inv_norm; a.n = (int)n; a.row_offset = (int)row_offset; a.c = (int)c; a.ldh = (int)ldh;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.rows = nullptr; a.n_rows = 0; a.skip_deg = 0;
     a.top_k = top_k > 0 ? top_k : 0; a.thr = thr; a.out = out; a.ldo = (int)ldo;
+    a.inv_denom = inv_denom;
     a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt;
     a.wt = wt; a.ldw = (int)ldw; a.b_w = b_w; a.beta = beta; a.bias = bias; a.diff = diff;
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab); a.n_chunks = staged ? (int)n_chunks : -1;
@@ -2109,11 +2131,26 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
         a.tmp_a0 = w;
     }
     SNG_DISPATCH_G(c,
-        if (wt) { if (top_k > 0) launch_edge_fwd<G, true, false>(a, rows_hub, n_hub, st);
-                  else launch_edge_fwd<G, true, true>(a, rows_hub, n_hub, st); }
-        else { if (top_k > 0) launch_edge_fwd<G, false, false>(a, rows_hub, n_hub, st);
-               else launch_edge_fwd<G, false, true>(a, rows_hub, n_hub, st); });
+        if (wt) { if (top_k <= 0) launch_edge_fwd<G, true, true, false>(a, rows_hub, n_hub, st);
+                  else if (denominator) launch_edge_fwd<G, true, false, true>(a, rows_hub, n_hub, st);
+                  else launch_edge_fwd<G, true, false, false>(a, rows_hub, n_hub, st); }
+        else { if (top_k <= 0) launch_edge_fwd<G, false, true, false>(a, rows_hub, n_hub, st);
+               else if (denominator) launch_edge_fwd<G, false, false, true>(a, rows_hub, n_hub, st);
+               else launch_edge_fwd<G, false, false, false>(a, rows_hub, n_hub, st); });
     return check_launch("sng_edge_fwd");
+}
+
+extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
+                            const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                            const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                            const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
+                            int top_k, float thr, float* out, int64_t ldo,
+                            int32_t* sel_src, float* sel_w, int32_t* sel_q, int32_t* sel_cnt, float* inv_norm, int inv_norm_ready,
+                            const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
+                            void* stream) {
+    return sng_edge_fwd_denom(h, n_total, n, row_offset, c, ldh, rowptr, col, tpos, chunk_tab, n_chunks, lrows, lrow_ptr, n_lrows,
+                              rows_hub, n_hub, workspace, workspace_bytes, top_k, thr, out, ldo, sel_src, sel_w, sel_q, sel_cnt,
+                              inv_norm, inv_norm_ready, wt, ldw, b_w, beta, bias, diff, 0, nullptr, stream);
 }
 
 namespace sng {
@@ -2180,16 +2217,17 @@ static int launch_edge_bwd(const EdgeBwdArgs& a, float* dbeta, cudaStream_t st, 
 }
 }  // namespace sng
 
-extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
-                            int64_t c, int64_t ld, int64_t ldg,
-                            const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
-                            const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
-                            int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
-                            const float* beta, const float* diff, int64_t lddiff, float* dbeta,
-                            float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
-                            const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
-                            int64_t n_lrows_out, float* chunk_partials, void* stream) {
+extern "C" int sng_edge_bwd_denom(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                                  int64_t c, int64_t ld, int64_t ldg,
+                                  const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                                  const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
+                                  int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
+                                  const float* beta, const float* diff, int64_t lddiff, float* dbeta,
+                                  float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
+                                  const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
+                                  int64_t n_lrows_out, float* chunk_partials, const float* inv_denom, void* stream) {
     if (int rc = check_rows("sng_edge_bwd", n_total, c, ld)) return rc;
+    SNG_REQUIRE(!inv_denom || top_k > 0, "sng_edge_bwd: inv_denom (denominator='selected') needs the selection lists (top_k > 0)");
     SNG_REQUIRE(n >= 0 && row_offset >= 0 && row_offset + n <= n_total, "sng_edge_bwd: bad n / row_offset / n_total");
     // (an empty shard, n == 0, has no rows of g / dn_target / the lists, and possibly no edges: those may be NULL)
     SNG_REQUIRE(h && inv_norm && rowptr && rowptr_out && (col_out || num_edges == 0) && coef && dh && ldg % 4 == 0 && ldg >= c &&
@@ -2210,7 +2248,7 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
     a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n_total; a.n = (int)n; a.row_offset = (int)row_offset;
     a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
     a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.top_k = top_k > 0 ? top_k : 0;
-    a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt; a.inv_denom = nullptr;
+    a.sel_src = sel_src; a.sel_w = sel_w; a.sel_q = sel_q; a.sel_cnt = sel_cnt; a.inv_denom = inv_denom;
     a.beta = beta; a.diff = dbeta ? diff : nullptr; a.lddiff = (int)lddiff; a.dbeta_part = dbeta ? partials : nullptr;
     a.coef = reinterpret_cast<float2*>(coef); a.dnT = dn_target;
     a.rowptr_out = rowptr_out; a.col_out = col_out; a.shift = (int)src_shift;
@@ -2218,6 +2256,21 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab_out); a.n_chunks = (int)n_chunks_out; a.lrows = lrows_out; a.lrow_ptr = lrow_ptr_out;
     a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials;
     return launch_edge_bwd(a, dbeta, st, "sng_edge_bwd");
+}
+
+extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                            int64_t c, int64_t ld, int64_t ldg,
+                            const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                            const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
+                            int top_k, const int32_t* sel_src, const float* sel_w, const int32_t* sel_q, const int32_t* sel_cnt,
+                            const float* beta, const float* diff, int64_t lddiff, float* dbeta,
+                            float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
+                            const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
+                            int64_t n_lrows_out, float* chunk_partials, void* stream) {
+    return sng_edge_bwd_denom(h, inv_norm, g, n_total, n, row_offset, c, ld, ldg, rowptr, col, tpos, rowptr_out, col_out, src_shift,
+                              num_edges, top_k, sel_src, sel_w, sel_q, sel_cnt, beta, diff, lddiff, dbeta, coef, dn_target, partials,
+                              dh, dwt, lddw, chunk_tab_out, n_chunks_out, lrows_out, lrow_ptr_out, n_lrows_out, chunk_partials,
+                              nullptr, stream);
 }
 
 extern "C" int sng_list_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,

@@ -94,9 +94,15 @@ def _check_h(h):
     return h.contiguous()
 
 
-def _edge_fwd(h_all, graph, row_offset, k, thr, train, fuse=None, want_q=False, inv_norm=None):
-    """sng_edge_fwd on the target rows of `graph` (a PreparedGraph or a row shard of one).  fuse = (wt [N, Cp], b_w [Cp],
-    beta [1], bias [Cp] | None) gathers the structural term and blends in the same pass (symmetric graphs only)."""
+_DENOMINATORS = {"candidates": 0, "selected": 1}
+
+
+def _edge_fwd(h_all, graph, row_offset, k, thr, train, fuse=None, want_q=False, inv_norm=None, denominator="candidates",
+              inv_denom=None):
+    """sng_edge_fwd_denom on the target rows of `graph` (a PreparedGraph or a row shard of one).  fuse = (wt [N, Cp], b_w [Cp],
+    beta [1], bias [Cp] | None) gathers the structural term and blends in the same pass (symmetric graphs only).
+    denominator='selected' divides each row by its selected count instead of its in-degree; inv_denom [graph.n] (optional)
+    then receives the factor each row was scaled by, the input of edge_bwd in that mode."""
     c = h_all.size(1)
     n = graph.n
     dev = h_all.device
@@ -123,11 +129,12 @@ def _edge_fwd(h_all, graph, row_offset, k, thr, train, fuse=None, want_q=False, 
         ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
     n_lrows = 0 if tab is None else int(graph.lrows.numel())
     n_hub = 0 if graph.rows_hub is None else int(graph.rows_hub.numel())
-    _C.call("sng_edge_fwd", h_all, _C.ptr(h_all), h_all.size(0), n, row_offset, c, c, _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
+    _C.call("sng_edge_fwd_denom", h_all, _C.ptr(h_all), h_all.size(0), n, row_offset, c, c, _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
             _C.ptr(graph.tpos if want_q else None), _C.ptr(tab), n_chunks, _C.ptr(graph.lrows), _C.ptr(graph.lrow_ptr), n_lrows,
             _C.ptr(graph.rows_hub), n_hub, _C.ptr(ws), wbytes, k,
             float(thr if thr is not None else 0.0), _C.ptr(out), c, _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_q), _C.ptr(sel_cnt),
-            _C.ptr(inv_norm), int(inv_ready), _C.ptr(wt), c, _C.ptr(bw), _C.ptr(beta), _C.ptr(bias), _C.ptr(diff))
+            _C.ptr(inv_norm), int(inv_ready), _C.ptr(wt), c, _C.ptr(bw), _C.ptr(beta), _C.ptr(bias), _C.ptr(diff),
+            _DENOMINATORS[denominator], _C.ptr(inv_denom))
     return out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff
 
 
@@ -158,10 +165,11 @@ class EdgeAgg(torch.autograd.Function):
     """The similarity-navigated aggregation of one layer: out_1 of R: models/models.py:132 / :239 / :326 and -- when the
     structural parameters are given and the graph's in-lists equal its out-lists -- the whole of
     R: models/models.py:124-136 (out = beta (A W^T + b_w) + (1 - beta) out_1 + bias) in the same pass over the edges.
-    Forward sng_edge_fwd, backward sng_edge_bwd (two gather passes, no float atomics, bit-reproducible)."""
+    Forward sng_edge_fwd, backward sng_edge_bwd (two gather passes, no float atomics, bit-reproducible).  With
+    denominator='selected' out_1 divides by each row's selected count; the backward reuses the forward's per-row factors."""
 
     @staticmethod
-    def forward(ctx, h, graph, top_k, thr, w_weight, w_bias, beta, bias, inv_norm=None):
+    def forward(ctx, h, graph, top_k, thr, w_weight, w_bias, beta, bias, inv_norm=None, denominator="candidates"):
         h = _check_h(h)
         n, cp = h.shape
         if n != graph.n:
@@ -180,31 +188,35 @@ class EdgeAgg(torch.autograd.Function):
                 raise RuntimeError("the fused SNGNN++ pass needs a graph whose in-lists equal its out-lists")
             fuse = _structural_operands(w_weight, w_bias, beta, bias, cp)
             ctx.c = c
-        out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = _edge_fwd(h, graph, 0, k, thr, train, fuse, want_q=True, inv_norm=inv_norm)
+        inv_denom = torch.empty(n, dtype=torch.float32, device=h.device) if train and k > 0 and denominator == "selected" else None
+        out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = _edge_fwd(h, graph, 0, k, thr, train, fuse, want_q=True, inv_norm=inv_norm,
+                                                                        denominator=denominator, inv_denom=inv_denom)
         ctx.graph, ctx.k, ctx.fused, ctx.has_bias = graph, k, fused, bias is not None
         if record_selection is not None and sel_cnt is not None:
             record_selection.append((sel_src, sel_cnt))
-        ctx.save_for_backward(h, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta if fused else None)
+        ctx.save_for_backward(h, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta if fused else None, inv_denom)
         if sel_cnt is not None:
             ctx.mark_non_differentiable(sel_src, sel_w, sel_cnt)
         return out, sel_src, sel_w, sel_cnt
 
     @staticmethod
     def backward(ctx, g, *_):
-        h, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
+        h, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta, inv_denom = ctx.saved_tensors
         graph, k, fused = ctx.graph, ctx.k, ctx.fused
         g = g.contiguous()
-        dh, dwt, dbeta = edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta if fused else None, diff)
+        dh, dwt, dbeta = edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta if fused else None, diff,
+                                  inv_denom=inv_denom)
         if not fused:
-            return dh, None, None, None, None, None, None, None, None
+            return dh, None, None, None, None, None, None, None, None, None
         c = ctx.c
         gsum = g.sum(0)[:c]
-        return dh, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None
+        return dh, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None, None
 
 
-def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None, *, row_offset=0):
-    """sng_edge_bwd: dL/dh [N, Cp] of the aggregation -- two gather passes, no float atomics -- and, with `beta` (the fused
-    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout.
+def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None, *, row_offset=0, inv_denom=None):
+    """sng_edge_bwd_denom: dL/dh [N, Cp] of the aggregation -- two gather passes, no float atomics -- and, with `beta` (the fused
+    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout.  inv_denom = the per-row factors _edge_fwd wrote under
+    denominator='selected' (None: 1 / max(in-degree, 1)).
     Row shard (`graph` = PreparedGraph.row_slice(lo, hi), row_offset = lo, `h` / `inv_norm` of all N nodes, `g` / `diff` / the
     lists of the shard's rows): dh is the shard's contribution to dL/dh of every node and dbeta its part of dL/dbeta, both
     bit-reproducible; dL/dW^T is not computed (None): the caller assembles it from the g0 of every shard."""
@@ -229,13 +241,14 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
         while cg < cp:
             cg *= 2
         cpart = torch.empty(n_chunks * 3 * cg, dtype=torch.float32, device=dev)
-    _C.call("sng_edge_bwd", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
+    _C.call("sng_edge_bwd_denom", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
             _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
             _C.ptr(graph.tpos), _C.ptr(graph.rowptr_tr), _C.ptr(graph.col_tr), graph.src_shift, graph.num_edges, k,
             _C.ptr(sel_src), _C.ptr(sel_w), _C.ptr(sel_q), _C.ptr(sel_cnt), _C.ptr(beta), _C.ptr(diff if fused else None), cp,
             _C.ptr(dbeta), _C.ptr(coef), _C.ptr(dnt), _C.ptr(part), _C.ptr(dh), _C.ptr(dwt), cp,
             _C.ptr(tab), n_chunks, _C.ptr(graph.lrows_out if tab is not None else None),
-            _C.ptr(graph.lrow_ptr_out if tab is not None else None), 0 if tab is None else int(graph.lrows_out.numel()), _C.ptr(cpart))
+            _C.ptr(graph.lrow_ptr_out if tab is not None else None), 0 if tab is None else int(graph.lrows_out.numel()), _C.ptr(cpart),
+            _C.ptr(inv_denom))
     return dh, dwt, dbeta
 
 
@@ -282,11 +295,13 @@ class ShardedEdgeTopkAgg(torch.autograd.Function):
         return dh, None, None, None, None
 
 
-def edge_topk_agg(h, graph, top_k=None, thr=None, return_selection=False, structural=None, inv_norm=None):
+def edge_topk_agg(h, graph, top_k=None, thr=None, return_selection=False, structural=None, inv_norm=None, denominator="candidates"):
     """out_1 (structural=None) or the fused SNGNN++ layer output (structural = (w.weight, w.bias, beta, bias)).
-    inv_norm = 1 / max(||h_i||, 1e-12) when the caller already has it (lin_norm), else it is computed here."""
+    inv_norm = 1 / max(||h_i||, 1e-12) when the caller already has it (lin_norm), else it is computed here.
+    denominator = 'candidates' (mean over the in-degree, PyG aggr='mean') | 'selected' (mean over the selected neighbours;
+    needs top_k > 0)."""
     w_weight, w_bias, beta, bias = structural if structural is not None else (None, None, None, None)
-    out, sel_src, sel_w, sel_cnt = EdgeAgg.apply(h, graph, top_k, thr, w_weight, w_bias, beta, bias, inv_norm)
+    out, sel_src, sel_w, sel_cnt = EdgeAgg.apply(h, graph, top_k, thr, w_weight, w_bias, beta, bias, inv_norm, denominator)
     if return_selection:
         return out, (sel_src, sel_w, sel_cnt)
     return out

@@ -111,14 +111,7 @@ class SNConv_plus(_SNConvBase):
         if self.top_k <= 0:
             return h * 0.0
         if self.candidates == "edges":
-            if self.denominator == "selected":
-                h = h if h.requires_grad else h.detach().requires_grad_(torch.is_grad_enabled())   # the lists are only emitted in training mode
-                out1, (_, _, sel_cnt) = SF.edge_topk_agg(h, g, self.top_k, self.thr, return_selection=True, inv_norm=inv)
-                if sel_cnt is None:
-                    raise RuntimeError("denominator='selected' needs grad mode (the selection lists are not emitted in inference)")
-                scale = (sel_cnt.clamp(min=1).float() * g.inv_deg).reciprocal()      # deg / max(cnt,1)
-                return out1 * scale[:, None]
-            return SF.edge_topk_agg(h, g, self.top_k, self.thr, inv_norm=inv)
+            return SF.edge_topk_agg(h, g, self.top_k, self.thr, inv_norm=inv, denominator=self.denominator)
         from . import simknn
         return simknn.allpairs_topk_agg(h, self.top_k, self.thr, bool(self.is_remove_self_loops), self.denominator)
 
@@ -168,9 +161,10 @@ class SNConv_plus_plus(SNConv_plus):
         self._check_options()
         g = G.prepare(edge_index, x.size(0), remove_self_loops=bool(self.is_remove_self_loops))
         h, inv = self._hidden_norm(x)
-        if self.top_k > 0 and self.candidates == "edges" and self.denominator == "candidates" and g.symmetric:
+        if self.top_k > 0 and self.candidates == "edges" and g.symmetric:
             # in-lists == out-lists: the structural term rides on the aggregation's own pass over the edges (one kernel)
-            out = SF.edge_topk_agg(h, g, self.top_k, self.thr, structural=(self.w.weight, self.w.bias, self.beta, self.bias), inv_norm=inv)
+            out = SF.edge_topk_agg(h, g, self.top_k, self.thr, structural=(self.w.weight, self.w.bias, self.beta, self.bias), inv_norm=inv,
+                                   denominator=self.denominator)
         else:
             out = SF.PPFuse.apply(self._aggregate(h, g, inv), self.w.weight, self.w.bias, self.beta, self.bias, g)
         return out[:, :self.lin.out_features]
