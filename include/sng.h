@@ -246,6 +246,31 @@ SNG_API int sng_nll_loss_bwd(int64_t n, int64_t c, int64_t ld, const int64_t* y,
                      void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * ReLU + BatchNorm1d over the rows of a shard (R: models/models.py:81-84 `x = F.relu(conv(x)); x = self.bns[i](x)`), with the
+ * batch statistics taken over all n_total rows of every shard: each rank computes its shard's sums, the caller all-reduces the
+ * FP64 [2, c] sums, every rank applies.  z [n, ldz] = the conv output (pre-activation), a = max(z, 0); 1 <= c <= SNG_MAX_CHANNELS.
+ * Sums are FP64 with per-CTA partials added in a fixed order (no atomics): bit-reproducible on a given device.  An empty shard
+ * (n = 0) writes zero sums.  workspace >= sng_bn_workspace_bytes(n, c) (0 = c rejected).
+ *   sng_bn_fwd_stats: sums [2, c] = (sum_i a_i, sum_i a_i^2) over this shard.
+ *   sng_bn_fwd_apply: y [n, ldy] = gamma (a - mu) rstd + beta.  sums != NULL (training): the global sums over n_total rows give
+ *     mu = S1 / N and rstd = 1 / sqrt(S2 / N - mu^2 + eps) (biased variance, as torch normalises), written to mean / rstd [c];
+ *     sums == NULL (eval): mean / rstd are INPUTS (running_mean, 1 / sqrt(running_var + eps)); n_total and eps are unused.
+ *   sng_bn_bwd_stats: sums [2, c] = (sum_i g_i, sum_i g_i ahat_i) over this shard, ahat = (a - mean) rstd recomputed from z.
+ *   sng_bn_bwd_apply: dz [n, lddz] = 1[z > 0] gamma rstd (g - S1 / N - ahat S2 / N) with the global backward sums over n_total rows;
+ *     sums == NULL (eval-mode statistics, constants): dz = 1[z > 0] gamma rstd g.
+ *   The global backward sums are also dL/dbeta (S1) and dL/dgamma (S2).
+ */
+SNG_API size_t sng_bn_workspace_bytes(int64_t n, int64_t c);
+SNG_API int sng_bn_fwd_stats(const float* z, int64_t n, int64_t c, int64_t ldz, double* sums, void* workspace, size_t workspace_bytes,
+                     void* stream);
+SNG_API int sng_bn_fwd_apply(const float* z, int64_t n, int64_t c, int64_t ldz, const double* sums, int64_t n_total, double eps,
+                     const float* gamma, const float* beta, float* mean, float* rstd, float* y, int64_t ldy, void* stream);
+SNG_API int sng_bn_bwd_stats(const float* z, const float* g, int64_t n, int64_t c, int64_t ldz, int64_t ldg, const float* mean,
+                     const float* rstd, double* sums, void* workspace, size_t workspace_bytes, void* stream);
+SNG_API int sng_bn_bwd_apply(const float* z, const float* g, int64_t n, int64_t c, int64_t ldz, int64_t ldg, const double* sums,
+                     int64_t n_total, const float* gamma, const float* mean, const float* rstd, float* dz, int64_t lddz, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * lin + bias + 1/norm in one pass (SURVEY.md §8(f) 2):  h [n, cp] = x W^T + b with cp = 4 * ceil(c / 4) zero-padded channels,
  * inv_norm[i] = 1 / max(||h_i||, 1e-12).  replaces `x = self.lin(x); norm = F.normalize(x)` at R: models/models.py:121-122,
  * 237-238, 324-325 (FP32 FMA; supported when cp is a power of two in [4, 128] and f * cp <= 24576 -- sng_lin_norm_supported --

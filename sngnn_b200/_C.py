@@ -24,6 +24,11 @@ SIGNATURES = {
                             _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _P]),
     "sng_edge_fwd_denom": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P, _P, _I64, _P, _I64, _P, _SZ, _I32, _F32, _P,
                                   _I64, _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _I32, _P, _P]),
+    "sng_bn_workspace_bytes": (_SZ, [_I64, _I64]),
+    "sng_bn_fwd_stats": (_I32, [_P, _I64, _I64, _I64, _P, _P, _SZ, _P]),
+    "sng_bn_fwd_apply": (_I32, [_P, _I64, _I64, _I64, _P, _I64, ctypes.c_double, _P, _P, _P, _P, _P, _I64, _P]),
+    "sng_bn_bwd_stats": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _SZ, _P]),
+    "sng_bn_bwd_apply": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _P, _I64, _P, _P, _P, _P, _I64, _P]),
     "sng_lin_norm_supported": (_I32, [_I64, _I64]),
     "sng_lin_norm_fwd": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _P, _P, _P, _P]),
     "sng_lin_bwd_supported": (_I32, [_I64, _I64]),

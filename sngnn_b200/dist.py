@@ -246,6 +246,68 @@ class _ShardedFusedAgg(torch.autograd.Function):
         return dh, dw, g0.sum(0)[:c], dbeta, dbias, None, None, None, None, None
 
 
+def _all_reduce_sums(sums):
+    ws, _ = world()
+    if ws > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM)
+    return sums
+
+
+def _update_running_stats(bn, sums, n):
+    """running_mean / running_var (unbiased: N / (N - 1)) / num_batches_tracked, as nn.BatchNorm1d updates them in training,
+    from the global FP64 sums (identical on every rank, so the buffers are too)."""
+    bn.num_batches_tracked.add_(1)
+    f = 1.0 / float(bn.num_batches_tracked) if bn.momentum is None else bn.momentum
+    mean = sums[0] / n
+    var = (sums[1] / n - mean * mean).clamp_min(0.0) * (n / (n - 1))
+    bn.running_mean.mul_(1.0 - f).add_(mean.to(bn.running_mean.dtype), alpha=f)
+    bn.running_var.mul_(1.0 - f).add_(var.to(bn.running_var.dtype), alpha=f)
+
+
+class _ShardedBatchNorm(torch.autograd.Function):
+    """y = bn(relu(z)) on a row shard with the batch statistics of all n rows (R: models/models.py:81-84).  Forward: the shard's
+    FP64 sums, ONE all-reduce of the [2, C] sums, apply; backward: the same with (sum g, sum g ahat), which are also the complete
+    dL/dbeta and dL/dgamma on every rank (the caller marks both parameters `_sng_grad_complete`).  Eval mode: the running
+    statistics, no collective in the forward.  `ops` = the four launch helpers of functional.py (or the tests' CPU stand-ins)."""
+
+    @staticmethod
+    def forward(ctx, z, weight, bias, bn, n, ops):
+        if bn.training:
+            sums = _all_reduce_sums(ops.bn_fwd_stats(z))
+            y, mean, rstd = ops.bn_fwd_apply(z, sums, n, bn.eps, weight, bias)
+            _update_running_stats(bn, sums, n)
+        else:
+            mean, rstd = bn.running_mean.clone(), torch.rsqrt(bn.running_var + bn.eps)
+            y, mean, rstd = ops.bn_fwd_apply(z, None, n, bn.eps, weight, bias, mean, rstd)
+        ctx.n, ctx.training, ctx.ops = n, bn.training, ops
+        ctx.save_for_backward(z, weight, mean, rstd)
+        return y
+
+    @staticmethod
+    def backward(ctx, g):
+        z, weight, mean, rstd = ctx.saved_tensors
+        sums = _all_reduce_sums(ctx.ops.bn_bwd_stats(z, g, mean, rstd))
+        dz = ctx.ops.bn_bwd_apply(z, g, sums if ctx.training else None, ctx.n, weight, mean, rstd)
+        return dz, sums[1].to(weight.dtype), sums[0].to(weight.dtype), None, None, None
+
+
+def _check_batch_norm(bn, n):
+    if not (bn.affine and bn.track_running_stats):
+        raise NotImplementedError("sharded_forward: BatchNorm needs affine=True and track_running_stats=True (what the models build)")
+    if bn.training and n <= 1:
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size {torch.Size([n, bn.num_features])}")
+
+
+def sharded_batch_norm(z, bn, n, ops=None):
+    """bn(relu(z)) for this rank's rows z [hi - lo, C] of an n-row batch, `bn` an nn.BatchNorm1d replicated on every rank: in
+    training the statistics span all n rows (one all-reduce each way) and the running buffers come out identical on every rank.
+    `ops` defaults to functional's CUDA helpers (bn_fwd_stats / bn_fwd_apply / bn_bwd_stats / bn_bwd_apply)."""
+    _check_batch_norm(bn, n)
+    bn.weight._sng_grad_complete = True                   # the backward returns the global sums: allreduce_grads skips them
+    bn.bias._sng_grad_complete = True
+    return _ShardedBatchNorm.apply(z, bn.weight, bn.bias, bn, n, SF if ops is None else ops)
+
+
 def allreduce_grads(params):
     """Sum the (partial, per-shard) parameter gradients over ranks: every parameter is replicated, every rank holds the
     gradient contribution of its own rows.  Structural weights whose gradient the sharded backward already assembled on
@@ -258,37 +320,51 @@ def allreduce_grads(params):
             dist.all_reduce(p.grad, op=dist.ReduceOp.SUM)
 
 
-def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
+def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None, bn_ops=None):
     """Row-sharded forward of an SNGNN / SNGNN_Plus / SNGNN_Plus_Plus model (replicated parameters): this rank holds the
     feature rows [lo, hi) and returns the log-probabilities of those rows.  Mirrors _SNStack.forward / the conv forwards of
     models.py (R: models/models.py:76-86,116-137,233-242,322-329) with the aggregation and the ++ fusion replaced by their
-    sharded forms.  BatchNorm needs statistics over all nodes and is not supported here (the reference default is bn=False);
-    neither is denominator='selected' with candidates='edges'.
+    sharded forms.  denominator='selected' with candidates='edges' is not supported here.
     candidates='all_pairs' (either denominator): h is all-gathered, the rank builds the kNN lists of its own rows over every
     node (simknn.allpairs_topk_agg with rows = [lo, hi)) and aggregates them; the SNGNN++ structural term goes through
-    pp_fuse_sharded."""
+    pp_fuse_sharded.
+    top_k <= 0: out_1 = 0 on the local rows (the reference runs no selection round), with zero gradients; SNGNN++ still adds
+    its structural term through pp_fuse_sharded.
+    bn=True: relu + BatchNorm of the hidden layers run as sharded_batch_norm, with the statistics of all n rows (training) or
+    the running statistics (eval); `bn_ops` replaces its four CUDA helpers (the tests inject CPU stand-ins)."""
     import torch.nn.functional as F
     from . import graph as G, models as M, simknn
-    if getattr(model, "bn", False):
-        raise NotImplementedError("sharded_forward: bn=True needs cross-rank batch statistics")
+    convs = list(model.lins)
+    for conv in convs:                                       # reject unsupported options before any collective or kernel
+        if type(conv) is not M.SNConv and conv.candidates != "all_pairs" and conv.denominator != "candidates":
+            raise NotImplementedError("sharded_forward: candidates='edges' with denominator='selected'")
+    use_bn = getattr(model, "bn", False)
+    if use_bn:
+        for bn in model.bns:
+            _check_batch_norm(bn, n)
     ws, rank = world()
     lo, hi = shard_bounds(n, ws, rank)
     x = x_local
-    convs = list(model.lins)
     for i, conv in enumerate(convs):
         base = type(conv) is M.SNConv
         plus_plus = isinstance(conv, M.SNConv_plus_plus)
         all_pairs = not base and conv.candidates == "all_pairs"
-        if not base and not all_pairs and conv.denominator != "candidates":
-            raise NotImplementedError("sharded_forward: candidates='edges' with denominator='selected'")
-        if not base and conv.top_k <= 0:
-            raise NotImplementedError("sharded_forward: top_k <= 0")
+        no_select = not base and conv.top_k <= 0
         g = G.prepare(edge_index, n, remove_self_loops=False if base else bool(conv.is_remove_self_loops))
         h = conv._hidden_norm(x)[0]                          # lin + bias in the library's kernel (its backward is the one-pass dW / db)
         injected = agg is not None or fuse is not None
         if plus_plus:
             conv.w.weight._sng_grad_complete = not injected      # the CUDA backward assembles the complete gradient itself
-        if plus_plus and not all_pairs and not injected and g.symmetric:
+        if no_select:
+            out = h * 0.0                                    # SNConv_plus._aggregate: zero out_1, zero (not missing) gradients
+            if plus_plus:
+                out = pp_fuse_sharded(out, conv.w.weight, conv.w.bias, conv.beta, conv.bias, g.row_slice(lo, hi), n, lo, fuse=fuse)
+                out = out[:, :conv.lin.out_features]
+            else:
+                out = out[:, :conv.lin.out_features]
+                if conv.bias is not None:
+                    out = out + conv.bias
+        elif plus_plus and not all_pairs and not injected and g.symmetric:
             h_all = AllGatherRows.apply(h, n)
             out = _ShardedFusedAgg.apply(h_all, conv.w.weight, conv.w.bias, conv.beta, conv.bias, g.row_slice(lo, hi), n, lo,
                                          conv.top_k, conv.thr)
@@ -309,6 +385,7 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None):
                 if conv.bias is not None:
                     out = out + conv.bias
         if i < len(convs) - 1:
-            out = model.dropout(F.relu(out))
+            out = sharded_batch_norm(out, model.bns[i], n, bn_ops) if use_bn else F.relu(out)
+            out = model.dropout(out)
         x = out
     return F.log_softmax(x, dim=1)

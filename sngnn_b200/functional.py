@@ -478,6 +478,69 @@ def pp_beta_grad(out0, out1, g):
     return dbeta
 
 
+def _bn_rows(t):
+    """A float32 CUDA [n, c] tensor with unit column stride (a column slice of a padded tensor is fine); else a contiguous copy."""
+    _C.require_cuda(t)
+    if t.dtype != torch.float32 or t.dim() != 2:
+        raise RuntimeError("expected a float32 [N, C] tensor")
+    return t if t.stride(1) == 1 and t.stride(0) >= t.size(1) else t.contiguous()
+
+
+def _bn_workspace(n, c, dev):
+    nb = _C.lib().sng_bn_workspace_bytes(n, c)
+    if nb == 0:
+        raise RuntimeError(f"sng_bn_workspace_bytes rejected c={c} (1 <= c <= {_C.MAX_CHANNELS})")
+    return torch.empty(nb, dtype=torch.uint8, device=dev), nb
+
+
+def bn_fwd_stats(z):
+    """sng_bn_fwd_stats: FP64 [2, C] = (sum of a, sum of a^2) over the rows of z [n, C], a = relu(z); zeros for n = 0."""
+    z = _bn_rows(z)
+    n, c = z.shape
+    sums = torch.empty(2, c, dtype=torch.float64, device=z.device)
+    ws, nb = _bn_workspace(n, c, z.device)
+    _C.call("sng_bn_fwd_stats", z, _C.ptr(z), n, c, max(z.stride(0), c), _C.ptr(sums), _C.ptr(ws), nb)
+    return sums
+
+
+def bn_fwd_apply(z, sums, n_total, eps, gamma, beta, mean=None, rstd=None):
+    """sng_bn_fwd_apply: (y [n, C] = gamma (relu(z) - mean) rstd + beta, mean [C], rstd [C]).  Training: `sums` = the global
+    bn_fwd_stats over n_total rows, mean / rstd are computed (biased variance).  Eval: sums = None, mean / rstd given."""
+    z = _bn_rows(z)
+    n, c = z.shape
+    if sums is None:
+        mean, rstd = mean.float().contiguous(), rstd.float().contiguous()
+    else:
+        mean = torch.empty(c, dtype=torch.float32, device=z.device)
+        rstd = torch.empty(c, dtype=torch.float32, device=z.device)
+    y = torch.empty(n, c, dtype=torch.float32, device=z.device)
+    _C.call("sng_bn_fwd_apply", z, _C.ptr(z), n, c, max(z.stride(0), c), _C.ptr(sums), int(n_total), float(eps),
+            _C.ptr(gamma.detach().contiguous()), _C.ptr(beta.detach().contiguous()), _C.ptr(mean), _C.ptr(rstd), _C.ptr(y), c)
+    return y, mean, rstd
+
+
+def bn_bwd_stats(z, g, mean, rstd):
+    """sng_bn_bwd_stats: FP64 [2, C] = (sum of g, sum of g * ahat) over the rows, ahat = (relu(z) - mean) rstd; zeros for n = 0."""
+    z, g = _bn_rows(z), _bn_rows(g)
+    n, c = z.shape
+    sums = torch.empty(2, c, dtype=torch.float64, device=z.device)
+    ws, nb = _bn_workspace(n, c, z.device)
+    _C.call("sng_bn_bwd_stats", z, _C.ptr(z), _C.ptr(g), n, c, max(z.stride(0), c), max(g.stride(0), c), _C.ptr(mean), _C.ptr(rstd),
+            _C.ptr(sums), _C.ptr(ws), nb)
+    return sums
+
+
+def bn_bwd_apply(z, g, sums, n_total, gamma, mean, rstd):
+    """sng_bn_bwd_apply: dL/dz [n, C] of y = batch_norm(relu(z)) from the global bn_bwd_stats `sums` over n_total rows
+    (sums = None: eval-mode statistics, dz = 1[z > 0] gamma rstd g)."""
+    z, g = _bn_rows(z), _bn_rows(g)
+    n, c = z.shape
+    dz = torch.empty(n, c, dtype=torch.float32, device=z.device)
+    _C.call("sng_bn_bwd_apply", z, _C.ptr(z), _C.ptr(g), n, c, max(z.stride(0), c), max(g.stride(0), c), _C.ptr(sums), int(n_total),
+            _C.ptr(gamma.detach().contiguous()), _C.ptr(mean), _C.ptr(rstd), _C.ptr(dz), c)
+    return dz
+
+
 def rownorm(x, want_f32=True, want_f16=False, f16_ld=None, want_inv=False):
     """K0: F.normalize(x, p=2, dim=-1) (R: models/models.py:122).  Returns (xhat_f32, xhat_f16, inv_norm)."""
     _C.require_cuda(x)
