@@ -43,6 +43,7 @@ extern "C" {
 #define SNG_MAX_CHANNELS 512     /* padded row width c of sng_edge_fwd / _bwd, sng_edge_agg_bwd, sng_list_agg_fwd, sng_spmm_fwd,
                                     sng_pp_fuse_fwd / _bwd; wider rows return SNG_ERR_UNSUPPORTED */
 #define SNG_KNN_MAX_TOPK 64      /* all-pairs builder */
+#define SNG_SIMHIST_MAX_BINS 4096 /* sng_simhist_f16: two 32-bit sub-histograms of this many bins take half of its 64 KiB */
 
 SNG_API int sng_version(void);
 SNG_API const char* sng_last_error(void);
@@ -324,6 +325,16 @@ SNG_API int sng_sddmm_dot(const float* xhat, int64_t n, int64_t d, int64_t ld,
  *   B = [hi | lo | hi] of the FP16 split x-hat = hi + lo the product equals the FP32 one to ~2^-22; and of the
  *   adjacency-as-features metrics (R: SimGFAToolbox/sparse.py:8-41): 0/1 columns are exact in FP16, the accumulators hold
  *   exact common-neighbour counts and the scales apply 1 / (|a_i| |a_j|).
+ * sng_simhist_f16: counts[b] += number of ORDERED pairs i != j (i, j < n) whose score s = sum_k A[i, k] B[j, k] falls in bin b
+ *   of [lo, hi) cut into `bins` equal bins, without the n x n matrix (tcgen05 contraction, binning epilogue).  s is
+ *   clamped to [-1, 1]; bin = floor((s - lo) * bins / (hi - lo)), s == hi goes into the last bin (numpy.histogram), scores
+ *   outside [lo, hi] are not counted.  With A = [hi | hi | lo], B = [hi | lo | hi] of the FP16 split of x-hat (as for
+ *   sng_gemm_nt_f16) this is the distribution of the off-diagonal cosines of R: SimGFAToolbox/dense.py:144-149.  Each
+ *   unordered pair of 128-row tiles is scored once: row tile I pairs with (I + s) mod T, s = 0 .. floor(T / 2), T = ceil(n
+ *   / 128), the pair at s = T / 2 (T even) only for I < T / 2.  Only row tiles [tile_lo, tile_hi) are run (shards, split
+ *   calls; an empty range adds nothing), so the counts of a split add up to those of [0, T).  Integer counting: the result
+ *   is the same bits whatever the split.  counts [bins] uint64 is zeroed by the caller.  Requires 0 < n < 2^31,
+ *   1 <= bins <= SNG_SIMHIST_MAX_BINS, lo < hi finite, lda / ldb % 8 == 0, 16-byte aligned operands.
  * sng_sparse_col_cos: the same cosine between two COLUMNS of a CSC matrix (sorted, duplicate-free indices) at given column
  *   pairs, by merging the two index lists -- the edge metrics of R: SimGFAToolbox/sparse.py:44-119 without densifying.
  * sng_class_sums_f64: sums[c, :] += sum_{i: y[i]==c} xhat[i, :] and counts[c] += |class c| (both zero-initialised,
@@ -332,6 +343,8 @@ SNG_API int sng_sddmm_dot(const float* xhat, int64_t n, int64_t d, int64_t ld,
  */
 SNG_API int sng_gemm_nt_f16(const uint16_t* a, int64_t lda, const uint16_t* b, int64_t ldb, int64_t m, int64_t n, int64_t k,
                     const float* row_scale, const float* col_scale, float* out, int64_t ldo, void* stream);
+SNG_API int sng_simhist_f16(const uint16_t* a, int64_t lda, const uint16_t* b, int64_t ldb, int64_t n, int64_t k, int64_t tile_lo,
+                    int64_t tile_hi, float lo, float hi, int bins, uint64_t* counts, void* stream);
 SNG_API int sng_sparse_col_cos(const int32_t* indptr, const int32_t* indices, const float* data, const float* inv_norm,
                        const int32_t* a, const int32_t* b, int64_t num_pairs, float* s, void* stream);
 SNG_API int sng_class_sums_f64(const float* xhat, const int32_t* y, int64_t n, int64_t d, int64_t ld, int num_classes,

@@ -55,6 +55,7 @@ SIGNATURES = {
     "sng_segment_mean": (_I32, [_P, _P, _I64, _I64, _P, _P, _SZ, _P]),
     "sng_sddmm_dot": (_I32, [_P, _I64, _I64, _I64, _P, _P, _I64, _P, _P]),
     "sng_gemm_nt_f16": (_I32, [_P, _I64, _P, _I64, _I64, _I64, _I64, _P, _P, _P, _I64, _P]),
+    "sng_simhist_f16": (_I32, [_P, _I64, _P, _I64, _I64, _I64, _I64, _I64, _F32, _F32, _I32, _P, _P]),
     "sng_sparse_col_cos": (_I32, [_P, _P, _P, _P, _P, _P, _I64, _P, _P]),
     "sng_class_sums_f64": (_I32, [_P, _P, _I64, _I64, _I64, _I32, _P, _P, _P]),
     "sng_graph_prepare_workspace_bytes": (_SZ, [_I64, _I64]),

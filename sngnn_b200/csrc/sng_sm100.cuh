@@ -1,6 +1,7 @@
-// tcgen05 / TMA primitives shared by the two tensor-core kernels, K1 (sng_simknn.cu) and the N x N producer (sng_gemm.cu):
-// mbarriers with the bounded wait, tcgen05 fences and TMEM loads, the descriptors of a K-major FP16 MMA and the TMA map
-// of its operands.  Forms that only one kernel uses (cta_group::2, cluster, multicast) stay in that kernel's file.
+// tcgen05 / TMA primitives shared by the tensor-core kernels, K1 (sng_simknn.cu), the N x N producer (sng_gemm.cu) and the
+// similarity histogram (sng_simhist.cu): mbarriers with the bounded wait, tcgen05 fences and TMEM loads, the cta_group::1
+// TMA load / MMA / commit, the descriptors of a K-major FP16 MMA and the TMA map of its operands.  Forms that only one
+// kernel uses (cta_group::2, cluster, multicast) stay in that kernel's file.
 #pragma once
 #include "sng_common.cuh"
 #include <cuda.h>        // CUtensorMap + enums only; cuTensorMapEncodeTiled is resolved at run time
@@ -53,6 +54,23 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
         : "r"(taddr) : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+
+// cta_group::1 forms: TMA tile load into this CTA's shared memory, one kind::f16 MMA into TMEM, and the commit that arrives
+// on an mbarrier when every MMA issued before it has retired
+__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1) {
+    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+                 ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+                 ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
 
 // K-major, 128-byte-swizzled shared-memory matrix descriptor (sm_100 "version 1"):
 // rows are 128 B apart, 8-row groups 1024 B apart (SBO); LBO unused for swizzled K-major.

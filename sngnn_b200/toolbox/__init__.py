@@ -6,7 +6,7 @@ Plotting (R: SimGFAToolbox/plot.py) is presentation and out of scope: the two pl
 from .dense import (node_similarity_dense_small, node_similarity_dense_large_parted, class_similarity_dense_small,
                     class_similarity_dense_large, linked_node_similarity_dense_large, linked_node_similarity_dense_small,
                     neighborhood_similarity_dense_large, neighborhood_similarity_dense_small, cosine_similarity_dense_small,
-                    cosine_similarity, edge_similarity_weight)
+                    cosine_similarity, edge_similarity_weight, node_similarity_histogram)
 from . import sharded  # noqa: F401  (row-sharded forms: one all-reduce of the class sums)
 from .sparse import (cosine_similarity_sparse, class_similarity_sparse, neighborhood_similarity_sparse, node_similarity_sparse,
                      linked_node_similarity_sparse, edge_index_to_sparse_csc_tensor)

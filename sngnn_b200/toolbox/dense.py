@@ -4,7 +4,11 @@
   sums over all pairs      -> sng_class_sums_f64 closed form <S_a, S_b> (R materialises 1000-row blocks, dense.py:17-27,108-128)
   the N x N matrix itself  -> sng_gemm_nt_f16 on the tensor cores (tcgen05 / TMEM / TMA) with the FP16 split x-hat = hi + lo
                               ([hi|hi|lo] x [hi|lo|hi]^T = FP32 product to ~2^-22), only for the *_small functions that return it
+  the distribution of the  -> sng_simhist_f16: the same split contraction with a binning epilogue, each unordered pair of
+  N x N values                row tiles scored once, integer counts (nothing N x N is stored)
 """
+import math
+
 import torch
 
 from .. import _C
@@ -57,6 +61,46 @@ def gemm_nt(a, b, k, row_scale=None, col_scale=None):
     out = torch.empty(m, n, dtype=torch.float32, device=a.device)
     _C.call("sng_gemm_nt_f16", a, _C.ptr(a), a.size(1), _C.ptr(b), b.size(1), m, n, k, _C.ptr(row_scale), _C.ptr(col_scale), _C.ptr(out), n)
     return out
+
+
+TILE_ROWS = 128        # rows per tile of sng_simhist_f16's schedule (include/sng.h)
+
+
+def _hist_range(bins, range):
+    lo, hi = float(range[0]), float(range[1])
+    if isinstance(bins, bool) or not isinstance(bins, int) or bins < 1:
+        raise ValueError(f"bins must be a positive int, got {bins!r}")
+    if not (math.isfinite(lo) and math.isfinite(hi) and lo < hi):
+        raise ValueError(f"range must be finite with lo < hi, got {range!r}")
+    return lo, hi
+
+
+def _hist_edges(lo, hi, bins, device):
+    return torch.linspace(lo, hi, bins + 1, dtype=torch.float64, device=device)
+
+
+def simhist_tiles(xhat, bins, lo, hi, tile_lo, tile_hi):
+    """int64 [bins] counts of the ordered off-diagonal cosines scored by the row tiles [tile_lo, tile_hi) of sng_simhist_f16's
+    symmetric schedule (128-row tiles; the counts of a split of [0, ceil(N / 128)) add up to the whole histogram)."""
+    _C.require_cuda(xhat)
+    a, b, k = split_f16_operands(xhat.contiguous())
+    counts = torch.zeros(bins, dtype=torch.int64, device=xhat.device)
+    _C.call("sng_simhist_f16", a, _C.ptr(a), a.size(1), _C.ptr(b), b.size(1), xhat.size(0), k, tile_lo, tile_hi, lo, hi, bins,
+            _C.ptr(counts))
+    return counts
+
+
+def node_similarity_histogram(x, bins=200, range=(-1.0, 1.0)):
+    """Histogram of the N (N - 1) off-diagonal cosines that node_similarity_dense_small returns, without the N x N matrix:
+    (counts int64 [bins], edges float64 [bins + 1]) as numpy.histogram(values, bins, range) -- equal bins, the last one
+    closed, values outside the range not counted.  Scores are the FP32 cosines of the split tensor-core contraction
+    (error ~1e-5 or less, DESIGN.md §7), clamped to [-1, 1]; an all-zero row scores 0 with every row."""
+    src, _ = _dev(x)
+    lo, hi = _hist_range(bins, range)
+    xhat = _normalised(x)
+    t = (xhat.size(0) + TILE_ROWS - 1) // TILE_ROWS
+    counts = simhist_tiles(xhat, bins, lo, hi, 0, t)
+    return counts.to(src), _hist_edges(lo, hi, bins, src)
 
 
 def cosine_similarity_dense_small(x):

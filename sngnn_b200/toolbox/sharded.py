@@ -2,7 +2,8 @@
 holds the feature rows [lo, hi) of `dist.shard_bounds`, computes the FP64 class sums of its rows with `sng_class_sums_f64`,
 and ONE all-reduce of the [K, d] sums (+ the [K] counts) gives every rank the closed forms <S_a, S_b> behind
 R: SimGFAToolbox/dense.py:9-30 (node similarity) and :104-130 (class similarity).  The edge metrics shard by edges: each rank
-scores its slice of the edge list against the all-gathered x-hat and the scalar mean is all-reduced.
+scores its slice of the edge list against the all-gathered x-hat and the scalar mean is all-reduced.  The similarity
+histogram shards by row tiles of its symmetric schedule over the all-gathered x-hat and all-reduces the integer counts.
 Works with any torch.distributed backend (NCCL on the B200 box; the CPU tests inject the local kernels and use gloo)."""
 import torch
 import torch.distributed as dist
@@ -62,3 +63,22 @@ def linked_node_similarity_dense_sharded(x_local, edge_index, n, edge_cos=None):
     acc = torch.stack([s.double().sum(), torch.tensor(float(hi - lo), dtype=torch.float64, device=s.device)])
     acc = _allreduce(acc)
     return s, (acc[0] / acc[1].clamp(min=1)).float()
+
+
+def node_similarity_histogram_sharded(x_local, n, bins=200, range=(-1.0, 1.0), hist=None):
+    """node_similarity_histogram of all n rows from row shards: x-hat all-gathered once (FP32), rank r scores a contiguous,
+    equal share of the T = ceil(n / 128) row tiles of sng_simhist_f16's schedule (every row tile does the same work), and
+    ONE all-reduce of the int64 counts.  Every rank returns (counts, edges), the counts equal bit for bit to the
+    single-GPU call.  `hist(xhat, bins, lo, hi, tile_lo, tile_hi)` stands in for the kernel (CPU tests)."""
+    from . import dense as D
+    ws, rank = sdist.world()
+    lo, hi = D._hist_range(bins, range)
+    if hist is None:
+        xhat = sdist.all_gather_rows(D._normalised(x_local), n)
+        hist = D.simhist_tiles
+    else:
+        xhat = sdist.all_gather_rows(torch.nn.functional.normalize(x_local.float(), dim=-1), n)
+    t = (n + D.TILE_ROWS - 1) // D.TILE_ROWS
+    per = (t + ws - 1) // ws
+    counts = hist(xhat, bins, lo, hi, min(t, rank * per), min(t, (rank + 1) * per))
+    return _allreduce(counts), D._hist_edges(lo, hi, bins, counts.device)
