@@ -39,7 +39,7 @@ extern "C" {
 #define SNG_ERR_CUDA (-3)        /* CUDA runtime/driver error */
 #define SNG_ERR_WORKSPACE (-4)   /* workspace too small */
 
-#define SNG_MAX_TOPK 64          /* edge path: top_k <= 64; top_k <= 0 means "select every edge" */
+#define SNG_MAX_TOPK 64          /* edge path lists: top_k <= 64 (larger: sng_edge_fwd_wide); top_k <= 0 means "select every edge" */
 #define SNG_MAX_CHANNELS 512     /* padded row width c of sng_edge_fwd / _bwd, sng_edge_agg_bwd, sng_list_agg_fwd, sng_spmm_fwd,
                                     sng_pp_fuse_fwd / _bwd; wider rows return SNG_ERR_UNSUPPORTED */
 #define SNG_KNN_MAX_TOPK 64      /* all-pairs builder */
@@ -158,6 +158,42 @@ SNG_API int sng_edge_bwd_denom(const float* h, const float* inv_norm, const floa
                  float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
                  const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
                  int64_t n_lrows_out, float* chunk_partials, const float* inv_denom, void* stream);
+
+/* Per-edge selection form of sng_edge_fwd_denom / sng_edge_bwd_denom for top_k > SNG_MAX_TOPK (any top_k: every value
+ * >= max_deg selects the same set, so callers clamp to that).  The selection rule is the same, S_i = {e : s_e >= thr and
+ * rank_i(e) < top_k} with ranks by (s desc, position asc); it is saved as one flag per in-edge instead of [n, top_k] lists.
+ * A row with deg <= top_k selects {e : s_e >= thr} in the aggregation pass itself.  A row with deg > top_k (only rows with
+ * more than 32 in-edges can be: lrows, when given, lists them) is cut first, once: one block per row scores its edges,
+ * radix-selects the top_k-th key and flags the winners, ties at the cut going to the lowest positions.  The aggregation reads
+ * those flags and weights edge e by s_e when selected, with the denominator 0 (1/max(deg_i,1)) or 1 (1/max(|S_i|,1), written
+ * to inv_denom [n] when given).
+ * num_edges = rowptr[n] (edges of the call's rows), max_deg >= every row's in-degree: no row is cut when top_k >= max_deg.
+ * sel_flag [num_edges] uint8 (CSR-by-target positions): required when top_k < max_deg or train != 0; with train != 0 every
+ * edge's flag is written (the input of sng_edge_bwd_wide).  workspace >= sng_edge_fwd_wide_workspace_bytes(n_chunks, c,
+ * num_edges, max_deg) (may be 0).  Other arguments, the fused epilogue and row sharding as sng_edge_fwd_denom; no selection
+ * lists are written. */
+SNG_API size_t sng_edge_fwd_wide_workspace_bytes(int64_t n_chunks, int64_t c, int64_t num_edges, int64_t max_deg);
+SNG_API int sng_edge_fwd_wide(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
+                 const int32_t* rowptr, const int32_t* col, int64_t num_edges,
+                 const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                 const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
+                 int top_k, int64_t max_deg, float thr, float* out, int64_t ldo, uint8_t* sel_flag, int train,
+                 float* inv_norm, int inv_norm_ready,
+                 const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
+                 int denominator, float* inv_denom, void* stream);
+/* Backward of sng_edge_fwd_wide: sng_edge_bwd_denom's two gather passes over every in-edge of the CSR (col, tpos), an edge
+ * counting only when sel_flag (the forward's, written with train != 0) marks it selected -- also when its score is 0.
+ * inv_denom: the forward's factors (denominator 1) or NULL (1/max(deg_i,1)).  No float atomics, bit-reproducible; workspaces,
+ * fused epilogue and row sharding as sng_edge_bwd. */
+SNG_API int sng_edge_bwd_wide(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                 int64_t c, int64_t ld, int64_t ldg,
+                 const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                 const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
+                 const uint8_t* sel_flag, const float* inv_denom,
+                 const float* beta, const float* diff, int64_t lddiff, float* dbeta,
+                 float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
+                 const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
+                 int64_t n_lrows_out, float* chunk_partials, void* stream);
 
 /* Gather form of the backward of sng_list_agg_fwd (explicit neighbour lists: the all-pairs mode) -- the same two passes and
  * kernels as sng_edge_bwd, no float atomics, bit-reproducible.  The lists are those of sng_simknn_build: idx / sim [n, top_k]

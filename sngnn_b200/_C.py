@@ -24,6 +24,11 @@ SIGNATURES = {
                             _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _P]),
     "sng_edge_fwd_denom": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _I64, _P, _P, _I64, _P, _I64, _P, _SZ, _I32, _F32, _P,
                                   _I64, _P, _P, _P, _P, _P, _I32, _P, _I64, _P, _P, _P, _P, _I32, _P, _P]),
+    "sng_edge_fwd_wide_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64]),
+    "sng_edge_fwd_wide": (_I32, [_P, _I64, _I64, _I64, _I64, _I64, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _I64, _P, _SZ, _I32, _I64,
+                                 _F32, _P, _I64, _P, _I32, _P, _I32, _P, _I64, _P, _P, _P, _P, _I32, _P, _P]),
+    "sng_edge_bwd_wide": (_I32, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _P, _I64, _I64, _P, _P,
+                                 _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _P]),
     "sng_bn_workspace_bytes": (_SZ, [_I64, _I64]),
     "sng_bn_fwd_stats": (_I32, [_P, _I64, _I64, _I64, _P, _P, _SZ, _P]),
     "sng_bn_fwd_apply": (_I32, [_P, _I64, _I64, _I64, _P, _I64, ctypes.c_double, _P, _P, _P, _P, _P, _I64, _P]),
@@ -106,6 +111,7 @@ def ptr(t):
 
 PARTIALS = 4096          # SNG_PARTIALS of include/sng.h
 MAX_CHANNELS = 512       # SNG_MAX_CHANNELS of include/sng.h
+MAX_TOPK = 64            # SNG_MAX_TOPK of include/sng.h: larger top_k take the per-edge form (sng_edge_fwd_wide)
 
 
 def stream(t=None):

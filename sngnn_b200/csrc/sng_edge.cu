@@ -4,7 +4,7 @@
 // G = C/4 lanes owns one in-edge at a time and fetches its source row with ONE 128-bit load per lane, so
 // a warp step touches 32/G full rows (coalesced 16..512-byte segments).  Wider rows (C > 128, up to SNG_MAX_CHANNELS) take the
 // whole warp, G/32 loads per lane (RowShape).  Scores, selection and the weighted reduction never leave registers / shared
-// memory; nothing of size E is written.
+// memory; nothing of size E is written (except the per-edge form of top_k > SNG_MAX_TOPK: one selection byte per edge).
 //
 // Reference call sites replaced: R: models/models.py:121-137,139-158 (++), :233-263 (+), :322-334 (base).
 #include "sng_common.cuh"
@@ -127,6 +127,10 @@ struct EdgeFwdArgs {
     int* sel_src; float* sel_w; int* sel_q; int* sel_cnt;      // saved for backward; all nullptr in inference
     const float* wt; int ldw; const float* b_w; const float* beta; const float* bias; float* diff;   // fused SNGNN++ epilogue
     int slots;                               // staged kernel: row slots per warp (>= 33, fused >= 65: any single item fits)
+    // per-edge form (WK instances, top_k > SNG_MAX_TOPK): eflag [E] = selection flag per in-edge position.  edge_cut_kernel
+    // writes the rows with deg > top_k; the aggregation reads those and decides every other row by s >= thr in place,
+    // writing its flags too when eflag_write (training).  cut_keys [E]: keys of rows too long for the cut kernel's stage.
+    unsigned char* eflag; int eflag_write; unsigned* cut_keys;
 };
 
 constexpr unsigned kFull = 0xffffffffu;
@@ -195,7 +199,7 @@ __device__ __forceinline__ float lds32(uint32_t addr) {
 // bytes of a staged row slot: the row padded by one 16-byte chunk (G > 1), so that slot strides are odd multiples of 16 B
 template <int G> constexpr int staged_row_bytes() { return G == 1 ? 16 : 16 * G + 16; }
 
-template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK, bool DSEL = false>
+template <int G, bool FUSE, bool SELECT_ALL, bool CHUNK, bool DSEL = false, bool WK = false>
 __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_kernel(const EdgeFwdArgs a) {
     constexpr int C = 4 * G;                    // channels of a padded row
     constexpr int RB = staged_row_bytes<G>();
@@ -315,7 +319,16 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_k
             float acc = 0.f, a0 = 0.f;
             int cnt = 0, myrank = -1;
             if (SELECT_ALL) {
-                const float wsel = has ? my_s : 0.f;
+                bool sel = has;
+                if (WK) {
+                    // a row of <= 32 edges is never cut (top_k > 64); a chunk reads its long row's flags when that row is cut
+                    bool cut = false;
+                    if (CHUNK) cut = __ldg(a.rowptr + trA + 1) - __ldg(a.rowptr + trA) > a.top_k;
+                    sel = has && (cut ? a.eflag[begA + lane] != 0 : my_s >= a.thr);
+                    if (!cut && a.eflag_write && has) a.eflag[begA + lane] = sel;
+                    cnt = __popc(__ballot_sync(kFull, sel));
+                }
+                const float wsel = sel ? my_s : 0.f;
 #pragma unroll 4
                 for (int e = 0; e < deg; ++e) acc = fmaf(__shfl_sync(kFull, wsel, e), lds32(rd + (uint32_t)(e * RB)), acc);
             } else {
@@ -340,6 +353,7 @@ __global__ void __launch_bounds__(kStWarps * 32, kStMinBlocks) edge_fwd_staged_k
                     if (myrank >= 0) { a.tmp_s[(int64_t)row * kk + myrank] = my_s; a.tmp_p[(int64_t)row * kk + myrank] = begA + lane; }
                     if (lane == 0) a.tmp_cnt[row] = cnt;
                 }
+                if (WK && lane == 0) a.tmp_cnt[row] = cnt;
                 if (lane < C) {
                     if (SELECT_ALL) a.tmp_acc[(int64_t)row * C + ch] = acc;
                     if (FUSE) a.tmp_a0[(int64_t)row * C + ch] = a0;
@@ -411,7 +425,7 @@ __device__ __forceinline__ float lane_reduce_scatter(float (&v)[K], int lane) {
 
 struct NarrowGather { float4 hj, wj, hi; float irl, iri; int tq; };
 
-template <bool FUSE, bool SELECT_ALL, bool DSEL = false>
+template <bool FUSE, bool SELECT_ALL, bool DSEL = false, bool WK = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_narrow_kernel(const EdgeFwdArgs a) {
     constexpr int K = FUSE ? 8 : 4;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -466,7 +480,13 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_narrow_kernel(const EdgeFwd
             int cnt = 0, myrank = -1;
             float wgt;
             if (SELECT_ALL) {
-                wgt = has ? my_s : 0.f;
+                bool sel = has;
+                if (WK) {                                                            // <= 32 edges: never cut (top_k > 64)
+                    sel = has && my_s >= a.thr;
+                    if (a.eflag_write && has) a.eflag[begA + lane] = sel;
+                    cnt = __popc(__ballot_sync(kFull, sel));
+                }
+                wgt = sel ? my_s : 0.f;
             } else {
                 const bool cand = has && my_s >= a.thr;
                 unsigned key = cand ? okey(my_s) : 0u;
@@ -555,20 +575,24 @@ struct TopList {
 // score); a group of RowShape<G>::L lanes fetches one source row per step.  SELECT_ALL accumulates the weighted rows on the
 // fly, the selection variant only maintains the warp's top-k list (winners are re-gathered afterwards: they were loaded
 // moments ago).  hb / wb / ni / ch_ok / acc / a0 hold one entry per float4 slot of the lane (RowShape<G>::V).
-template <int G, bool FUSE, bool SELECT_ALL>
+// WK (per-edge form, SELECT_ALL): an edge weighs s_e only when selected -- by eflag when the row is `cut`, else by s_e >= thr
+// (written to eflag when eflag_write); L.cnt receives the warp's selected count.
+template <int G, bool FUSE, bool SELECT_ALL, bool WK = false>
 __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* const (&hb)[RowShape<G>::V], const float* const (&wb)[RowShape<G>::V],
                                          int grow, int end, int first, int step, const float4 (&ni)[RowShape<G>::V],
                                          const bool (&ch_ok)[RowShape<G>::V], int lane, TopList& L, float4 (&acc)[RowShape<G>::V],
-                                         float4 (&a0)[RowShape<G>::V]) {
+                                         float4 (&a0)[RowShape<G>::V], bool cut = false) {
     using S = RowShape<G>;
     constexpr int EPW = S::EPW, V = S::V;
     constexpr int U = (G <= 8) ? G : 8 / V;     // steps whose loads are issued together (eight 16-byte loads per lane from G = 8 on)
     const int grp = lane / S::L;
+    int nsel = 0;                               // WK: selected edges counted by this lane (the first lane of a group)
     for (int base = first; base < end; base += step) {
         const int nchunk = min(32, end - base);
         const bool has = lane < nchunk;
         const int jl = has ? __ldg(a.col + base + lane) : grow;                          // missing edges read the target row itself
         const float irl = __ldg(a.inv_r + jl);
+        const int fl = (WK && cut && has) ? a.eflag[base + lane] : 0;
         float my_d = 0.f;                                                               // <n_i, h_j> of edge base + lane
         for (int st = 0; st < nchunk; st += EPW * U) {
             float4 v[U][V];
@@ -589,9 +613,20 @@ __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* cons
                 if (SELECT_ALL) {
                     const int e = st + u * EPW + grp;
                     const float w = __shfl_sync(kFull, irl, e & 31);
+                    float wk = 0.f;                                                  // WK: the edge's weight
+                    if (WK) {
+                        const float sc = d * w + 0.0f;
+                        const int f = __shfl_sync(kFull, fl, e & 31);
+                        const bool sel = cut ? f != 0 : sc >= a.thr;
+                        if (e < nchunk && lane % S::L == 0) {
+                            nsel += sel;
+                            if (!cut && a.eflag_write) a.eflag[base + e] = sel;
+                        }
+                        wk = sel ? sc : 0.f;
+                    }
 #pragma unroll
                     for (int s = 0; s < V; ++s)
-                        if (e < nchunk && ch_ok[s]) fma4(acc[s], d * w + 0.0f, v[u][s]);
+                        if (e < nchunk && ch_ok[s]) fma4(acc[s], WK ? wk : d * w + 0.0f, v[u][s]);
                 } else {
                     const float t = __shfl_sync(kFull, d, (lane % EPW) * S::L);          // hand (step, group) to the edge's lane
                     if (lane / EPW == st / EPW + u) my_d = t;
@@ -625,6 +660,7 @@ __device__ __forceinline__ void scan_row(const EdgeFwdArgs& a, const float* cons
             }
         }
     }
+    if (WK) L.cnt = (int)__reduce_add_sync(kFull, (unsigned)nsel);
 }
 
 // weighted sum of the <= top_k winners of a finished list (source ids re-read through their positions) + the saved lists
@@ -655,7 +691,7 @@ __device__ __forceinline__ void finish_list(const EdgeFwdArgs& a, const float* c
     if (DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(cnt);
 }
 
-template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false, bool WK = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdArgs a) {
     using S = RowShape<G>;
     constexpr int V = S::V;
@@ -695,8 +731,9 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdAr
             acc[s] = z4; a0[s] = z4;
         }
         L.cnt = 0; L.kth = -CUDART_INF_F;
-        scan_row<G, FUSE, SELECT_ALL>(a, hb, wb, grow, end, beg, 32, ni, ch_ok, lane, L, acc, a0);
+        scan_row<G, FUSE, SELECT_ALL, WK>(a, hb, wb, grow, end, beg, 32, ni, ch_ok, lane, L, acc, a0, WK && end - beg > a.top_k);
         if (!SELECT_ALL) { finish_list<G, DSEL>(a, hb, row, L.s, L.p, L.cnt, lane, acc); __syncwarp(); }
+        if (WK && DSEL && lane == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(L.cnt);
         const int den = DSEL ? L.cnt : end - beg;
 #pragma unroll
         for (int s = 0; s < V; ++s) {
@@ -714,7 +751,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_long_kernel(const EdgeFwdAr
 // candidates of as many further chunks as fit, and top_k rounds of a warp max pick the new winners; lane order equals edge
 // position order, so the lowest lane among equal scores is the reference's tie-break.  Larger top_k: sorted insertion into
 // a shared-memory list (a newcomer loses every tie).
-template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false, bool WK = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdArgs a) {
     constexpr int C = 4 * G;
     extern __shared__ float smem[];
@@ -739,6 +776,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
             for (int ci = c0; ci < c1; ++ci) {
                 if (SELECT_ALL) acc += __ldg(a.tmp_acc + (int64_t)ci * C + ch);
                 if (FUSE) a0 += __ldg(a.tmp_a0 + (int64_t)ci * C + ch);
+                if (WK) nsel += __ldg(a.tmp_cnt + ci);                      // the chunks' selected counts
             }
         }
         if (!SELECT_ALL) {
@@ -837,7 +875,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_merge_kernel(const EdgeFwdA
 // Hub rows (in-degree > 1024): one block per row.  Warp w scans chunks w, w + 8, ... with its own top-k list; the 8 lists
 // are merged by ranking their <= 8 top_k entries against each other (positions are unique, so (score, position) is a
 // strict order and the ranks are the final ranks); warp 0 then finishes the row exactly like the long-row kernel.
-template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL = false, bool WK = false>
 __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArgs a) {
     using S = RowShape<G>;
     constexpr int V = S::V;
@@ -846,7 +884,7 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int q = lane % S::L, grp = lane / S::L;
     const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-    const int k1 = max(a.top_k, 1);
+    const int k1 = WK ? 1 : max(a.top_k, 1);   // (the shared memory of WK instances is sized for top_k = 0, see hub_smem)
     bool ch_ok[V];
     const float* hb[V];
     const float* wb[V];
@@ -884,7 +922,8 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
             acc[s] = z4; a0[s] = z4;
         }
         L.cnt = 0; L.kth = -CUDART_INF_F;
-        scan_row<G, FUSE, SELECT_ALL>(a, hb, wb, grow, end, beg + 32 * warp, 32 * kWarpsPerBlock, ni, ch_ok, lane, L, acc, a0);
+        scan_row<G, FUSE, SELECT_ALL, WK>(a, hb, wb, grow, end, beg + 32 * warp, 32 * kWarpsPerBlock, ni, ch_ok, lane, L, acc, a0,
+                                          WK && end - beg > a.top_k);
 #pragma unroll
         for (int s = 0; s < V; ++s) {
             cross_group_sum4<G>(acc[s]);
@@ -918,6 +957,9 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
                 if (rank < a.top_k) { fin_s[rank] = s; fin_p[rank] = p; }
             }
             __syncthreads();
+        } else if (WK) {
+            for (int w = 0; w < kWarpsPerBlock; ++w) cnt += wcnt[w];
+            if (DSEL && threadIdx.x == 0 && a.inv_denom) a.inv_denom[row] = sel_factor(cnt);
         }
         if (warp == 0) {
             float4 sacc[V], sa0[V];
@@ -941,6 +983,124 @@ __global__ void __launch_bounds__(kThreads) edge_fwd_hub_kernel(const EdgeFwdArg
                 if (grp == 0 && ch_ok[s]) write_row<FUSE>(a, row, slot_c4(q, s), sacc[s], sa0[s], DSEL ? cnt : end - beg, beta, bw[s], bb[s]);
         }
         __syncthreads();
+    }
+}
+
+// ---- per-edge form, top_k > SNG_MAX_TOPK: the cut --------------------------------------------------------------------------
+// A row with deg <= top_k selects {e : s_e >= thr}, which the aggregation decides in place.  Only a row with deg > top_k needs
+// ranks: one block scores its in-edges once (keys = okey(s) for s >= thr, 0 otherwise; in shared memory up to kCutKeys edges,
+// else in the caller's workspace at the row's edge positions), finds the top_k-th key T by a radix select (four 8-bit digits,
+// integer histograms in shared memory), and flags the edges with key > T plus the first `need` edges with key == T in position
+// order (a block-wide prefix count) -- the rule (s desc, position asc) of R: models/models.py:145-154.  The aggregation
+// reads the flags of these rows and never re-derives the cut from its own scores, so |S_i| is decided once.
+constexpr int kCutKeys = 8192;
+template <int G>
+__global__ void __launch_bounds__(kThreads) edge_cut_kernel(const EdgeFwdArgs a) {
+    using S = RowShape<G>;
+    constexpr int EPW = S::EPW, V = S::V;
+    constexpr int U = (G <= 8) ? G : 8 / V;
+    __shared__ unsigned skeys[kCutKeys];
+    __shared__ unsigned hist[256];
+    __shared__ int s_nc, s_digit, s_need, s_wtot[kWarpsPerBlock];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int q = lane % S::L, grp = lane / S::L;
+    const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    bool ch_ok[V];
+    const float* hb[V];
+#pragma unroll
+    for (int s = 0; s < V; ++s) { ch_ok[s] = slot_c4(q, s) < a.c; hb[s] = a.h + (ch_ok[s] ? slot_c4(q, s) : 0); }
+    const int total = a.rows ? a.n_rows : a.n;
+    for (int ri = blockIdx.x; ri < total; ri += gridDim.x) {
+        const int row = a.rows ? __ldg(a.rows + ri) : ri;
+        const int beg = __ldg(a.rowptr + row), deg = __ldg(a.rowptr + row + 1) - beg;
+        if (deg <= a.top_k) continue;                                        // block-uniform
+        unsigned* keys = deg <= kCutKeys ? skeys : a.cut_keys + beg;
+        const int grow = a.row_offset + row;
+        float4 ni[V];
+#pragma unroll
+        for (int s = 0; s < V; ++s) ni[s] = ch_ok[s] ? scale4(ldg4(hb[s] + (int64_t)grow * a.ldh), __ldg(a.inv_r + grow)) : z4;
+        if (threadIdx.x == 0) s_nc = 0;
+        __syncthreads();
+        // 1. keys, the scores computed as the long-row kernel computes them; warp w takes the 32-edge chunks w, w + 8, ...
+        int nc = 0;
+        for (int base = 32 * warp; base < deg; base += 32 * kWarpsPerBlock) {
+            const int nchunk = min(32, deg - base);
+            const int jl = lane < nchunk ? __ldg(a.col + beg + base + lane) : grow;
+            const float irl = __ldg(a.inv_r + jl);
+            for (int st = 0; st < nchunk; st += EPW * U) {
+                float4 v[U][V];
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    const int j = __shfl_sync(kFull, jl, (st + u * EPW + grp) & 31);
+#pragma unroll
+                    for (int s = 0; s < V; ++s) v[u][s] = ldg4(hb[s] + (int64_t)j * a.ldh);
+                }
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    const int e = st + u * EPW + grp;
+                    const float d = group_sum<S::L>(dotv<V>(ni, v[u]));
+                    const float sc = d * __shfl_sync(kFull, irl, e & 31) + 0.0f;
+                    if (q == 0 && e < nchunk) {
+                        const bool cand = sc >= a.thr;
+                        keys[base + e] = cand ? okey(sc) : 0u;
+                        nc += cand;
+                    }
+                }
+            }
+        }
+        nc = (int)__reduce_add_sync(kFull, (unsigned)nc);
+        if (lane == 0) atomicAdd(&s_nc, nc);
+        __syncthreads();
+        // 2. radix select of the top_k-th largest key T among the candidates; need = how many edges with key == T are taken.
+        // With no more candidates than top_k every candidate is selected: T = 0, need = 0.
+        unsigned prefix = 0u, mask = 0u;
+        int need = 0;
+        if (s_nc > a.top_k) {
+            need = a.top_k;
+            for (int shift = 24; shift >= 0; shift -= 8) {
+                for (int i = threadIdx.x; i < 256; i += kThreads) hist[i] = 0u;
+                __syncthreads();
+                for (int e = threadIdx.x; e < deg; e += kThreads) {
+                    const unsigned k = keys[e];
+                    if ((k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+                }
+                __syncthreads();
+                if (warp == 0) {                                             // lane l: digits 255 - 8 l down to 248 - 8 l
+                    int h8[8], sum = 0;
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) { h8[i] = (int)hist[255 - 8 * lane - i]; sum += h8[i]; }
+                    int inc = sum;
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(kFull, inc, o); if (lane >= o) inc += t; }
+                    int c = inc - sum;
+                    if (c < need && inc >= need) {
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) {
+                            if (c + h8[i] >= need) { s_digit = 255 - 8 * lane - i; s_need = need - c; break; }
+                            c += h8[i];
+                        }
+                    }
+                }
+                __syncthreads();
+                prefix |= (unsigned)s_digit << shift; mask |= 255u << shift; need = s_need;
+            }
+        }
+        // 3. flags in position order: key > T, or key == T among the first `need` such edges
+        int before = 0;
+        for (int t0 = 0; t0 < deg; t0 += kThreads) {
+            const int e = t0 + threadIdx.x;
+            const unsigned k = e < deg ? keys[e] : 0u;
+            const bool tie = e < deg && need > 0 && k == prefix;
+            const unsigned bal = __ballot_sync(kFull, tie);
+            if (lane == 0) s_wtot[warp] = __popc(bal);
+            __syncthreads();
+            int rank = before + __popc(bal & ((1u << lane) - 1u)), tot = 0;
+#pragma unroll
+            for (int w = 0; w < kWarpsPerBlock; ++w) { const int c = s_wtot[w]; rank += w < warp ? c : 0; tot += c; }
+            if (e < deg) a.eflag[beg + e] = (k > prefix || (tie && rank < need)) ? 1 : 0;
+            before += tot;
+            __syncthreads();
+        }
     }
 }
 
@@ -1131,6 +1291,7 @@ struct EdgeBwdArgs {
     const int4* chunk_tab; int n_chunks; const int* lrows; const int* lrow_ptr; int n_lrows;
     float* tmp_part;                         // [n_chunks, 3, 4G]
     int slots;                               // staged source pass: row slots per warp (>= 64: any single item fits)
+    const unsigned char* eflag;              // per-edge form: the forward's selection flags [E] (edge_bwd_target_kernel<.., WK>)
 };
 
 // source row j is one of the call's target rows: pass T wrote its target-side dn at dnT[j - row_offset]
@@ -1138,7 +1299,10 @@ __device__ __forceinline__ bool owns_row(const EdgeBwdArgs& a, int j) { return (
 
 // LIST: the saved lists come with a.inv_denom -- neighbour lists, or edges under denominator='selected' (a template flag: a
 // runtime branch costs the edge instances at C = 32 / 64 an 8-byte spill)
-template <int G, bool SELECT_ALL, bool LIST = false>
+// WK (per-edge form, with SELECT_ALL): eflag [E] says which in-edges the forward selected; an unselected edge gets coefficients
+// (0, 0) and adds nothing to dn_i, a selected one -- even with s_e = 0 -- carries its gradient.  inv_denom, when given, holds
+// the forward's per-row factors (denominator='selected').
+template <int G, bool SELECT_ALL, bool LIST = false, bool WK = false>
 __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwdArgs a) {
     using S = RowShape<G>;
     constexpr int EPW = S::EPW, V = S::V;
@@ -1156,7 +1320,10 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
         const int grow = a.row_offset + row;
         int beg = 0, cnt;
         float invd;
-        if (SELECT_ALL) { beg = __ldg(a.rowptr + row); cnt = __ldg(a.rowptr + row + 1) - beg; invd = 1.0f / (float)max(cnt, 1); }
+        if (SELECT_ALL) {
+            beg = __ldg(a.rowptr + row); cnt = __ldg(a.rowptr + row + 1) - beg;
+            invd = (WK && a.inv_denom) ? __ldg(a.inv_denom + row) : 1.0f / (float)max(cnt, 1);
+        }
         else {
             cnt = __ldg(a.sel_cnt + row);
             invd = LIST ? __ldg(a.inv_denom + row) : 1.0f / (float)max(__ldg(a.rowptr + row + 1) - __ldg(a.rowptr + row), 1);
@@ -1179,13 +1346,16 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
 #pragma unroll
         for (int s = 0; s < V; ++s) dni[s] = z4;
         for (int st = 0; st < cnt; st += EPW * U) {
-            float4 v[U][V]; int j[U], qp[U]; float w[U];
+            float4 v[U][V]; int j[U], qp[U]; float w[U]; bool fs[U];
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int t = st + u * EPW + grp;
-                j[u] = -1; w[u] = 0.f; qp[u] = 0;
+                j[u] = -1; w[u] = 0.f; qp[u] = 0; fs[u] = true;
                 if (t < cnt) {
-                    if (SELECT_ALL) { j[u] = __ldg(a.col + beg + t); qp[u] = __ldg(a.tpos + beg + t); }
+                    if (SELECT_ALL) {
+                        j[u] = __ldg(a.col + beg + t); qp[u] = __ldg(a.tpos + beg + t);
+                        if (WK) fs[u] = a.eflag[beg + t] != 0;
+                    }
                     else {
                         const int64_t o = (int64_t)row * a.top_k + t;
                         j[u] = __ldg(a.sel_src + o); w[u] = __ldg(a.sel_w + o); qp[u] = __ldg(a.sel_q + o);
@@ -1200,10 +1370,12 @@ __global__ void __launch_bounds__(kThreads) edge_bwd_target_kernel(const EdgeBwd
                 const float irj = j[u] >= 0 ? __ldg(a.inv_r + j[u]) : 0.f;
                 const float ds = group_sum<S::L>(dotv<V>(v[u], gs));         // dL/ds_e
                 const float sc = SELECT_ALL ? group_sum<S::L>(dotv<V>(ni, v[u])) * irj + 0.0f : w[u];
-                if (j[u] >= 0) {
+                if (j[u] >= 0 && (!WK || fs[u])) {
 #pragma unroll
                     for (int s = 0; s < V; ++s) fma4(dni[s], ds * irj, v[u][s]);   // ds_e n_j
                     if (q == 0) a.coef[qp[u]] = make_float2(sc * invd * gscale, ds * iri);
+                } else if (WK && j[u] >= 0 && q == 0) {
+                    a.coef[qp[u]] = make_float2(0.f, 0.f);                   // not selected
                 }
             }
         }
@@ -2038,9 +2210,9 @@ static size_t hub_smem(int top_k) {
 static int forward_slots(bool fuse) {
     return fuse ? 66 : 40;                  // measured (pokec shape, C = 32): smaller pools win -- occupancy beats prefetch depth
 }
-template <int G, bool FUSE, bool SELECT_ALL, bool DSEL>
+template <int G, bool FUSE, bool SELECT_ALL, bool DSEL, bool WK = false>
 static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hub, cudaStream_t st) {
-    const size_t ls = long_smem(a.top_k), hs = hub_smem<G>(a.top_k);
+    const size_t ls = long_smem(WK ? 0 : a.top_k), hs = hub_smem<G>(WK ? 0 : a.top_k);     // (WK keeps no top-k lists)
     if constexpr (G <= 8) {
         if (a.n_chunks >= 0) {
             // degree lists known, rows of <= 128 bytes: staged kernel over the short rows, then over the <= 32-edge chunks of the
@@ -2049,15 +2221,15 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
             const size_t ss = (size_t)kStWarps * a.slots * staged_row_bytes<G>();
             if constexpr (G == 1) {
                 // 16-byte rows: everything in registers (edge_fwd_narrow_kernel); the chunk pass of the long rows stays staged
-                edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL>, a.n, kWarpsPerBlock), kThreads, 0, st>>>(a);
+                edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL, WK><<<grid_resident(edge_fwd_narrow_kernel<FUSE, SELECT_ALL, DSEL, WK>, a.n, kWarpsPerBlock), kThreads, 0, st>>>(a);
             } else {
-                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
-                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL>, a.n, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
+                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL, WK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
+                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL, WK><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, false, DSEL, WK>, a.n, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
             }
             if (a.n_chunks > 0) {
-                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
-                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true>, a.n_chunks, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
-                edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL>, a.n_lrows, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
+                cudaFuncSetAttribute(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true, false, WK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ss);
+                edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true, false, WK><<<grid_resident(edge_fwd_staged_kernel<G, FUSE, SELECT_ALL, true, false, WK>, a.n_chunks, kStWarps, ss, kStWarps * 32), kStWarps * 32, ss, st>>>(a);
+                edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL, WK><<<grid_resident(edge_fwd_merge_kernel<G, FUSE, SELECT_ALL, DSEL, WK>, a.n_lrows, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
             }
             return;
         }
@@ -2065,10 +2237,10 @@ static void launch_edge_fwd(EdgeFwdArgs a, const int32_t* rows_hub, int64_t n_hu
     // wide rows (C > 32) or no degree lists: the chunked kernel runs every row; listed hubs still get their block kernel
     a.rows = nullptr; a.n_rows = 0;
     a.skip_deg = n_hub > 0 ? 1024 : 0;
-    edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_resident(edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL>, a.n, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
+    edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL, WK><<<grid_resident(edge_fwd_long_kernel<G, FUSE, SELECT_ALL, DSEL, WK>, a.n, kWarpsPerBlock, ls), kThreads, ls, st>>>(a);
     if (a.skip_deg) {
         a.rows = rows_hub; a.n_rows = (int)n_hub; a.skip_deg = 0;
-        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL, DSEL><<<grid_capped(n_hub, 1, 4), kThreads, hs, st>>>(a);
+        edge_fwd_hub_kernel<G, FUSE, SELECT_ALL, DSEL, WK><<<grid_capped(n_hub, 1, 4), kThreads, hs, st>>>(a);
     }
 }
 }  // namespace sng
@@ -2121,6 +2293,7 @@ extern "C" int sng_edge_fwd_denom(const float* h, int64_t n_total, int64_t n, in
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab); a.n_chunks = staged ? (int)n_chunks : -1;
     a.lrows = lrows; a.lrow_ptr = lrow_ptr; a.n_lrows = (int)n_lrows;
     a.tmp_s = nullptr; a.tmp_p = nullptr; a.tmp_cnt = nullptr; a.tmp_acc = nullptr; a.tmp_a0 = nullptr;
+    a.eflag = nullptr; a.eflag_write = 0; a.cut_keys = nullptr;
     if (staged && n_chunks > 0) {
         const int64_t kk = a.top_k < 32 ? a.top_k : 32, cg = 4 * group_lanes(c);
         float* w = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
@@ -2151,6 +2324,83 @@ extern "C" int sng_edge_fwd(const float* h, int64_t n_total, int64_t n, int64_t 
     return sng_edge_fwd_denom(h, n_total, n, row_offset, c, ldh, rowptr, col, tpos, chunk_tab, n_chunks, lrows, lrow_ptr, n_lrows,
                               rows_hub, n_hub, workspace, workspace_bytes, top_k, thr, out, ldo, sel_src, sel_w, sel_q, sel_cnt,
                               inv_norm, inv_norm_ready, wt, ldw, b_w, beta, bias, diff, 0, nullptr, stream);
+}
+
+extern "C" size_t sng_edge_fwd_wide_workspace_bytes(int64_t n_chunks, int64_t c, int64_t num_edges, int64_t max_deg) {
+    // the chunk pass's partial sums and selected counts (c <= 32: the layout of sng_edge_fwd at top_k = 0), then the keys of
+    // the rows that do not fit the cut kernel's shared-memory stage
+    const size_t keys = max_deg > kCutKeys && num_edges > 0 ? (size_t)num_edges * sizeof(unsigned) + 256 : 0;
+    return sng_edge_fwd_workspace_bytes(n_chunks, c, 0) + keys;
+}
+
+extern "C" int sng_edge_fwd_wide(const float* h, int64_t n_total, int64_t n, int64_t row_offset, int64_t c, int64_t ldh,
+                                 const int32_t* rowptr, const int32_t* col, int64_t num_edges,
+                                 const int32_t* chunk_tab, int64_t n_chunks, const int32_t* lrows, const int32_t* lrow_ptr, int64_t n_lrows,
+                                 const int32_t* rows_hub, int64_t n_hub, void* workspace, size_t workspace_bytes,
+                                 int top_k, int64_t max_deg, float thr, float* out, int64_t ldo, uint8_t* sel_flag, int train,
+                                 float* inv_norm, int inv_norm_ready,
+                                 const float* wt, int64_t ldw, const float* b_w, const float* beta, const float* bias, float* diff,
+                                 int denominator, float* inv_denom, void* stream) {
+    if (int rc = check_rows("sng_edge_fwd_wide", n, c, ldh)) return rc;
+    SNG_REQUIRE(top_k > SNG_MAX_TOPK, "sng_edge_fwd_wide: top_k=%d must be > %d (smaller values: sng_edge_fwd)", top_k, SNG_MAX_TOPK);
+    SNG_REQUIRE(thr > -1.1f, "sng_edge_fwd_wide: thr must be > -1.1 (knock-out sentinel of R models.py:153)");
+    SNG_REQUIRE(denominator == 0 || denominator == 1, "sng_edge_fwd_wide: denominator=%d must be 0 (candidates) or 1 (selected)", denominator);
+    SNG_REQUIRE(!inv_denom || denominator == 1, "sng_edge_fwd_wide: inv_denom is an output of denominator=1 (selected)");
+    SNG_REQUIRE(h && rowptr && ((col && out) || n == 0) && ldo % 4 == 0 && ldo >= c, "sng_edge_fwd_wide: null pointer or bad ldo");
+    SNG_REQUIRE(row_offset >= 0 && row_offset + n <= n_total && n_total < (1ll << 31) && ldh < (1ll << 31) && ldo < (1ll << 31),
+                "sng_edge_fwd_wide: bad row_offset / n_total");
+    SNG_REQUIRE(num_edges >= 0 && num_edges < (1ll << 31) && max_deg >= 0, "sng_edge_fwd_wide: bad num_edges / max_deg");
+    SNG_REQUIRE(inv_norm, "sng_edge_fwd_wide: inv_norm [n_total] is required");
+    const bool cut = top_k < max_deg;                       // some row may have more in-edges than top_k
+    SNG_REQUIRE(sel_flag || (!train && !cut) || n == 0,
+                "sng_edge_fwd_wide: sel_flag [num_edges] is required in training and whenever top_k < max_deg");
+    SNG_REQUIRE(n_chunks <= 0 || (chunk_tab && lrows && lrow_ptr && n_lrows > 0 && n_chunks < (1ll << 31)), "sng_edge_fwd_wide: chunk tables missing");
+    SNG_REQUIRE(n_hub >= 0 && (n_hub == 0 || rows_hub), "sng_edge_fwd_wide: hub list missing");
+    SNG_REQUIRE(!wt || (b_w && beta && ldw % 4 == 0 && ldw >= c && ldw < (1ll << 31)), "sng_edge_fwd_wide: fused epilogue needs b_w, beta and a 16-byte aligned wt");
+    SNG_REQUIRE(wt || !diff, "sng_edge_fwd_wide: diff is an output of the fused epilogue");
+    if (n == 0 && (inv_norm_ready || n_total == 0)) return SNG_OK;
+    const bool staged = c <= 32 && n_chunks >= 0;
+    const size_t chunk_bytes = staged && n_chunks > 0 ? sng_edge_fwd_workspace_bytes(n_chunks, c, 0) : 0;
+    const bool global_keys = cut && max_deg > kCutKeys;
+    if ((chunk_bytes || global_keys) && (!workspace || workspace_bytes < sng_edge_fwd_wide_workspace_bytes(staged ? n_chunks : 0, c, num_edges, max_deg))) {
+        set_error("sng_edge_fwd_wide: workspace too small"); return SNG_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!inv_norm_ready)
+        SNG_DISPATCH_G(c, row_inv_norm_kernel<G><<<grid_resident(row_inv_norm_kernel<G>, n_total, kWarpsPerBlock * RowShape<G>::EPW * 4), kThreads, 0, st>>>(h, n_total, (int)c, ldh, inv_norm));
+    if (n == 0) return check_launch("sng_edge_fwd_wide");
+    EdgeFwdArgs a;
+    a.h = h; a.inv_r = inv_norm; a.n = (int)n; a.row_offset = (int)row_offset; a.c = (int)c; a.ldh = (int)ldh;
+    a.rowptr = rowptr; a.col = col; a.tpos = nullptr; a.rows = nullptr; a.n_rows = 0; a.skip_deg = 0;
+    a.top_k = top_k; a.thr = thr; a.out = out; a.ldo = (int)ldo;
+    a.inv_denom = inv_denom;
+    a.sel_src = nullptr; a.sel_w = nullptr; a.sel_q = nullptr; a.sel_cnt = nullptr;
+    a.wt = wt; a.ldw = (int)ldw; a.b_w = b_w; a.beta = beta; a.bias = bias; a.diff = diff;
+    a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab); a.n_chunks = staged ? (int)n_chunks : -1;
+    a.lrows = lrows; a.lrow_ptr = lrow_ptr; a.n_lrows = (int)n_lrows;
+    a.tmp_s = nullptr; a.tmp_p = nullptr; a.tmp_cnt = nullptr; a.tmp_acc = nullptr; a.tmp_a0 = nullptr;
+    a.eflag = sel_flag; a.eflag_write = train ? 1 : 0; a.cut_keys = nullptr;
+    if (chunk_bytes) {
+        const int64_t cg = 4 * group_lanes(c);
+        float* w = reinterpret_cast<float*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+        a.tmp_s = w; a.tmp_p = reinterpret_cast<int*>(w);            // (top_k = 0 layout: no candidate lists)
+        a.tmp_cnt = reinterpret_cast<int*>(w); w += n_chunks;
+        a.tmp_acc = w; w += n_chunks * cg;
+        a.tmp_a0 = w;
+    }
+    if (global_keys) a.cut_keys = reinterpret_cast<unsigned*>(((uintptr_t)workspace + chunk_bytes + 255) & ~(uintptr_t)255);
+    if (cut) {                                              // rows with deg > top_k are among the rows with deg > 32 (top_k > 64)
+        EdgeFwdArgs ac = a;
+        if (lrows && n_lrows > 0) { ac.rows = lrows; ac.n_rows = (int)n_lrows; }
+        const int64_t items = ac.rows ? n_lrows : n;
+        SNG_DISPATCH_G(c, edge_cut_kernel<G><<<grid_resident(edge_cut_kernel<G>, items, 1), kThreads, 0, st>>>(ac));
+    }
+    SNG_DISPATCH_G(c,
+        if (wt) { if (denominator) launch_edge_fwd<G, true, true, true, true>(a, rows_hub, n_hub, st);
+                  else launch_edge_fwd<G, true, true, false, true>(a, rows_hub, n_hub, st); }
+        else { if (denominator) launch_edge_fwd<G, false, true, true, true>(a, rows_hub, n_hub, st);
+               else launch_edge_fwd<G, false, true, false, true>(a, rows_hub, n_hub, st); });
+    return check_launch("sng_edge_fwd_wide");
 }
 
 namespace sng {
@@ -2200,7 +2450,8 @@ static int launch_edge_bwd(const EdgeBwdArgs& a, float* dbeta, cudaStream_t st, 
             if (staged_t) grid_t = launch_bwd_target_staged<G>(a, st);
         }
         if (!staged_t || G > 8) {
-            if (a.inv_denom) { grid_t = grid_resident(edge_bwd_target_kernel<G, false, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false, true><<<grid_t, kThreads, 0, st>>>(a); }
+            if (a.eflag) { grid_t = grid_resident(edge_bwd_target_kernel<G, true, false, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, true, false, true><<<grid_t, kThreads, 0, st>>>(a); }
+            else if (a.inv_denom) { grid_t = grid_resident(edge_bwd_target_kernel<G, false, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false, true><<<grid_t, kThreads, 0, st>>>(a); }
             else if (top_k > 0) { grid_t = grid_resident(edge_bwd_target_kernel<G, false>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, false><<<grid_t, kThreads, 0, st>>>(a); }
             else { grid_t = grid_resident(edge_bwd_target_kernel<G, true>, n, kWarpsPerBlock); edge_bwd_target_kernel<G, true><<<grid_t, kThreads, 0, st>>>(a); }
         }
@@ -2254,7 +2505,7 @@ extern "C" int sng_edge_bwd_denom(const float* h, const float* inv_norm, const f
     a.rowptr_out = rowptr_out; a.col_out = col_out; a.shift = (int)src_shift;
     a.dh = dh; a.dwt = dwt; a.lddw = (int)lddw;
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab_out); a.n_chunks = (int)n_chunks_out; a.lrows = lrows_out; a.lrow_ptr = lrow_ptr_out;
-    a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials;
+    a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials; a.eflag = nullptr;
     return launch_edge_bwd(a, dbeta, st, "sng_edge_bwd");
 }
 
@@ -2271,6 +2522,42 @@ extern "C" int sng_edge_bwd(const float* h, const float* inv_norm, const float* 
                               num_edges, top_k, sel_src, sel_w, sel_q, sel_cnt, beta, diff, lddiff, dbeta, coef, dn_target, partials,
                               dh, dwt, lddw, chunk_tab_out, n_chunks_out, lrows_out, lrow_ptr_out, n_lrows_out, chunk_partials,
                               nullptr, stream);
+}
+
+extern "C" int sng_edge_bwd_wide(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
+                                 int64_t c, int64_t ld, int64_t ldg,
+                                 const int32_t* rowptr, const int32_t* col, const int32_t* tpos,
+                                 const int32_t* rowptr_out, const int32_t* col_out, int64_t src_shift, int64_t num_edges,
+                                 const uint8_t* sel_flag, const float* inv_denom,
+                                 const float* beta, const float* diff, int64_t lddiff, float* dbeta,
+                                 float* coef, float* dn_target, float* partials, float* dh, float* dwt, int64_t lddw,
+                                 const int32_t* chunk_tab_out, int64_t n_chunks_out, const int32_t* lrows_out, const int32_t* lrow_ptr_out,
+                                 int64_t n_lrows_out, float* chunk_partials, void* stream) {
+    if (int rc = check_rows("sng_edge_bwd_wide", n_total, c, ld)) return rc;
+    SNG_REQUIRE(n >= 0 && row_offset >= 0 && row_offset + n <= n_total, "sng_edge_bwd_wide: bad n / row_offset / n_total");
+    SNG_REQUIRE(h && inv_norm && rowptr && rowptr_out && (col_out || num_edges == 0) && coef && dh && ldg % 4 == 0 && ldg >= c &&
+                (n == 0 || (g && dn_target)), "sng_edge_bwd_wide: null pointer or bad ldg");
+    SNG_REQUIRE(n == 0 || (col && tpos && sel_flag), "sng_edge_bwd_wide: missing CSR + tpos or the forward's sel_flag");
+    SNG_REQUIRE(!dwt || (beta && lddw % 4 == 0 && lddw >= c), "sng_edge_bwd_wide: dwt needs beta and a 16-byte aligned leading dimension");
+    SNG_REQUIRE(!dwt || (row_offset == 0 && n == n_total),
+                "sng_edge_bwd_wide: dwt needs a call over all rows (row_offset = 0, n = n_total); a row shard's pass S sees only its own out-edges");
+    SNG_REQUIRE(!dbeta || (beta && (diff || n == 0) && partials && lddiff % 4 == 0 && lddiff >= c), "sng_edge_bwd_wide: dbeta needs beta, diff and the partials workspace");
+    SNG_REQUIRE(src_shift >= 0 && num_edges >= 0 && num_edges < (1ll << 31), "sng_edge_bwd_wide: bad src_shift / num_edges");
+    SNG_REQUIRE(n_chunks_out <= 0 || (chunk_tab_out && lrows_out && lrow_ptr_out && n_lrows_out > 0 && chunk_partials),
+                "sng_edge_bwd_wide: by-source chunk tables / partials workspace missing");
+    if (n_total == 0) return SNG_OK;
+    EdgeBwdArgs a;
+    a.h = h; a.inv_r = inv_norm; a.g = g; a.n_total = (int)n_total; a.n = (int)n; a.row_offset = (int)row_offset;
+    a.c = (int)c; a.ld = (int)ld; a.ldg = (int)ldg;
+    a.rowptr = rowptr; a.col = col; a.tpos = tpos; a.top_k = 0;                // pass T walks every in-edge (select-every-edge form)
+    a.sel_src = nullptr; a.sel_w = nullptr; a.sel_q = nullptr; a.sel_cnt = nullptr; a.inv_denom = inv_denom;
+    a.beta = beta; a.diff = dbeta ? diff : nullptr; a.lddiff = (int)lddiff; a.dbeta_part = dbeta ? partials : nullptr;
+    a.coef = reinterpret_cast<float2*>(coef); a.dnT = dn_target;            // pass T writes every edge's coefficients: no memset
+    a.rowptr_out = rowptr_out; a.col_out = col_out; a.shift = (int)src_shift;
+    a.dh = dh; a.dwt = dwt; a.lddw = (int)lddw;
+    a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab_out); a.n_chunks = (int)n_chunks_out; a.lrows = lrows_out; a.lrow_ptr = lrow_ptr_out;
+    a.n_lrows = (int)n_lrows_out; a.tmp_part = chunk_partials; a.eflag = sel_flag;
+    return launch_edge_bwd(a, dbeta, (cudaStream_t)stream, "sng_edge_bwd_wide");
 }
 
 extern "C" int sng_list_bwd(const float* h, const float* inv_norm, const float* g, int64_t n_total, int64_t n, int64_t row_offset,
@@ -2299,7 +2586,7 @@ extern "C" int sng_list_bwd(const float* h, const float* inv_norm, const float* 
     a.rowptr_out = rowptr_tr; a.col_out = col_tr; a.shift = 0;
     a.dh = dh; a.dwt = nullptr; a.lddw = 0;
     a.chunk_tab = reinterpret_cast<const int4*>(chunk_tab); a.n_chunks = (int)n_chunks; a.lrows = lrows; a.lrow_ptr = lrow_ptr;
-    a.n_lrows = (int)n_lrows; a.tmp_part = chunk_partials;
+    a.n_lrows = (int)n_lrows; a.tmp_part = chunk_partials; a.eflag = nullptr;
     return launch_edge_bwd(a, nullptr, (cudaStream_t)stream, "sng_list_bwd");
 }
 

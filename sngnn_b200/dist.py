@@ -131,15 +131,15 @@ class AllGatherRows(torch.autograd.Function):
 def edge_agg_sharded(h_local, graph, top_k=None, thr=None, agg=None):
     """Differentiable out_1 rows [lo, hi): all-gather h (autograd-aware), then K2 on the shard; its backward produces the
     shard's contribution to dL/dh of every node, which AllGatherRows.backward reduce-scatters.
-    `agg(h_all, shard, row_offset, top_k, thr)` defaults to the CUDA kernels (functional.ShardedEdgeTopkAgg); the gloo tests
-    inject a differentiable CPU oracle."""
+    `agg(h_all, shard, row_offset, top_k, thr)` defaults to the CUDA kernels (functional.sharded_edge_agg: the selection lists,
+    or the per-edge form for top_k > SNG_MAX_TOPK); the gloo tests inject a differentiable CPU oracle."""
     ws, rank = world()
     n = graph.n
     lo, hi = shard_bounds(n, ws, rank)
     h_all = AllGatherRows.apply(h_local, n)
     shard = graph.row_slice(lo, hi)
     if agg is None:
-        agg = SF.ShardedEdgeTopkAgg.apply
+        agg = SF.sharded_edge_agg
     return agg(h_all, shard, lo, top_k, thr), shard
 
 
@@ -228,19 +228,27 @@ class _ShardedFusedAgg(torch.autograd.Function):
         h_all = SF._check_h(h_all)
         fuse = SF._structural_operands(w_weight, w_bias, beta, bias, h_all.size(1))
         train = any(ctx.needs_input_grad)
-        out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = SF._edge_fwd(h_all, shard, lo, int(top_k), thr, train, fuse, want_q=True)
+        if SF.per_edge_form(top_k):                              # selection saved as one flag per in-edge
+            out, flags, inv_norm, diff = SF._edge_fwd_wide(h_all, shard, lo, top_k, thr, train, fuse)
+            sel = (flags,)
+        else:
+            out, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff = SF._edge_fwd(h_all, shard, lo, int(top_k), thr, train, fuse, want_q=True)
+            sel = (sel_src, sel_w, sel_q, sel_cnt)
         ctx.shard, ctx.c, ctx.n, ctx.lo, ctx.k, ctx.has_bias = shard, w_weight.size(0), n, lo, int(top_k), bias is not None
-        ctx.save_for_backward(h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta)
+        ctx.save_for_backward(h_all, inv_norm, diff, beta, *sel)
         return out
 
     @staticmethod
     def backward(ctx, g):
-        h_all, sel_src, sel_w, sel_q, sel_cnt, inv_norm, diff, beta = ctx.saved_tensors
+        h_all, inv_norm, diff, beta, *sel = ctx.saved_tensors
         shard, c = ctx.shard, ctx.c
         g = g.contiguous()
         g0 = g * beta
         pending = _gather_row_blocks_async(g0, ctx.n)             # needed only for dL/dW^T below: overlaps the aggregation backward
-        dh, _, dbeta = SF.edge_bwd(h_all, inv_norm, g, shard, ctx.k, sel_src, sel_w, sel_q, sel_cnt, beta, diff, row_offset=ctx.lo)
+        if len(sel) == 1:
+            dh, _, dbeta = SF.edge_bwd_wide(h_all, inv_norm, g, shard, sel[0], beta, diff, row_offset=ctx.lo)
+        else:
+            dh, _, dbeta = SF.edge_bwd(h_all, inv_norm, g, shard, ctx.k, *sel, beta, diff, row_offset=ctx.lo)
         dw = _complete_dw(g0, shard, ctx.n, c, pending)
         dbias = g.sum(0)[:c] if ctx.has_bias else None
         return dh, dw, g0.sum(0)[:c], dbeta, dbias, None, None, None, None, None

@@ -213,17 +213,12 @@ class EdgeAgg(torch.autograd.Function):
         return dh, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None, None
 
 
-def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None, *, row_offset=0, inv_denom=None):
-    """sng_edge_bwd_denom: dL/dh [N, Cp] of the aggregation -- two gather passes, no float atomics -- and, with `beta` (the fused
-    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout.  inv_denom = the per-row factors _edge_fwd wrote under
-    denominator='selected' (None: 1 / max(in-degree, 1)).
-    Row shard (`graph` = PreparedGraph.row_slice(lo, hi), row_offset = lo, `h` / `inv_norm` of all N nodes, `g` / `diff` / the
-    lists of the shard's rows): dh is the shard's contribution to dL/dh of every node and dbeta its part of dL/dbeta, both
-    bit-reproducible; dL/dW^T is not computed (None): the caller assembles it from the g0 of every shard."""
-    n_total, cp = h.shape
+def _bwd_buffers(h, graph, fused):
+    """Outputs and workspaces of sng_edge_bwd_denom / sng_edge_bwd_wide: (coef, dn_target, dh, dbeta, dwt, partials, the
+    by-source chunk table (c <= 32) and its size, chunk partials)."""
+    cp = h.size(1)
     n = graph.n
     dev = h.device
-    fused = beta is not None
     coef = torch.empty(max(graph.num_edges, 1) * 2, dtype=torch.float32, device=dev)
     dnt = torch.empty(n, cp, dtype=torch.float32, device=dev)
     dh = torch.empty_like(h)
@@ -241,6 +236,20 @@ def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None
         while cg < cp:
             cg *= 2
         cpart = torch.empty(n_chunks * 3 * cg, dtype=torch.float32, device=dev)
+    return coef, dnt, dh, dbeta, dwt, part, tab, n_chunks, cpart
+
+
+def edge_bwd(h, inv_norm, g, graph, k, sel_src, sel_w, sel_q, sel_cnt, beta=None, diff=None, *, row_offset=0, inv_denom=None):
+    """sng_edge_bwd_denom: dL/dh [N, Cp] of the aggregation -- two gather passes, no float atomics -- and, with `beta` (the fused
+    SNGNN++ epilogue), dL/dW^T [N, Cp] and dL/dbeta.  `g` = dL/dout.  inv_denom = the per-row factors _edge_fwd wrote under
+    denominator='selected' (None: 1 / max(in-degree, 1)).
+    Row shard (`graph` = PreparedGraph.row_slice(lo, hi), row_offset = lo, `h` / `inv_norm` of all N nodes, `g` / `diff` / the
+    lists of the shard's rows): dh is the shard's contribution to dL/dh of every node and dbeta its part of dL/dbeta, both
+    bit-reproducible; dL/dW^T is not computed (None): the caller assembles it from the g0 of every shard."""
+    n_total, cp = h.shape
+    n = graph.n
+    fused = beta is not None
+    coef, dnt, dh, dbeta, dwt, part, tab, n_chunks, cpart = _bwd_buffers(h, graph, fused)
     _C.call("sng_edge_bwd_denom", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
             _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
             _C.ptr(graph.tpos), _C.ptr(graph.rowptr_tr), _C.ptr(graph.col_tr), graph.src_shift, graph.num_edges, k,
@@ -305,6 +314,124 @@ def edge_topk_agg(h, graph, top_k=None, thr=None, return_selection=False, struct
     if return_selection:
         return out, (sel_src, sel_w, sel_cnt)
     return out
+
+
+# ------------------------------------------------------------------------------------------ per-edge form (top_k > SNG_MAX_TOPK)
+def per_edge_form(top_k):
+    """True when `top_k` asks for more neighbours than the selection lists of sng_edge_fwd hold (SNG_MAX_TOPK): the layer then
+    runs the per-edge form (sng_edge_fwd_wide / sng_edge_bwd_wide), which saves one flag per in-edge instead of [N, top_k]
+    lists.  The one place where the models and the sharded forward choose between the two forms."""
+    return top_k is not None and int(top_k) > _C.MAX_TOPK
+
+
+def _edge_fwd_wide(h_all, graph, row_offset, top_k, thr, train, fuse=None, inv_norm=None, denominator="candidates", inv_denom=None):
+    """sng_edge_fwd_wide on the target rows of `graph` (a PreparedGraph or a row shard of one), arguments as _edge_fwd.
+    Returns (out, sel_flag [num_edges] uint8 | None, inv_norm, diff); sel_flag is written for every edge in training (the
+    backward's input) and exists in inference only when some row needs a cut.  Any top_k > SNG_MAX_TOPK: every value at or
+    above the largest in-degree selects the same set, so it is clamped there before the call."""
+    c = h_all.size(1)
+    n = graph.n
+    dev = h_all.device
+    k = max(_C.MAX_TOPK + 1, min(int(top_k), graph.max_deg))
+    out = torch.empty(n, c, dtype=torch.float32, device=dev)
+    flags = None
+    if train or k < graph.max_deg:
+        flags = torch.empty(max(graph.num_edges, 1), dtype=torch.uint8, device=dev)
+    inv_ready = inv_norm is not None
+    if not inv_ready:
+        inv_norm = torch.empty(h_all.size(0), dtype=torch.float32, device=dev)
+    wt = bw = beta = bias = diff = None
+    if fuse is not None:
+        wt, bw, beta, bias = fuse
+        if train:
+            diff = torch.empty_like(out)
+    tab = graph.chunk_tab
+    n_chunks = -1 if tab is None else int(tab.size(0))
+    wbytes = _C.lib().sng_edge_fwd_wide_workspace_bytes(n_chunks if c <= 32 else 0, c, graph.num_edges, graph.max_deg)
+    ws = torch.empty(wbytes, dtype=torch.uint8, device=dev) if wbytes else None
+    n_lrows = 0 if tab is None else int(graph.lrows.numel())
+    n_hub = 0 if graph.rows_hub is None else int(graph.rows_hub.numel())
+    _C.call("sng_edge_fwd_wide", h_all, _C.ptr(h_all), h_all.size(0), n, row_offset, c, c, _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in),
+            graph.num_edges, _C.ptr(tab), n_chunks, _C.ptr(graph.lrows), _C.ptr(graph.lrow_ptr), n_lrows, _C.ptr(graph.rows_hub), n_hub,
+            _C.ptr(ws), wbytes, k, graph.max_deg, float(thr if thr is not None else 0.0), _C.ptr(out), c, _C.ptr(flags), int(bool(train)),
+            _C.ptr(inv_norm), int(inv_ready), _C.ptr(wt), c, _C.ptr(bw), _C.ptr(beta), _C.ptr(bias), _C.ptr(diff),
+            _DENOMINATORS[denominator], _C.ptr(inv_denom))
+    return out, flags, inv_norm, diff
+
+
+def edge_bwd_wide(h, inv_norm, g, graph, flags, beta=None, diff=None, *, row_offset=0, inv_denom=None):
+    """sng_edge_bwd_wide: the backward of _edge_fwd_wide from its training flags -- edge_bwd's two gather passes, no float
+    atomics, bit-reproducible; outputs and row-shard convention as edge_bwd."""
+    n_total, cp = h.shape
+    n = graph.n
+    fused = beta is not None
+    coef, dnt, dh, dbeta, dwt, part, tab, n_chunks, cpart = _bwd_buffers(h, graph, fused)
+    _C.call("sng_edge_bwd_wide", h, _C.ptr(h), _C.ptr(inv_norm), _C.ptr(g), n_total, n, int(row_offset), cp, cp, cp,
+            _C.ptr(graph.rowptr_in), _C.ptr(graph.col_in), _C.ptr(graph.tpos), _C.ptr(graph.rowptr_tr), _C.ptr(graph.col_tr),
+            graph.src_shift, graph.num_edges, _C.ptr(flags), _C.ptr(inv_denom), _C.ptr(beta), _C.ptr(diff if fused else None), cp,
+            _C.ptr(dbeta), _C.ptr(coef), _C.ptr(dnt), _C.ptr(part), _C.ptr(dh), _C.ptr(dwt), cp,
+            _C.ptr(tab), n_chunks, _C.ptr(graph.lrows_out if tab is not None else None),
+            _C.ptr(graph.lrow_ptr_out if tab is not None else None), 0 if tab is None else int(graph.lrows_out.numel()), _C.ptr(cpart))
+    return dh, dwt, dbeta
+
+
+class EdgeWideAgg(torch.autograd.Function):
+    """EdgeAgg for top_k > SNG_MAX_TOPK (the per-edge form): the same layer outputs -- out_1, or with the structural parameters
+    the fused SNGNN++ layer on a graph whose in-lists equal its out-lists -- and the same gradients.  With row_offset / a
+    row shard of the graph, `h` holds every node and the backward returns the shard's contribution to dL/dh (fused: whole
+    graphs only; dist._ShardedFusedAgg assembles dL/dw.weight of a shard)."""
+
+    @staticmethod
+    def forward(ctx, h, graph, row_offset, top_k, thr, w_weight, w_bias, beta, bias, inv_norm=None, denominator="candidates"):
+        h = _check_h(h)
+        n, cp = h.shape
+        if not graph.is_shard and n != graph.n:
+            raise RuntimeError(f"h has {n} rows but the graph has {graph.n} nodes")
+        fused = w_weight is not None
+        train = any(ctx.needs_input_grad)
+        fuse = None
+        if fused:
+            _C.require_cuda(h, w_weight, w_bias, beta, bias)
+            if graph.is_shard or not graph.symmetric:
+                raise RuntimeError("the fused SNGNN++ pass needs a whole graph whose in-lists equal its out-lists")
+            if w_weight.size(1) != n:
+                raise RuntimeError(f"w.weight is [{w_weight.size(0)},{w_weight.size(1)}] but the graph has {n} nodes "
+                                   "(R builds w = Linear(num_nodes, out_channels), models.py:95)")
+            fuse = _structural_operands(w_weight, w_bias, beta, bias, cp)
+            ctx.c = w_weight.size(0)
+        inv_denom = torch.empty(graph.n, dtype=torch.float32, device=h.device) if train and denominator == "selected" else None
+        out, flags, inv_norm, diff = _edge_fwd_wide(h, graph, int(row_offset), top_k, thr, train, fuse, inv_norm, denominator, inv_denom)
+        ctx.graph, ctx.row_offset, ctx.fused, ctx.has_bias = graph, int(row_offset), fused, bias is not None
+        ctx.save_for_backward(h, flags, inv_norm, diff, beta if fused else None, inv_denom)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        h, flags, inv_norm, diff, beta, inv_denom = ctx.saved_tensors
+        g = g.contiguous()
+        dh, dwt, dbeta = edge_bwd_wide(h, inv_norm, g, ctx.graph, flags, beta, diff, row_offset=ctx.row_offset, inv_denom=inv_denom)
+        if not ctx.fused:
+            return dh, None, None, None, None, None, None, None, None, None, None
+        c = ctx.c
+        gsum = g.sum(0)[:c]
+        return dh, None, None, None, None, _weight_grad(dwt, c), gsum * beta, dbeta, (gsum if ctx.has_bias else None), None, None
+
+
+def edge_agg(h, graph, top_k, thr, structural=None, inv_norm=None, denominator="candidates"):
+    """The edge-candidate aggregation of the models at any top_k > 0: edge_topk_agg (selection lists) up to SNG_MAX_TOPK, the
+    per-edge form (EdgeWideAgg) above.  Arguments as edge_topk_agg."""
+    if not per_edge_form(top_k):
+        return edge_topk_agg(h, graph, top_k, thr, structural=structural, inv_norm=inv_norm, denominator=denominator)
+    w_weight, w_bias, beta, bias = structural if structural is not None else (None, None, None, None)
+    return EdgeWideAgg.apply(h, graph, 0, top_k, thr, w_weight, w_bias, beta, bias, inv_norm, denominator)
+
+
+def sharded_edge_agg(h_all, shard, row_offset, top_k, thr):
+    """out_1 of target rows [row_offset, row_offset + shard.n) from `h_all` (all nodes), differentiable: ShardedEdgeTopkAgg
+    up to SNG_MAX_TOPK, the per-edge form above (denominator='candidates')."""
+    if per_edge_form(top_k):
+        return EdgeWideAgg.apply(h_all, shard, int(row_offset), top_k, thr, None, None, None, None)
+    return ShardedEdgeTopkAgg.apply(h_all, shard, row_offset, top_k, thr)
 
 
 class ListTranspose:

@@ -111,7 +111,7 @@ class SNConv_plus(_SNConvBase):
         if self.top_k <= 0:
             return h * 0.0
         if self.candidates == "edges":
-            return SF.edge_topk_agg(h, g, self.top_k, self.thr, inv_norm=inv, denominator=self.denominator)
+            return SF.edge_agg(h, g, self.top_k, self.thr, inv_norm=inv, denominator=self.denominator)
         from . import simknn
         return simknn.allpairs_topk_agg(h, self.top_k, self.thr, bool(self.is_remove_self_loops), self.denominator)
 
@@ -163,8 +163,8 @@ class SNConv_plus_plus(SNConv_plus):
         h, inv = self._hidden_norm(x)
         if self.top_k > 0 and self.candidates == "edges" and g.symmetric:
             # in-lists == out-lists: the structural term rides on the aggregation's own pass over the edges (one kernel)
-            out = SF.edge_topk_agg(h, g, self.top_k, self.thr, structural=(self.w.weight, self.w.bias, self.beta, self.bias), inv_norm=inv,
-                                   denominator=self.denominator)
+            out = SF.edge_agg(h, g, self.top_k, self.thr, structural=(self.w.weight, self.w.bias, self.beta, self.bias), inv_norm=inv,
+                              denominator=self.denominator)
         else:
             out = SF.PPFuse.apply(self._aggregate(h, g, inv), self.w.weight, self.w.bias, self.beta, self.bias, g)
         return out[:, :self.lin.out_features]
