@@ -122,28 +122,29 @@ struct Stage1Params {
     int* phase;                   // [nsplit] sweep phase shared by all CTAs of a column split (see "Phase alignment"), or nullptr
 };
 
-// MMA issue loop of the SPLIT (four 128-column accumulator stages) mode for issuer W of NI, kblocks <= 2.  W / NI are compile
-// time so that every address, descriptor and ring index below is provably warp-uniform and stays in uniform registers: on a
-// busy SM the issuer's dependent instruction chain, not the tensor pipe, sets the tile period (per-tile clock stamps).
-template <int W, int NI>
+// MMA issue loop of the SPLIT mode (four 128-column accumulator stages, kblocks <= 2) for issuer W of two: tiles tt = W, W + 2,
+// ..., half h of a tile into stage 2 W + h.  On a busy SM the issuer's dependent instruction chain, not the tensor pipe, sets
+// the tile period (per-tile clock stamps), so everything is compile time that can be: W (every address, descriptor and ring
+// index stays warp-uniform, in uniform registers) and the K steps of the two K blocks, KS0 and KS1: runtime step counts put a
+// predicate set-up and register moves in front of every MMA (~230 instructions per tile in SASS), compile-time ones make a
+// half one straight run of KS0 + KS1 MMAs.
+template <int W, int KS0, int KS1>
 __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base, uint32_t a_off, uint32_t b_off, uint32_t bar_full, uint32_t bar_empty,
                                             uint32_t bar_tfull, uint32_t bar_tempty, int t_beg, int t_end, bool issuer) {
     constexpr uint32_t kIdescHalf = f16_idesc(256, 128);
+    constexpr int kKb = KS1 > 0 ? 2 : 1;                     // K blocks of a tile
+    constexpr int acc0 = 2 * W;                              // tt & 1 == W
     const uint64_t adesc0 = make_smem_desc(base + a_off);
     const uint64_t bdesc0 = make_smem_desc(base + b_off);
-    const int kb2 = p.kblocks == 2;                          // second K block present
-    const int ks0 = kb2 ? 4 : p.ksteps_last;                 // K steps of block 0
-    const int ks1 = kb2 ? p.ksteps_last : 0;                 // K steps of block 1
-    const int nst = p.stages, step = NI * p.kblocks;
-    int st0 = (W * p.kblocks) % nst;                         // ring slot of this tile's K block 0
-    uint32_t ph0 = (uint32_t)((W * p.kblocks) / nst) & 1u;
-    for (int tt = W; tt < t_end - t_beg; tt += NI) {
-        const int st1 = st0 + 1;                             // same ring lap: stages % kblocks == 0
+    const int nst = p.stages;
+    int st0 = (W * kKb) % nst;                               // ring slot of this tile's K block 0
+    uint32_t ph0 = (uint32_t)((W * kKb) / nst) & 1u;
+    for (int tt = W; tt < t_end - t_beg; tt += 2) {
         const uint32_t acc_phase = (uint32_t)(tt >> 1) & 1u;
-        const int acc0 = 2 * (tt & 1);
-        const uint64_t b0 = bdesc0 + (uint64_t)(st0 * (kTileBytes >> 4)), b1 = bdesc0 + (uint64_t)(st1 * (kTileBytes >> 4));
+        // K block 1 sits in the next ring slot (same ring lap: stages % kblocks == 0)
+        const uint64_t b0 = bdesc0 + (uint64_t)(st0 * (kTileBytes >> 4)), b1 = b0 + (uint64_t)(kTileBytes >> 4);
         mbar_wait(bar_full + 8 * st0, ph0);                  // every K block of the tile landed (one barrier per tile)
-        mbar_wait(bar_tempty + 8 * (tt & 1), acc_phase ^ 1); // both accumulator halves of this tile parity drained
+        mbar_wait(bar_tempty + 8 * W, acc_phase ^ 1);        // both accumulator halves of this tile parity drained
         tc_fence_after();
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
@@ -151,19 +152,37 @@ __device__ __forceinline__ void issue_split(const Stage1Params& p, uint32_t base
             const uint64_t hb = (uint64_t)(h * (kTileBytes >> 5));                       // + 64 rows x 128 B
             if (issuer) {
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks)
-                    if (ks < ks0) umma_f16_pair(tmem_d, adesc0 + (uint64_t)(ks * 2), b0 + hb + (uint64_t)(ks * 2), kIdescHalf, ks != 0 ? 1u : 0u);
+                for (int ks = 0; ks < KS0; ++ks)
+                    umma_f16_pair(tmem_d, adesc0 + (uint64_t)(ks * 2), b0 + hb + (uint64_t)(ks * 2), kIdescHalf, ks != 0 ? 1u : 0u);
 #pragma unroll
-                for (int ks = 0; ks < 4; ++ks)
-                    if (ks < ks1) umma_f16_pair(tmem_d, adesc0 + (uint64_t)((kTileBytes >> 4) + ks * 2), b1 + hb + (uint64_t)(ks * 2), kIdescHalf, 1u);
+                for (int ks = 0; ks < KS1; ++ks)
+                    umma_f16_pair(tmem_d, adesc0 + (uint64_t)((kTileBytes >> 4) + ks * 2), b1 + hb + (uint64_t)(ks * 2), kIdescHalf, 1u);
                 if (h == 1) umma_commit_pair(bar_empty + 8 * st0);                       // both halves read: free the tile's B slots
                 umma_commit_pair(bar_tfull + 8 * (acc0 + h));
             }
             __syncwarp();
         }
-        st0 += step;
+        st0 += 2 * kKb;
         while (st0 >= nst) { st0 -= nst; ph0 ^= 1u; }
     }
+}
+// the SPLIT plans: one K block of 1..4 K steps (d <= 64) or a full block plus 1..4 steps (64 < d <= 128)
+template <int W>
+__device__ __forceinline__ void issue_split_any(const Stage1Params& p, uint32_t base, uint32_t a_off, uint32_t b_off, uint32_t bar_full,
+                                                uint32_t bar_empty, uint32_t bar_tfull, uint32_t bar_tempty, int t_beg, int t_end, bool issuer) {
+#define SNG_ISSUE_SPLIT(KS0, KS1) issue_split<W, KS0, KS1>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer)
+    switch (p.kblocks * 8 + p.ksteps_last) {
+        case 9:  SNG_ISSUE_SPLIT(1, 0); break;
+        case 10: SNG_ISSUE_SPLIT(2, 0); break;
+        case 11: SNG_ISSUE_SPLIT(3, 0); break;
+        case 12: SNG_ISSUE_SPLIT(4, 0); break;
+        case 17: SNG_ISSUE_SPLIT(4, 1); break;
+        case 18: SNG_ISSUE_SPLIT(4, 2); break;
+        case 19: SNG_ISSUE_SPLIT(4, 3); break;
+        case 20: SNG_ISSUE_SPLIT(4, 4); break;
+        default: __trap();                                   // not a SPLIT plan: the epilogue would wait forever
+    }
+#undef SNG_ISSUE_SPLIT
 }
 
 // EW = epilogue warps per TMEM lane quarter; every epilogue thread owns one query row x (256/EW) columns of each tile; the
@@ -354,9 +373,8 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             auto advance = [&](int steps) { for (int i = 0; i < steps; ++i) if (++stage == p.stages) { stage = 0; phase ^= 1; } };
             advance(w * p.kblocks);
             if constexpr (SPLIT) {
-                if (p.issuers == 1) issue_split<0, 1>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
-                else if (warp == 1) issue_split<0, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
-                else issue_split<1, 2>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
+                if (warp == 1) issue_split_any<0>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
+                else issue_split_any<1>(p, base, a_off, b_off, bar_full, bar_empty, bar_tfull, bar_tempty, t_beg, t_end, issuer);
             } else {
             for (int tt = w; tt < T; tt += p.issuers) {
                 const int acc = tt & 1;
