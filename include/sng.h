@@ -42,7 +42,7 @@ extern "C" {
 #define SNG_MAX_TOPK 64          /* edge path lists: top_k <= 64 (larger: sng_edge_fwd_wide); top_k <= 0 means "select every edge" */
 #define SNG_MAX_CHANNELS 512     /* padded row width c of sng_edge_fwd / _bwd, sng_edge_agg_bwd, sng_list_agg_fwd, sng_spmm_fwd,
                                     sng_pp_fuse_fwd / _bwd; wider rows return SNG_ERR_UNSUPPORTED */
-#define SNG_KNN_MAX_TOPK 64      /* all-pairs builder */
+#define SNG_KNN_MAX_TOPK 64      /* all-pairs builder sng_simknn_build (larger top_k: sng_simknn_wide_count / _select) */
 #define SNG_SIMHIST_MAX_BINS 4096 /* sng_simhist_f16: two 32-bit sub-histograms of this many bins take half of its 64 KiB */
 
 SNG_API int sng_version(void);
@@ -196,7 +196,8 @@ SNG_API int sng_edge_bwd_wide(const float* h, const float* inv_norm, const float
                  int64_t n_lrows_out, float* chunk_partials, void* stream);
 
 /* Gather form of the backward of sng_list_agg_fwd (explicit neighbour lists: the all-pairs mode) -- the same two passes and
- * kernels as sng_edge_bwd, no float atomics, bit-reproducible.  The lists are those of sng_simknn_build: idx / sim [n, top_k]
+ * kernels as sng_edge_bwd, no float atomics, bit-reproducible.  Any list width top_k >= 1 (n * top_k < 2^31): lists longer
+ * than 32 are walked from memory by pass T.  The lists are those of sng_simknn_build / _wide_select: idx / sim [n, top_k]
  * (global column ids in rank order, sim = cosine of h_i and h_j), cnt [n]; entries t < cnt[i] <= top_k are node ids, the
  * rest is padding.  inv_denom [n] = the forward's per-row factor (1 / denominator).  g = dL/dout [n, ldg].
  * sel_q / rowptr_tr / col_tr: the transpose of the lists (sng_list_transpose), the by-source CSR over all n_total nodes.
@@ -466,6 +467,28 @@ SNG_API int sng_simknn_seed(const uint16_t* xq_f16, const uint16_t* xall_f16, in
 /* Launch plan of sng_simknn_build for a shape: out8 = {epilogue warps per lane quarter, candidate slots per list,
  * column splits, seed stride (0 = no seed pass), seed quantile, B ring stages, K blocks of 64, lists per row}. */
 SNG_API int sng_simknn_plan(int64_t nq, int64_t n, int64_t d, int top_k, int32_t* out8);
+
+/* Wide all-pairs build: any top_k >= 1 (int64; 2^40 = every column with cosine >= thr), the selection rule of
+ * sng_simknn_build.  Lists have k_eff = min(top_k, n - remove_self) entries: idx / sim [nq, k_eff], cnt [nq]; nq * k_eff
+ * must be < 2^31.  Query rows [q_offset, q_offset + nq) must be rows of the database.  Two calls on the same workspace
+ * (>= sng_simknn_wide_workspace_bytes(nq, n, d, top_k); the second call reads what the first left there):
+ *   sng_simknn_wide_count: seed pass (its stride chosen from k_eff) -> every row's emission threshold T_i -> a tensor-core
+ *     sweep counting the columns whose FP16 score is >= T_i -> offsets [nq + 1] int64 = their exclusive scan (a row with more
+ *     than 16384 candidates gets none); offsets[nq] = the candidate total.
+ *   sng_simknn_wide_select: a second sweep writes the candidate column ids into cand [offsets[nq]] int32 (allocated by the
+ *     caller from the total), then every row is rescored in FP32 (the exact score of sng_simknn_build), sorted by
+ *     (sim desc, index asc) and proven; rows that cannot be proven, or have too many candidates, are recomputed by an exact
+ *     FP32 scan of all n columns.  n_exact (device int32, may be NULL) = the number of such rows.
+ * Neither call synchronises; the caller reads offsets[nq] back to size cand. */
+SNG_API size_t sng_simknn_wide_workspace_bytes(int64_t nq, int64_t n, int64_t d, int64_t top_k);
+SNG_API int sng_simknn_wide_count(const uint16_t* xq_f16, const uint16_t* xall_f16, int64_t ldh,
+                      int64_t nq, int64_t q_offset, int64_t n, int64_t d, int64_t top_k, float thr, int remove_self,
+                      int64_t* offsets, void* workspace, size_t workspace_bytes, void* stream);
+SNG_API int sng_simknn_wide_select(const uint16_t* xq_f16, const uint16_t* xall_f16, int64_t ldh,
+                      const float* xq_f32, const float* xall_f32, int64_t ld32,
+                      int64_t nq, int64_t q_offset, int64_t n, int64_t d, int64_t top_k, float thr, int remove_self,
+                      const int64_t* offsets, int32_t* cand, int32_t* idx, float* sim, int32_t* cnt, int32_t* n_exact,
+                      void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -4,7 +4,10 @@ SNGNN_Plus and SNGNN_Plus_Plus (symmetric graph: the fused pass; asymmetric: agg
 denominators, hidden widths 32 and 128: one training forward + backward per library on the same seeded inputs and parameters,
 and every output and parameter gradient compared with torch.equal.
 
-    python scripts/lib_parity.py --ref-lib PATH [--out FILE]
+    python scripts/lib_parity.py --ref-lib PATH [--candidates all_pairs] [--out FILE]
+
+With --candidates all_pairs the models select among all nodes, and simknn.build_knn's lists at the same top_k are compared
+too.
 
 Prints one JSON object; exits non-zero when any tensor differs."""
 import argparse
@@ -42,6 +45,7 @@ def step(model, data, y):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--ref-lib", required=True)
+    ap.add_argument("--candidates", default="edges", choices=("edges", "all_pairs"))
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -51,6 +55,19 @@ def main():
     x = synth.make_features(n, fd, "clustered", seed=1).cuda()
     y = synth.make_labels(n, ncls, seed=3).cuda()
     rows, ok = [], True
+    if args.candidates == "all_pairs":
+        from sngnn_b200 import simknn
+        for k in (1, 10, 64):
+            new = simknn.build_knn(x, k, 0.2, True)
+            this, _C._lib = _C._lib, ref_lib
+            try:
+                old = simknn.build_knn(x, k, 0.2, True)
+            finally:
+                _C._lib = this
+            same = all(torch.equal(a, b) for a, b in zip(new, old))
+            ok &= same
+            rows.append(dict(build_knn=True, top_k=k, bit_identical=same))
+            print(json.dumps(rows[-1]), file=sys.stderr, flush=True)
     for symmetric in (True, False):
         ei = synth.make_graph(n, 300000, seed=2, symmetric=symmetric, hub_offset=3.0).cuda()
         data = synth.GraphData(x, ei)
@@ -62,7 +79,8 @@ def main():
                         torch.manual_seed(0)
                         cls = M.SNGNN_Plus if kind == "SNGNN_Plus" else M.SNGNN_Plus_Plus
                         extra = (0.5,) if kind == "SNGNN_Plus_Plus" else ()
-                        model = cls(fd, hid, ncls, n, 2, k, 0.2, *extra, 1, 0.0, denominator=den).cuda().train()
+                        model = cls(fd, hid, ncls, n, 2, k, 0.2, *extra, 1, 0.0, denominator=den,
+                                    candidates=args.candidates).cuda().train()
                         other = copy.deepcopy(model)
                         new = step(model, data, y)
                         this, _C._lib = _C._lib, ref_lib

@@ -72,6 +72,10 @@ SIGNATURES = {
                                  _P, _I32, _I32, _P, _P]),
     "sng_simknn_seed": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _I32, _I32, _P, _P]),
     "sng_simknn_plan": (_I32, [_I64, _I64, _I64, _I32, _P]),
+    "sng_simknn_wide_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64]),
+    "sng_simknn_wide_count": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _F32, _I32, _P, _P, _SZ, _P]),
+    "sng_simknn_wide_select": (_I32, [_P, _P, _I64, _P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _F32, _I32,
+                                      _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
 }
 
 
@@ -112,6 +116,7 @@ def ptr(t):
 PARTIALS = 4096          # SNG_PARTIALS of include/sng.h
 MAX_CHANNELS = 512       # SNG_MAX_CHANNELS of include/sng.h
 MAX_TOPK = 64            # SNG_MAX_TOPK of include/sng.h: larger top_k take the per-edge form (sng_edge_fwd_wide)
+KNN_MAX_TOPK = 64        # SNG_KNN_MAX_TOPK of include/sng.h: larger top_k take the wide all-pairs build (sng_simknn_wide_count)
 
 
 def stream(t=None):

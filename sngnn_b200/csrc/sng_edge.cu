@@ -2569,7 +2569,8 @@ extern "C" int sng_list_bwd(const float* h, const float* inv_norm, const float* 
                             float* chunk_partials, void* stream) {
     if (int rc = check_rows("sng_list_bwd", n_total, c, ld)) return rc;
     SNG_REQUIRE(n >= 0 && row_offset >= 0 && row_offset + n <= n_total, "sng_list_bwd: bad n / row_offset / n_total");
-    SNG_REQUIRE(top_k > 0 && top_k <= SNG_MAX_TOPK, "sng_list_bwd: list width top_k=%d must be in [1, %d]", top_k, SNG_MAX_TOPK);
+    // (any width: lists longer than 32 take the pass-T kernel that walks them from memory, edge_bwd_target_kernel<G, false, true>)
+    SNG_REQUIRE(top_k > 0 && n * (int64_t)top_k < (1ll << 31), "sng_list_bwd: list width top_k=%d must be >= 1 with n * top_k < 2^31", top_k);
     // (an empty shard, n == 0, has no rows of g / dn_target / the lists, and no transposed entries: those may be NULL)
     SNG_REQUIRE(h && inv_norm && rowptr_tr && dh && ldg % 4 == 0 && ldg >= c, "sng_list_bwd: null pointer or bad ldg");
     SNG_REQUIRE(n == 0 || (g && idx && sim && cnt && inv_denom && sel_q && col_tr && coef && dn_target), "sng_list_bwd: missing lists / transpose / workspace");

@@ -180,7 +180,7 @@ extern "C" int sng_graph_prepare(const int64_t* edge_index, int64_t num_edges, i
 }
 
 extern "C" size_t sng_list_transpose_workspace_bytes(int64_t nq, int64_t k, int64_t n_total) {
-    if (nq < 0 || k <= 0 || k > SNG_MAX_TOPK || n_total < 0 || n_total >= (1ll << 31) || nq * k >= (1ll << 31)) return 0;
+    if (nq < 0 || k <= 0 || k >= (1ll << 31) || n_total < 0 || n_total >= (1ll << 31) || nq * k >= (1ll << 31)) return 0;
     const int64_t total = nq * k;
     return 4 * al256((size_t)total * 4) + al256(sort_temp_bytes(total, key_bits(n_total))) + 256;
 }

@@ -22,6 +22,8 @@
 // smaller; kind::f16 runs FP16 and BF16 at the same rate.
 #include "sng_sm100.cuh"
 #include <cuda_fp16.h>
+#include <cub/block/block_scan.cuh>
+#include <cub/device/device_scan.cuh>
 #include <math_constants.h>
 #include <stdlib.h>
 
@@ -195,7 +197,13 @@ __device__ __forceinline__ void issue_split_any(const Stage1Params& p, uint32_t 
 // score >= tau, so >= top_k columns of the full set do unless >= seed_q of the row's true top_k fell into the 1/stride
 // sample (probability chosen < 2e-5 on the host).  As with every pruning threshold here, a bad tau costs time, never
 // correctness: tau is reported through cand_min and stage 2 sends unproven rows to the exact scan.
-template <int EW, bool SEED>
+//
+// WIDE (the wide build, top_k > SNG_KNN_MAX_TOPK; see "Wide build" below): no lists, no queue, no list warp.  Every row has a
+// fixed emission threshold T (p.seeds = T [nq]); a column passes when its FP16 score is >= T.  WIDE == 1 (count) adds the
+// passing columns of each row into p.cand_idx [nq]; WIDE == 2 (emit) appends their ids to the row's slice of the candidate
+// buffer: p.cand_min holds the buffer (int32), p.cand_val the slice offsets (int64 [nq + 1]), p.cand_idx the per-row cursor.
+// (Stage1Params gains no field for this: its size is part of how ptxas schedules the existing instances.)
+template <int EW, bool SEED, int WIDE = 0>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kNonEpiThreads + 128 * EW, 1)
 simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_db, const Stage1Params p) {
     constexpr int CPT = BN / EW;                                  // columns per thread per tile
@@ -268,7 +276,8 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
             float tau = p.thr_lo;
             const int grow = row0 + i;
             if (!SEED && grow >= nq_eff) tau = CUDART_INF_F;         // rows beyond the query matrix (TMA zero fill / stale retry slots) never hit
-            if (!SEED && p.seeds != nullptr && grow < nq_eff) {
+            if (WIDE != 0 && grow < nq_eff) tau = __ldg(p.seeds + grow);
+            if (WIDE == 0 && !SEED && p.seeds != nullptr && grow < nq_eff) {
                 const int srow = p.row_ids ? __ldg(p.row_ids + grow) : grow;     // retry pass: the seeds belong to the original row
                 float g[kSeedGroups];
 #pragma unroll
@@ -410,7 +419,7 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         // columns).  Everything data dependent and slow happens here, off the warps whose pace gates the tensor pipe: an
         // accumulator stage is reusable only once ALL 32 epilogue warps of the pair have drained it, and on a busy SM a
         // dependent chain of ~150 instructions (the former in-line insert) costs ~1900 cycles, three tile periods.
-        if (!SEED) {
+        if (!SEED && WIDE == 0) {
             const int L = p.cand;
             unsigned tail = 0;
             while (true) {
@@ -507,6 +516,7 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
         float gmax[2 * CT];                                        // SEED: running maxima of this thread's column groups
 #pragma unroll
         for (int i = 0; i < 2 * CT; ++i) gmax[i] = -CUDART_INF_F;
+        int wcnt = 0;                                              // WIDE == 1: passing columns of this thread's share of the row
 
         // Pruning thresholds are heuristics: ANY threshold is safe because the row reports the largest threshold anything
         // was pruned with (cand_min) and stage 2 only accepts a row whose k-th exact score clears it.
@@ -521,6 +531,30 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 return max3(max3(m0, m1, m2), m[9], m[10]);
             };
             float mx = tree();
+            if constexpr (WIDE != 0) {
+                if (mx >= thr_cur) {
+                    if ((unsigned)(self_col - col0) < 32u || col0 + 32 > n) {
+#pragma unroll
+                        for (int i = 0; i < 32; ++i) if (col0 + i == self_col || col0 + i >= n) v[i] = 0xff800000u;
+                    }
+                    unsigned m = 0u;
+#pragma unroll
+                    for (int i = 0; i < 32; ++i) m |= (__uint_as_float(v[i]) >= thr_cur ? 1u : 0u) << i;
+                    if (WIDE == 1) {
+                        wcnt += __popc(m);
+                    } else if (m != 0u) {
+                        const long long* off = reinterpret_cast<const long long*>(p.cand_val);
+                        const long long o = off[grow];
+                        const int len = (int)(off[grow + 1] - o);
+                        int at = atomicAdd(p.cand_idx + grow, __popc(m));
+                        int* buf = reinterpret_cast<int*>(p.cand_min);
+#pragma unroll
+                        for (int i = 0; i < 32; ++i)
+                            if ((m >> i) & 1u) { if (at < len) buf[o + at] = col0 + i; ++at; }   // (a row over its slice: see wide_select_kernel)
+                    }
+                }
+                return;
+            }
             if (SEED) {
                 if (col0 + 32 > n) {                                 // last tile: zero-filled columns beyond n must not count
                     mx = -CUDART_INF_F;
@@ -610,6 +644,8 @@ simknn_stage1_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_con
                 for (int i = 0; i < 2 * CT; ++i)
                     p.seed_out[(size_t)grow * kSeedGroups + (i / CT) * 8 + (tile_col >> 5) + (i % CT)] = gmax[i];
             }
+        } else if (WIDE != 0) {
+            if (WIDE == 1 && grow < nq_eff && wcnt > 0) atomicAdd(p.cand_idx + grow, wcnt);
         } else {
             __syncwarp();
             __threadfence_block();
@@ -940,6 +976,243 @@ __global__ void __launch_bounds__(256) simknn_fb_stream_kernel(
     }
 }
 
+// ------------------------------------------------------------------------------------------ wide build (top_k > SNG_KNN_MAX_TOPK)
+// Lists longer than 64 do not fit in shared memory next to the pipeline, so the wide build keeps no list there.  It bounds
+// every row from below instead and keeps every column that can reach the bound:
+//   1. T_i, the row's emission threshold: the seed pass's q-th largest group maximum tau_i minus 2 eps, raised to thr - eps.
+//      q sampled columns score >= tau_i in FP16, so with high probability >= k_eff columns of the database score >= tau_i
+//      - eps = T_i + eps exactly (q and the stride come from k_eff, see wide_plan).
+//   2. count sweep (stage-1 kernel, WIDE = 1): c_i = the columns whose FP16 score is >= T_i; an exclusive scan of the c_i
+//      gives every row its slice of the caller's candidate buffer (sng_simknn_wide_count);
+//   3. emit sweep (WIDE = 2): the same test appends the ids of those columns to the row's slice;
+//   4. wide_select_kernel: exact FP32 rescore (dot_seq: the score of K1's stage 2, so a pair scores the same bits in both
+//      builders), sort by (score desc, index asc), cut at thr and k_eff.  A column left out scores < T_i + eps exactly
+//      (|FP16 score - exact| <= eps), so the row is proven when its k_eff-th exact score is > T_i + eps, or when fewer than
+//      k_eff columns reach thr and T_i was not raised above thr - eps (then every column >= thr was emitted);
+//   5. wide_exact_kernel: rows that are not proven, or have more than kWideSortCap candidates, are recomputed by an exact
+//      FP32 scan of all n columns: a radix select of the cut, no candidate buffer.  No path is heuristic.
+constexpr int kWideSortCap = 16384;     // candidates a block sorts in shared memory: 128 KiB of 64-bit keys
+constexpr int kWideThreads = 256;
+constexpr size_t kWideSmem = (size_t)kWideSortCap * 8;
+
+__device__ __forceinline__ uint32_t order_key(float s) {      // order-preserving: larger score <-> larger key
+    const uint32_t u = __float_as_uint(s);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key_score(uint32_t k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
+// ascending 64-bit sort key = (score desc, index asc)
+__device__ __forceinline__ unsigned long long rank_key(float s, int j) { return ((unsigned long long)(~order_key(s)) << 32) | (uint32_t)j; }
+__device__ __forceinline__ float rank_key_score(unsigned long long k) { return key_score(~(uint32_t)(k >> 32)); }
+
+// ascending bitonic sort of key[0, p2) (p2 a power of two) by the whole block
+__device__ void block_bitonic(unsigned long long* key, int p2) {
+    for (int k = 2; k <= p2; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < p2; i += blockDim.x) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const unsigned long long a = key[i], b = key[ixj];
+                    if ((a > b) == ((i & k) == 0)) { key[i] = b; key[ixj] = a; }
+                }
+            }
+        }
+    __syncthreads();
+}
+
+// T_i (step 1).  seeds == nullptr (no seed pass): T_i = thr - eps, every column that can reach thr is a candidate.
+__global__ void __launch_bounds__(256) wide_tau_kernel(const float* __restrict__ seeds, int nq, int q_offset, int remove_self, int seed_q,
+                                                       int seed_stride, float eps, float t_floor, float* __restrict__ tau) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nq; i += gridDim.x * blockDim.x) {
+        float t = t_floor;
+        if (seeds) {
+            float g[kSeedGroups];
+            for (int j = 0; j < kSeedGroups; ++j) g[j] = seeds[(size_t)i * kSeedGroups + j];
+            const int self = q_offset + i;                             // the row itself may sit in the sample: drop its group
+            if (remove_self && self % seed_stride == 0) {
+                const int cs = self / seed_stride;
+                g[((cs >> 8) & 1) * 8 + ((cs & 255) >> 5)] = -CUDART_INF_F;
+            }
+            float cur = CUDART_INF_F;
+            for (int r = 0; r < seed_q; ++r) {                         // seed_q-th largest by repeated removal of the maximum
+                int at = 0;
+                for (int j = 1; j < kSeedGroups; ++j) if (g[j] > g[at]) at = j;
+                cur = g[at];
+                g[at] = -CUDART_INF_F;
+            }
+            t = fmaxf(t, cur - 2.0f * eps);
+        }
+        tau[i] = t;
+    }
+}
+
+// slice lengths for the scan: rows with more candidates than a block sorts get none (wide_select_kernel sends them to the scan)
+__global__ void __launch_bounds__(256) wide_len_kernel(const int* __restrict__ cnt, int nq, long long* __restrict__ len) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i <= nq; i += gridDim.x * blockDim.x)
+        len[i] = (i < nq && cnt[i] <= kWideSortCap) ? cnt[i] : 0;
+}
+
+// step 4: one block per row
+__global__ void __launch_bounds__(kWideThreads) wide_select_kernel(
+    const float* __restrict__ xq, const float* __restrict__ xall, int64_t ld32, int d4, int nq, int n, int q_offset, int remove_self,
+    int k_eff, float thr, float eps, float t_floor, const float* __restrict__ tau, const int* __restrict__ cnt, const int* __restrict__ cursor,
+    const long long* __restrict__ off, const int* __restrict__ cand, int* __restrict__ idx_out, float* __restrict__ sim_out,
+    int* __restrict__ cnt_out, int* __restrict__ ex_rows, int* __restrict__ n_ex) {
+    extern __shared__ unsigned long long wkey[];
+    __shared__ int s_nv;
+    for (int row = blockIdx.x; row < nq; row += gridDim.x) {
+        const float* a = xq + (int64_t)row * ld32;
+        const int self_col = remove_self ? q_offset + row : -1;
+        int* io = idx_out + (size_t)row * k_eff;
+        float* so = sim_out + (size_t)row * k_eff;
+        bool nz = false;
+        for (int k4 = threadIdx.x; k4 < d4; k4 += blockDim.x) { const float4 v = ldg4(a + 4 * k4); nz = nz || v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f; }
+        if (threadIdx.x == 0) s_nv = 0;
+        if (!__syncthreads_or(nz)) {
+            // all-zero row (as in stage 2): every score is exactly 0, the list is the lowest column ids when 0 >= thr
+            const int avail = n - ((self_col >= 0 && self_col < n) ? 1 : 0);
+            const int c0 = 0.0f >= thr ? min(k_eff, avail) : 0;
+            for (int t = threadIdx.x; t < k_eff; t += blockDim.x) {
+                io[t] = t < c0 ? ((self_col >= 0 && t >= self_col) ? t + 1 : t) : -1;
+                so[t] = 0.f;
+            }
+            if (threadIdx.x == 0) cnt_out[row] = c0;
+            continue;
+        }
+        const int c = cnt[row];
+        if (c > kWideSortCap || cursor[row] != c) {                 // (cursor != count: the sweeps disagreed; never seen, but exact anyway)
+            if (threadIdx.x == 0) ex_rows[atomicAdd(n_ex, 1)] = row;
+            continue;
+        }
+        const long long o = off[row];
+        int p2 = 1;
+        while (p2 < c) p2 <<= 1;
+        int nv = 0;
+        for (int m = threadIdx.x; m < p2; m += blockDim.x) {
+            unsigned long long key = ~0ull;
+            if (m < c) {
+                const int j = cand[o + m];
+                const float s = dot_seq(a, xall + (int64_t)j * ld32, d4);
+                if (s >= thr) { key = rank_key(s, j); ++nv; }
+            }
+            wkey[m] = key;
+        }
+        if (nv) atomicAdd(&s_nv, nv);
+        block_bitonic(wkey, p2);
+        nv = s_nv;
+        const float T = tau[row];
+        const bool proven = nv >= k_eff ? rank_key_score(wkey[k_eff - 1]) > T + eps : T <= t_floor;
+        if (!proven) {
+            if (threadIdx.x == 0) ex_rows[atomicAdd(n_ex, 1)] = row;
+        } else {
+            const int sel = min(nv, k_eff);
+            for (int t = threadIdx.x; t < k_eff; t += blockDim.x) {
+                io[t] = t < sel ? (int)(uint32_t)wkey[t] : -1;
+                so[t] = t < sel ? rank_key_score(wkey[t]) : 0.f;
+            }
+            if (threadIdx.x == 0) cnt_out[row] = sel;
+        }
+        __syncthreads();
+    }
+}
+
+// step 5: exact scan of the rows wide_select_kernel could not answer, one block per row.  Radix select (8-bit digits, most
+// significant first) of the k_eff-th largest order key among the columns with score >= thr, each digit pass rescoring all n
+// columns; then the selected columns in index order (ties at the cut: the lowest indices), sorted into rank order -- in
+// shared memory up to kWideSortCap entries, else ranked by counting over the block's slice of `big`.
+__global__ void __launch_bounds__(kWideThreads) wide_exact_kernel(
+    const float* __restrict__ xq, const float* __restrict__ xall, int64_t ld32, int d4, int n, int q_offset, int remove_self, int k_eff,
+    float thr, const int* __restrict__ ex_rows, const int* __restrict__ n_ex, unsigned long long* __restrict__ big,
+    int* __restrict__ idx_out, float* __restrict__ sim_out, int* __restrict__ cnt_out) {
+    extern __shared__ unsigned long long wkey[];
+    __shared__ int hist[256];
+    __shared__ int s_bin, s_acc, s_all;
+    typedef cub::BlockScan<int, kWideThreads> Scan;
+    __shared__ typename Scan::TempStorage scan_ts;
+    const int nex = *n_ex;
+    unsigned long long* mybig = big ? big + (size_t)blockIdx.x * k_eff : nullptr;
+    for (int f = blockIdx.x; f < nex; f += gridDim.x) {
+        const int row = ex_rows[f];
+        const float* a = xq + (int64_t)row * ld32;
+        const int self_col = remove_self ? q_offset + row : -1;
+        uint32_t prefix = 0u, pmask = 0u;
+        int need = k_eff, total = 0;
+        bool all = false;
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            for (int i = threadIdx.x; i < 256; i += blockDim.x) hist[i] = 0;
+            __syncthreads();
+            for (int j = threadIdx.x; j < n; j += blockDim.x) {
+                if (j == self_col) continue;
+                const float s = dot_seq(a, xall + (int64_t)j * ld32, d4);
+                if (!(s >= thr)) continue;
+                const uint32_t key = order_key(s);
+                if ((key & pmask) == prefix) atomicAdd(&hist[(key >> shift) & 255], 1);
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                int acc = 0, b = 255;
+                if (shift == 24) {
+                    int t = 0;
+                    for (int i = 0; i < 256; ++i) t += hist[i];
+                    s_all = t;
+                }
+                for (; b > 0; --b) { if (acc + hist[b] >= need) break; acc += hist[b]; }
+                s_bin = b; s_acc = acc;
+            }
+            __syncthreads();
+            if (shift == 24) { total = s_all; all = total <= k_eff; }
+            if (all) break;
+            need -= s_acc;
+            prefix |= (uint32_t)s_bin << shift;
+            pmask |= 255u << shift;
+            __syncthreads();
+        }
+        const int sel = all ? total : k_eff;
+        const bool in_smem = sel <= kWideSortCap;
+        int m_run = 0, ties_run = 0;
+        for (int base = 0; base < n; base += blockDim.x) {
+            const int j = base + threadIdx.x;
+            float s = 0.f;
+            bool valid = false;
+            if (j < n && j != self_col) { s = dot_seq(a, xall + (int64_t)j * ld32, d4); valid = s >= thr; }
+            const uint32_t key = valid ? order_key(s) : 0u;
+            const bool tie = !all && valid && key == prefix;
+            int tie_pos, tie_tot, pos, tot;
+            Scan(scan_ts).ExclusiveSum(tie ? 1 : 0, tie_pos, tie_tot);
+            __syncthreads();
+            const bool take = valid && (all || key > prefix || (tie && ties_run + tie_pos < need));
+            Scan(scan_ts).ExclusiveSum(take ? 1 : 0, pos, tot);
+            __syncthreads();
+            if (take) {
+                if (in_smem) wkey[m_run + pos] = rank_key(s, j);
+                else mybig[m_run + pos] = rank_key(s, j);
+            }
+            m_run += tot; ties_run += tie_tot;
+        }
+        int* io = idx_out + (size_t)row * k_eff;
+        float* so = sim_out + (size_t)row * k_eff;
+        if (in_smem) {
+            int p2 = 1;
+            while (p2 < sel) p2 <<= 1;
+            for (int i = sel + threadIdx.x; i < p2; i += blockDim.x) wkey[i] = ~0ull;
+            block_bitonic(wkey, p2);
+            for (int t = threadIdx.x; t < sel; t += blockDim.x) { io[t] = (int)(uint32_t)wkey[t]; so[t] = rank_key_score(wkey[t]); }
+        } else {
+            __syncthreads();
+            __threadfence_block();
+            for (int e = threadIdx.x; e < sel; e += blockDim.x) {
+                const unsigned long long ke = mybig[e];
+                int r = 0;
+                for (int x = 0; x < sel; ++x) r += mybig[x] < ke ? 1 : 0;
+                io[r] = (int)(uint32_t)ke; so[r] = rank_key_score(ke);
+            }
+        }
+        for (int t = sel + threadIdx.x; t < k_eff; t += blockDim.x) { io[t] = -1; so[t] = 0.f; }
+        if (threadIdx.x == 0) cnt_out[row] = sel;
+        __syncthreads();
+    }
+}
+
 // ------------------------------------------------------------------------------------------ host side
 struct Plan {
     int ew, stages, cand, qcap, nsplit, kblocks, ksteps_last, tiles, stream_a;
@@ -1074,11 +1347,11 @@ static int make_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int top_k, int 
     return SNG_OK;
 }
 
-template <int EW, bool SEED>
+template <int EW, bool SEED, int WIDE = 0>
 static cudaError_t launch_ew(dim3 grid, size_t smem, cudaStream_t st, const CUtensorMap& mq, const CUtensorMap& mdb, const Stage1Params& p) {
-    cudaError_t e = cudaFuncSetAttribute(simknn_stage1_kernel<EW, SEED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(simknn_stage1_kernel<EW, SEED, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    simknn_stage1_kernel<EW, SEED><<<grid, kNonEpiThreads + 128 * EW, smem, st>>>(mq, mdb, p);
+    simknn_stage1_kernel<EW, SEED, WIDE><<<grid, kNonEpiThreads + 128 * EW, smem, st>>>(mq, mdb, p);
     return cudaSuccess;
 }
 
@@ -1127,6 +1400,24 @@ static int check_common(const char* fn, const void* xq, const void* xall, int64_
 constexpr float kScoreEps = 0.0009765625f + 1.2e-4f;
 static float score_eps(int64_t d) { return 0.0009765625f + 1.2e-4f * (d > 640 ? (float)d / 640.0f : 1.0f); }
 static int64_t retry_ld(int64_t d) { return (d + 15) / 16 * 16 + 64; }   // widest ldb (FP16 row pitch) the build accepts: the retry query matrix is sized for it
+
+// Wide build: the sweeps' launch plan (no lists: the smallest list layout the planner knows) and the seed sample.  The stride
+// is the smallest power of two whose quantile fits the 16 group maxima (<= 14: one group may be the row's own) at the main
+// pass's 2e-5 miss probability; the sample must hold >= 512 columns so that every group has 32 of them.  Without a usable
+// stride (a database small for the top_k: k = 100 needs n >= 16,384, k = 256 n >= 65,536, k = 1,000 n >= 262,144) T_i =
+// thr - eps: then every column >= thr - eps is a candidate, and rows with more than kWideSortCap of them take the exact scan.
+static int wide_plan(Plan* pl, int64_t nq, int64_t n, int64_t d, int64_t k_eff) {
+    if (int rc = make_plan(pl, nq, n, d, 0, 8, 0)) return rc;
+    pl->seed_stride = pl->seed_q = 0;
+    const int k = (int)(k_eff < (1 << 30) ? k_eff : (1 << 30));
+    for (int64_t stride = 2; stride <= n / 512 && !pl->seed_stride; stride *= 2) {
+        const int q = seed_quantile(k, (int)stride, 2e-5);
+        if (q <= kSeedGroups - 2) { pl->seed_stride = (int)stride; pl->seed_q = q; }
+    }
+    return SNG_OK;
+}
+static int64_t wide_k_eff(int64_t n, int64_t top_k, int remove_self) { const int64_t avail = n - (remove_self ? 1 : 0); return top_k < avail ? top_k : avail; }
+static int wide_exact_grid() { return sm_count(); }       // one 128 KiB-shared-memory block per SM
 
 }  // namespace knn
 }  // namespace sng
@@ -1323,4 +1614,144 @@ extern "C" int sng_simknn_build(const uint16_t* xq, const uint16_t* xall, int64_
     simknn_fb_stream_kernel<<<fb_grid, 256, 0, st>>>(xq32, xall32, ld32, d4, (int)n, (int)q_offset, top_k, thr, remove_self, fb2_rows,
                                                     n_fallback, kFbWaves * kFbWaveRows, idx, sim, cnt);
     return check_launch("simknn stage 3");
+}
+
+// ------------------------------------------------------------------------------------------ wide build entry points
+namespace {
+struct WideWs {
+    float* seeds; float* tau; int* cnt; int* cursor; long long* len; void* scan_tmp; size_t scan_bytes; int* phase; int* ex_rows; int* n_ex;
+    unsigned long long* big;
+};
+size_t wide_scan_bytes(int64_t nq) {
+    size_t t = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, t, (const long long*)nullptr, (long long*)nullptr, (int)(nq + 1));
+    return t;
+}
+size_t wide_big_bytes(int64_t k_eff) { return k_eff > kWideSortCap ? (size_t)wide_exact_grid() * (size_t)k_eff * 8 : 0; }
+WideWs wide_carve(void* workspace, int64_t nq, int64_t k_eff) {
+    WideWs w;
+    uint8_t* p = reinterpret_cast<uint8_t*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    w.seeds = reinterpret_cast<float*>(p); p += align256((size_t)nq * kSeedGroups * 4);
+    w.tau = reinterpret_cast<float*>(p); p += align256((size_t)nq * 4);
+    w.cnt = reinterpret_cast<int*>(p); p += align256((size_t)nq * 4);
+    w.cursor = reinterpret_cast<int*>(p); p += align256((size_t)nq * 4);
+    w.len = reinterpret_cast<long long*>(p); p += align256((size_t)(nq + 1) * 8);
+    w.ex_rows = reinterpret_cast<int*>(p); p += align256((size_t)nq * 4);
+    w.phase = reinterpret_cast<int*>(p); p += 256;
+    w.n_ex = reinterpret_cast<int*>(p); p += 256;
+    w.big = wide_big_bytes(k_eff) ? reinterpret_cast<unsigned long long*>(p) : nullptr; p += align256(wide_big_bytes(k_eff));
+    w.scan_bytes = wide_scan_bytes(nq);
+    w.scan_tmp = p;
+    return w;
+}
+int wide_check(const char* fn, const uint16_t* xq, const uint16_t* xall, int64_t ldb, int64_t nq, int64_t q_offset, int64_t n, int64_t d,
+               int64_t top_k, int remove_self, void* workspace, size_t workspace_bytes) {
+    if (int rc = check_common(fn, xq, xall, ldb, nq, q_offset, n, d)) return rc;
+    SNG_REQUIRE(q_offset + nq <= n, "%s: query rows [%lld, %lld) beyond the %lld database rows", fn, (long long)q_offset, (long long)(q_offset + nq), (long long)n);
+    SNG_REQUIRE(top_k >= 1, "%s: top_k=%lld must be >= 1", fn, (long long)top_k);
+    const int64_t k_eff = wide_k_eff(n, top_k, remove_self);
+    SNG_REQUIRE(k_eff >= 1, "%s: no candidate column (n=%lld, remove_self=%d)", fn, (long long)n, remove_self);
+    SNG_REQUIRE(nq * k_eff < (1ll << 31), "%s: nq * min(top_k, n - remove_self) = %lld lists entries >= 2^31", fn, (long long)(nq * k_eff));
+    SNG_REQUIRE(ldb <= retry_ld(d), "%s: ldb=%lld > %lld (rows padded far beyond d)", fn, (long long)ldb, (long long)retry_ld(d));
+    SNG_REQUIRE(workspace, "%s: null workspace", fn);
+    const size_t need = sng_simknn_wide_workspace_bytes(nq, n, d, top_k);
+    if (workspace_bytes < need) { set_error("%s: workspace too small (%zu < %zu)", fn, workspace_bytes, need); return SNG_ERR_WORKSPACE; }
+    return SNG_OK;
+}
+// one count (WIDE = 1) or emit (WIDE = 2) sweep over all n columns; the row thresholds come from `tau`
+template <int WIDE>
+int launch_wide(const Plan& pl, const uint16_t* xq, const uint16_t* xall, int64_t ldb, int64_t nq, int64_t q_offset, int64_t n, int remove_self,
+                const float* tau, int* cnt_or_cursor, const long long* off, int* cand, int* phase, cudaStream_t st) {
+    CUtensorMap mq, mdb;
+    if (int rc = make_tma_map_f16(&mq, xq, nq, ldb, ldb, 1)) return rc;
+    if (int rc = make_tma_map_f16(&mdb, xall, n, ldb, ldb, 1)) return rc;
+    Stage1Params p;
+    p.nq = (int)nq; p.n = (int)n; p.q_offset = (int)q_offset;
+    p.kblocks = pl.kblocks; p.ksteps_last = pl.ksteps_last; p.stages = pl.stages; p.stream_a = pl.stream_a; p.cand = pl.cand; p.qcap = pl.qcap;
+    p.nsplit = pl.nsplit; p.tiles_total = pl.tiles; p.thr_lo = -3.0e38f; p.remove_self = remove_self;
+    p.issuers = pl.stream_a ? 1 : (pl.kblocks <= 3 ? 2 : 1);
+    p.cand_idx = cnt_or_cursor;
+    p.cand_val = reinterpret_cast<float*>(const_cast<long long*>(off));
+    p.cand_min = reinterpret_cast<float*>(cand);
+    p.phase = phase;
+    p.nq_dev = nullptr; p.row_ids = nullptr;
+    p.seeds = tau; p.seed_out = nullptr; p.seed_q = 0; p.seed_stride = 1;
+    dim3 grid((unsigned)(2 * ((nq + 2 * BM - 1) / (2 * BM))), (unsigned)p.nsplit);
+    const cudaError_t e = pl.ew == 4 ? launch_ew<4, false, WIDE>(grid, pl.smem, st, mq, mdb, p)
+                        : pl.ew == 2 ? launch_ew<2, false, WIDE>(grid, pl.smem, st, mq, mdb, p)
+                                     : launch_ew<1, false, WIDE>(grid, pl.smem, st, mq, mdb, p);
+    if (e != cudaSuccess) { cudaGetLastError(); set_error("simknn wide sweep: cudaFuncSetAttribute(%zu B smem): %s", pl.smem, cudaGetErrorString(e)); return SNG_ERR_CUDA; }
+    return check_launch(WIDE == 1 ? "simknn wide count sweep" : "simknn wide emit sweep");
+}
+}  // namespace
+
+extern "C" size_t sng_simknn_wide_workspace_bytes(int64_t nq, int64_t n, int64_t d, int64_t top_k) {
+    if (nq <= 0 || n <= 0 || d <= 0 || top_k < 1 || nq >= (1ll << 31) || n >= (1ll << 31)) return 0;
+    const int64_t k_eff = top_k < n ? top_k : n;
+    if (nq * k_eff >= (1ll << 31)) return 0;
+    Plan pl;
+    if (wide_plan(&pl, nq, n, d, k_eff)) return 0;
+    return align256((size_t)nq * kSeedGroups * 4) + 3 * align256((size_t)nq * 4) + align256((size_t)(nq + 1) * 8) + align256((size_t)nq * 4) +
+           512 + align256(wide_big_bytes(k_eff)) + align256(wide_scan_bytes(nq)) + 256;
+}
+
+extern "C" int sng_simknn_wide_count(const uint16_t* xq, const uint16_t* xall, int64_t ldb, int64_t nq, int64_t q_offset, int64_t n, int64_t d,
+                                     int64_t top_k, float thr, int remove_self, int64_t* offsets, void* workspace, size_t workspace_bytes,
+                                     void* stream) {
+    if (int rc = wide_check("sng_simknn_wide_count", xq, xall, ldb, nq, q_offset, n, d, top_k, remove_self, workspace, workspace_bytes)) return rc;
+    SNG_REQUIRE(offsets, "sng_simknn_wide_count: null offsets");
+    const int64_t k_eff = wide_k_eff(n, top_k, remove_self);
+    Plan pl;
+    if (int rc = wide_plan(&pl, nq, n, d, k_eff)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    WideWs w = wide_carve(workspace, nq, k_eff);
+    const float eps = score_eps(d);
+    if (cudaMemsetAsync(w.cnt, 0, (size_t)nq * 4, st) != cudaSuccess || cudaMemsetAsync(w.phase, 0, 256, st) != cudaSuccess)
+        return check_launch("sng_simknn_wide_count memset");
+    if (pl.seed_stride > 0)
+        if (int rc = launch_stage1(pl, xq, xall, ldb, nq, q_offset, n, -3.0e38f, remove_self, nullptr, nullptr, nullptr, nullptr, w.seeds, nullptr, st)) return rc;
+    const int g = grid_capped(nq + 1, 256, 4);
+    wide_tau_kernel<<<g, 256, 0, st>>>(pl.seed_stride > 0 ? w.seeds : nullptr, (int)nq, (int)q_offset, remove_self, pl.seed_q,
+                                       pl.seed_stride > 0 ? pl.seed_stride : 1, eps, thr - eps, w.tau);
+    if (int rc = launch_wide<1>(pl, xq, xall, ldb, nq, q_offset, n, remove_self, w.tau, w.cnt, nullptr, nullptr, w.phase, st)) return rc;
+    wide_len_kernel<<<g, 256, 0, st>>>(w.cnt, (int)nq, w.len);
+    size_t tb = w.scan_bytes;
+    if (cub::DeviceScan::ExclusiveSum(w.scan_tmp, tb, w.len, reinterpret_cast<long long*>(offsets), (int)(nq + 1), st) != cudaSuccess)
+        return check_launch("sng_simknn_wide_count scan");
+    return check_launch("sng_simknn_wide_count");
+}
+
+extern "C" int sng_simknn_wide_select(const uint16_t* xq, const uint16_t* xall, int64_t ldb, const float* xq32, const float* xall32, int64_t ld32,
+                                      int64_t nq, int64_t q_offset, int64_t n, int64_t d, int64_t top_k, float thr, int remove_self,
+                                      const int64_t* offsets, int32_t* cand, int32_t* idx, float* sim, int32_t* cnt, int32_t* n_exact,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = wide_check("sng_simknn_wide_select", xq, xall, ldb, nq, q_offset, n, d, top_k, remove_self, workspace, workspace_bytes)) return rc;
+    SNG_REQUIRE(xq32 && xall32 && ld32 % 4 == 0 && ld32 >= d, "sng_simknn_wide_select: FP32 rows must be padded to a multiple of 4 floats (ld32=%lld)", (long long)ld32);
+    SNG_REQUIRE(offsets && cand && idx && sim && cnt, "sng_simknn_wide_select: null offsets / candidate buffer / output");
+    const int64_t k_eff = wide_k_eff(n, top_k, remove_self);
+    Plan pl;
+    if (int rc = wide_plan(&pl, nq, n, d, k_eff)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    WideWs w = wide_carve(workspace, nq, k_eff);
+    const float eps = score_eps(d);
+    if (cudaMemsetAsync(w.cursor, 0, (size_t)nq * 4, st) != cudaSuccess || cudaMemsetAsync(w.phase, 0, 256, st) != cudaSuccess ||
+        cudaMemsetAsync(w.n_ex, 0, 4, st) != cudaSuccess)
+        return check_launch("sng_simknn_wide_select memset");
+    const long long* off = reinterpret_cast<const long long*>(offsets);
+    if (int rc = launch_wide<2>(pl, xq, xall, ldb, nq, q_offset, n, remove_self, w.tau, w.cursor, off, cand, w.phase, st)) return rc;
+    const int d4 = (int)((d + 3) / 4);
+    if (cudaFuncSetAttribute(wide_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWideSmem) != cudaSuccess ||
+        cudaFuncSetAttribute(wide_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWideSmem) != cudaSuccess) {
+        cudaGetLastError(); set_error("sng_simknn_wide_select: cannot raise the shared-memory limit"); return SNG_ERR_CUDA;
+    }
+    wide_select_kernel<<<grid_capped(nq, 1, 1), kWideThreads, kWideSmem, st>>>(
+        xq32, xall32, ld32, d4, (int)nq, (int)n, (int)q_offset, remove_self, (int)k_eff, thr, eps, thr - eps, w.tau, w.cnt, w.cursor, off, cand,
+        idx, sim, cnt, w.ex_rows, w.n_ex);
+    if (int rc = check_launch("simknn wide select")) return rc;
+    wide_exact_kernel<<<wide_exact_grid(), kWideThreads, kWideSmem, st>>>(xq32, xall32, ld32, d4, (int)n, (int)q_offset, remove_self, (int)k_eff,
+                                                                          thr, w.ex_rows, w.n_ex, w.big, idx, sim, cnt);
+    if (int rc = check_launch("simknn wide exact scan")) return rc;
+    if (n_exact && cudaMemcpyAsync(n_exact, w.n_ex, sizeof(int), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+        return check_launch("sng_simknn_wide_select n_exact");
+    return SNG_OK;
 }

@@ -29,14 +29,29 @@ def normalize_operands(x):
     return xf, xh
 
 
+def list_width(n, top_k, remove_self):
+    """Width of the lists a build returns: top_k up to SNG_KNN_MAX_TOPK (64), above it k_eff = min(top_k, n - remove_self),
+    at least 1 (top_k = 2**40 asks for every neighbour with cosine >= thr)."""
+    top_k = int(top_k)
+    return top_k if top_k <= _C.KNN_MAX_TOPK else max(1, min(top_k, n - (1 if remove_self else 0)))
+
+
 def build_knn_normalized(xf, xh, d, top_k, thr, remove_self=True, q_lo=0, q_hi=None, return_fallback=False):
     """K1 on already normalised operands (what a rank calls after the all-gather of x-hat).  return_fallback adds a device
-    int32[2] = [rows that needed the exact scan, rows that needed the retry pass]."""
+    int32[2] = [rows that needed the exact scan, rows that needed the retry pass].
+    The lists are list_width(n, top_k, remove_self) wide.  Up to SNG_KNN_MAX_TOPK (64) that is sng_simknn_build; wider lists
+    take the wide build (sng_simknn_wide_count + _select), which reads the candidate total back to allocate the candidate
+    buffer: one host synchronisation, so a wide build cannot be captured in a CUDA graph."""
     n = xf.size(0)
     q_hi = n if q_hi is None else q_hi
     nq = q_hi - q_lo
     if nq <= 0:
         raise ValueError("empty query range")
+    if int(top_k) < 1:
+        raise ValueError(f"top_k={top_k} must be >= 1")
+    top_k = list_width(n, top_k, remove_self)
+    if top_k > _C.KNN_MAX_TOPK:
+        return _build_wide(xf, xh, d, top_k, thr, remove_self, q_lo, nq, return_fallback)
     dev = xf.device
     idx = torch.empty(nq, top_k, dtype=torch.int32, device=dev)
     sim = torch.empty(nq, top_k, dtype=torch.float32, device=dev)
@@ -55,8 +70,36 @@ def build_knn_normalized(xf, xh, d, top_k, thr, remove_self=True, q_lo=0, q_hi=N
     return idx, sim, cnt
 
 
+def _build_wide(xf, xh, d, k_eff, thr, remove_self, q_lo, nq, return_fallback):
+    n = xf.size(0)
+    if nq * k_eff >= 2 ** 31:
+        raise ValueError(f"{nq} query rows x {k_eff} neighbours = {nq * k_eff} list entries: the lists are limited to < 2**31 "
+                         "entries (int32 positions of the list transpose); use fewer rows per call or a smaller top_k")
+    dev = xf.device
+    _C.require_cuda(xf, xh)
+    wbytes = _C.lib().sng_simknn_wide_workspace_bytes(nq, n, d, k_eff)
+    if wbytes == 0:
+        raise RuntimeError(f"sng_simknn_wide_workspace_bytes rejected nq={nq} n={n} d={d} top_k={k_eff}")
+    ws = torch.empty(wbytes, dtype=torch.uint8, device=dev)
+    offsets = torch.empty(nq + 1, dtype=torch.int64, device=dev)
+    common = (_C.ptr(xh[q_lo:]), _C.ptr(xh), xh.size(1))
+    _C.call("sng_simknn_wide_count", xf, *common, nq, q_lo, n, d, k_eff, float(thr), int(bool(remove_self)), _C.ptr(offsets),
+            _C.ptr(ws), wbytes)
+    total = int(offsets[nq])                                 # the wide build's one host synchronisation
+    cand = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+    idx = torch.empty(nq, k_eff, dtype=torch.int32, device=dev)
+    sim = torch.empty(nq, k_eff, dtype=torch.float32, device=dev)
+    cnt = torch.empty(nq, dtype=torch.int32, device=dev)
+    nfb = torch.zeros(2, dtype=torch.int32, device=dev)      # [rows that needed the exact scan, 0: the wide build has no retry pass]
+    _C.call("sng_simknn_wide_select", xf, *common, _C.ptr(xf[q_lo:]), _C.ptr(xf), xf.size(1), nq, q_lo, n, d, k_eff, float(thr),
+            int(bool(remove_self)), _C.ptr(offsets), _C.ptr(cand), _C.ptr(idx), _C.ptr(sim), _C.ptr(cnt), _C.ptr(nfb), _C.ptr(ws), wbytes)
+    if return_fallback:
+        return idx, sim, cnt, nfb
+    return idx, sim, cnt
+
+
 def build_knn(x, top_k, thr=-1.0, remove_self=True, q_lo=0, q_hi=None, return_fallback=False):
-    """idx [nq, top_k] int32 (-1 padded, rank order), sim [nq, top_k] float32, cnt [nq] int32."""
+    """idx [nq, k] int32 (-1 padded, rank order), sim [nq, k] float32, cnt [nq] int32; k = list_width(n, top_k, remove_self)."""
     xf, xh = normalize_operands(x)
     return build_knn_normalized(xf, xh, x.size(1), top_k, thr, remove_self, q_lo, q_hi, return_fallback)
 
@@ -133,8 +176,9 @@ def allpairs_topk_agg(h, top_k, thr, remove_self, denominator="candidates", rows
     n = h.size(0)
     lo, hi = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
     if hi <= lo:                                          # empty shard: no build (it rejects empty ranges), zero contribution
-        idx = torch.empty(0, top_k, dtype=torch.int32, device=h.device)
-        sim = torch.empty(0, top_k, dtype=torch.float32, device=h.device)
+        k = list_width(n, top_k, remove_self)
+        idx = torch.empty(0, k, dtype=torch.int32, device=h.device)
+        sim = torch.empty(0, k, dtype=torch.float32, device=h.device)
         cnt = torch.empty(0, dtype=torch.int32, device=h.device)
     else:
         xf, xh = normalize_operands(h.detach())
