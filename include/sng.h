@@ -309,6 +309,22 @@ SNG_API int sng_bn_bwd_apply(const float* z, const float* g, int64_t n, int64_t 
                      int64_t n_total, const float* gamma, const float* mean, const float* rstd, float* dz, int64_t lddz, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Counter-based dropout over the rows [row_offset, row_offset + n) of a layer of logical width c (R: models/models.py:85
+ * `x = self.dropout(x)`, optionally fused with the ReLU before it).  The mask depends only on (seed, call, global row, channel):
+ * element e = (row_offset + i) c + j keeps iff (w >> 8) >= round(p 2^24), w = word (e & 3) of Philox4x32-10 (Random123 constants)
+ * with key (seed lo, seed hi) and counter (e >> 2 lo, e >> 2 hi, call lo, call hi).  Row shards of any split therefore draw the
+ * masks of the whole layer, and the backward regenerates the mask: no [n, c] mask is stored.  s = 1.0f / (1.0f - p) in FP32.
+ *   sng_row_dropout_fwd: y [n, ldy] = keep ? a s : 0, a = relu ? max(z, 0) : z (a select: p = 1 gives zeros).
+ *   sng_row_dropout_bwd: dz [n, lddz] = keep && (!relu || z > 0) ? g s : 0; z is read only with relu (else it may be NULL).
+ * 0 <= p <= 1, c >= 1, every ld >= c, n >= 0 (n = 0 launches nothing), row_offset >= 0, (row_offset + n) c < 2^63 - 4.
+ * Rows whose pointers and strides are 16-byte aligned with c % 4 == 0 take float4 accesses; others a scalar path.
+ */
+SNG_API int sng_row_dropout_fwd(const float* z, int64_t n, int64_t c, int64_t ldz, int64_t row_offset, uint64_t seed, uint64_t call,
+                     float p, int relu, float* y, int64_t ldy, void* stream);
+SNG_API int sng_row_dropout_bwd(const float* z, const float* g, int64_t n, int64_t c, int64_t ldz, int64_t ldg, int64_t row_offset,
+                     uint64_t seed, uint64_t call, float p, int relu, float* dz, int64_t lddz, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * lin + bias + 1/norm in one pass (SURVEY.md §8(f) 2):  h [n, cp] = x W^T + b with cp = 4 * ceil(c / 4) zero-padded channels,
  * inv_norm[i] = 1 / max(||h_i||, 1e-12).  replaces `x = self.lin(x); norm = F.normalize(x)` at R: models/models.py:121-122,
  * 237-238, 324-325 (FP32 FMA; supported when cp is a power of two in [4, 128] and f * cp <= 24576 -- sng_lin_norm_supported --

@@ -11,6 +11,7 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "lib
 _lib = None
 
 _P, _I64, _I32, _F32, _SZ = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float, ctypes.c_size_t
+_U64 = ctypes.c_uint64
 
 # name -> (restype, argtypes); mirrors include/sng.h one to one (tests/test_abi.py checks the symbol list)
 SIGNATURES = {
@@ -34,6 +35,8 @@ SIGNATURES = {
     "sng_bn_fwd_apply": (_I32, [_P, _I64, _I64, _I64, _P, _I64, ctypes.c_double, _P, _P, _P, _P, _P, _I64, _P]),
     "sng_bn_bwd_stats": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _P, _P, _P, _P, _SZ, _P]),
     "sng_bn_bwd_apply": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _P, _I64, _P, _P, _P, _P, _I64, _P]),
+    "sng_row_dropout_fwd": (_I32, [_P, _I64, _I64, _I64, _I64, _U64, _U64, _F32, _I32, _P, _I64, _P]),
+    "sng_row_dropout_bwd": (_I32, [_P, _P, _I64, _I64, _I64, _I64, _I64, _U64, _U64, _F32, _I32, _P, _I64, _P]),
     "sng_lin_norm_supported": (_I32, [_I64, _I64]),
     "sng_lin_norm_fwd": (_I32, [_P, _I64, _I64, _I64, _P, _I64, _I64, _P, _P, _P, _P]),
     "sng_lin_bwd_supported": (_I32, [_I64, _I64]),

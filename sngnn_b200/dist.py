@@ -328,7 +328,29 @@ def allreduce_grads(params):
             dist.all_reduce(p.grad, op=dist.ReduceOp.SUM)
 
 
-def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None, bn_ops=None):
+class RowDropout:
+    """Dropout of row shards whose masks do not depend on the shard split: element (row, channel) of the c-wide activation of a
+    layer is kept or dropped by a pure function of (seed, call, GLOBAL row, channel) (sng_row_dropout_fwd), so every node draws
+    the same mask at any world size.  `calls` counts the dropout sites run in training with p > 0: it advances identically on
+    every rank (a host counter, no device synchronisation), so each site of each training forward draws fresh masks.
+    `ops` replaces the two launch helpers of functional.py (row_dropout_fwd / row_dropout_bwd; the tests inject CPU stand-ins)."""
+
+    def __init__(self, seed, ops=None):
+        self.seed = int(seed) % (1 << 64)
+        self.calls = 0
+        self.ops = SF if ops is None else ops
+
+    def __call__(self, z, row_offset, p, training=True, relu=False):
+        """[relu +] dropout of the rows [row_offset, row_offset + z.size(0)) of a layer; identity (after the relu) in eval mode or at
+        p = 0, where the counter does not advance."""
+        if not training or p == 0:
+            return torch.relu(z) if relu else z
+        call = self.calls
+        self.calls += 1
+        return SF.RowDropout.apply(z, int(row_offset), self.seed, call, float(p), bool(relu), self.ops)
+
+
+def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None, bn_ops=None, dropout=None):
     """Row-sharded forward of an SNGNN / SNGNN_Plus / SNGNN_Plus_Plus model (replicated parameters): this rank holds the
     feature rows [lo, hi) and returns the log-probabilities of those rows.  Mirrors _SNStack.forward / the conv forwards of
     models.py (R: models/models.py:76-86,116-137,233-242,322-329) with the aggregation and the ++ fusion replaced by their
@@ -339,7 +361,10 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None, bn_ops=N
     top_k <= 0: out_1 = 0 on the local rows (the reference runs no selection round), with zero gradients; SNGNN++ still adds
     its structural term through pp_fuse_sharded.
     bn=True: relu + BatchNorm of the hidden layers run as sharded_batch_norm, with the statistics of all n rows (training) or
-    the running statistics (eval); `bn_ops` replaces its four CUDA helpers (the tests inject CPU stand-ins)."""
+    the running statistics (eval); `bn_ops` replaces its four CUDA helpers (the tests inject CPU stand-ins).
+    dropout: a RowDropout replaces model.dropout (same p) by the counter-based dropout of the GLOBAL rows, fused with the ReLU
+    before it (or applied after sharded_batch_norm), so the masks are those of the unsharded layer at any world size.  With None,
+    model.dropout runs on the local rows: each rank draws from its own generator, so ranks seeded alike repeat each other's masks."""
     import torch.nn.functional as F
     from . import graph as G, models as M, simknn
     convs = list(model.lins)
@@ -392,7 +417,13 @@ def sharded_forward(model, x_local, edge_index, n, agg=None, fuse=None, bn_ops=N
                 out = out[:, :conv.lin.out_features]
                 if conv.bias is not None:
                     out = out + conv.bias
-        if i < len(convs) - 1:
+        if i < len(convs) - 1 and dropout is not None:
+            p = model.dropout.p
+            if use_bn:
+                out = dropout(sharded_batch_norm(out, model.bns[i], n, bn_ops), lo, p, model.dropout.training)
+            else:
+                out = dropout(out, lo, p, model.dropout.training, relu=True)
+        elif i < len(convs) - 1:
             out = sharded_batch_norm(out, model.bns[i], n, bn_ops) if use_bn else F.relu(out)
             out = model.dropout(out)
         x = out

@@ -668,6 +668,45 @@ def bn_bwd_apply(z, g, sums, n_total, gamma, mean, rstd):
     return dz
 
 
+def row_dropout_fwd(z, row_offset, seed, call, p, relu):
+    """sng_row_dropout_fwd: y [n, C] = keep ? a / (1 - p) : 0, a = relu(z) if `relu` else z, for the rows [row_offset, row_offset + n)
+    of a layer; the keep bit of element (row, channel) depends only on (seed, call, global row, channel)."""
+    z = _bn_rows(z)
+    n, c = z.shape
+    y = torch.empty(n, c, dtype=torch.float32, device=z.device)
+    _C.call("sng_row_dropout_fwd", z, _C.ptr(z), n, c, max(z.stride(0), c), int(row_offset), int(seed), int(call), float(p), int(relu),
+            _C.ptr(y), c)
+    return y
+
+
+def row_dropout_bwd(z, g, row_offset, seed, call, p, relu):
+    """sng_row_dropout_bwd: dL/dz [n, C] = keep && (!relu || z > 0) ? g / (1 - p) : 0, the mask regenerated from its counters
+    (z is read only with `relu`; pass None without)."""
+    g = _bn_rows(g)
+    n, c = g.shape
+    z = _bn_rows(z) if relu else None
+    dz = torch.empty(n, c, dtype=torch.float32, device=g.device)
+    _C.call("sng_row_dropout_bwd", g, _C.ptr(z), _C.ptr(g), n, c, max(z.stride(0), c) if relu else c, max(g.stride(0), c), int(row_offset),
+            int(seed), int(call), float(p), int(relu), _C.ptr(dz), c)
+    return dz
+
+
+class RowDropout(torch.autograd.Function):
+    """[relu +] counter-based dropout of a row block (row_dropout_fwd / row_dropout_bwd): saves z only, and only with relu -- the
+    backward regenerates the mask.  `ops` supplies the two launch helpers (this module's, or the tests' CPU stand-ins)."""
+
+    @staticmethod
+    def forward(ctx, z, row_offset, seed, call, p, relu, ops):
+        ctx.args, ctx.ops = (row_offset, seed, call, p, relu), ops
+        ctx.save_for_backward(z if relu else None)
+        return ops.row_dropout_fwd(z, row_offset, seed, call, p, relu)
+
+    @staticmethod
+    def backward(ctx, g):
+        z, = ctx.saved_tensors
+        return ctx.ops.row_dropout_bwd(z, g.contiguous(), *ctx.args), None, None, None, None, None, None
+
+
 def rownorm(x, want_f32=True, want_f16=False, f16_ld=None, want_inv=False):
     """K0: F.normalize(x, p=2, dim=-1) (R: models/models.py:122).  Returns (xhat_f32, xhat_f16, inv_norm)."""
     _C.require_cuda(x)

@@ -171,9 +171,131 @@ def train(model, data, optimizer, cfg, log=print):
     return final_test_acc, history
 
 
+class ShardedData:
+    """This rank's part of a dataset for the row-sharded trainer: rows [lo, hi) of x, y and the three masks, the whole edge_index,
+    and the global mask counts (every rank loads the whole dataset, so they are known before training starts)."""
+
+    def __init__(self, data, n, lo, hi):
+        self.n, self.lo, self.hi = n, lo, hi
+        self.x, self.edge_index, self.y = data.x[lo:hi].contiguous(), data.edge_index, data.y[lo:hi]
+        self.masks, self.counts = {}, {}
+        for k in ("train", "val", "test"):
+            m = getattr(data, k + "_mask")
+            self.masks[k] = m[lo:hi]
+            self.counts[k] = int(m.sum())
+        self.local_counts = {k: int(m.sum()) for k, m in self.masks.items()}
+
+
+def _sharded_pass(sd, split, forward, loss_fn):
+    """(loss term, local loss sum, local correct count) of one split on this rank's rows.  The loss term is the local masked
+    mean times local / global count, so the terms of all ranks add up to the global masked mean; a rank without rows of the
+    split contributes an exact 0 that still carries a gradient, because the backward runs collectives on every rank."""
+    out = forward()
+    mask, cnt = sd.masks[split], sd.local_counts[split]
+    correct = (out.max(dim=1)[1].eq(sd.y) & mask).sum()
+    if cnt == 0:
+        return out.sum() * 0.0, out.new_zeros((), dtype=torch.float64), correct
+    local = loss_fn(out, sd.y, mask)
+    return local * (cnt / max(sd.counts[split], 1)), local.detach().double() * cnt, correct
+
+
+def train_sharded(model, sd, optimizer, cfg, log=print, dropout=None, agg=None, fuse=None, bn_ops=None, loss_fn=None):
+    """The epoch loop of `train` on row shards (dist.sharded_forward): a training step with `dropout` (a dist.RowDropout), then
+    allreduce_grads and the optimizer; a validation and a test forward in eval mode; ONE all-reduce of an FP64 vector of loss sums
+    and correct counts -- the epoch's host synchronisation -- from which every rank takes the same history and the same stopping
+    decision.  `log` = None on the ranks that do not print.  agg / fuse / bn_ops / loss_fn replace the CUDA paths (gloo tests)."""
+    from . import dist as D
+    loss_fn = SF.nll_loss if loss_fn is None else loss_fn
+    fwd = lambda: D.sharded_forward(model, sd.x, sd.edge_index, sd.n, agg=agg, fuse=fuse, bn_ops=bn_ops, dropout=dropout)
+    dur, history = [], []
+    final_test_acc, smallest_val_loss, curr_step = 0, float("inf"), 0
+    for epoch in range(cfg["epochs"]):
+        if sd.x.is_cuda:
+            torch.cuda.synchronize(sd.x.device)
+        t0 = time.time()
+        model.train()
+        optimizer.zero_grad()
+        term, tr_sum, tr_cor = _sharded_pass(sd, "train", fwd, loss_fn)
+        term.backward()
+        D.allreduce_grads(model.parameters())
+        optimizer.step()
+        model.eval()
+        with torch.no_grad():
+            _, va_sum, va_cor = _sharded_pass(sd, "val", fwd, loss_fn)
+            _, te_sum, te_cor = _sharded_pass(sd, "test", fwd, loss_fn)
+        stats = torch.stack([v.to(torch.float64) for v in (tr_sum, tr_cor, va_sum, va_cor, te_sum, te_cor)])
+        stats = D._all_reduce_sums(stats).tolist()                             # device -> host: ends the epoch
+        dur.append(time.time() - t0)
+        cnt = [max(sd.counts[k], 1) for k in ("train", "val", "test")]
+        train_loss, val_loss, test_loss = stats[0] / cnt[0], stats[2] / cnt[1], stats[4] / cnt[2]
+        train_acc, val_acc, test_acc = int(stats[1]) / cnt[0], int(stats[3]) / cnt[1], int(stats[5]) / cnt[2]
+        history.append((train_loss, train_acc, val_loss, val_acc, test_loss, test_acc))
+        if log is not None and cfg.get("log_every", 1) and epoch % cfg["log_every"] == 0:
+            log("Epoch: {:d} | Train_loss: {:.4f}, Train_acc:{:.4f}, Val_loss: {:.4f}, Val_acc:{:.4f}, Test_loss: {:.4f}, "
+                "Test_acc:{:.4f}, Time(s): {:.4f}".format(epoch, train_loss, train_acc, val_loss, val_acc, test_loss, test_acc,
+                                                          sum(dur) / len(dur)))
+        if val_loss < smallest_val_loss:
+            smallest_val_loss, final_test_acc, curr_step = val_loss, test_acc, 0
+        else:
+            curr_step += 1
+        if curr_step == cfg["patience"]:
+            break
+    return final_test_acc, history
+
+
+def broadcast_parameters(model, src=0):
+    """Make every rank's parameters and buffers rank `src`'s (w.weight lives in transposed storage: broadcast a contiguous copy)."""
+    import torch.distributed as dist
+    for t in list(model.parameters()) + list(model.buffers()):
+        buf = t.data if t.data.is_contiguous() else t.data.contiguous()
+        dist.broadcast(buf, src)
+        if buf is not t.data:
+            t.data.copy_(buf)
+
+
+def main_sharded(cfg, log=print):
+    """One rank of a torchrun launch (WORLD_SIZE, RANK, LOCAL_RANK set): NCCL on cuda:LOCAL_RANK, rows [lo, hi) of every node-level
+    tensor, rank 0's initial parameters, train_sharded with a RowDropout seeded from --seed.  Every rank returns the same
+    (final test accuracy, history); rank 0 logs."""
+    import torch.distributed as dist
+    from . import dist as D
+    if not torch.cuda.is_available():
+        raise RuntimeError("sngnn_b200.train needs a CUDA device (there is no CPU path)")
+    device = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
+    asked = torch.device(cfg["device"])
+    if asked.type != "cuda" or (asked.index is not None and asked.index != device.index):
+        raise ValueError(f"--device {cfg['device']} contradicts LOCAL_RANK={device.index}: under torchrun each rank runs on cuda:LOCAL_RANK")
+    torch.cuda.set_device(device)
+    dist.init_process_group("nccl", device_id=device)
+    try:
+        ws, rank = D.world()
+        say = log if rank == 0 else (lambda *_: None)
+        set_random_seed(cfg["seed"])
+        cfg = dict(cfg, world_size=ws)
+        say(f"Config:\n{cfg}")
+        data, num_classes = load_data(cfg["dataset"], cfg["part_id"], device)
+        n = data.x.size(0)
+        say("train dataset len:{}, val dataset len:{}, test dataset len:{}".format(int(data.train_mask.sum()), int(data.val_mask.sum()),
+                                                                                   int(data.test_mask.sum())))
+        model = build_model(cfg, data.x.size(1), num_classes, n).to(device)
+        broadcast_parameters(model)
+        sd = ShardedData(data, n, *D.shard_bounds(n, ws, rank))
+        del data
+        optimizer = torch.optim.Adam(model.parameters(), lr=cfg["lr"], weight_decay=cfg["weight_decay"])
+        say("number of epoch: {}".format(cfg["epochs"]))
+        final_test_acc, history = train_sharded(model, sd, optimizer, cfg, log if rank == 0 else None, dropout=D.RowDropout(cfg["seed"]))
+        say("Part {} final test acc: {:.4f}".format(cfg["part_id"], final_test_acc))
+        return final_test_acc, history
+    finally:
+        dist.destroy_process_group()
+
+
 def main(argv=None, log=print):
+    """Single-GPU training; under torchrun (WORLD_SIZE set, 1 included) the row-sharded trainer, one rank per GPU."""
     args = parse_args(argv)
     cfg = dict(vars(args))
+    if "WORLD_SIZE" in os.environ:
+        return main_sharded(cfg, log)
     if not torch.cuda.is_available():
         raise RuntimeError("sngnn_b200.train needs a CUDA device (there is no CPU path)")
     device = torch.device(cfg["device"])
